@@ -2,6 +2,7 @@
 """bench.py - grid-cell-years/s of the two HDP hot paths (thresholds + heatwave metrics) on B200.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload NAME] [--scaling weak|strong]
+                    [--dump-outputs DIR]
 
 One "step" = thresholds for every measure of the workload, then the full percentile x definition metric
 sweep for every measure (BASELINE.json configs[1]: CMIP6-like 180x360, 30 y + 86 y, 3 measures, 10 x 6).
@@ -48,7 +49,12 @@ def parse_args():
     ap.add_argument("--scaling", default="weak", choices=["weak", "strong"], help="what N > 1 ranks share (see the module docstring)")
     ap.add_argument("--no-extra", action="store_true", help="skip the extra records (strong / lens50 / configs)")
     ap.add_argument("--no-gather", action="store_true", help="skip the output gather timing (N > 1)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step computed (a fixed sample of cells) to DIR/<name>.npy")
+    args = ap.parse_args()
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes what the GPU path computed; --impl reference times a CPU sample of other cells")
+    return args
 
 
 def peaks():
@@ -527,6 +533,32 @@ def parity_on_sample(job, n, threads):
     return res
 
 
+DUMP_BYTES = 63_000_000      # under 64 MB with the .npy headers and cells.npy
+DUMP_SEED = 2026
+
+
+def dump_outputs(job, out_dir):
+    """What the timed path handed back in its last step, so that two builds can be compared output for output: on a fixed,
+    seeded sample of this rank's cells, every measure's thresholds (float64 [cells, n_doy, P]) and metrics (uint16
+    [4, P, D, Y, cells], stored as float32, which holds them exactly), plus the sampled cell indices."""
+    import torch
+    per_cell = job.M * (job.n_doy * job.P * 8 + (4 * job.P * job.D * job.Y * 4 if job.wl.run_years else 0))
+    n = max(1, min(job.C, DUMP_BYTES // per_cell))
+    sel = np.sort(np.random.default_rng(DUMP_SEED).choice(job.C, n, replace=False))
+    if job.shared_thr:           # thresholds are per grid cell: the grid cell of every sampled (member, cell)
+        thr_rows, thr = np.concatenate([np.arange(g0, g1) for _, g0, g1 in job.pieces])[sel], job.thr_full
+    else:
+        thr_rows, thr = sel, job.thr
+    sel_t, rows_t = torch.as_tensor(sel, device=job.dev), torch.as_tensor(thr_rows, device=job.dev)
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "cells.npy"), (job.c0 + sel).astype(np.float64))
+    for m in range(job.M):
+        np.save(os.path.join(out_dir, f"thresholds_m{m}.npy"), thr[m][rows_t].cpu().numpy())
+        if job.out[m] is not None:
+            met = job.out[m].view(torch.int16)[..., sel_t].cpu().numpy().view(np.uint16)
+            np.save(os.path.join(out_dir, f"metrics_m{m}.npy"), met.astype(np.float32))
+
+
 def sub_record(job, res, steps, peak):
     bytes_step = job.bytes_per_step_global()
     ms = res["ms"] / steps
@@ -573,6 +605,8 @@ def main():
     sampler = ClockSampler(gpu_id) if rank == 0 else None
     res = timed_steps(job, args.steps, args.warmup, world, dev, with_kernels=True)
     clocks = sampler.stop(res["t0"], res["t1"]) if sampler else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(job, args.dump_outputs)
     elapsed_ms = res["ms"]
     value = job.cell_years() * args.steps / (elapsed_ms / 1e3)
 
