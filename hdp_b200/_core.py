@@ -7,6 +7,8 @@ These are the two seams of the reference that the CUDA library replaces:
 * :func:`metrics_array`     <- ``compute_heatwave_metrics`` + the percentile x definition sweep
   (reference hdp/metric.py:304-369)
 * :func:`hot_days_array`    <- ``indicate_hot_days`` (reference hdp/metric.py:280-301)
+* :func:`intensity_array`   heatwave intensity (HWC, HWI, HWP: cumulative, mean and peak exceedance of the threshold over the
+  heatwave days of a season), which the reference does not have; optionally with the four metrics from the same pass
 * :func:`index_heatwaves_array`, :func:`season_metrics_array` <- ``index_heatwaves`` and ``heatwave_frequency`` / ``number`` /
   ``duration`` / ``average`` (reference hdp/metric.py:11-172), the building blocks the hot path never materialises
 
@@ -25,6 +27,7 @@ from . import _lib
 from ._tables import WindowTables
 
 METRIC_NAMES = ("HWF", "HWN", "HWD", "HWA")      # plane order of the metric output (reference metric.py:336-340)
+INTENSITY_NAMES = ("HWC", "HWI", "HWP")          # plane order of the intensity output
 
 _workspaces = {}
 
@@ -130,31 +133,48 @@ def _check_thr(thr, C):
         raise TypeError("thresholds must be a contiguous float64 CUDA tensor [C, n_doy, P]")
 
 
+def _south_tensor(is_south, C, device):
+    if is_south is None:
+        return None
+    torch = _torch()
+    south_t = torch.as_tensor(np.ascontiguousarray(is_south, dtype=np.uint8) if not isinstance(is_south, torch.Tensor) else is_south)
+    south_t = south_t.to(device=device, dtype=torch.uint8).contiguous()
+    if south_t.numel() != C:
+        raise ValueError("is_south must have one entry per cell")
+    return south_t
+
+
+def _device_out(out, dtype, shape, device, message):
+    torch = _torch()
+    if out is None:
+        return torch.empty(shape, dtype=dtype, device=device)
+    if not (out.is_cuda and out.dtype == dtype and out.is_contiguous() and tuple(out.shape) == shape):
+        raise TypeError(message)
+    return out
+
+
+def _metric_call(measure, thresholds, doy_map, defs, season_north, season_south):
+    _check_measure(measure, "measure")
+    T, C = measure.shape
+    _check_thr(thresholds, C)
+    n_doy, P = int(thresholds.shape[1]), int(thresholds.shape[2])
+    dm, df, sn, ss = _metric_tables(doy_map, defs, season_north, season_south)
+    if dm.size != T:
+        raise ValueError("doy_map must have one entry per time step")
+    return T, C, n_doy, P, dm, df, sn, ss
+
+
 def metrics_array(measure, thresholds, doy_map, defs, season_north, season_south, is_south=None, out=None, units=None):
     """``measure`` f32 ``[T, C]``, ``thresholds`` f64 ``[C, n_doy, P]`` -> uint16 ``[4, P, D, Y, C]``
     (planes HWF, HWN, HWD, HWA; the reference's int64 ``[P, D, C, 4, Y]`` is ``out.permute(1, 2, 4, 0, 3)`` widened).
     ``units`` of the measure's samples as for :func:`thresholds_array`."""
     torch = _torch()
     unit = _unit_code(units)
-    _check_measure(measure, "measure")
-    T, C = measure.shape
-    _check_thr(thresholds, C)
+    T, C, n_doy, P, dm, df, sn, ss = _metric_call(measure, thresholds, doy_map, defs, season_north, season_south)
     L = _lib.lib()
-    n_doy, P = int(thresholds.shape[1]), int(thresholds.shape[2])
-    dm, df, sn, ss = _metric_tables(doy_map, defs, season_north, season_south)
-    if dm.size != T:
-        raise ValueError("doy_map must have one entry per time step")
     D, Y = int(df.shape[0]), int(sn.shape[0])
-    south_t = None
-    if is_south is not None:
-        south_t = torch.as_tensor(np.ascontiguousarray(is_south, dtype=np.uint8) if not isinstance(is_south, torch.Tensor) else is_south)
-        south_t = south_t.to(device=measure.device, dtype=torch.uint8).contiguous()
-        if south_t.numel() != C:
-            raise ValueError("is_south must have one entry per cell")
-    if out is None:
-        out = torch.empty((4, P, D, Y, C), dtype=torch.uint16, device=measure.device)
-    elif not (out.is_cuda and out.dtype == torch.uint16 and out.is_contiguous() and tuple(out.shape) == (4, P, D, Y, C)):
-        raise TypeError("out must be a contiguous uint16 CUDA tensor [4, P, D, Y, C]")
+    south_t = _south_tensor(is_south, C, measure.device)
+    out = _device_out(out, torch.uint16, (4, P, D, Y, C), measure.device, "out must be a contiguous uint16 CUDA tensor [4, P, D, Y, C]")
     ld_t, ld_c = _strides(measure)
     with torch.cuda.device(measure.device):
         nbytes = L.hdp_b200_metrics_workspace_bytes(C, T, ld_t, ld_c, n_doy, P, D, Y, _hp(dm))
@@ -164,6 +184,36 @@ def metrics_array(measure, thresholds, doy_map, defs, season_north, season_south
                                 south_t.data_ptr() if south_t is not None else None,
                                 out.data_ptr(), ws.data_ptr(), ws.numel(), torch.cuda.current_stream().cuda_stream, unit)
     _lib.check(rc, "hdp_b200_metrics")
+    return out
+
+
+def intensity_array(measure, thresholds, doy_map, defs, season_north, season_south, is_south=None, out=None, metrics_out=None,
+                    units=None):
+    """Heatwave intensity: ``measure`` f32 ``[T, C]``, ``thresholds`` f64 ``[C, n_doy, P]`` -> float32 ``[3, P, D, Y, C]``, planes
+    HWC (cumulative), HWI (mean) and HWP (peak) exceedance ``measure - threshold`` over the heatwave days of every season (the
+    days HWF counts; 0 where there are none).  ``metrics_out``: an optional uint16 CUDA tensor ``[4, P, D, Y, C]`` that also
+    receives exactly what :func:`metrics_array` returns, from the same pass.  The non-empty seasons of each hemisphere's table must
+    be disjoint (every table compute_hemisphere_ranges builds is)."""
+    torch = _torch()
+    unit = _unit_code(units)
+    T, C, n_doy, P, dm, df, sn, ss = _metric_call(measure, thresholds, doy_map, defs, season_north, season_south)
+    L = _lib.lib()
+    D, Y = int(df.shape[0]), int(sn.shape[0])
+    south_t = _south_tensor(is_south, C, measure.device)
+    out = _device_out(out, torch.float32, (3, P, D, Y, C), measure.device, "out must be a contiguous float32 CUDA tensor [3, P, D, Y, C]")
+    if metrics_out is not None:
+        metrics_out = _device_out(metrics_out, torch.uint16, (4, P, D, Y, C), measure.device,
+                                  "metrics_out must be a contiguous uint16 CUDA tensor [4, P, D, Y, C]")
+    ld_t, ld_c = _strides(measure)
+    with torch.cuda.device(measure.device):
+        nbytes = L.hdp_b200_intensity_workspace_bytes(C, T, ld_t, ld_c, n_doy, P, D, Y, _hp(dm))
+        ws = _workspace(measure.device, nbytes)
+        rc = L.hdp_b200_intensity(measure.data_ptr(), C, T, ld_t, ld_c, thresholds.data_ptr(), n_doy, P, _hp(dm),
+                                  _hp(df), D, _hp(sn), _hp(ss), Y,
+                                  south_t.data_ptr() if south_t is not None else None, out.data_ptr(),
+                                  metrics_out.data_ptr() if metrics_out is not None else None,
+                                  ws.data_ptr(), ws.numel(), torch.cuda.current_stream().cuda_stream, unit)
+    _lib.check(rc, "hdp_b200_intensity")
     return out
 
 
@@ -407,12 +457,8 @@ def thresholds_host(temps: np.ndarray, tables: WindowTables, percentiles: Sequen
     return out
 
 
-def metrics_host(measure: np.ndarray, thresholds, doy_map, defs, season_north, season_south,
-                 is_south=None, out: Optional[np.ndarray] = None, units=None) -> np.ndarray:
-    """``thresholds``: float64 ``[C, n_doy, P]`` as a host array, or as a CUDA tensor (device-resident: no upload).  A host
-    array that :func:`thresholds_host` returned with ``keep=True`` is recognised and its device copy used."""
+def _host_metric_call(measure, thresholds, doy_map, defs, season_north, season_south, is_south):
     torch = _torch()
-    L = _lib.lib()
     measure, ld_t, ld_c = _host_measure(measure, "measure")
     T, C = measure.shape
     d_thr = None
@@ -429,15 +475,44 @@ def metrics_host(measure: np.ndarray, thresholds, doy_map, defs, season_north, s
     dm, df, sn, ss = _metric_tables(doy_map, defs, season_north, season_south)
     if dm.size != T:
         raise ValueError("doy_map must have one entry per time step")
-    D, Y = df.shape[0], sn.shape[0]
     south = None if is_south is None else np.ascontiguousarray(is_south, dtype=np.uint8)
+    args = (_hp(measure), C, T, ld_t, ld_c, _hp(thr) if thr is not None else None, d_thr.data_ptr() if d_thr is not None else None,
+            n_doy, P, _hp(dm), _hp(df), df.shape[0], _hp(sn), _hp(ss), sn.shape[0], _hp(south) if south is not None else None)
+    return args, (P, df.shape[0], sn.shape[0], C)
+
+
+def _host_out(out, dtype, shape, message):
+    if out is None:
+        return np.empty(shape, dtype)
+    if not (isinstance(out, np.ndarray) and out.flags.c_contiguous and out.dtype == dtype and out.shape == shape):
+        raise TypeError(message)
+    return out
+
+
+def metrics_host(measure: np.ndarray, thresholds, doy_map, defs, season_north, season_south,
+                 is_south=None, out: Optional[np.ndarray] = None, units=None) -> np.ndarray:
+    """``thresholds``: float64 ``[C, n_doy, P]`` as a host array, or as a CUDA tensor (device-resident: no upload).  A host
+    array that :func:`thresholds_host` returned with ``keep=True`` is recognised and its device copy used."""
+    args, (P, D, Y, C) = _host_metric_call(measure, thresholds, doy_map, defs, season_north, season_south, is_south)
     if out is None:
         out = np.empty((4, P, D, Y, C), np.uint16)
     assert out.flags.c_contiguous and out.dtype == np.uint16 and out.shape == (4, P, D, Y, C)
-    rc = L.hdp_b200_metrics_host(_hp(measure), C, T, ld_t, ld_c, _hp(thr) if thr is not None else None,
-                                 d_thr.data_ptr() if d_thr is not None else None, n_doy, P, _hp(dm), _hp(df), D, _hp(sn), _hp(ss), Y,
-                                 _hp(south) if south is not None else None, _hp(out), _unit_code(units))
+    rc = _lib.lib().hdp_b200_metrics_host(*args, _hp(out), _unit_code(units))
     _lib.check(rc, "hdp_b200_metrics_host")
+    return out
+
+
+def intensity_host(measure: np.ndarray, thresholds, doy_map, defs, season_north, season_south, is_south=None,
+                   out: Optional[np.ndarray] = None, metrics_out: Optional[np.ndarray] = None, units=None) -> np.ndarray:
+    """Host-array counterpart of :func:`intensity_array`: float32 ``[3, P, D, Y, C]`` (HWC, HWI, HWP); ``metrics_out`` an
+    optional uint16 host array ``[4, P, D, Y, C]`` that also receives what :func:`metrics_host` returns (the samples cross PCIe
+    once for both).  Thresholds as for :func:`metrics_host` (host array, CUDA tensor, or a resident copy)."""
+    args, (P, D, Y, C) = _host_metric_call(measure, thresholds, doy_map, defs, season_north, season_south, is_south)
+    out = _host_out(out, np.float32, (3, P, D, Y, C), "out must be a C-contiguous float32 array [3, P, D, Y, C]")
+    if metrics_out is not None:
+        metrics_out = _host_out(metrics_out, np.uint16, (4, P, D, Y, C), "metrics_out must be a C-contiguous uint16 array [4, P, D, Y, C]")
+    rc = _lib.lib().hdp_b200_intensity_host(*args, _hp(out), _hp(metrics_out) if metrics_out is not None else None, _unit_code(units))
+    _lib.check(rc, "hdp_b200_intensity_host")
     return out
 
 
@@ -452,7 +527,8 @@ def launch_count() -> int:
 
 
 KERNEL_NAMES = {1: "normalize", 2: "k_thr_generic", 3: "k_hot_words", 4: "k_scan", 5: "k_unpack_mask",
-                6: "k_thr_seg", 7: "k_thr_ranked", 8: "k_measure", 9: "k_thr_cand", 10: "k_thr_net", 11: "k_seam"}
+                6: "k_thr_seg", 7: "k_thr_ranked", 8: "k_measure", 9: "k_thr_cand", 10: "k_thr_net", 11: "k_seam",
+                12: "k_intensity"}
 
 
 def timing_enable(on: bool) -> None:

@@ -30,6 +30,9 @@ SIGNATURES = {
     "hdp_b200_metrics_workspace_bytes": (_sz, [_i64, _i64, _i64, _i64, _int, _int, _int, _int, _p]),
     "hdp_b200_metrics": (_int, [_p, _i64, _i64, _i64, _i64, _p, _int, _int, _p, _p, _int, _p, _p, _int, _p, _p, _p, _sz, _p, _int]),
     "hdp_b200_metrics_host": (_int, [_p, _i64, _i64, _i64, _i64, _p, _p, _int, _int, _p, _p, _int, _p, _p, _int, _p, _p, _int]),
+    "hdp_b200_intensity_workspace_bytes": (_sz, [_i64, _i64, _i64, _i64, _int, _int, _int, _int, _p]),
+    "hdp_b200_intensity": (_int, [_p, _i64, _i64, _i64, _i64, _p, _int, _int, _p, _p, _int, _p, _p, _int, _p, _p, _p, _p, _sz, _p, _int]),
+    "hdp_b200_intensity_host": (_int, [_p, _i64, _i64, _i64, _i64, _p, _p, _int, _int, _p, _p, _int, _p, _p, _int, _p, _p, _p, _int]),
     "hdp_b200_host_release": (None, []),
     "hdp_b200_metrics_run_filter": (None, [_int]),
     "hdp_b200_heat_index": (_int, [_p, _p, _i64, _p, _p]),
@@ -69,7 +72,7 @@ def lib() -> ctypes.CDLL:
             fn = getattr(L, name)          # AttributeError if the library does not export the symbol
             fn.restype = res
             fn.argtypes = args
-        if L.hdp_b200_abi_version() != 4:
+        if L.hdp_b200_abi_version() != 5:
             raise RuntimeError("libhdp_b200.so ABI version mismatch; rebuild with `python -m hdp_b200.build --force`")
         _LIB = L
     return _LIB

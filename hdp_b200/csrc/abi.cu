@@ -120,7 +120,8 @@ const char *hdp_b200_strerror(int code)
         return "invalid argument (null pointer, negative size, quantile outside [0,1] or NaN, table entry out of range)";
     case HDP_B200_ERR_UNSUPPORTED:
         return "unsupported shape (more than 32 percentiles or definitions, a window of more than 32768 samples, "
-               "or a season longer than 65535 days)";
+               "a season longer than 65535 days, or - for the intensity metrics - two overlapping non-empty seasons in one "
+               "hemisphere's table)";
     case HDP_B200_ERR_WORKSPACE: return "workspace missing or smaller than *_workspace_bytes()";
     case HDP_B200_ERR_NO_DEVICE: return "no CUDA device available";
     case HDP_B200_ERR_NOMEM: return "host allocation failed";

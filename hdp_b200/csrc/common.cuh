@@ -30,7 +30,7 @@ inline int cuda_status(cudaError_t e) { return e == cudaSuccess ? HDP_B200_OK : 
     } while (0)
 
 // Optional per-kernel CUDA-event timing (hdp_b200_timing_enable / hdp_b200_timing_read).
-enum KernelId { kNormalize = 1, kThrGeneric = 2, kHotWords = 3, kScan = 4, kUnpackMask = 5, kThrSeg = 6, kThrRanked = 7, kMeasure = 8, kThrCand = 9, kThrNet = 10, kSeam = 11 };
+enum KernelId { kNormalize = 1, kThrGeneric = 2, kHotWords = 3, kScan = 4, kUnpackMask = 5, kThrSeg = 6, kThrRanked = 7, kMeasure = 8, kThrCand = 9, kThrNet = 10, kSeam = 11, kIntensity = 12 };
 struct KernelTimer {
     bool on;
     cudaStream_t st;

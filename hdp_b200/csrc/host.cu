@@ -42,6 +42,12 @@ int metrics_launch(const float *d_measure, int64_t C, int64_t T, int64_t ld_t, i
                    const int32_t *h_season_north, const int32_t *h_season_south, int Y,
                    const uint8_t *d_is_south, uint16_t *d_out,
                    void *d_workspace, size_t workspace_bytes, void *stream, int64_t carve_cells, bool tables_resident, int input_unit);
+int intensity_launch(const float *d_measure, int64_t C, int64_t T, int64_t ld_t, int64_t ld_c,
+                     const double *d_thr, int n_doy, int P, const int32_t *h_doy_map,
+                     const int32_t *h_defs, int D,
+                     const int32_t *h_season_north, const int32_t *h_season_south, int Y,
+                     const uint8_t *d_is_south, float *d_int, uint16_t *d_out,
+                     void *d_workspace, size_t workspace_bytes, void *stream, int64_t carve_cells, bool tables_resident, int input_unit);
 
 constexpr int kSlots = 3;
 constexpr int kMaxDevices = 64;
@@ -163,7 +169,7 @@ struct HostCtx {
     bool ready = false;
     cudaStream_t s_in = nullptr, s_k = nullptr, s_out = nullptr;
     cudaEvent_t in_ready[kSlots] = {}, k_done[kSlots] = {}, out_done[kSlots] = {};
-    DeviceBuf x[kSlots], aux[kSlots], south[kSlots], out[kSlots], ws;
+    DeviceBuf x[kSlots], aux[kSlots], south[kSlots], out[kSlots], out_f[kSlots], ws;
     PinnedRing ring_in, ring_out;                    // staging for pageable sources / destinations (allocated on first use)
     std::deque<PendingOut> pending;                  // D2H blocks on their way through ring_out
 
@@ -269,7 +275,7 @@ struct HostCtx {
             for (int i = 0; i < kSlots; i++) { cudaEventDestroy(in_ready[i]); cudaEventDestroy(k_done[i]); cudaEventDestroy(out_done[i]); }
             ready = false;
         }
-        for (int i = 0; i < kSlots; i++) { x[i].release(); aux[i].release(); south[i].release(); out[i].release(); }
+        for (int i = 0; i < kSlots; i++) { x[i].release(); aux[i].release(); south[i].release(); out[i].release(); out_f[i].release(); }
         ws.release();
         ring_in.release(); ring_out.release();
     }
@@ -330,6 +336,84 @@ using namespace hdp;
         if (_rc != HDP_B200_OK) { ctx->drain(); return _rc; }\
     } while (0)
 #define HDP_HOST_CUDA(expr) HDP_HOST_TRY(cuda_status(expr))
+
+// hdp_b200_metrics_host (h_int == NULL) and hdp_b200_intensity_host: the same chunk pipeline; with h_int the chunk's kernels are
+// those of hdp_b200_intensity, and the f32 planes (and the u16 ones when h_out is given) go back to the host.
+static int metric_pass_host(const float *h_measure, int64_t C, int64_t T, int64_t ld_t, int64_t ld_c,
+                            const double *h_thr, const double *d_thr, int n_doy, int P, const int32_t *h_doy_map,
+                            const int32_t *h_defs, int D,
+                            const int32_t *h_season_north, const int32_t *h_season_south, int Y,
+                            const uint8_t *h_is_south, float *h_int, uint16_t *h_out, int input_unit)
+{
+    if (C < 0 || T <= 0 || n_doy <= 0 || P <= 0 || D <= 0 || Y < 0 || !h_doy_map) return HDP_B200_ERR_INVALID;
+    if (C == 0 || Y == 0) return HDP_B200_OK;
+    if (!h_measure || (!h_thr && !d_thr)) return HDP_B200_ERR_INVALID;
+    if (ld_t <= 0 || ld_c <= 0) return HDP_B200_ERR_INVALID;
+    if (ld_c != 1 && ld_t != 1) return HDP_B200_ERR_UNSUPPORTED;
+    HostCtx *ctx = nullptr;
+    int rc = current_ctx(&ctx);
+    if (rc) return rc;
+    std::lock_guard<std::mutex> lock(ctx->mu);
+    if ((rc = ctx->init())) return rc;
+
+    const size_t thr_per_cell = (size_t)n_doy * P * sizeof(double);
+    const size_t rows = (size_t)4 * P * D * Y;                                 // output rows of C cells each
+    const size_t rows_f = (size_t)3 * P * D * Y;
+    const int64_t chunk = pick_chunk(C, (size_t)T * sizeof(float) + thr_per_cell, (size_t)320 << 20);
+    const int64_t dl_t = ld_c == 1 ? chunk : 1, dl_c = ld_c == 1 ? 1 : T;
+    const size_t ws_bytes = h_int ? hdp_b200_intensity_workspace_bytes(chunk, T, dl_t, dl_c, n_doy, P, D, Y, h_doy_map)
+                                  : hdp_b200_metrics_workspace_bytes(chunk, T, dl_t, dl_c, n_doy, P, D, Y, h_doy_map);
+    if ((rc = ctx->ws.reserve(ws_bytes))) return rc;
+    for (int i = 0; i < kSlots; i++) {
+        if ((rc = ctx->x[i].reserve((size_t)chunk * T * sizeof(float)))) return rc;
+        if (!d_thr && (rc = ctx->aux[i].reserve((size_t)chunk * thr_per_cell))) return rc;
+        if ((rc = ctx->south[i].reserve((size_t)chunk))) return rc;
+        if (h_out && (rc = ctx->out[i].reserve(rows * chunk * sizeof(uint16_t)))) return rc;
+        if (h_int && (rc = ctx->out_f[i].reserve(rows_f * chunk * sizeof(float)))) return rc;
+    }
+    const bool page_x = is_pageable(h_measure), page_thr = !d_thr && is_pageable(h_thr), page_out = h_out && is_pageable(h_out);
+    const bool page_int = h_int && is_pageable(h_int);
+    const bool page_south = h_is_south && is_pageable(h_is_south);
+    int64_t i = 0;
+    for (int64_t c0 = 0; c0 < C; c0 += chunk, i++) {
+        const int slot = (int)(i % kSlots);
+        const int64_t nc = std::min(chunk, C - c0);
+        int64_t a, b;
+        HDP_HOST_CUDA(cudaStreamWaitEvent(ctx->s_in, ctx->k_done[slot], 0));
+        HDP_HOST_TRY(upload_cells(ctx, h_measure, page_x, T, ld_t, ld_c, c0, nc, (float *)ctx->x[slot].p, &a, &b, ctx->s_in));
+        if (!d_thr)                                                            // device-resident thresholds never cross PCIe again
+            HDP_HOST_TRY(ctx->h2d((char *)ctx->aux[slot].p, 0, (const char *)(h_thr + (size_t)c0 * n_doy * P), 0, (size_t)nc * thr_per_cell, 1,
+                                  page_thr, ctx->s_in));
+        if (h_is_south)
+            HDP_HOST_TRY(ctx->h2d((char *)ctx->south[slot].p, 0, (const char *)(h_is_south + c0), 0, (size_t)nc, 1, page_south, ctx->s_in));
+        HDP_HOST_CUDA(cudaEventRecord(ctx->in_ready[slot], ctx->s_in));
+
+        HDP_HOST_CUDA(cudaStreamWaitEvent(ctx->s_k, ctx->in_ready[slot], 0));
+        HDP_HOST_CUDA(cudaStreamWaitEvent(ctx->s_k, ctx->out_done[slot], 0));
+        const double *thr_chunk = d_thr ? d_thr + (size_t)c0 * n_doy * P : (const double *)ctx->aux[slot].p;
+        const uint8_t *south_chunk = h_is_south ? (const uint8_t *)ctx->south[slot].p : nullptr;
+        if (h_int)
+            HDP_HOST_TRY(intensity_launch((const float *)ctx->x[slot].p, nc, T, a, b, thr_chunk, n_doy, P, h_doy_map,
+                                          h_defs, D, h_season_north, h_season_south, Y, south_chunk, (float *)ctx->out_f[slot].p,
+                                          h_out ? (uint16_t *)ctx->out[slot].p : nullptr, ctx->ws.p, ws_bytes, ctx->s_k, chunk, i > 0, input_unit));
+        else
+            HDP_HOST_TRY(metrics_launch((const float *)ctx->x[slot].p, nc, T, a, b, thr_chunk, n_doy, P, h_doy_map,
+                                        h_defs, D, h_season_north, h_season_south, Y, south_chunk,
+                                        (uint16_t *)ctx->out[slot].p, ctx->ws.p, ws_bytes, ctx->s_k, chunk, i > 0, input_unit));
+        HDP_HOST_CUDA(cudaEventRecord(ctx->k_done[slot], ctx->s_k));
+
+        // device chunk is [rows, nc]; host array is [rows, C]
+        HDP_HOST_CUDA(cudaStreamWaitEvent(ctx->s_out, ctx->k_done[slot], 0));
+        if (h_out)
+            HDP_HOST_TRY(ctx->d2h((char *)(h_out + c0), (size_t)C * sizeof(uint16_t), (const char *)ctx->out[slot].p, (size_t)nc * sizeof(uint16_t),
+                                  (size_t)nc * sizeof(uint16_t), rows, page_out, ctx->s_out));
+        if (h_int)
+            HDP_HOST_TRY(ctx->d2h((char *)(h_int + c0), (size_t)C * sizeof(float), (const char *)ctx->out_f[slot].p, (size_t)nc * sizeof(float),
+                                  (size_t)nc * sizeof(float), rows_f, page_int, ctx->s_out));
+        HDP_HOST_CUDA(cudaEventRecord(ctx->out_done[slot], ctx->s_out));
+    }
+    return ctx->drain();
+}
 
 extern "C" {
 
@@ -399,61 +483,20 @@ int hdp_b200_metrics_host(const float *h_measure, int64_t C, int64_t T, int64_t 
                           const int32_t *h_season_north, const int32_t *h_season_south, int Y,
                           const uint8_t *h_is_south, uint16_t *h_out, int input_unit)
 {
-    if (C < 0 || T <= 0 || n_doy <= 0 || P <= 0 || D <= 0 || Y < 0 || !h_doy_map) return HDP_B200_ERR_INVALID;
-    if (C == 0 || Y == 0) return HDP_B200_OK;
-    if (!h_measure || (!h_thr && !d_thr) || !h_out) return HDP_B200_ERR_INVALID;
-    if (ld_t <= 0 || ld_c <= 0) return HDP_B200_ERR_INVALID;
-    if (ld_c != 1 && ld_t != 1) return HDP_B200_ERR_UNSUPPORTED;
-    HostCtx *ctx = nullptr;
-    int rc = current_ctx(&ctx);
-    if (rc) return rc;
-    std::lock_guard<std::mutex> lock(ctx->mu);
-    if ((rc = ctx->init())) return rc;
+    if (!h_out && C > 0 && Y > 0) return HDP_B200_ERR_INVALID;
+    return metric_pass_host(h_measure, C, T, ld_t, ld_c, h_thr, d_thr, n_doy, P, h_doy_map, h_defs, D, h_season_north, h_season_south, Y,
+                            h_is_south, nullptr, h_out, input_unit);
+}
 
-    const size_t thr_per_cell = (size_t)n_doy * P * sizeof(double);
-    const size_t rows = (size_t)4 * P * D * Y;                                 // output rows of C cells each
-    const int64_t chunk = pick_chunk(C, (size_t)T * sizeof(float) + thr_per_cell, (size_t)320 << 20);
-    const int64_t dl_t = ld_c == 1 ? chunk : 1, dl_c = ld_c == 1 ? 1 : T;
-    const size_t ws_bytes = hdp_b200_metrics_workspace_bytes(chunk, T, dl_t, dl_c, n_doy, P, D, Y, h_doy_map);
-    if ((rc = ctx->ws.reserve(ws_bytes))) return rc;
-    for (int i = 0; i < kSlots; i++) {
-        if ((rc = ctx->x[i].reserve((size_t)chunk * T * sizeof(float)))) return rc;
-        if (!d_thr && (rc = ctx->aux[i].reserve((size_t)chunk * thr_per_cell))) return rc;
-        if ((rc = ctx->south[i].reserve((size_t)chunk))) return rc;
-        if ((rc = ctx->out[i].reserve(rows * chunk * sizeof(uint16_t)))) return rc;
-    }
-    const bool page_x = is_pageable(h_measure), page_thr = !d_thr && is_pageable(h_thr), page_out = is_pageable(h_out);
-    const bool page_south = h_is_south && is_pageable(h_is_south);
-    int64_t i = 0;
-    for (int64_t c0 = 0; c0 < C; c0 += chunk, i++) {
-        const int slot = (int)(i % kSlots);
-        const int64_t nc = std::min(chunk, C - c0);
-        int64_t a, b;
-        HDP_HOST_CUDA(cudaStreamWaitEvent(ctx->s_in, ctx->k_done[slot], 0));
-        HDP_HOST_TRY(upload_cells(ctx, h_measure, page_x, T, ld_t, ld_c, c0, nc, (float *)ctx->x[slot].p, &a, &b, ctx->s_in));
-        if (!d_thr)                                                            // device-resident thresholds never cross PCIe again
-            HDP_HOST_TRY(ctx->h2d((char *)ctx->aux[slot].p, 0, (const char *)(h_thr + (size_t)c0 * n_doy * P), 0, (size_t)nc * thr_per_cell, 1,
-                                  page_thr, ctx->s_in));
-        if (h_is_south)
-            HDP_HOST_TRY(ctx->h2d((char *)ctx->south[slot].p, 0, (const char *)(h_is_south + c0), 0, (size_t)nc, 1, page_south, ctx->s_in));
-        HDP_HOST_CUDA(cudaEventRecord(ctx->in_ready[slot], ctx->s_in));
-
-        HDP_HOST_CUDA(cudaStreamWaitEvent(ctx->s_k, ctx->in_ready[slot], 0));
-        HDP_HOST_CUDA(cudaStreamWaitEvent(ctx->s_k, ctx->out_done[slot], 0));
-        HDP_HOST_TRY(metrics_launch((const float *)ctx->x[slot].p, nc, T, a, b,
-                                    d_thr ? d_thr + (size_t)c0 * n_doy * P : (const double *)ctx->aux[slot].p, n_doy, P, h_doy_map,
-                                    h_defs, D, h_season_north, h_season_south, Y,
-                                    h_is_south ? (const uint8_t *)ctx->south[slot].p : nullptr,
-                                    (uint16_t *)ctx->out[slot].p, ctx->ws.p, ws_bytes, ctx->s_k, chunk, i > 0, input_unit));
-        HDP_HOST_CUDA(cudaEventRecord(ctx->k_done[slot], ctx->s_k));
-
-        // device chunk is [rows, nc]; host array is [rows, C]
-        HDP_HOST_CUDA(cudaStreamWaitEvent(ctx->s_out, ctx->k_done[slot], 0));
-        HDP_HOST_TRY(ctx->d2h((char *)(h_out + c0), (size_t)C * sizeof(uint16_t), (const char *)ctx->out[slot].p, (size_t)nc * sizeof(uint16_t),
-                              (size_t)nc * sizeof(uint16_t), rows, page_out, ctx->s_out));
-        HDP_HOST_CUDA(cudaEventRecord(ctx->out_done[slot], ctx->s_out));
-    }
-    return ctx->drain();
+int hdp_b200_intensity_host(const float *h_measure, int64_t C, int64_t T, int64_t ld_t, int64_t ld_c,
+                            const double *h_thr, const double *d_thr, int n_doy, int P, const int32_t *h_doy_map,
+                            const int32_t *h_defs, int D,
+                            const int32_t *h_season_north, const int32_t *h_season_south, int Y,
+                            const uint8_t *h_is_south, float *h_int, uint16_t *h_out, int input_unit)
+{
+    if (!h_int && C > 0 && Y > 0) return HDP_B200_ERR_INVALID;
+    return metric_pass_host(h_measure, C, T, ld_t, ld_c, h_thr, d_thr, n_doy, P, h_doy_map, h_defs, D, h_season_north, h_season_south, Y,
+                            h_is_south, h_int, h_out, input_unit);
 }
 
 }  // extern "C"

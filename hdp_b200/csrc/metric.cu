@@ -22,7 +22,7 @@
 #include <vector>
 #include <algorithm>
 
-#include "common.cuh"
+#include "metric.cuh"
 
 namespace hdp {
 
@@ -508,13 +508,6 @@ k_scan(const uint32_t *__restrict__ hot, int64_t C, int K, int T, const int4 *__
 // ----------------------------------------------------------------------------------------------------
 // host side
 // ----------------------------------------------------------------------------------------------------
-struct WordPlan {
-    std::vector<int4> words;        // {t0, nbits, doy of bit 0, 0}
-    std::vector<int> blk_start;     // [n_blk + 1]
-    std::vector<int> blk_words;     // word ids grouped by day-of-year block
-    int n_blk = 0;
-};
-
 // Cuts the time axis into words of <= 32 consecutive days whose days of year are consecutive and stay
 // inside one 32-day block of the day-of-year axis (so that every word of a block shares one threshold tile).
 static int build_words(const int32_t *doy_map, int64_t T, int n_doy, WordPlan &plan)
@@ -543,14 +536,14 @@ static int build_words(const int32_t *doy_map, int64_t T, int n_doy, WordPlan &p
     return HDP_B200_OK;
 }
 
-static int64_t words_upper_bound(int64_t T, int n_doy)
+int64_t words_upper_bound(int64_t T, int n_doy)
 {
     // regular daily calendars: every (partial) year contributes at most n_blk + 1 words
     const int64_t n_blk = (n_doy + kTileDoy - 1) / kTileDoy;
     return (T / std::max(n_doy, 1) + 2) * (n_blk + 1) + 1;
 }
 
-static int64_t count_words(const int32_t *doy_map, int64_t T)
+int64_t count_words(const int32_t *doy_map, int64_t T)
 {
     int64_t K = 0, t = 0;
     while (t < T) {
@@ -578,17 +571,7 @@ static int pick_pg(int P)
     return best;
 }
 
-struct Layout {
-    size_t total = 0;
-    float *xn = nullptr;
-    int4 *words = nullptr;
-    int *blk_start = nullptr, *blk_words = nullptr;
-    int4 *seasons = nullptr;
-    uint32_t *lut = nullptr;
-    uint32_t *hot = nullptr;
-};
-
-static Layout carve(void *ws, size_t ws_bytes, int64_t C, int64_t T, bool need_norm, int64_t K, int n_doy, int P, int Y)
+Layout carve(void *ws, size_t ws_bytes, int64_t C, int64_t T, bool need_norm, int64_t K, int n_doy, int P, int Y, bool intensity)
 {
     Layout L;
     Carver cv(ws, ws_bytes);
@@ -599,27 +582,27 @@ static Layout carve(void *ws, size_t ws_bytes, int64_t C, int64_t T, bool need_n
     L.seasons = cv.take<int4>((size_t)2 * (Y + 1));
     L.lut = cv.take<uint32_t>((size_t)2 * 8192);
     L.hot = cv.take<uint32_t>((size_t)P * K * C);
+    if (intensity) L.int_seasons = cv.take<int4>((size_t)2 * (Y + 1));
     L.total = cv.off;
     return L;
 }
 
-static bool bad_dims(int64_t C, int64_t T, int n_doy, int P)
+bool bad_dims(int64_t C, int64_t T, int n_doy, int P)
 {
     return C < 0 || T < 0 || n_doy <= 0 || P <= 0 || T > 0x3fffffff;
 }
 
-// Runs k_hot_words; on success *plan_out/*L_out describe what lives in the workspace.
-static int run_hot_words(const float *d_measure, int64_t C, int64_t T, int64_t ld_t, int64_t ld_c,
-                         const double *d_thr, int n_doy, int P, const int32_t *h_doy_map,
-                         int Y, void *ws, size_t ws_bytes, cudaStream_t st, WordPlan &plan, Layout &L,
-                         int64_t carve_cells = 0, bool tables_resident = false, int input_unit = 0)
+int run_hot_words(const float *d_measure, int64_t C, int64_t T, int64_t ld_t, int64_t ld_c,
+                  const double *d_thr, int n_doy, int P, const int32_t *h_doy_map,
+                  int Y, void *ws, size_t ws_bytes, cudaStream_t st, WordPlan &plan, Layout &L,
+                  int64_t carve_cells, bool tables_resident, int input_unit, bool intensity)
 {
     if (input_unit < 0 || input_unit > 2) return HDP_B200_ERR_INVALID;
     int rc = build_words(h_doy_map, T, n_doy, plan);
     if (rc != HDP_B200_OK) return rc;
     const int K = (int)plan.words.size();
     const bool need_norm = ld_c != 1;
-    L = carve(ws, ws_bytes, std::max(C, carve_cells), T, need_norm, K, n_doy, P, Y);
+    L = carve(ws, ws_bytes, std::max(C, carve_cells), T, need_norm, K, n_doy, P, Y, intensity);
     if (ws == nullptr || L.total > ws_bytes) return HDP_B200_ERR_WORKSPACE;
     if (C == 0 || T == 0) return HDP_B200_OK;
     const float *x = d_measure;
@@ -673,6 +656,28 @@ static void clamp_season(int64_t a, int64_t b, int64_t T, int &lo, int &hi)
     lo = (int)a; hi = (int)b;
 }
 
+int scan_passes(const int32_t *h_season_north, const int32_t *h_season_south, int Y, int64_t T, ScanPasses (&passes)[2])
+{
+    for (int h = 0; h < 2; h++) {
+        const int32_t *tab = h == 0 ? h_season_north : h_season_south;
+        std::vector<ScanSeason> all(Y);
+        for (int y = 0; y < Y; y++) {
+            clamp_season(tab[2 * y], tab[2 * y + 1], T, all[y].a, all[y].b);
+            all[y].row = y;
+            if (all[y].b - all[y].a > 65535) return HDP_B200_ERR_UNSUPPORTED;
+        }
+        std::stable_sort(all.begin(), all.end(), [](const ScanSeason &l, const ScanSeason &r) { return l.a < r.a; });
+        for (const ScanSeason &s : all) {
+            size_t i = 0;
+            for (; i < passes[h].size(); i++)
+                if (passes[h][i].back().b <= s.a) break;
+            if (i == passes[h].size()) passes[h].emplace_back();
+            passes[h][i].push_back(s);
+        }
+    }
+    return HDP_B200_OK;
+}
+
 // The whole of hdp_b200_metrics; carve_cells / tables_resident as in thresholds_launch (threshold.cu).
 int metrics_launch(const float *d_measure, int64_t C, int64_t T, int64_t ld_t, int64_t ld_c,
                    const double *d_thr, int n_doy, int P, const int32_t *h_doy_map,
@@ -688,33 +693,22 @@ int metrics_launch(const float *d_measure, int64_t C, int64_t T, int64_t ld_t, i
     if (P > HDP_B200_MAX_PERCENTILES || D > HDP_B200_MAX_DEFINITIONS) return HDP_B200_ERR_UNSUPPORTED;
     cudaStream_t st = (cudaStream_t)stream;
 
-    // season tables: clamp, then split into passes of sorted, disjoint seasons per hemisphere
-    struct Season { int a, b, row; };
-    std::vector<std::vector<Season>> passes[2];
-    for (int h = 0; h < 2; h++) {
-        const int32_t *tab = h == 0 ? h_season_north : h_season_south;
-        std::vector<Season> all(Y);
-        for (int y = 0; y < Y; y++) {
-            clamp_season(tab[2 * y], tab[2 * y + 1], T, all[y].a, all[y].b);
-            all[y].row = y;
-            if (all[y].b - all[y].a > 65535) return HDP_B200_ERR_UNSUPPORTED;
-        }
-        std::stable_sort(all.begin(), all.end(), [](const Season &l, const Season &r) { return l.a < r.a; });
-        for (const Season &s : all) {
-            size_t i = 0;
-            for (; i < passes[h].size(); i++)
-                if (passes[h][i].back().b <= s.a) break;
-            if (i == passes[h].size()) passes[h].emplace_back();
-            passes[h][i].push_back(s);
-        }
-    }
-    const size_t n_pass = std::max(passes[0].size(), passes[1].size());
+    ScanPasses passes[2];
+    int rc = scan_passes(h_season_north, h_season_south, Y, T, passes);
+    if (rc != HDP_B200_OK) return rc;
 
     WordPlan plan;
     Layout L;
-    int rc = run_hot_words(d_measure, C, T, ld_t, ld_c, d_thr, n_doy, P, h_doy_map, Y, d_workspace, workspace_bytes, st, plan, L,
-                            carve_cells, tables_resident, input_unit);
+    rc = run_hot_words(d_measure, C, T, ld_t, ld_c, d_thr, n_doy, P, h_doy_map, Y, d_workspace, workspace_bytes, st, plan, L,
+                       carve_cells, tables_resident, input_unit);
     if (rc != HDP_B200_OK || C == 0 || Y == 0) return rc;
+    return run_scan(L, plan, C, T, P, h_defs, D, passes, Y, d_is_south, d_out, st, tables_resident);
+}
+
+int run_scan(const Layout &L, const WordPlan &plan, int64_t C, int64_t T, int P, const int32_t *h_defs, int D,
+             const ScanPasses (&passes)[2], int Y, const uint8_t *d_is_south, uint16_t *d_out, cudaStream_t st, bool tables_resident)
+{
+    const size_t n_pass = std::max(passes[0].size(), passes[1].size());
     const int K = (int)plan.words.size();
 
     // bit-sliced definition tables (see k_scan)
@@ -758,7 +752,7 @@ int metrics_launch(const float *d_measure, int64_t C, int64_t T, int64_t ld_t, i
     int max_season = 0;
     for (int h = 0; h < 2; h++)
         for (const auto &pass : passes[h])
-            for (const Season &se : pass) max_season = std::max(max_season, se.b - se.a);
+            for (const ScanSeason &se : pass) max_season = std::max(max_season, se.b - se.a);
     const bool bytes = max_season <= 255;
     const int per = bytes ? 4 : 2;
     int ng = (D + per - 1) / per;
@@ -771,7 +765,7 @@ int metrics_launch(const float *d_measure, int64_t C, int64_t T, int64_t ld_t, i
     for (int h = 0; h < 2; h++)
         for (const auto &pass : passes[h]) {
             off[h].push_back(tab.size());
-            for (const Season &s : pass) tab.push_back(make_int4(s.a, s.b, s.row, 0));
+            for (const ScanSeason &s : pass) tab.push_back(make_int4(s.a, s.b, s.row, 0));
         }
     if (!tables_resident) HDP_CUDA_TRY(cudaMemcpyAsync(L.seasons, tab.data(), sizeof(int4) * tab.size(), cudaMemcpyHostToDevice, st));
     for (size_t ip = 0; ip < n_pass; ip++) {

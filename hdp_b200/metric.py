@@ -23,6 +23,17 @@ METRIC_ATTRS = {          # metric.py:473-492
             "description": "Average length of heatwaves during a heatwave season"},
 }
 
+# The opt-in intensity variables (compute_individual_metrics(..., intensity=True)); their units are the measure's.
+_EXCEEDANCE = "exceedance e = measure - threshold (float64) on the days that fall within a heatwave during a heatwave season"
+INTENSITY_ATTRS = {
+    "HWC": {"long_name": "Heatwave Cumulative Intensity",
+            "description": f"Sum of the {_EXCEEDANCE}, added heatwave by heatwave in time order; 0 without heatwave days"},
+    "HWI": {"long_name": "Heatwave Mean Intensity",
+            "description": f"Cumulative intensity divided by the heatwave frequency: mean of the {_EXCEEDANCE}; 0 without heatwave days"},
+    "HWP": {"long_name": "Heatwave Peak Intensity",
+            "description": f"Largest {_EXCEEDANCE}; 0 without heatwave days"},
+}
+
 
 # ----------------------------------------------------------------------------------------------
 # The building blocks under the reference's names (its unit tests import exactly these: hdp/tests/test_index_heatwaves.py,
@@ -163,9 +174,10 @@ def _widen_int64(a: np.ndarray) -> np.ndarray:
     return out
 
 
-def _metric_sweep(measure, threshold, hw_definitions, time_axis, doy_map=None):
+def _metric_sweep(measure, threshold, hw_definitions, time_axis, doy_map=None, intensity=False):
     """The percentile x definition x cell sweep of compute_heatwave_metrics_wrapper (metric.py:344-369) as ONE library call:
-    -> (uint16 [4, P, D, Y, C], season tables, cell dims, cell shape, P, D)."""
+    -> (uint16 [4, P, D, Y, C], season tables, cell dims, cell shape, P, D).  With ``intensity`` the call is the intensity pass
+    and the first item is (uint16 [4, P, D, Y, C], float32 [3, P, D, Y, C])."""
     st = _tables.hemisphere_ranges(time_axis)                       # compute_hemisphere_ranges, :410
     if doy_map is None:
         doy_map = _tables.doy_map(time_axis.dayofyr)                # build_doy_map, :413
@@ -185,6 +197,10 @@ def _metric_sweep(measure, threshold, hw_definitions, time_axis, doy_map=None):
     thr_cdp = np.ascontiguousarray(thr_vals).reshape(-1, n_doy, P)
 
     defs = np.asarray(hw_definitions, dtype=np.int64).reshape(-1, 3)
+    if intensity:
+        out = np.empty((4, P, defs.shape[0], st.n_years, x.shape[1]), np.uint16)
+        heat = _core.intensity_host(x, thr_cdp, doy_map, defs, st.north, st.south, south, metrics_out=out)   # float32 [3, P, D, Y, C]
+        return (out, heat), st, cell_dims, cell_shape, P, defs.shape[0]
     out = _core.metrics_host(x, thr_cdp, doy_map, defs, st.north, st.south, south)     # uint16 [4, P, D, Y, C]
     return out, st, cell_dims, cell_shape, P, defs.shape[0]
 
@@ -200,8 +216,11 @@ def compute_heatwave_metrics_wrapper(measure, threshold, doy_map, hw_definitions
     return xr.DataArray(data, dims=["percentile", "definition", *cell_dims, "metric", "year"], coords=coords)
 
 
-def compute_individual_metrics(measure, threshold, hw_definitions: list, include_threshold: bool = True, check_variables: bool = True):
-    """metric.py:372-506."""
+def compute_individual_metrics(measure, threshold, hw_definitions: list, include_threshold: bool = True, check_variables: bool = True,
+                               *, intensity: bool = False):
+    """metric.py:372-506.  ``intensity=True`` adds three float32 variables to the four metrics (which stay identical): HWC, HWI
+    and HWP, the cumulative, mean and peak exceedance ``measure - threshold`` over the heatwave days of every season, in the
+    measure's units (see hdp_b200_intensity in include/hdp_b200.h for the exact arithmetic).  Same dims and coords as HWF."""
     time_axis = time_axis_of(measure)
     if check_variables:                                             # :393-398
         assert "hdp_type" in threshold.attrs
@@ -219,7 +238,9 @@ def compute_individual_metrics(measure, threshold, hw_definitions: list, include
             if entry != '':
                 combined_history += (f"(Threshold) {entry}\n")
 
-    out, st, cell_dims, cell_shape, P, D = _metric_sweep(measure, threshold, hw_definitions, time_axis)
+    out, st, cell_dims, cell_shape, P, D = _metric_sweep(measure, threshold, hw_definitions, time_axis, intensity=intensity)
+    if intensity:
+        out, heat = out
     Y = st.n_years
 
     coords = dict(xr.non_time_coords(measure))
@@ -232,6 +253,9 @@ def compute_individual_metrics(measure, threshold, hw_definitions: list, include
         wide = out[i] if np.dtype(METRIC_DTYPE) == np.uint16 else _widen_int64(out[i]).astype(METRIC_DTYPE, copy=False)   # [P, D, Y, C]
         plane = wide.transpose(0, 1, 3, 2).reshape(P, D, *cell_shape, Y)                # view: no host transposition
         data_vars[name] = xr.DataArray(plane, dims=dims, coords=coords)
+    if intensity:
+        for i, name in enumerate(_core.INTENSITY_NAMES):            # float32 [P, D, Y, C]
+            data_vars[name] = xr.DataArray(heat[i].transpose(0, 1, 3, 2).reshape(P, D, *cell_shape, Y), dims=dims, coords=coords)
     ds = xr.Dataset(data_vars)
     ds.attrs.update({
         "description": f"Heatwave metric dataset generated by Heatwave Diagnostics Package (HDP v{get_version()})",
@@ -240,6 +264,9 @@ def compute_individual_metrics(measure, threshold, hw_definitions: list, include
     })
     for name, attrs in METRIC_ATTRS.items():
         ds[name].attrs.update(attrs)
+    if intensity:
+        for name, attrs in INTENSITY_ATTRS.items():
+            ds[name].attrs.update({"units": measure.attrs["units"], **attrs} if "units" in measure.attrs else attrs)
     xr.set_coord_attrs(ds, "percentile", {"range": "(0, 1)"})
     xr.set_coord_attrs(ds, "definition", {
         "first_number": "Minimum number of consecutively hot days",
@@ -252,15 +279,18 @@ def compute_individual_metrics(measure, threshold, hw_definitions: list, include
     return ds
 
 
-def compute_group_metrics(measures, thresholds, hw_definitions: list, include_threshold: bool = False, check_variables: bool = True):
-    """metric.py:509-523: every measure against every threshold of the same baseline variable."""
+def compute_group_metrics(measures, thresholds, hw_definitions: list, include_threshold: bool = False, check_variables: bool = True,
+                          *, intensity: bool = False):
+    """metric.py:509-523: every measure against every threshold of the same baseline variable.  ``intensity=True`` adds the
+    HWC / HWI / HWP variables of :func:`compute_individual_metrics` under the same ``{measure}.{threshold}.{metric}`` names."""
     metric_sets = []
     for measure_name in list(measures.keys()):
         measure = measures[measure_name]
         for threshold_name in list(thresholds.keys()):
             threshold = thresholds[threshold_name]
             if threshold.attrs["baseline_variable"] == measure.attrs["baseline_variable"]:
-                hw_metrics = compute_individual_metrics(measure, threshold, hw_definitions, include_threshold, check_variables)
+                hw_metrics = compute_individual_metrics(measure, threshold, hw_definitions, include_threshold, check_variables,
+                                                        intensity=intensity)
                 var_renames = {name: f"{measure_name}.{threshold_name}.{name}" for name in list(hw_metrics.keys())}
                 metric_sets.append(hw_metrics.rename(var_renames))
     aggr_ds = xr.merge(metric_sets)

@@ -13,6 +13,8 @@
  *                                    heatwave_frequency/number/duration/average :63-172)
  *                                   + compute_heatwave_metrics_wrapper     hdp/metric.py:344-369
  *   hdp_b200_hot_days     replaces  indicate_hot_days                     hdp/metric.py:280-301
+ *   hdp_b200_intensity    (no reference counterpart) heatwave intensity: cumulative, mean and peak exceedance of the
+ *                         threshold over the heatwave days of every season, optionally with the metrics in the same pass
  *   hdp_b200_index_heatwaves   replaces  index_heatwaves                  hdp/metric.py:11-60     (the building blocks under
  *   hdp_b200_season_metrics    replaces  heatwave_frequency / number / duration / average  hdp/metric.py:63-172   their own names)
  *   *_host variants       the same calls with HOST buffers (cell chunks pipelined H2D -> kernels -> D2H on three streams).
@@ -42,7 +44,7 @@
 extern "C" {
 #endif
 
-#define HDP_B200_ABI_VERSION 4
+#define HDP_B200_ABI_VERSION 5
 
 #define HDP_B200_OK                 0
 #define HDP_B200_ERR_INVALID       (-1)  /* null pointer, negative size, quantile outside [0,1] or NaN, bad table entry */
@@ -156,6 +158,45 @@ int hdp_b200_metrics_host(const float *h_measure, int64_t C, int64_t T, int64_t 
                           const uint8_t *h_is_south,
                           uint16_t *h_out, int input_unit);
 
+/* ---------------------------------------------------------------------------------------------------
+ * Path 2 - heatwave intensity (opt-in; hdp_b200_metrics is unchanged).  Same inputs as hdp_b200_metrics.  For cell c,
+ * percentile p, definition d and season y, with e_t = (double)x_c(t) - thr[c, doy_map[t], p] (x after the input_unit
+ * conversion) over the days t of the season slice whose heatwave id is > 0 (exactly the days HWF counts, so e_t > 0):
+ *
+ *   HWC  cumulative intensity: per maximal block of consecutive such days, in time order, r = 0, r = r + e_t, then S = S + r
+ *   HWI  mean intensity S / HWF (0 when HWF = 0)
+ *   HWP  peak intensity: the largest e_t (0 when there is no heatwave day)
+ *
+ *   d_int         f32 [3, P, D, Y, C]  planes HWC, HWI, HWP, each rounded once from float64 (the canonical order above makes
+ *                 the result reproducible bit for bit)
+ *   d_out         optional u16 [4, P, D, Y, C]: when given, also exactly what hdp_b200_metrics writes, from the same hot-day
+ *                 pass over the samples
+ * The non-empty seasons of each hemisphere's table must be pairwise disjoint after slice clamping (every table built by
+ * compute_hemisphere_ranges / get_range_indices is); other tables return HDP_B200_ERR_UNSUPPORTED.
+ * ------------------------------------------------------------------------------------------------- */
+/* h_doy_map may be NULL: the size is then an upper bound for regular daily calendars. */
+size_t hdp_b200_intensity_workspace_bytes(int64_t C, int64_t T, int64_t ld_t, int64_t ld_c,
+                                          int n_doy, int P, int D, int Y, const int32_t *h_doy_map);
+
+int hdp_b200_intensity(const float *d_measure, int64_t C, int64_t T, int64_t ld_t, int64_t ld_c,
+                       const double *d_thr, int n_doy, int P,
+                       const int32_t *h_doy_map,
+                       const int32_t *h_defs, int D,
+                       const int32_t *h_season_north, const int32_t *h_season_south, int Y,
+                       const uint8_t *d_is_south,
+                       float *d_int, uint16_t *d_out,
+                       void *d_workspace, size_t workspace_bytes, void *stream, int input_unit);
+
+/* Host-buffer variant (the pipeline of hdp_b200_metrics_host: each measure chunk crosses PCIe once for both outputs).
+ * h_out may be NULL; thresholds from h_thr unless d_thr (DEVICE) is given. */
+int hdp_b200_intensity_host(const float *h_measure, int64_t C, int64_t T, int64_t ld_t, int64_t ld_c,
+                            const double *h_thr, const double *d_thr, int n_doy, int P,
+                            const int32_t *h_doy_map,
+                            const int32_t *h_defs, int D,
+                            const int32_t *h_season_north, const int32_t *h_season_south, int Y,
+                            const uint8_t *h_is_south,
+                            float *h_int, uint16_t *h_out, int input_unit);
+
 /* The *_host variants keep their streams, events and device buffers (grown on demand) in a per-device context between
  * calls; this frees them.  Safe to call at any time no *_host call is running. */
 void hdp_b200_host_release(void);
@@ -225,6 +266,7 @@ int64_t hdp_b200_launch_count(void);
 #define HDP_B200_KERNEL_THR_CAND     9   /* k_thr_cand */
 #define HDP_B200_KERNEL_THR_NET     10   /* k_thr_net / k_thr_net_tm / k_thr_net_irr */
 #define HDP_B200_KERNEL_SEAM        11   /* k_index_heatwaves, k_season_metrics */
+#define HDP_B200_KERNEL_INTENSITY   12   /* k_intensity */
 void hdp_b200_timing_enable(int on);
 int  hdp_b200_timing_read(int *ids, float *ms, int cap);
 
