@@ -153,7 +153,12 @@ def _device_out(out, dtype, shape, device, message):
     return out
 
 
-def _metric_call(measure, thresholds, doy_map, defs, season_north, season_south):
+def _metric_pass(measure, thresholds, doy_map, defs, season_north, season_south, is_south, units, met, heat, intensity):
+    """hdp_b200_metrics, or with ``intensity`` hdp_b200_intensity, on CUDA tensors.  ``met`` / ``heat``: the uint16 metrics /
+    float32 intensity output or None; the metrics are allocated unless the intensity pass runs without them.  Returns the
+    intensity output of the intensity pass, else the metrics."""
+    torch = _torch()
+    unit = _unit_code(units)
     _check_measure(measure, "measure")
     T, C = measure.shape
     _check_thr(thresholds, C)
@@ -161,30 +166,33 @@ def _metric_call(measure, thresholds, doy_map, defs, season_north, season_south)
     dm, df, sn, ss = _metric_tables(doy_map, defs, season_north, season_south)
     if dm.size != T:
         raise ValueError("doy_map must have one entry per time step")
-    return T, C, n_doy, P, dm, df, sn, ss
+    L = _lib.lib()
+    D, Y = int(df.shape[0]), int(sn.shape[0])
+    south_t = _south_tensor(is_south, C, measure.device)
+    if intensity:
+        heat = _device_out(heat, torch.float32, (3, P, D, Y, C), measure.device,
+                           "out must be a contiguous float32 CUDA tensor [3, P, D, Y, C]")
+    if met is not None or not intensity:
+        met = _device_out(met, torch.uint16, (4, P, D, Y, C), measure.device,
+                          f"{'metrics_out' if intensity else 'out'} must be a contiguous uint16 CUDA tensor [4, P, D, Y, C]")
+    outs = (heat.data_ptr(), met.data_ptr() if met is not None else None) if intensity else (met.data_ptr(),)
+    name = "hdp_b200_intensity" if intensity else "hdp_b200_metrics"
+    ld_t, ld_c = _strides(measure)
+    with torch.cuda.device(measure.device):
+        nbytes = getattr(L, name + "_workspace_bytes")(C, T, ld_t, ld_c, n_doy, P, D, Y, _hp(dm))
+        ws = _workspace(measure.device, nbytes)
+        rc = getattr(L, name)(measure.data_ptr(), C, T, ld_t, ld_c, thresholds.data_ptr(), n_doy, P, _hp(dm),
+                              _hp(df), D, _hp(sn), _hp(ss), Y, south_t.data_ptr() if south_t is not None else None,
+                              *outs, ws.data_ptr(), ws.numel(), torch.cuda.current_stream().cuda_stream, unit)
+    _lib.check(rc, name)
+    return heat if intensity else met
 
 
 def metrics_array(measure, thresholds, doy_map, defs, season_north, season_south, is_south=None, out=None, units=None):
     """``measure`` f32 ``[T, C]``, ``thresholds`` f64 ``[C, n_doy, P]`` -> uint16 ``[4, P, D, Y, C]``
     (planes HWF, HWN, HWD, HWA; the reference's int64 ``[P, D, C, 4, Y]`` is ``out.permute(1, 2, 4, 0, 3)`` widened).
     ``units`` of the measure's samples as for :func:`thresholds_array`."""
-    torch = _torch()
-    unit = _unit_code(units)
-    T, C, n_doy, P, dm, df, sn, ss = _metric_call(measure, thresholds, doy_map, defs, season_north, season_south)
-    L = _lib.lib()
-    D, Y = int(df.shape[0]), int(sn.shape[0])
-    south_t = _south_tensor(is_south, C, measure.device)
-    out = _device_out(out, torch.uint16, (4, P, D, Y, C), measure.device, "out must be a contiguous uint16 CUDA tensor [4, P, D, Y, C]")
-    ld_t, ld_c = _strides(measure)
-    with torch.cuda.device(measure.device):
-        nbytes = L.hdp_b200_metrics_workspace_bytes(C, T, ld_t, ld_c, n_doy, P, D, Y, _hp(dm))
-        ws = _workspace(measure.device, nbytes)
-        rc = L.hdp_b200_metrics(measure.data_ptr(), C, T, ld_t, ld_c, thresholds.data_ptr(), n_doy, P, _hp(dm),
-                                _hp(df), D, _hp(sn), _hp(ss), Y,
-                                south_t.data_ptr() if south_t is not None else None,
-                                out.data_ptr(), ws.data_ptr(), ws.numel(), torch.cuda.current_stream().cuda_stream, unit)
-    _lib.check(rc, "hdp_b200_metrics")
-    return out
+    return _metric_pass(measure, thresholds, doy_map, defs, season_north, season_south, is_south, units, out, None, False)
 
 
 def intensity_array(measure, thresholds, doy_map, defs, season_north, season_south, is_south=None, out=None, metrics_out=None,
@@ -194,27 +202,7 @@ def intensity_array(measure, thresholds, doy_map, defs, season_north, season_sou
     days HWF counts; 0 where there are none).  ``metrics_out``: an optional uint16 CUDA tensor ``[4, P, D, Y, C]`` that also
     receives exactly what :func:`metrics_array` returns, from the same pass.  The non-empty seasons of each hemisphere's table must
     be disjoint (every table compute_hemisphere_ranges builds is)."""
-    torch = _torch()
-    unit = _unit_code(units)
-    T, C, n_doy, P, dm, df, sn, ss = _metric_call(measure, thresholds, doy_map, defs, season_north, season_south)
-    L = _lib.lib()
-    D, Y = int(df.shape[0]), int(sn.shape[0])
-    south_t = _south_tensor(is_south, C, measure.device)
-    out = _device_out(out, torch.float32, (3, P, D, Y, C), measure.device, "out must be a contiguous float32 CUDA tensor [3, P, D, Y, C]")
-    if metrics_out is not None:
-        metrics_out = _device_out(metrics_out, torch.uint16, (4, P, D, Y, C), measure.device,
-                                  "metrics_out must be a contiguous uint16 CUDA tensor [4, P, D, Y, C]")
-    ld_t, ld_c = _strides(measure)
-    with torch.cuda.device(measure.device):
-        nbytes = L.hdp_b200_intensity_workspace_bytes(C, T, ld_t, ld_c, n_doy, P, D, Y, _hp(dm))
-        ws = _workspace(measure.device, nbytes)
-        rc = L.hdp_b200_intensity(measure.data_ptr(), C, T, ld_t, ld_c, thresholds.data_ptr(), n_doy, P, _hp(dm),
-                                  _hp(df), D, _hp(sn), _hp(ss), Y,
-                                  south_t.data_ptr() if south_t is not None else None, out.data_ptr(),
-                                  metrics_out.data_ptr() if metrics_out is not None else None,
-                                  ws.data_ptr(), ws.numel(), torch.cuda.current_stream().cuda_stream, unit)
-    _lib.check(rc, "hdp_b200_intensity")
-    return out
+    return _metric_pass(measure, thresholds, doy_map, defs, season_north, season_south, is_south, units, metrics_out, out, True)
 
 
 def hot_days_array(measure, thresholds, doy_map):
@@ -457,7 +445,16 @@ def thresholds_host(temps: np.ndarray, tables: WindowTables, percentiles: Sequen
     return out
 
 
-def _host_metric_call(measure, thresholds, doy_map, defs, season_north, season_south, is_south):
+def _host_out(out, dtype, shape, message):
+    if out is None:
+        return np.empty(shape, dtype)
+    if not (isinstance(out, np.ndarray) and out.flags.c_contiguous and out.dtype == dtype and out.shape == shape):
+        raise TypeError(message)
+    return out
+
+
+def _metric_pass_host(measure, thresholds, doy_map, defs, season_north, season_south, is_south, units, met, heat, intensity):
+    """:func:`_metric_pass` with host arrays: hdp_b200_metrics_host, or with ``intensity`` hdp_b200_intensity_host."""
     torch = _torch()
     measure, ld_t, ld_c = _host_measure(measure, "measure")
     T, C = measure.shape
@@ -476,30 +473,26 @@ def _host_metric_call(measure, thresholds, doy_map, defs, season_north, season_s
     if dm.size != T:
         raise ValueError("doy_map must have one entry per time step")
     south = None if is_south is None else np.ascontiguousarray(is_south, dtype=np.uint8)
-    args = (_hp(measure), C, T, ld_t, ld_c, _hp(thr) if thr is not None else None, d_thr.data_ptr() if d_thr is not None else None,
-            n_doy, P, _hp(dm), _hp(df), df.shape[0], _hp(sn), _hp(ss), sn.shape[0], _hp(south) if south is not None else None)
-    return args, (P, df.shape[0], sn.shape[0], C)
-
-
-def _host_out(out, dtype, shape, message):
-    if out is None:
-        return np.empty(shape, dtype)
-    if not (isinstance(out, np.ndarray) and out.flags.c_contiguous and out.dtype == dtype and out.shape == shape):
-        raise TypeError(message)
-    return out
+    D, Y = df.shape[0], sn.shape[0]
+    if intensity:
+        heat = _host_out(heat, np.float32, (3, P, D, Y, C), "out must be a C-contiguous float32 array [3, P, D, Y, C]")
+    if met is not None or not intensity:
+        met = _host_out(met, np.uint16, (4, P, D, Y, C),
+                        f"{'metrics_out' if intensity else 'out'} must be a C-contiguous uint16 array [4, P, D, Y, C]")
+    outs = (_hp(heat), _hp(met) if met is not None else None) if intensity else (_hp(met),)
+    name = "hdp_b200_intensity_host" if intensity else "hdp_b200_metrics_host"
+    rc = getattr(_lib.lib(), name)(_hp(measure), C, T, ld_t, ld_c, _hp(thr) if thr is not None else None,
+                                   d_thr.data_ptr() if d_thr is not None else None, n_doy, P, _hp(dm), _hp(df), D, _hp(sn), _hp(ss), Y,
+                                   _hp(south) if south is not None else None, *outs, _unit_code(units))
+    _lib.check(rc, name)
+    return heat if intensity else met
 
 
 def metrics_host(measure: np.ndarray, thresholds, doy_map, defs, season_north, season_south,
                  is_south=None, out: Optional[np.ndarray] = None, units=None) -> np.ndarray:
     """``thresholds``: float64 ``[C, n_doy, P]`` as a host array, or as a CUDA tensor (device-resident: no upload).  A host
     array that :func:`thresholds_host` returned with ``keep=True`` is recognised and its device copy used."""
-    args, (P, D, Y, C) = _host_metric_call(measure, thresholds, doy_map, defs, season_north, season_south, is_south)
-    if out is None:
-        out = np.empty((4, P, D, Y, C), np.uint16)
-    assert out.flags.c_contiguous and out.dtype == np.uint16 and out.shape == (4, P, D, Y, C)
-    rc = _lib.lib().hdp_b200_metrics_host(*args, _hp(out), _unit_code(units))
-    _lib.check(rc, "hdp_b200_metrics_host")
-    return out
+    return _metric_pass_host(measure, thresholds, doy_map, defs, season_north, season_south, is_south, units, out, None, False)
 
 
 def intensity_host(measure: np.ndarray, thresholds, doy_map, defs, season_north, season_south, is_south=None,
@@ -507,13 +500,7 @@ def intensity_host(measure: np.ndarray, thresholds, doy_map, defs, season_north,
     """Host-array counterpart of :func:`intensity_array`: float32 ``[3, P, D, Y, C]`` (HWC, HWI, HWP); ``metrics_out`` an
     optional uint16 host array ``[4, P, D, Y, C]`` that also receives what :func:`metrics_host` returns (the samples cross PCIe
     once for both).  Thresholds as for :func:`metrics_host` (host array, CUDA tensor, or a resident copy)."""
-    args, (P, D, Y, C) = _host_metric_call(measure, thresholds, doy_map, defs, season_north, season_south, is_south)
-    out = _host_out(out, np.float32, (3, P, D, Y, C), "out must be a C-contiguous float32 array [3, P, D, Y, C]")
-    if metrics_out is not None:
-        metrics_out = _host_out(metrics_out, np.uint16, (4, P, D, Y, C), "metrics_out must be a C-contiguous uint16 array [4, P, D, Y, C]")
-    rc = _lib.lib().hdp_b200_intensity_host(*args, _hp(out), _hp(metrics_out) if metrics_out is not None else None, _unit_code(units))
-    _lib.check(rc, "hdp_b200_intensity_host")
-    return out
+    return _metric_pass_host(measure, thresholds, doy_map, defs, season_north, season_south, is_south, units, metrics_out, out, True)
 
 
 def host_release() -> None:

@@ -92,4 +92,21 @@ int to_celsius_launch(const float *src, int64_t n, int unit, float *dst, cudaStr
 // Copies the strided measure array into a time-major, cell-contiguous [T, C] buffer.
 int normalize_layout(const float *src, int64_t C, int64_t T, int64_t ld_t, int64_t ld_c, float *dst, cudaStream_t st);
 
+// The whole of hdp_b200_thresholds (threshold.cu).  `carve_cells` sizes the workspace layout (>= C; the host pipeline passes its
+// chunk capacity so that every chunk sees the tables at the same place) and `tables_resident` skips the table uploads when the
+// previous call on this workspace and stream used identical tables.
+int thresholds_launch(const float *d_temps, int64_t C, int64_t T_b, int64_t ld_t, int64_t ld_c,
+                      const int32_t *h_time_index, const int32_t *h_win_rows, int n_doy, int n_y, int W,
+                      const double *h_q, int P, double *d_out,
+                      void *d_workspace, size_t workspace_bytes, void *stream, int64_t carve_cells, bool tables_resident, int input_unit);
+
+// The whole of hdp_b200_metrics and hdp_b200_intensity (metric.cu): k_hot_words, then k_scan on its hot words when d_out is given
+// (u16 [4, P, D, Y, C]) and k_intensity when d_int is given (f32 [3, P, D, Y, C]).  carve_cells / tables_resident as above.
+int metric_pass(const float *d_measure, int64_t C, int64_t T, int64_t ld_t, int64_t ld_c,
+                const double *d_thr, int n_doy, int P, const int32_t *h_doy_map,
+                const int32_t *h_defs, int D,
+                const int32_t *h_season_north, const int32_t *h_season_south, int Y,
+                const uint8_t *d_is_south, uint16_t *d_out, float *d_int,
+                void *d_workspace, size_t workspace_bytes, void *stream, int64_t carve_cells, bool tables_resident, int input_unit);
+
 }  // namespace hdp

@@ -10,7 +10,7 @@
 //
 // with kSlots input and output buffers handed from stage to stage by events, so both PCIe directions and the SMs are
 // busy at the same time and the call runs at the rate of its slowest stage (on B200 + PCIe Gen5: the H2D copy).
-// Index tables are uploaded with the first chunk only and stay in the workspace (thresholds_launch / metrics_launch
+// Index tables are uploaded with the first chunk only and stay in the workspace (thresholds_launch / metric_pass
 // `tables_resident`), so nothing blocks the host between chunks and the whole call is enqueued ahead of the GPU.
 // Streams, events and device buffers live in a per-device context that is kept between calls (grown on demand;
 // hdp_b200_host_release frees it): cudaMalloc / cudaFree of GB-sized buffers would otherwise cost as much as the copies.
@@ -31,23 +31,6 @@
 #include "common.cuh"
 
 namespace hdp {
-
-int thresholds_launch(const float *d_temps, int64_t C, int64_t T_b, int64_t ld_t, int64_t ld_c,
-                      const int32_t *h_time_index, const int32_t *h_win_rows, int n_doy, int n_y, int W,
-                      const double *h_q, int P, double *d_out,
-                      void *d_workspace, size_t workspace_bytes, void *stream, int64_t carve_cells, bool tables_resident, int input_unit);
-int metrics_launch(const float *d_measure, int64_t C, int64_t T, int64_t ld_t, int64_t ld_c,
-                   const double *d_thr, int n_doy, int P, const int32_t *h_doy_map,
-                   const int32_t *h_defs, int D,
-                   const int32_t *h_season_north, const int32_t *h_season_south, int Y,
-                   const uint8_t *d_is_south, uint16_t *d_out,
-                   void *d_workspace, size_t workspace_bytes, void *stream, int64_t carve_cells, bool tables_resident, int input_unit);
-int intensity_launch(const float *d_measure, int64_t C, int64_t T, int64_t ld_t, int64_t ld_c,
-                     const double *d_thr, int n_doy, int P, const int32_t *h_doy_map,
-                     const int32_t *h_defs, int D,
-                     const int32_t *h_season_north, const int32_t *h_season_south, int Y,
-                     const uint8_t *d_is_south, float *d_int, uint16_t *d_out,
-                     void *d_workspace, size_t workspace_bytes, void *stream, int64_t carve_cells, bool tables_resident, int input_unit);
 
 constexpr int kSlots = 3;
 constexpr int kMaxDevices = 64;
@@ -337,8 +320,8 @@ using namespace hdp;
     } while (0)
 #define HDP_HOST_CUDA(expr) HDP_HOST_TRY(cuda_status(expr))
 
-// hdp_b200_metrics_host (h_int == NULL) and hdp_b200_intensity_host: the same chunk pipeline; with h_int the chunk's kernels are
-// those of hdp_b200_intensity, and the f32 planes (and the u16 ones when h_out is given) go back to the host.
+// hdp_b200_metrics_host and hdp_b200_intensity_host: metric_pass chunk by chunk; the u16 planes (h_out) and the f32 planes (h_int),
+// whichever are given, go back to the host.
 static int metric_pass_host(const float *h_measure, int64_t C, int64_t T, int64_t ld_t, int64_t ld_c,
                             const double *h_thr, const double *d_thr, int n_doy, int P, const int32_t *h_doy_map,
                             const int32_t *h_defs, int D,
@@ -392,14 +375,9 @@ static int metric_pass_host(const float *h_measure, int64_t C, int64_t T, int64_
         HDP_HOST_CUDA(cudaStreamWaitEvent(ctx->s_k, ctx->out_done[slot], 0));
         const double *thr_chunk = d_thr ? d_thr + (size_t)c0 * n_doy * P : (const double *)ctx->aux[slot].p;
         const uint8_t *south_chunk = h_is_south ? (const uint8_t *)ctx->south[slot].p : nullptr;
-        if (h_int)
-            HDP_HOST_TRY(intensity_launch((const float *)ctx->x[slot].p, nc, T, a, b, thr_chunk, n_doy, P, h_doy_map,
-                                          h_defs, D, h_season_north, h_season_south, Y, south_chunk, (float *)ctx->out_f[slot].p,
-                                          h_out ? (uint16_t *)ctx->out[slot].p : nullptr, ctx->ws.p, ws_bytes, ctx->s_k, chunk, i > 0, input_unit));
-        else
-            HDP_HOST_TRY(metrics_launch((const float *)ctx->x[slot].p, nc, T, a, b, thr_chunk, n_doy, P, h_doy_map,
-                                        h_defs, D, h_season_north, h_season_south, Y, south_chunk,
-                                        (uint16_t *)ctx->out[slot].p, ctx->ws.p, ws_bytes, ctx->s_k, chunk, i > 0, input_unit));
+        HDP_HOST_TRY(metric_pass((const float *)ctx->x[slot].p, nc, T, a, b, thr_chunk, n_doy, P, h_doy_map, h_defs, D,
+                                 h_season_north, h_season_south, Y, south_chunk, h_out ? (uint16_t *)ctx->out[slot].p : nullptr,
+                                 h_int ? (float *)ctx->out_f[slot].p : nullptr, ctx->ws.p, ws_bytes, ctx->s_k, chunk, i > 0, input_unit));
         HDP_HOST_CUDA(cudaEventRecord(ctx->k_done[slot], ctx->s_k));
 
         // device chunk is [rows, nc]; host array is [rows, C]

@@ -101,74 +101,23 @@ k_intensity(const uint32_t *__restrict__ hot, const float *__restrict__ x, int64
     };
 
     const uint32_t *hp = hot + (int64_t)p * K * C + c;
-    int run_start = -1, run_word = 0;                               // hot run still open at the end of the previous word
-    uint32_t carry = 0u;                                             // the last day of the previous word was hot
-    for (int k = 0; k <= K; k++) {                                   // word K: a virtual cold day at T closes an open run
+    HotRuns runs{&word_s[0].x, 2, K, T};
+    for (int k = 0; k <= K; k++) {
         if (!__any_sync(0xffffffffu, L.open())) break;
         const uint32_t w = k < K ? __ldg(hp + (int64_t)k * C) : 0u;
         if (!L.open()) continue;
-        const int t0 = k < K ? word_s[k].x : T;
-        const int nb = k + 1 < K ? word_s[k + 1].x - t0 : k < K ? T - t0 : 1;
-        const uint32_t vmask = nb == 32 ? 0xffffffffu : (1u << nb) - 1u;
-        const uint32_t prev = (w << 1) | carry;
-        uint32_t starts = w & ~prev, ends = ~w & prev & vmask;
-        carry = (w >> (nb - 1)) & 1u;
-        while (ends != 0u) {
-            int s, ks;
-            if (run_start >= 0) { s = run_start; ks = run_word; run_start = -1; }
-            else { s = t0 + __ffs(starts) - 1; ks = k; starts &= starts - 1u; }
-            const int e = t0 + __ffs(ends) - 1;
-            ends &= ends - 1u;
-            uint32_t lab = 0u;
-            for (int d = 0; d < D; d++) {
-                IndexState sd = ist[d * 32 + lane];
-                if (index_run(sd, s, e, defs.v[3 * d], defs.v[3 * d + 1], defs.v[3 * d + 2]) != 0) lab |= 1u << d;
-                ist[d * 32 + lane] = sd;
-            }
-            kw = ks;
-            intensity_run(L, s, e, lab, acc + lane, 32, block, flush);
-        }
-        if (starts != 0u) { run_start = t0 + __ffs(starts) - 1; run_word = k; }
+        runs.word(k, w);
+        int s, e;
+        while (runs.pop(s, e, kw)) intensity_run(L, s, e, label_run(ist + lane, 32, defs.v, D, s, e), acc + lane, 32, block, flush);
     }
     while (L.open()) { flush(); L.next(); }
 }
 
-// The whole of hdp_b200_intensity; carve_cells / tables_resident as in metrics_launch.
-int intensity_launch(const float *d_measure, int64_t C, int64_t T, int64_t ld_t, int64_t ld_c,
-                     const double *d_thr, int n_doy, int P, const int32_t *h_doy_map,
-                     const int32_t *h_defs, int D,
-                     const int32_t *h_season_north, const int32_t *h_season_south, int Y,
-                     const uint8_t *d_is_south, float *d_int, uint16_t *d_out,
-                     void *d_workspace, size_t workspace_bytes, void *stream, int64_t carve_cells, bool tables_resident, int input_unit)
+int run_intensity(const Layout &L, const WordPlan &plan, const float *d_measure, int64_t C, int64_t T, int64_t ld_t, int64_t ld_c,
+                  const double *d_thr, int n_doy, int P, const int32_t *h_defs, int D, const std::vector<int32_t> &seasons, int Y,
+                  const uint8_t *d_is_south, float *d_int, cudaStream_t st, bool tables_resident, int input_unit)
 {
-    if (bad_dims(C, T, n_doy, P) || D <= 0 || Y < 0) return HDP_B200_ERR_INVALID;
-    if ((T > 0 && !h_doy_map) || !h_defs || (Y > 0 && (!h_season_north || !h_season_south))) return HDP_B200_ERR_INVALID;
-    if (C > 0 && T > 0 && (!d_measure || !d_thr)) return HDP_B200_ERR_INVALID;
-    if (C > 0 && Y > 0 && !d_int) return HDP_B200_ERR_INVALID;
-    if (P > HDP_B200_MAX_PERCENTILES || D > HDP_B200_MAX_DEFINITIONS) return HDP_B200_ERR_UNSUPPORTED;
-    cudaStream_t st = (cudaStream_t)stream;
-
-    // one open season per lane: each hemisphere's non-empty seasons must be disjoint
-    std::vector<int32_t> tab((size_t)8 * (Y + 1), 0);
-    if (!intensity_season_table(h_season_north, Y, T, tab.data()) || !intensity_season_table(h_season_south, Y, T, tab.data() + 4 * (Y + 1)))
-        return HDP_B200_ERR_UNSUPPORTED;
-    ScanPasses passes[2];
-    if (d_out) {
-        const int rc = scan_passes(h_season_north, h_season_south, Y, T, passes);
-        if (rc != HDP_B200_OK) return rc;
-    }
-
-    WordPlan plan;
-    Layout L;
-    int rc = run_hot_words(d_measure, C, T, ld_t, ld_c, d_thr, n_doy, P, h_doy_map, Y, d_workspace, workspace_bytes, st, plan, L,
-                           carve_cells, tables_resident, input_unit, true);
-    if (rc != HDP_B200_OK || C == 0 || Y == 0) return rc;
     const int K = (int)plan.words.size();
-    if (d_out) {
-        rc = run_scan(L, plan, C, T, P, h_defs, D, passes, Y, d_is_south, d_out, st, tables_resident);
-        if (rc != HDP_B200_OK) return rc;
-    }
-
     const size_t words_bytes = ((size_t)K * sizeof(int2) + 15) & ~(size_t)15;
     const size_t per_warp = int_warp_bytes(D);
     if (words_bytes + per_warp > kIntSmemMax) return HDP_B200_ERR_UNSUPPORTED;
@@ -177,7 +126,7 @@ int intensity_launch(const float *d_measure, int64_t C, int64_t T, int64_t ld_t,
     IntensityDefs defs;
     for (int i = 0; i < 3 * HDP_B200_MAX_DEFINITIONS; i++) defs.v[i] = i < 3 * D ? h_defs[i] : 0;
     if (!tables_resident)
-        HDP_CUDA_TRY(cudaMemcpyAsync(L.int_seasons, tab.data(), sizeof(int32_t) * tab.size(), cudaMemcpyHostToDevice, st));
+        HDP_CUDA_TRY(cudaMemcpyAsync(L.int_seasons, seasons.data(), sizeof(int32_t) * seasons.size(), cudaMemcpyHostToDevice, st));
     const float *x = ld_c != 1 ? L.xn : d_measure;                  // run_hot_words normalised other layouts into L.xn
     const int64_t x_ld_t = ld_c != 1 ? C : ld_t;
     const int64_t n_warps = ((C + 31) / 32) * P;
@@ -200,9 +149,7 @@ size_t hdp_b200_intensity_workspace_bytes(int64_t C, int64_t T, int64_t ld_t, in
                                           int n_doy, int P, int D, int Y, const int32_t *h_doy_map)
 {
     (void)ld_t; (void)D;
-    if (bad_dims(C, T, n_doy, P) || Y < 0) return 0;
-    const int64_t K = h_doy_map ? count_words(h_doy_map, T) : words_upper_bound(T, n_doy);
-    return carve(nullptr, 0, C, T, ld_c != 1, K, n_doy, P, Y, true).total;
+    return metric_pass_workspace_bytes(C, T, ld_c, n_doy, P, Y, h_doy_map, true);
 }
 
 int hdp_b200_intensity(const float *d_measure, int64_t C, int64_t T, int64_t ld_t, int64_t ld_c,
@@ -212,8 +159,9 @@ int hdp_b200_intensity(const float *d_measure, int64_t C, int64_t T, int64_t ld_
                        const uint8_t *d_is_south, float *d_int, uint16_t *d_out,
                        void *d_workspace, size_t workspace_bytes, void *stream, int input_unit)
 {
-    return intensity_launch(d_measure, C, T, ld_t, ld_c, d_thr, n_doy, P, h_doy_map, h_defs, D, h_season_north, h_season_south, Y,
-                            d_is_south, d_int, d_out, d_workspace, workspace_bytes, stream, C, false, input_unit);
+    if (C > 0 && Y > 0 && !d_int) return HDP_B200_ERR_INVALID;
+    return metric_pass(d_measure, C, T, ld_t, ld_c, d_thr, n_doy, P, h_doy_map, h_defs, D, h_season_north, h_season_south, Y,
+                       d_is_south, d_out, d_int, d_workspace, workspace_bytes, stream, C, false, input_unit);
 }
 
 }  // extern "C"

@@ -48,22 +48,22 @@ HDP_HD void intensity_values(const IntensityAcc &a, float &hwc, float &hwi, floa
     hwp = (float)a.peak;
 }
 
+// index of the lowest set bit of v != 0
+HDP_HD int low_bit(uint32_t v)
+{
+#ifdef __CUDA_ARCH__
+    return __ffs(v) - 1;
+#else
+    return __builtin_ctz(v);
+#endif
+}
+
 // ---- season tables ------------------------------------------------------------------------------------------------------
-// A lane keeps ONE open season, so a hemisphere's seasons must be disjoint.  raw i32 [Y, 2] (Python slice semantics) ->
-// tab i32 [Y, 4] {lo, hi, row, 0} sorted by lo (stable).  Empty seasons may sit anywhere; any two non-empty seasons must not
-// overlap.  Returns false otherwise.
+// A lane keeps ONE open season, so a hemisphere's seasons must be disjoint.  Builds tab as season_table (seams.h) does and returns
+// whether it qualifies: empty seasons may sit anywhere, but no two non-empty seasons may overlap.
 HDP_HD bool intensity_season_table(const int32_t *raw, int Y, int64_t T, int32_t *tab)
 {
-    for (int y = 0; y < Y; y++) {
-        int64_t lo, hi;
-        season_slice(raw[2 * y], raw[2 * y + 1], T, lo, hi);
-        int i = y;                                                          // insertion sort by lo, stable
-        while (i > 0 && tab[4 * (i - 1)] > lo) {
-            for (int k = 0; k < 4; k++) tab[4 * i + k] = tab[4 * (i - 1) + k];
-            i--;
-        }
-        tab[4 * i] = (int32_t)lo; tab[4 * i + 1] = (int32_t)hi; tab[4 * i + 2] = y; tab[4 * i + 3] = 0;
-    }
+    season_table(raw, Y, T, tab);
     int64_t end = INT64_MIN;                                                // end of the last non-empty season
     for (int y = 0; y < Y; y++) {
         if (tab[4 * y + 1] == tab[4 * y]) continue;
@@ -74,8 +74,59 @@ HDP_HD bool intensity_season_table(const int32_t *raw, int Y, int64_t T, int32_t
 }
 
 // ---- one lane --------------------------------------------------------------------------------------------------------------
+// The hot runs [s, e) of one lane in time order, popped from its hot-day words (k_hot_words).  Word k starts at day
+// word_t0[k * stride] and ends where word k + 1 starts (the last one at T); bit j is day t0 + j.  Word K is a virtual cold day at
+// T that closes a run still open at the end of the series.
+struct HotRuns {
+    const int *word_t0;
+    int stride, K, T;
+    int k = 0, t0 = 0;                   // the current word and its first day
+    uint32_t starts = 0u, ends = 0u;     // its run starts and run ends not popped yet
+    uint32_t carry = 0u;                 // the last day of the previous word was hot
+    int open_s = -1, open_k = 0;         // the run still open at the end of the previous word: first day, word of that day
+
+    // word k_ with hot-day bits w (0 for word K)
+    HDP_HD void word(int k_, uint32_t w)
+    {
+        k = k_;
+        t0 = k < K ? word_t0[k * stride] : T;
+        const int nb = k + 1 < K ? word_t0[(k + 1) * stride] - t0 : k < K ? T - t0 : 1;
+        const uint32_t vmask = nb == 32 ? 0xffffffffu : (1u << nb) - 1u;
+        const uint32_t prev = (w << 1) | carry;
+        starts = w & ~prev;
+        ends = ~w & prev & vmask;
+        carry = (w >> (nb - 1)) & 1u;
+    }
+    // the next run that ends in the current word, and the word ks of its first day; false when none is left
+    HDP_HD bool pop(int &s, int &e, int &ks)
+    {
+        if (ends == 0u) {
+            if (starts != 0u) { open_s = t0 + low_bit(starts); open_k = k; starts = 0u; }   // (at most one: it ends later)
+            return false;
+        }
+        if (open_s >= 0) { s = open_s; ks = open_k; open_s = -1; }
+        else { s = t0 + low_bit(starts); ks = k; starts &= starts - 1u; }
+        e = t0 + low_bit(ends);
+        ends &= ends - 1u;
+        return true;
+    }
+};
+
+// The hot run [s, e) through every definition's index_heatwaves state machine (st[d * stride]; defs i32 [D, 3]): bit d of the
+// result is set when definition d labels the run.
+HDP_HD uint32_t label_run(IndexState *st, int stride, const int *defs, int D, int64_t s, int64_t e)
+{
+    uint32_t lab = 0u;
+    for (int d = 0; d < D; d++) {
+        IndexState sd = st[d * stride];
+        if (index_run(sd, s, e, defs[3 * d], defs[3 * d + 1], defs[3 * d + 2]) != 0) lab |= 1u << d;
+        st[d * stride] = sd;
+    }
+    return lab;
+}
+
 struct IntensityLane {
-    const int32_t *seas = nullptr;   // i32 [n, 4] as built by intensity_season_table
+    const int32_t *seas = nullptr;   // i32 [n, 4] as built by season_table
     int n = 0, ys = 0;
     int64_t a = 0, b = 0;            // the open season [a, b)
     int row = 0;                     // its output row
@@ -104,14 +155,7 @@ HDP_HD void intensity_run(IntensityLane &L, int64_t s, int64_t e, uint32_t lab, 
         if (hi > lo) {
             double r = 0.0, m = 0.0;
             block(lo, hi, r, m);
-            for (uint32_t bits = lab; bits != 0u; bits &= bits - 1u) {
-#ifdef __CUDA_ARCH__
-                const int d = __ffs(bits) - 1;
-#else
-                const int d = __builtin_ctz(bits);
-#endif
-                intensity_block(acc[d * stride], r, m, hi - lo);
-            }
+            for (uint32_t bits = lab; bits != 0u; bits &= bits - 1u) intensity_block(acc[low_bit(bits) * stride], r, m, hi - lo);
         }
         if (e <= L.b) break;
         flush();

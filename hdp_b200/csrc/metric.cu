@@ -22,6 +22,7 @@
 #include <vector>
 #include <algorithm>
 
+#include "intensity.h"
 #include "metric.cuh"
 
 namespace hdp {
@@ -508,21 +509,16 @@ k_scan(const uint32_t *__restrict__ hot, int64_t C, int K, int T, const int4 *__
 // ----------------------------------------------------------------------------------------------------
 // host side
 // ----------------------------------------------------------------------------------------------------
-// Cuts the time axis into words of <= 32 consecutive days whose days of year are consecutive and stay
-// inside one 32-day block of the day-of-year axis (so that every word of a block shares one threshold tile).
+static_assert(kTileDoy == 32, "word_length (seams.h) cuts words at 32-day blocks of the day-of-year axis");
+
+// Cuts the time axis into hot-day words (word_length) and groups them by day-of-year block.
 static int build_words(const int32_t *doy_map, int64_t T, int n_doy, WordPlan &plan)
 {
     plan.n_blk = (n_doy + kTileDoy - 1) / kTileDoy;
-    int64_t t = 0;
-    while (t < T) {
+    for (int64_t t = 0; t < T;) {
         const int d0 = doy_map[t];
         if (d0 < 0 || d0 >= n_doy) return HDP_B200_ERR_INVALID;
-        int nb = 1;
-        while (t + nb < T && nb < 32) {
-            const int d = doy_map[t + nb];
-            if (d != d0 + nb || (d & (kTileDoy - 1)) == 0) break;
-            nb++;
-        }
+        const int nb = word_length(doy_map, t, T);
         plan.words.push_back(make_int4((int)t, nb, d0, 0));
         t += nb;
     }
@@ -536,27 +532,17 @@ static int build_words(const int32_t *doy_map, int64_t T, int n_doy, WordPlan &p
     return HDP_B200_OK;
 }
 
-int64_t words_upper_bound(int64_t T, int n_doy)
+static int64_t words_upper_bound(int64_t T, int n_doy)
 {
     // regular daily calendars: every (partial) year contributes at most n_blk + 1 words
     const int64_t n_blk = (n_doy + kTileDoy - 1) / kTileDoy;
     return (T / std::max(n_doy, 1) + 2) * (n_blk + 1) + 1;
 }
 
-int64_t count_words(const int32_t *doy_map, int64_t T)
+static int64_t count_words(const int32_t *doy_map, int64_t T)
 {
-    int64_t K = 0, t = 0;
-    while (t < T) {
-        const int d0 = doy_map[t];
-        int nb = 1;
-        while (t + nb < T && nb < 32) {
-            const int d = doy_map[t + nb];
-            if (d != d0 + nb || (d & (kTileDoy - 1)) == 0) break;
-            nb++;
-        }
-        K++;
-        t += nb;
-    }
+    int64_t K = 0;
+    for (int64_t t = 0; t < T; K++) t += word_length(doy_map, t, T);
     return K;
 }
 
@@ -571,7 +557,8 @@ static int pick_pg(int P)
     return best;
 }
 
-Layout carve(void *ws, size_t ws_bytes, int64_t C, int64_t T, bool need_norm, int64_t K, int n_doy, int P, int Y, bool intensity)
+// Workspace layout; `intensity` appends the intensity pass's season tables behind what the metric pass uses.
+static Layout carve(void *ws, size_t ws_bytes, int64_t C, int64_t T, bool need_norm, int64_t K, int n_doy, int P, int Y, bool intensity)
 {
     Layout L;
     Carver cv(ws, ws_bytes);
@@ -587,15 +574,24 @@ Layout carve(void *ws, size_t ws_bytes, int64_t C, int64_t T, bool need_norm, in
     return L;
 }
 
-bool bad_dims(int64_t C, int64_t T, int n_doy, int P)
+static bool bad_dims(int64_t C, int64_t T, int n_doy, int P)
 {
     return C < 0 || T < 0 || n_doy <= 0 || P <= 0 || T > 0x3fffffff;
 }
 
-int run_hot_words(const float *d_measure, int64_t C, int64_t T, int64_t ld_t, int64_t ld_c,
-                  const double *d_thr, int n_doy, int P, const int32_t *h_doy_map,
-                  int Y, void *ws, size_t ws_bytes, cudaStream_t st, WordPlan &plan, Layout &L,
-                  int64_t carve_cells, bool tables_resident, int input_unit, bool intensity)
+size_t metric_pass_workspace_bytes(int64_t C, int64_t T, int64_t ld_c, int n_doy, int P, int Y, const int32_t *h_doy_map, bool intensity)
+{
+    if (bad_dims(C, T, n_doy, P) || Y < 0) return 0;
+    const int64_t K = h_doy_map ? count_words(h_doy_map, T) : words_upper_bound(T, n_doy);
+    return carve(nullptr, 0, C, T, ld_c != 1, K, n_doy, P, Y, intensity).total;
+}
+
+// Runs k_hot_words (after the layout-normalising copy when ld_c != 1: the samples then live in L.xn, time-major, ld_t = C);
+// on success plan / L describe what lives in the workspace.
+static int run_hot_words(const float *d_measure, int64_t C, int64_t T, int64_t ld_t, int64_t ld_c,
+                         const double *d_thr, int n_doy, int P, const int32_t *h_doy_map,
+                         int Y, void *ws, size_t ws_bytes, cudaStream_t st, WordPlan &plan, Layout &L,
+                         int64_t carve_cells = 0, bool tables_resident = false, int input_unit = 0, bool intensity = false)
 {
     if (input_unit < 0 || input_unit > 2) return HDP_B200_ERR_INVALID;
     int rc = build_words(h_doy_map, T, n_doy, plan);
@@ -645,68 +641,28 @@ int run_hot_words(const float *d_measure, int64_t C, int64_t T, int64_t ld_t, in
     return HDP_B200_OK;
 }
 
-// Python-slice semantics of hw_ts[a:b] (metric.py:79,100,122,157) resolved to 0 <= lo <= hi <= T.
-static void clamp_season(int64_t a, int64_t b, int64_t T, int &lo, int &hi)
-{
-    if (a < 0) { a += T; if (a < 0) a = 0; }
-    if (b < 0) { b += T; if (b < 0) b = 0; }
-    if (a > T) a = T;
-    if (b > T) b = T;
-    if (b < a) b = a;
-    lo = (int)a; hi = (int)b;
-}
+// k_scan's season tables: per hemisphere, passes of sorted, disjoint seasons (one launch each).
+struct ScanSeason { int a, b, row; };
+using ScanPasses = std::vector<std::vector<ScanSeason>>;
 
-int scan_passes(const int32_t *h_season_north, const int32_t *h_season_south, int Y, int64_t T, ScanPasses (&passes)[2])
+// Splits a hemisphere's season table (season_table, sorted by start) into passes: each season goes to the first pass it does
+// not overlap.  Seasons of more than 65 535 days do not fit the u16 output.
+static int scan_passes(const int32_t *tab, int Y, ScanPasses &passes)
 {
-    for (int h = 0; h < 2; h++) {
-        const int32_t *tab = h == 0 ? h_season_north : h_season_south;
-        std::vector<ScanSeason> all(Y);
-        for (int y = 0; y < Y; y++) {
-            clamp_season(tab[2 * y], tab[2 * y + 1], T, all[y].a, all[y].b);
-            all[y].row = y;
-            if (all[y].b - all[y].a > 65535) return HDP_B200_ERR_UNSUPPORTED;
-        }
-        std::stable_sort(all.begin(), all.end(), [](const ScanSeason &l, const ScanSeason &r) { return l.a < r.a; });
-        for (const ScanSeason &s : all) {
-            size_t i = 0;
-            for (; i < passes[h].size(); i++)
-                if (passes[h][i].back().b <= s.a) break;
-            if (i == passes[h].size()) passes[h].emplace_back();
-            passes[h][i].push_back(s);
-        }
+    for (int y = 0; y < Y; y++) {
+        const ScanSeason s = {tab[4 * y], tab[4 * y + 1], tab[4 * y + 2]};
+        if (s.b - s.a > 65535) return HDP_B200_ERR_UNSUPPORTED;
+        size_t i = 0;
+        while (i < passes.size() && passes[i].back().b > s.a) i++;
+        if (i == passes.size()) passes.emplace_back();
+        passes[i].push_back(s);
     }
     return HDP_B200_OK;
 }
 
-// The whole of hdp_b200_metrics; carve_cells / tables_resident as in thresholds_launch (threshold.cu).
-int metrics_launch(const float *d_measure, int64_t C, int64_t T, int64_t ld_t, int64_t ld_c,
-                   const double *d_thr, int n_doy, int P, const int32_t *h_doy_map,
-                   const int32_t *h_defs, int D,
-                   const int32_t *h_season_north, const int32_t *h_season_south, int Y,
-                   const uint8_t *d_is_south, uint16_t *d_out,
-                   void *d_workspace, size_t workspace_bytes, void *stream, int64_t carve_cells, bool tables_resident, int input_unit)
-{
-    if (bad_dims(C, T, n_doy, P) || D <= 0 || Y < 0) return HDP_B200_ERR_INVALID;
-    if ((T > 0 && !h_doy_map) || !h_defs || (Y > 0 && (!h_season_north || !h_season_south))) return HDP_B200_ERR_INVALID;
-    if (C > 0 && T > 0 && (!d_measure || !d_thr)) return HDP_B200_ERR_INVALID;
-    if (C > 0 && Y > 0 && !d_out) return HDP_B200_ERR_INVALID;
-    if (P > HDP_B200_MAX_PERCENTILES || D > HDP_B200_MAX_DEFINITIONS) return HDP_B200_ERR_UNSUPPORTED;
-    cudaStream_t st = (cudaStream_t)stream;
-
-    ScanPasses passes[2];
-    int rc = scan_passes(h_season_north, h_season_south, Y, T, passes);
-    if (rc != HDP_B200_OK) return rc;
-
-    WordPlan plan;
-    Layout L;
-    rc = run_hot_words(d_measure, C, T, ld_t, ld_c, d_thr, n_doy, P, h_doy_map, Y, d_workspace, workspace_bytes, st, plan, L,
-                       carve_cells, tables_resident, input_unit);
-    if (rc != HDP_B200_OK || C == 0 || Y == 0) return rc;
-    return run_scan(L, plan, C, T, P, h_defs, D, passes, Y, d_is_south, d_out, st, tables_resident);
-}
-
-int run_scan(const Layout &L, const WordPlan &plan, int64_t C, int64_t T, int P, const int32_t *h_defs, int D,
-             const ScanPasses (&passes)[2], int Y, const uint8_t *d_is_south, uint16_t *d_out, cudaStream_t st, bool tables_resident)
+// k_scan over the hot words in L (one launch per pass): the integer metrics u16 [4, P, D, Y, C].
+static int run_scan(const Layout &L, const WordPlan &plan, int64_t C, int64_t T, int P, const int32_t *h_defs, int D,
+                    const ScanPasses (&passes)[2], int Y, const uint8_t *d_is_south, uint16_t *d_out, cudaStream_t st, bool tables_resident)
 {
     const size_t n_pass = std::max(passes[0].size(), passes[1].size());
     const int K = (int)plan.words.size();
@@ -824,6 +780,47 @@ int run_scan(const Layout &L, const WordPlan &plan, int64_t C, int64_t T, int P,
     return HDP_B200_OK;
 }
 
+int metric_pass(const float *d_measure, int64_t C, int64_t T, int64_t ld_t, int64_t ld_c,
+                const double *d_thr, int n_doy, int P, const int32_t *h_doy_map,
+                const int32_t *h_defs, int D,
+                const int32_t *h_season_north, const int32_t *h_season_south, int Y,
+                const uint8_t *d_is_south, uint16_t *d_out, float *d_int,
+                void *d_workspace, size_t workspace_bytes, void *stream, int64_t carve_cells, bool tables_resident, int input_unit)
+{
+    if (bad_dims(C, T, n_doy, P) || D <= 0 || Y < 0) return HDP_B200_ERR_INVALID;
+    if ((T > 0 && !h_doy_map) || !h_defs || (Y > 0 && (!h_season_north || !h_season_south))) return HDP_B200_ERR_INVALID;
+    if (C > 0 && T > 0 && (!d_measure || !d_thr)) return HDP_B200_ERR_INVALID;
+    if (P > HDP_B200_MAX_PERCENTILES || D > HDP_B200_MAX_DEFINITIONS) return HDP_B200_ERR_UNSUPPORTED;
+    cudaStream_t st = (cudaStream_t)stream;
+
+    // the season tables of both hemispheres, north then south (Y + 1 rows apart, as k_intensity reads them)
+    std::vector<int32_t> seasons((size_t)8 * (Y + 1), 0);
+    ScanPasses passes[2];
+    for (int h = 0; h < 2; h++) {
+        int32_t *tab = seasons.data() + (size_t)4 * (Y + 1) * h;
+        const bool disjoint = intensity_season_table(h == 0 ? h_season_north : h_season_south, Y, T, tab);
+        if (d_int && !disjoint) return HDP_B200_ERR_UNSUPPORTED;                        // k_intensity: one open season per lane
+        if (d_out) {
+            const int rc = scan_passes(tab, Y, passes[h]);
+            if (rc != HDP_B200_OK) return rc;
+        }
+    }
+
+    WordPlan plan;
+    Layout L;
+    int rc = run_hot_words(d_measure, C, T, ld_t, ld_c, d_thr, n_doy, P, h_doy_map, Y, d_workspace, workspace_bytes, st, plan, L,
+                           carve_cells, tables_resident, input_unit, d_int != nullptr);
+    if (rc != HDP_B200_OK || C == 0 || Y == 0) return rc;
+    if (d_out) {
+        rc = run_scan(L, plan, C, T, P, h_defs, D, passes, Y, d_is_south, d_out, st, tables_resident);
+        if (rc != HDP_B200_OK) return rc;
+    }
+    if (d_int)
+        rc = run_intensity(L, plan, d_measure, C, T, ld_t, ld_c, d_thr, n_doy, P, h_defs, D, seasons, Y, d_is_south, d_int, st,
+                           tables_resident, input_unit);
+    return rc;
+}
+
 }  // namespace hdp
 
 using namespace hdp;
@@ -834,9 +831,7 @@ size_t hdp_b200_metrics_workspace_bytes(int64_t C, int64_t T, int64_t ld_t, int6
                                         int n_doy, int P, int D, int Y, const int32_t *h_doy_map)
 {
     (void)ld_t; (void)D;
-    if (bad_dims(C, T, n_doy, P) || Y < 0) return 0;
-    const int64_t K = h_doy_map ? count_words(h_doy_map, T) : words_upper_bound(T, n_doy);
-    return carve(nullptr, 0, C, T, ld_c != 1, K, n_doy, P, Y).total;
+    return metric_pass_workspace_bytes(C, T, ld_c, n_doy, P, Y, h_doy_map, false);
 }
 
 void hdp_b200_metrics_run_filter(int on) { g_scan_filter = on != 0; }
@@ -869,8 +864,9 @@ int hdp_b200_metrics(const float *d_measure, int64_t C, int64_t T, int64_t ld_t,
                      const uint8_t *d_is_south, uint16_t *d_out,
                      void *d_workspace, size_t workspace_bytes, void *stream, int input_unit)
 {
-    return metrics_launch(d_measure, C, T, ld_t, ld_c, d_thr, n_doy, P, h_doy_map, h_defs, D, h_season_north, h_season_south, Y,
-                          d_is_south, d_out, d_workspace, workspace_bytes, stream, C, false, input_unit);
+    if (C > 0 && Y > 0 && !d_out) return HDP_B200_ERR_INVALID;
+    return metric_pass(d_measure, C, T, ld_t, ld_c, d_thr, n_doy, P, h_doy_map, h_defs, D, h_season_north, h_season_south, Y,
+                       d_is_south, d_out, nullptr, d_workspace, workspace_bytes, stream, C, false, input_unit);
 }
 
 }  // extern "C"

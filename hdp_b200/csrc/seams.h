@@ -1,6 +1,7 @@
 // seams.h - the per-run and per-season logic of the reference's path-2 BUILDING BLOCKS, as plain functions that compile for
 // the device (seams.cu) and for the host (tests/seams_host.cpp, which replays the kernels' lane loops on the CPU against the
-// oracle: the logic below is checked without a GPU, the kernels add only the warp plumbing around it).
+// oracle: the logic below is checked without a GPU, the kernels add only the warp plumbing around it).  It also holds the two
+// rules of the fused pass that its host replay (tests/intensity_host.cpp) shares: the season table and the cut into hot-day words.
 //
 // Reference = AgentOxygen/HDP v1.0.2:
 //   index_heatwaves      hdp/metric.py:11-60
@@ -73,6 +74,33 @@ HDP_HD void season_slice(int64_t a, int64_t b, int64_t T, int64_t &lo, int64_t &
     if (b < a) b = a;
     lo = a;
     hi = b;
+}
+
+// raw i32 [Y, 2] (season_slice semantics) -> tab i32 [Y, 4] {lo, hi, row, 0}, stably sorted by lo: the season table of one
+// hemisphere as the fused metric pass (metric.cu) and its intensity kernel walk it.
+HDP_HD void season_table(const int32_t *raw, int Y, int64_t T, int32_t *tab)
+{
+    for (int y = 0; y < Y; y++) {
+        int64_t lo, hi;
+        season_slice(raw[2 * y], raw[2 * y + 1], T, lo, hi);
+        int i = y;                                                          // insertion sort by lo, stable
+        while (i > 0 && tab[4 * (i - 1)] > lo) {
+            for (int k = 0; k < 4; k++) tab[4 * i + k] = tab[4 * (i - 1) + k];
+            i--;
+        }
+        tab[4 * i] = (int32_t)lo; tab[4 * i + 1] = (int32_t)hi; tab[4 * i + 2] = y; tab[4 * i + 3] = 0;
+    }
+}
+
+// ---- hot-day words --------------------------------------------------------------------------------------------------------
+// The fused metric pass cuts the time axis into words of <= 32 consecutive days whose days of year are consecutive and stay inside
+// one 32-day block of the day-of-year axis, so that every word of a block shares one threshold tile (k_hot_words, metric.cu).
+// Length of the word that starts at day t.
+HDP_HD int word_length(const int32_t *doy_map, int64_t t, int64_t T)
+{
+    int nb = 1;
+    while (t + nb < T && nb < 32 && doy_map[t + nb] == doy_map[t] + nb && (doy_map[t + nb] & 31) != 0) nb++;
+    return nb;
 }
 
 // What one lane of a warp adds up over its elements i = lane, lane + n_lanes, ... of the slice v[0 .. n).

@@ -1792,9 +1792,6 @@ static std::shared_ptr<ThrPlans> thr_plans(const int32_t *h_time_index, const in
     return cached;
 }
 
-// The whole of hdp_b200_thresholds.  `carve_cells` sizes the workspace layout (>= C; the host pipeline passes its chunk
-// capacity so that every chunk sees the tables at the same place) and `tables_resident` skips the table uploads when
-// the previous call on this workspace and stream used identical tables.
 int thresholds_launch(const float *d_temps, int64_t C, int64_t T_b, int64_t ld_t, int64_t ld_c,
                       const int32_t *h_time_index, const int32_t *h_win_rows, int n_doy, int n_y, int W,
                       const double *h_q, int P, double *d_out,

@@ -176,8 +176,8 @@ def _widen_int64(a: np.ndarray) -> np.ndarray:
 
 def _metric_sweep(measure, threshold, hw_definitions, time_axis, doy_map=None, intensity=False):
     """The percentile x definition x cell sweep of compute_heatwave_metrics_wrapper (metric.py:344-369) as ONE library call:
-    -> (uint16 [4, P, D, Y, C], season tables, cell dims, cell shape, P, D).  With ``intensity`` the call is the intensity pass
-    and the first item is (uint16 [4, P, D, Y, C], float32 [3, P, D, Y, C])."""
+    -> ((uint16 [4, P, D, Y, C], float32 [3, P, D, Y, C] or None), season tables, cell dims, cell shape, P, D).  With
+    ``intensity`` the call is the intensity pass, which also returns the intensity metrics."""
     st = _tables.hemisphere_ranges(time_axis)                       # compute_hemisphere_ranges, :410
     if doy_map is None:
         doy_map = _tables.doy_map(time_axis.dayofyr)                # build_doy_map, :413
@@ -200,16 +200,16 @@ def _metric_sweep(measure, threshold, hw_definitions, time_axis, doy_map=None, i
     if intensity:
         out = np.empty((4, P, defs.shape[0], st.n_years, x.shape[1]), np.uint16)
         heat = _core.intensity_host(x, thr_cdp, doy_map, defs, st.north, st.south, south, metrics_out=out)   # float32 [3, P, D, Y, C]
-        return (out, heat), st, cell_dims, cell_shape, P, defs.shape[0]
-    out = _core.metrics_host(x, thr_cdp, doy_map, defs, st.north, st.south, south)     # uint16 [4, P, D, Y, C]
-    return out, st, cell_dims, cell_shape, P, defs.shape[0]
+    else:
+        out, heat = _core.metrics_host(x, thr_cdp, doy_map, defs, st.north, st.south, south), None       # uint16 [4, P, D, Y, C]
+    return (out, heat), st, cell_dims, cell_shape, P, defs.shape[0]
 
 
 def compute_heatwave_metrics_wrapper(measure, threshold, doy_map, hw_definitions):
     """metric.py:344-369: the four metrics of every cell for every percentile and definition as one int64 array with dims
     ``(percentile, definition, <cells>, metric, year)``; ``metric`` = HWF, HWN, HWD, HWA in this order (:336-340)."""
     dm = None if doy_map is None else np.asarray(getattr(doy_map, "values", doy_map))
-    out, st, cell_dims, cell_shape, P, D = _metric_sweep(measure, threshold, hw_definitions, time_axis_of(measure), dm)
+    (out, _), st, cell_dims, cell_shape, P, D = _metric_sweep(measure, threshold, hw_definitions, time_axis_of(measure), dm)
     data = out.astype(np.int64).transpose(1, 2, 4, 0, 3).reshape(P, D, *cell_shape, 4, st.n_years)
     coords = {"definition": [f"{hw_def[0]}-{hw_def[1]}-{hw_def[2]}" for hw_def in hw_definitions],      # :347-350
               "percentile": np.asarray(xr.coord_values(threshold, "percentile"))}
@@ -238,9 +238,7 @@ def compute_individual_metrics(measure, threshold, hw_definitions: list, include
             if entry != '':
                 combined_history += (f"(Threshold) {entry}\n")
 
-    out, st, cell_dims, cell_shape, P, D = _metric_sweep(measure, threshold, hw_definitions, time_axis, intensity=intensity)
-    if intensity:
-        out, heat = out
+    (out, heat), st, cell_dims, cell_shape, P, D = _metric_sweep(measure, threshold, hw_definitions, time_axis, intensity=intensity)
     Y = st.n_years
 
     coords = dict(xr.non_time_coords(measure))

@@ -1,5 +1,5 @@
 // intensity_host.cpp - TEST INFRASTRUCTURE: replays the lane loop of k_intensity (hdp_b200/csrc/intensity.cu) on the CPU around
-// the very same per-run / per-season functions (hdp_b200/csrc/intensity.h, and index_run of seams.h), so that
+// the very same functions (hdp_b200/csrc/intensity.h; the season table, the cut into words and index_run of seams.h), so that
 // tests/test_intensity_host.py can check that logic against the oracle without a GPU.  Not part of the product.
 //     g++ -O2 -shared -fPIC -I hdp_b200/csrc tests/intensity_host.cpp -o <tmp>/libintensity_host.so
 #include <stdint.h>
@@ -18,13 +18,16 @@ int intensity_host_cell(const float *x, const double *thr, const int32_t *doy_ma
 {
     std::vector<int32_t> tab((size_t)4 * (Y + 1));
     if (!intensity_season_table(seasons, Y, T, tab.data())) return -2;
-    // words of at most 32 days with consecutive days of year that do not cross a 32-day block (metric.cu build_words)
     std::vector<int> w_t0, w_doy;
+    std::vector<uint32_t> w_hot;                                            // the hot-day words of k_hot_words
     for (int64_t t = 0; t < T;) {
-        int nb = 1;
-        while (t + nb < T && nb < 32 && doy_map[t + nb] == doy_map[t] + nb && (doy_map[t + nb] & 31) != 0) nb++;
+        const int nb = word_length(doy_map, t, T);
+        uint32_t w = 0u;
+        for (int j = 0; j < nb; j++)
+            if ((double)x[t + j] > thr[doy_map[t] + j]) w |= 1u << j;
         w_t0.push_back((int)t);
         w_doy.push_back(doy_map[t]);
+        w_hot.push_back(w);
         t += nb;
     }
     const int K = (int)w_t0.size();
@@ -46,31 +49,11 @@ int intensity_host_cell(const float *x, const double *thr, const int32_t *doy_ma
             intensity_day(r, m, intensity_excess(x[t], thr[doy]));
         }
     };
-    int run_start = -1, run_word = 0;
-    uint32_t carry = 0u;
+    HotRuns runs{w_t0.data(), 1, K, (int)T};
     for (int k = 0; k <= K && L.open(); k++) {
-        const int t0 = k < K ? w_t0[k] : (int)T;
-        const int nb = k + 1 < K ? w_t0[k + 1] - t0 : k < K ? (int)T - t0 : 1;
-        uint32_t w = 0u;                                                    // the hot-day word of k_hot_words
-        for (int j = 0; j < nb && k < K; j++)
-            if ((double)x[t0 + j] > thr[w_doy[k] + j]) w |= 1u << j;
-        const uint32_t vmask = nb == 32 ? 0xffffffffu : (1u << nb) - 1u;
-        const uint32_t prev = (w << 1) | carry;
-        uint32_t starts = w & ~prev, ends = ~w & prev & vmask;
-        carry = (w >> (nb - 1)) & 1u;
-        while (ends != 0u) {
-            int s, ks;
-            if (run_start >= 0) { s = run_start; ks = run_word; run_start = -1; }
-            else { s = t0 + __builtin_ctz(starts); ks = k; starts &= starts - 1u; }
-            const int e = t0 + __builtin_ctz(ends);
-            ends &= ends - 1u;
-            uint32_t lab = 0u;
-            for (int d = 0; d < D; d++)
-                if (index_run(ist[d], s, e, defs[3 * d], defs[3 * d + 1], defs[3 * d + 2]) != 0) lab |= 1u << d;
-            kw = ks;
-            intensity_run(L, s, e, lab, acc.data(), 1, block, flush);
-        }
-        if (starts != 0u) { run_start = t0 + __builtin_ctz(starts); run_word = k; }
+        runs.word(k, k < K ? w_hot[k] : 0u);
+        int s, e;
+        while (runs.pop(s, e, kw)) intensity_run(L, s, e, label_run(ist.data(), 1, defs, D, s, e), acc.data(), 1, block, flush);
     }
     while (L.open()) { flush(); L.next(); }
     return 0;
