@@ -35,6 +35,7 @@ SIGNATURES = {
     "hdp_b200_intensity_host": (_int, [_p, _i64, _i64, _i64, _i64, _p, _p, _int, _int, _p, _p, _int, _p, _p, _int, _p, _p, _p, _int]),
     "hdp_b200_host_release": (None, []),
     "hdp_b200_metrics_run_filter": (None, [_int]),
+    "hdp_b200_metrics_kernel_choice": (_int, [_p, _int, _p, _p, _int, _i64, _p]),
     "hdp_b200_heat_index": (_int, [_p, _p, _i64, _p, _p]),
     "hdp_b200_heat_index_measure": (_int, [_p, _p, _i64, _int, _p, _p]),
     "hdp_b200_to_celsius": (_int, [_p, _i64, _int, _p, _p]),
@@ -72,7 +73,7 @@ def lib() -> ctypes.CDLL:
             fn = getattr(L, name)          # AttributeError if the library does not export the symbol
             fn.restype = res
             fn.argtypes = args
-        if L.hdp_b200_abi_version() != 5:
+        if L.hdp_b200_abi_version() != 6:
             raise RuntimeError("libhdp_b200.so ABI version mismatch; rebuild with `python -m hdp_b200.build --force`")
         _LIB = L
     return _LIB

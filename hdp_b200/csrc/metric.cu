@@ -546,6 +546,36 @@ static int64_t count_words(const int32_t *doy_map, int64_t T)
     return K;
 }
 
+// A threshold table without a day-of-year axis (n_doy = 1: the no-season and fixed-value variants, every day reads row 0) would
+// cut the series into one-day words, because word_length needs consecutive days of year, and a run of a few decades would then
+// have more words than k_scan and k_intensity keep in shared memory.  The pass sees such a table as kTileDoy identical rows
+// instead (replicated into the workspace, replicate_rows) with day t on row t mod kTileDoy, so its words are 32 days long.
+static int pass_n_doy(int n_doy) { return n_doy == 1 ? kTileDoy : n_doy; }
+
+// The day-of-year map the pass cuts into words: h_doy_map itself, or for n_doy = 1 (where every entry must be 0) t mod kTileDoy.
+static int pass_doy_map(const int32_t *h_doy_map, int64_t T, int n_doy, std::vector<int32_t> &own, const int32_t *&map)
+{
+    map = h_doy_map;
+    if (n_doy != 1) return HDP_B200_OK;
+    own.resize((size_t)T);
+    for (int64_t t = 0; t < T; t++) {
+        if (h_doy_map[t] != 0) return HDP_B200_ERR_INVALID;
+        own[(size_t)t] = (int32_t)(t % kTileDoy);
+    }
+    map = own.data();
+    return HDP_B200_OK;
+}
+
+// thr [C, 1, P] -> rep [C, kTileDoy, P]: row 0 of every cell, then copies that double the rows already there.
+static int replicate_rows(const double *thr, int64_t C, int P, double *rep, cudaStream_t st)
+{
+    const size_t row = (size_t)P * sizeof(double), pitch = kTileDoy * row;
+    HDP_CUDA_TRY(cudaMemcpy2DAsync(rep, pitch, thr, row, row, (size_t)C, cudaMemcpyDeviceToDevice, st));
+    for (int n = 1; n < kTileDoy; n *= 2)
+        HDP_CUDA_TRY(cudaMemcpy2DAsync(rep + (size_t)n * P, pitch, rep, pitch, n * row, (size_t)C, cudaMemcpyDeviceToDevice, st));
+    return HDP_B200_OK;
+}
+
 static int pick_pg(int P)
 {
     const int cand[] = {4, 8, 10, 16, 20};
@@ -564,12 +594,13 @@ static Layout carve(void *ws, size_t ws_bytes, int64_t C, int64_t T, bool need_n
     Carver cv(ws, ws_bytes);
     if (need_norm) L.xn = cv.take<float>((size_t)C * T);
     L.words = cv.take<int4>((size_t)K + 1);
-    L.blk_start = cv.take<int>((size_t)(n_doy + kTileDoy - 1) / kTileDoy + 1);
+    L.blk_start = cv.take<int>((size_t)(pass_n_doy(n_doy) + kTileDoy - 1) / kTileDoy + 1);
     L.blk_words = cv.take<int>((size_t)K + 1);
     L.seasons = cv.take<int4>((size_t)2 * (Y + 1));
     L.lut = cv.take<uint32_t>((size_t)2 * 8192);
     L.hot = cv.take<uint32_t>((size_t)P * K * C);
     if (intensity) L.int_seasons = cv.take<int4>((size_t)2 * (Y + 1));
+    if (n_doy == 1) L.thr_rep = cv.take<double>((size_t)C * kTileDoy * P);
     L.total = cv.off;
     return L;
 }
@@ -582,25 +613,36 @@ static bool bad_dims(int64_t C, int64_t T, int n_doy, int P)
 size_t metric_pass_workspace_bytes(int64_t C, int64_t T, int64_t ld_c, int n_doy, int P, int Y, const int32_t *h_doy_map, bool intensity)
 {
     if (bad_dims(C, T, n_doy, P) || Y < 0) return 0;
-    const int64_t K = h_doy_map ? count_words(h_doy_map, T) : words_upper_bound(T, n_doy);
+    const int64_t K = n_doy == 1 ? (T + kTileDoy - 1) / kTileDoy : h_doy_map ? count_words(h_doy_map, T) : words_upper_bound(T, n_doy);
     return carve(nullptr, 0, C, T, ld_c != 1, K, n_doy, P, Y, intensity).total;
 }
 
 // Runs k_hot_words (after the layout-normalising copy when ld_c != 1: the samples then live in L.xn, time-major, ld_t = C);
-// on success plan / L describe what lives in the workspace.
+// on success plan / L describe what lives in the workspace, and L.thr / L.n_doy the thresholds the kernels read.
 static int run_hot_words(const float *d_measure, int64_t C, int64_t T, int64_t ld_t, int64_t ld_c,
                          const double *d_thr, int n_doy, int P, const int32_t *h_doy_map,
                          int Y, void *ws, size_t ws_bytes, cudaStream_t st, WordPlan &plan, Layout &L,
                          int64_t carve_cells = 0, bool tables_resident = false, int input_unit = 0, bool intensity = false)
 {
     if (input_unit < 0 || input_unit > 2) return HDP_B200_ERR_INVALID;
-    int rc = build_words(h_doy_map, T, n_doy, plan);
+    std::vector<int32_t> own_map;
+    const int32_t *doy_map = nullptr;
+    int rc = pass_doy_map(h_doy_map, T, n_doy, own_map, doy_map);
+    if (rc != HDP_B200_OK) return rc;
+    rc = build_words(doy_map, T, pass_n_doy(n_doy), plan);
     if (rc != HDP_B200_OK) return rc;
     const int K = (int)plan.words.size();
     const bool need_norm = ld_c != 1;
     L = carve(ws, ws_bytes, std::max(C, carve_cells), T, need_norm, K, n_doy, P, Y, intensity);
     if (ws == nullptr || L.total > ws_bytes) return HDP_B200_ERR_WORKSPACE;
+    L.thr = d_thr;
+    L.n_doy = pass_n_doy(n_doy);
     if (C == 0 || T == 0) return HDP_B200_OK;
+    if (L.thr_rep) {
+        rc = replicate_rows(d_thr, C, P, L.thr_rep, st);
+        if (rc != HDP_B200_OK) return rc;
+        L.thr = L.thr_rep;
+    }
     const float *x = d_measure;
     if (need_norm) {
         rc = normalize_layout(d_measure, C, T, ld_t, ld_c, L.xn, st);
@@ -620,7 +662,7 @@ static int run_hot_words(const float *d_measure, int64_t C, int64_t T, int64_t l
 #define HDP_LAUNCH_HOT_U(PG, U)                                                                                    \
     do {                                                                                                           \
         HDP_CUDA_TRY(cudaFuncSetAttribute(k_hot_words<PG, U>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)); \
-        k_hot_words<PG, U><<<grid, 256, smem, st>>>(x, C, ld_t, d_thr, n_doy, P, L.words, L.blk_start, L.blk_words, K, L.hot); \
+        k_hot_words<PG, U><<<grid, 256, smem, st>>>(x, C, ld_t, L.thr, L.n_doy, P, L.words, L.blk_start, L.blk_words, K, L.hot); \
     } while (0)
 #define HDP_LAUNCH_HOT(PG)                                                                                         \
     do {                                                                                                           \
@@ -660,15 +702,22 @@ static int scan_passes(const int32_t *tab, int Y, ScanPasses &passes)
     return HDP_B200_OK;
 }
 
-// k_scan over the hot words in L (one launch per pass): the integer metrics u16 [4, P, D, Y, C].
-static int run_scan(const Layout &L, const WordPlan &plan, int64_t C, int64_t T, int P, const int32_t *h_defs, int D,
-                    const ScanPasses (&passes)[2], int Y, const uint8_t *d_is_south, uint16_t *d_out, cudaStream_t st, bool tables_resident)
-{
-    const size_t n_pass = std::max(passes[0].size(), passes[1].size());
-    const int K = (int)plan.words.size();
-
-    // bit-sliced definition tables (see k_scan)
+// What k_scan runs for a definition set and its season passes: the bit-sliced definition tables and the instantiation.
+// run_scan launches it and hdp_b200_metrics_kernel_choice reports it.
+struct ScanConfig {
     ScanTables tabs;
+    std::vector<uint32_t> lut;       // [ge_len] definitions with min_dur <= len, then [brk_len] definitions with max_break < gap
+    bool bytes = true;               // 8-bit accumulator lanes (four definitions per register), else 16-bit (two)
+    int ng = 0, ks = 0;              // accumulator registers (template NG), bit planes of the max_subs counters (template KS)
+    int lmin = 0, bmax = 0;          // compile-time run-filter constants of the instantiation; 0, 0 = run-time values
+    size_t n_pass = 0;               // launches: the larger pass count of the two hemispheres
+};
+
+static int scan_config(const int32_t *h_defs, int D, int64_t T, const ScanPasses (&passes)[2], ScanConfig &cfg)
+{
+    cfg.n_pass = std::max(passes[0].size(), passes[1].size());
+    // bit-sliced definition tables (see k_scan)
+    ScanTables &tabs = cfg.tabs;
     int max_min_dur = 0, max_break_all = 0;
     int64_t max_subs_all = 0;
     std::vector<int64_t> subs(D);
@@ -687,33 +736,50 @@ static int run_scan(const Layout &L, const WordPlan &plan, int64_t C, int64_t T,
         tabs.max_subs_plane[k] = 0u;
         for (int i = 0; i < D; i++) tabs.max_subs_plane[k] |= (uint32_t)((subs[i] >> k) & 1) << i;
     }
-    std::vector<uint32_t> lut(tabs.ge_len + tabs.brk_len, 0u);
+    cfg.lut.assign(tabs.ge_len + tabs.brk_len, 0u);
     for (int l = 0; l < tabs.ge_len; l++)
-        for (int i = 0; i < D; i++) if (h_defs[3 * i] <= l) lut[l] |= 1u << i;
+        for (int i = 0; i < D; i++) if (h_defs[3 * i] <= l) cfg.lut[l] |= 1u << i;
     for (int g = 0; g < tabs.brk_len; g++)
-        for (int i = 0; i < D; i++) if (h_defs[3 * i + 1] < g) lut[tabs.ge_len + g] |= 1u << i;
-    if (!tables_resident) HDP_CUDA_TRY(cudaMemcpyAsync(L.lut, lut.data(), sizeof(uint32_t) * lut.size(), cudaMemcpyHostToDevice, st));
-    const uint32_t *ge_tab = L.lut, *brk_tab = L.lut + tabs.ge_len;
+        for (int i = 0; i < D; i++) if (h_defs[3 * i + 1] < g) cfg.lut[tabs.ge_len + g] |= 1u << i;
     // run filter (see k_scan): only when the look-back / look-ahead fits the 32-day neighbourhood
     int min_min_dur = INT_MAX;
     for (int i = 0; i < D; i++) min_min_dur = std::min(min_min_dur, h_defs[3 * i]);
     tabs.f_lmin = min_min_dur;
     tabs.f_bmax = max_break_all;
     tabs.f_on = (min_min_dur >= 2 && min_min_dur <= 32 && max_break_all >= 0 && max_break_all <= 30 && g_scan_filter) ? 1 : 0;
-    const size_t scan_smem = (((size_t)kScanWarps * kScanQueueWords + lut.size() + 3) & ~(size_t)3) * sizeof(uint32_t) + ((size_t)K + 1) * sizeof(int4);
-    if (scan_smem > 200 * 1024) return HDP_B200_ERR_UNSUPPORTED;             // > ~9 000 hot words (~800 years of daily data)
-    const int64_t n_warps = ((C + 31) / 32) * P;                             // one warp per (32 cells, percentile)
-    const unsigned scan_grid = (unsigned)((n_warps + kScanWarps - 1) / kScanWarps);
     // accumulators: four definitions per register when every season fits 8-bit lanes, else two
     int max_season = 0;
     for (int h = 0; h < 2; h++)
         for (const auto &pass : passes[h])
             for (const ScanSeason &se : pass) max_season = std::max(max_season, se.b - se.a);
-    const bool bytes = max_season <= 255;
-    const int per = bytes ? 4 : 2;
-    int ng = (D + per - 1) / per;
-    ng = ng <= 2 ? 2 : ng <= 3 ? 3 : ng <= 4 ? 4 : ng <= 6 ? 6 : ng <= 8 ? 8 : ng <= 12 ? 12 : 16;
-    const int ks = ks_needed <= 1 ? 1 : ks_needed <= 2 ? 2 : 32;      // bit planes of the max_subs counters: 1, 2 or all 32
+    cfg.bytes = max_season <= 255;
+    const int per = cfg.bytes ? 4 : 2;
+    const int ng = (D + per - 1) / per;
+    cfg.ng = ng <= 2 ? 2 : ng <= 3 ? 3 : ng <= 4 ? 4 : ng <= 6 ? 6 : ng <= 8 ? 8 : ng <= 12 ? 12 : 16;
+    cfg.ks = ks_needed <= 1 ? 1 : ks_needed <= 2 ? 2 : 32;          // bit planes of the max_subs counters: 1, 2 or all 32
+    // compile-time filter constants for the usual shapes (seasons of at most 255 days, common definition sets)
+    if (cfg.bytes && cfg.ks == 1 && tabs.f_on && tabs.f_lmin == 3 && (tabs.f_bmax == 1 || tabs.f_bmax == 2)) {
+        cfg.lmin = 3;
+        cfg.bmax = tabs.f_bmax;
+    }
+    return HDP_B200_OK;
+}
+
+// k_scan over the hot words in L (one launch per pass): the integer metrics u16 [4, P, D, Y, C].
+static int run_scan(const Layout &L, const WordPlan &plan, int64_t C, int64_t T, int P, const int32_t *h_defs, int D,
+                    const ScanPasses (&passes)[2], int Y, const uint8_t *d_is_south, uint16_t *d_out, cudaStream_t st, bool tables_resident)
+{
+    const int K = (int)plan.words.size();
+    ScanConfig cfg;
+    const int rc = scan_config(h_defs, D, T, passes, cfg);
+    if (rc != HDP_B200_OK) return rc;
+    const ScanTables &tabs = cfg.tabs;
+    if (!tables_resident) HDP_CUDA_TRY(cudaMemcpyAsync(L.lut, cfg.lut.data(), sizeof(uint32_t) * cfg.lut.size(), cudaMemcpyHostToDevice, st));
+    const uint32_t *ge_tab = L.lut, *brk_tab = L.lut + tabs.ge_len;
+    const size_t scan_smem = (((size_t)kScanWarps * kScanQueueWords + cfg.lut.size() + 3) & ~(size_t)3) * sizeof(uint32_t) + ((size_t)K + 1) * sizeof(int4);
+    if (scan_smem > 200 * 1024) return HDP_B200_ERR_UNSUPPORTED;             // > ~9 000 hot words (~800 years of daily data)
+    const int64_t n_warps = ((C + 31) / 32) * P;                             // one warp per (32 cells, percentile)
+    const unsigned scan_grid = (unsigned)((n_warps + kScanWarps - 1) / kScanWarps);
 
     // all passes of both hemispheres live side by side in the workspace: north passes, then south passes
     std::vector<int4> tab;
@@ -724,7 +790,7 @@ static int run_scan(const Layout &L, const WordPlan &plan, int64_t C, int64_t T,
             for (const ScanSeason &s : pass) tab.push_back(make_int4(s.a, s.b, s.row, 0));
         }
     if (!tables_resident) HDP_CUDA_TRY(cudaMemcpyAsync(L.seasons, tab.data(), sizeof(int4) * tab.size(), cudaMemcpyHostToDevice, st));
-    for (size_t ip = 0; ip < n_pass; ip++) {
+    for (size_t ip = 0; ip < cfg.n_pass; ip++) {
         const int4 *sn = ip < passes[0].size() ? L.seasons + off[0][ip] : L.seasons;
         const int4 *ss = ip < passes[1].size() ? L.seasons + off[1][ip] : L.seasons;
         const int nn = ip < passes[0].size() ? (int)passes[0][ip].size() : 0;
@@ -743,18 +809,17 @@ static int run_scan(const Layout &L, const WordPlan &plan, int64_t C, int64_t T,
                                                                                      brk_tab, sn, nn, ss, ns, Y, d_is_south, d_out); \
         } while (0)
 #define HDP_SCAN_KS(NG, BY)                                                \
-        switch (ks) {                                                      \
+        switch (cfg.ks) {                                                  \
         case 1:                                                            \
-            /* compile-time filter constants for the usual shapes (seasons of at most 255 days, common definition sets) */ \
-            if (BY && tabs.f_on && tabs.f_lmin == 3 && tabs.f_bmax == 1) HDP_LAUNCH_SCAN_F(NG, true, 3, 1);       \
-            else if (BY && tabs.f_on && tabs.f_lmin == 3 && tabs.f_bmax == 2) HDP_LAUNCH_SCAN_F(NG, true, 3, 2);  \
+            if (BY && cfg.lmin == 3 && cfg.bmax == 1) HDP_LAUNCH_SCAN_F(NG, true, 3, 1);                          \
+            else if (BY && cfg.lmin == 3 && cfg.bmax == 2) HDP_LAUNCH_SCAN_F(NG, true, 3, 2);                     \
             else HDP_LAUNCH_SCAN(NG, 1, BY);                               \
             break;                                                         \
         case 2: HDP_LAUNCH_SCAN(NG, 2, BY); break;                         \
         default: HDP_LAUNCH_SCAN(NG, 32, BY); break;                       \
         }
-        if (bytes) {
-            switch (ng) {                                                  // D <= 32: at most 8 registers of 4
+        if (cfg.bytes) {
+            switch (cfg.ng) {                                                  // D <= 32: at most 8 registers of 4
             case 2: HDP_SCAN_KS(2, true); break;
             case 3: HDP_SCAN_KS(3, true); break;
             case 4: HDP_SCAN_KS(4, true); break;
@@ -762,7 +827,7 @@ static int run_scan(const Layout &L, const WordPlan &plan, int64_t C, int64_t T,
             default: HDP_SCAN_KS(8, true); break;
             }
         } else {
-            switch (ng) {
+            switch (cfg.ng) {
             case 2: HDP_SCAN_KS(2, false); break;
             case 3: HDP_SCAN_KS(3, false); break;
             case 4: HDP_SCAN_KS(4, false); break;
@@ -816,7 +881,7 @@ int metric_pass(const float *d_measure, int64_t C, int64_t T, int64_t ld_t, int6
         if (rc != HDP_B200_OK) return rc;
     }
     if (d_int)
-        rc = run_intensity(L, plan, d_measure, C, T, ld_t, ld_c, d_thr, n_doy, P, h_defs, D, seasons, Y, d_is_south, d_int, st,
+        rc = run_intensity(L, plan, d_measure, C, T, ld_t, ld_c, L.thr, L.n_doy, P, h_defs, D, seasons, Y, d_is_south, d_int, st,
                            tables_resident, input_unit);
     return rc;
 }
@@ -835,6 +900,27 @@ size_t hdp_b200_metrics_workspace_bytes(int64_t C, int64_t T, int64_t ld_t, int6
 }
 
 void hdp_b200_metrics_run_filter(int on) { g_scan_filter = on != 0; }
+
+int hdp_b200_metrics_kernel_choice(const int32_t *h_defs, int D, const int32_t *h_season_north, const int32_t *h_season_south, int Y,
+                                   int64_t T, int *info)
+{
+    if (!h_defs || !info || D <= 0 || Y < 0 || T < 0 || T > 0x3fffffff || (Y > 0 && (!h_season_north || !h_season_south)))
+        return HDP_B200_ERR_INVALID;
+    if (D > HDP_B200_MAX_DEFINITIONS) return HDP_B200_ERR_UNSUPPORTED;
+    std::vector<int32_t> tab((size_t)4 * (Y + 1));
+    ScanPasses passes[2];
+    for (int h = 0; h < 2; h++) {
+        season_table(h == 0 ? h_season_north : h_season_south, Y, T, tab.data());
+        const int rc = scan_passes(tab.data(), Y, passes[h]);
+        if (rc != HDP_B200_OK) return rc;
+    }
+    ScanConfig cfg;
+    const int rc = scan_config(h_defs, D, T, passes, cfg);
+    if (rc != HDP_B200_OK) return rc;
+    info[0] = cfg.bytes ? 8 : 16; info[1] = cfg.ng; info[2] = cfg.ks; info[3] = cfg.tabs.f_on;
+    info[4] = cfg.lmin; info[5] = cfg.bmax; info[6] = (int)cfg.n_pass;
+    return HDP_B200_OK;
+}
 
 int hdp_b200_hot_days(const float *d_measure, int64_t C, int64_t T, int64_t ld_t, int64_t ld_c,
                       const double *d_thr, int n_doy, int P, const int32_t *h_doy_map,

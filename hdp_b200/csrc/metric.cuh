@@ -24,6 +24,9 @@ struct Layout {
     uint32_t *lut = nullptr;
     uint32_t *hot = nullptr;
     int4 *int_seasons = nullptr;    // intensity pass only: its season tables (north, then south)
+    double *thr_rep = nullptr;      // n_doy = 1 only: the thresholds replicated to kTileDoy rows (metric.cu, pass_n_doy)
+    const double *thr = nullptr;    // the thresholds the kernels read, [C, n_doy, P]: the caller's, or thr_rep
+    int n_doy = 0;
 };
 
 // Workspace of metric_pass; `intensity` appends the intensity pass's season tables behind what the metric pass uses.

@@ -44,7 +44,7 @@
 extern "C" {
 #endif
 
-#define HDP_B200_ABI_VERSION 5
+#define HDP_B200_ABI_VERSION 6
 
 #define HDP_B200_OK                 0
 #define HDP_B200_ERR_INVALID       (-1)  /* null pointer, negative size, quantile outside [0,1] or NaN, bad table entry */
@@ -147,6 +147,14 @@ int hdp_b200_metrics(const float *d_measure, int64_t C, int64_t T, int64_t ld_t,
 /* Test hook: 0 makes k_scan feed every hot run to the definitions' state machines instead of first dropping the runs
  * that cannot change any result (short runs after long breaks, see metric.cu); the outputs must be identical. */
 void hdp_b200_metrics_run_filter(int on);
+
+/* Which k_scan instantiation hdp_b200_metrics would launch for these definitions and season tables over T days (host logic
+ * only: no device needed; the run filter setting above is taken into account).  info[0..6] = {accumulator lane bits: 8 (four
+ * definitions per register) or 16 (two), accumulator registers NG, bit planes of the max_subs counters KS, run filter on,
+ * compile-time filter constants LMIN and BMAX (0, 0 = the generic instantiation), launches (season passes)}.  Returns what
+ * hdp_b200_metrics would return for the definitions and tables (e.g. HDP_B200_ERR_UNSUPPORTED for a season over 65 535 days). */
+int hdp_b200_metrics_kernel_choice(const int32_t *h_defs, int D, const int32_t *h_season_north, const int32_t *h_season_south, int Y,
+                                   int64_t T, int *info);
 
 /* Host-buffer variant.  Thresholds come from h_thr (host, uploaded chunk by chunk) unless d_thr (DEVICE f64
  * [C, n_doy, P], e.g. the d_keep of hdp_b200_thresholds_host) is given, in which case h_thr may be NULL. */

@@ -177,7 +177,7 @@ def test_intensity_is_positive_exactly_where_there_are_heatwave_days():
 def test_abi_entry_points():
     from hdp_b200 import _lib
     L = _lib.lib()
-    assert L.hdp_b200_abi_version() == 5
+    assert L.hdp_b200_abi_version() == 6
     raw = ctypes.CDLL(L._name)
     for name in ("hdp_b200_intensity", "hdp_b200_intensity_host", "hdp_b200_intensity_workspace_bytes"):
         assert hasattr(raw, name)
