@@ -9,6 +9,8 @@ These are the two seams of the reference that the CUDA library replaces:
 * :func:`hot_days_array`    <- ``indicate_hot_days`` (reference hdp/metric.py:280-301)
 * :func:`intensity_array`   heatwave intensity (HWC, HWI, HWP: cumulative, mean and peak exceedance of the threshold over the
   heatwave days of a season), which the reference does not have; optionally with the four metrics from the same pass
+* ``cold=True`` on the metric and intensity calls: cold spells (CSF ... CSA, CSC ... CSP), the same sweep over the days below the
+  threshold, which the reference does not have either
 * :func:`index_heatwaves_array`, :func:`season_metrics_array` <- ``index_heatwaves`` and ``heatwave_frequency`` / ``number`` /
   ``duration`` / ``average`` (reference hdp/metric.py:11-172), the building blocks the hot path never materialises
 
@@ -28,6 +30,9 @@ from ._tables import WindowTables
 
 METRIC_NAMES = ("HWF", "HWN", "HWD", "HWA")      # plane order of the metric output (reference metric.py:336-340)
 INTENSITY_NAMES = ("HWC", "HWI", "HWP")          # plane order of the intensity output
+COLD_METRIC_NAMES = ("CSF", "CSN", "CSD", "CSA")  # the same planes of a cold-spell pass (cold=True)
+COLD_INTENSITY_NAMES = ("CSC", "CSI", "CSP")
+COLD = 0x100                                      # HDP_B200_COLD, OR-ed into the unit code of the metric entry points
 
 _workspaces = {}
 
@@ -153,12 +158,12 @@ def _device_out(out, dtype, shape, device, message):
     return out
 
 
-def _metric_pass(measure, thresholds, doy_map, defs, season_north, season_south, is_south, units, met, heat, intensity):
+def _metric_pass(measure, thresholds, doy_map, defs, season_north, season_south, is_south, units, met, heat, intensity, cold):
     """hdp_b200_metrics, or with ``intensity`` hdp_b200_intensity, on CUDA tensors.  ``met`` / ``heat``: the uint16 metrics /
     float32 intensity output or None; the metrics are allocated unless the intensity pass runs without them.  Returns the
-    intensity output of the intensity pass, else the metrics."""
+    intensity output of the intensity pass, else the metrics.  ``cold``: the cold-spell pass."""
     torch = _torch()
-    unit = _unit_code(units)
+    unit = _unit_code(units) | (COLD if cold else 0)
     _check_measure(measure, "measure")
     T, C = measure.shape
     _check_thr(thresholds, C)
@@ -188,21 +193,25 @@ def _metric_pass(measure, thresholds, doy_map, defs, season_north, season_south,
     return heat if intensity else met
 
 
-def metrics_array(measure, thresholds, doy_map, defs, season_north, season_south, is_south=None, out=None, units=None):
+def metrics_array(measure, thresholds, doy_map, defs, season_north, season_south, is_south=None, out=None, units=None, *,
+                  cold=False):
     """``measure`` f32 ``[T, C]``, ``thresholds`` f64 ``[C, n_doy, P]`` -> uint16 ``[4, P, D, Y, C]``
     (planes HWF, HWN, HWD, HWA; the reference's int64 ``[P, D, C, 4, Y]`` is ``out.permute(1, 2, 4, 0, 3)`` widened).
-    ``units`` of the measure's samples as for :func:`thresholds_array`."""
-    return _metric_pass(measure, thresholds, doy_map, defs, season_north, season_south, is_south, units, out, None, False)
+    ``units`` of the measure's samples as for :func:`thresholds_array`.  ``cold=True``: cold spells - the same rules over the
+    days with ``measure < threshold``, planes CSF, CSN, CSD, CSA (the season tables are used as given; the cold season of a
+    hemisphere is usually the other one's warm season)."""
+    return _metric_pass(measure, thresholds, doy_map, defs, season_north, season_south, is_south, units, out, None, False, cold)
 
 
 def intensity_array(measure, thresholds, doy_map, defs, season_north, season_south, is_south=None, out=None, metrics_out=None,
-                    units=None):
+                    units=None, *, cold=False):
     """Heatwave intensity: ``measure`` f32 ``[T, C]``, ``thresholds`` f64 ``[C, n_doy, P]`` -> float32 ``[3, P, D, Y, C]``, planes
     HWC (cumulative), HWI (mean) and HWP (peak) exceedance ``measure - threshold`` over the heatwave days of every season (the
     days HWF counts; 0 where there are none).  ``metrics_out``: an optional uint16 CUDA tensor ``[4, P, D, Y, C]`` that also
     receives exactly what :func:`metrics_array` returns, from the same pass.  The non-empty seasons of each hemisphere's table must
-    be disjoint (every table compute_hemisphere_ranges builds is)."""
-    return _metric_pass(measure, thresholds, doy_map, defs, season_north, season_south, is_south, units, metrics_out, out, True)
+    be disjoint (every table compute_hemisphere_ranges builds is).  ``cold=True``: CSC, CSI, CSP - the deficit
+    ``threshold - measure`` over the cold-spell days (and CSF ... CSA in ``metrics_out``), see :func:`metrics_array`."""
+    return _metric_pass(measure, thresholds, doy_map, defs, season_north, season_south, is_south, units, metrics_out, out, True, cold)
 
 
 def hot_days_array(measure, thresholds, doy_map):
@@ -453,7 +462,7 @@ def _host_out(out, dtype, shape, message):
     return out
 
 
-def _metric_pass_host(measure, thresholds, doy_map, defs, season_north, season_south, is_south, units, met, heat, intensity):
+def _metric_pass_host(measure, thresholds, doy_map, defs, season_north, season_south, is_south, units, met, heat, intensity, cold):
     """:func:`_metric_pass` with host arrays: hdp_b200_metrics_host, or with ``intensity`` hdp_b200_intensity_host."""
     torch = _torch()
     measure, ld_t, ld_c = _host_measure(measure, "measure")
@@ -483,24 +492,28 @@ def _metric_pass_host(measure, thresholds, doy_map, defs, season_north, season_s
     name = "hdp_b200_intensity_host" if intensity else "hdp_b200_metrics_host"
     rc = getattr(_lib.lib(), name)(_hp(measure), C, T, ld_t, ld_c, _hp(thr) if thr is not None else None,
                                    d_thr.data_ptr() if d_thr is not None else None, n_doy, P, _hp(dm), _hp(df), D, _hp(sn), _hp(ss), Y,
-                                   _hp(south) if south is not None else None, *outs, _unit_code(units))
+                                   _hp(south) if south is not None else None, *outs, _unit_code(units) | (COLD if cold else 0))
     _lib.check(rc, name)
     return heat if intensity else met
 
 
 def metrics_host(measure: np.ndarray, thresholds, doy_map, defs, season_north, season_south,
-                 is_south=None, out: Optional[np.ndarray] = None, units=None) -> np.ndarray:
+                 is_south=None, out: Optional[np.ndarray] = None, units=None, *, cold=False) -> np.ndarray:
     """``thresholds``: float64 ``[C, n_doy, P]`` as a host array, or as a CUDA tensor (device-resident: no upload).  A host
-    array that :func:`thresholds_host` returned with ``keep=True`` is recognised and its device copy used."""
-    return _metric_pass_host(measure, thresholds, doy_map, defs, season_north, season_south, is_south, units, out, None, False)
+    array that :func:`thresholds_host` returned with ``keep=True`` is recognised and its device copy used.  ``cold`` as for
+    :func:`metrics_array`."""
+    return _metric_pass_host(measure, thresholds, doy_map, defs, season_north, season_south, is_south, units, out, None, False, cold)
 
 
 def intensity_host(measure: np.ndarray, thresholds, doy_map, defs, season_north, season_south, is_south=None,
-                   out: Optional[np.ndarray] = None, metrics_out: Optional[np.ndarray] = None, units=None) -> np.ndarray:
+                   out: Optional[np.ndarray] = None, metrics_out: Optional[np.ndarray] = None, units=None, *,
+                   cold=False) -> np.ndarray:
     """Host-array counterpart of :func:`intensity_array`: float32 ``[3, P, D, Y, C]`` (HWC, HWI, HWP); ``metrics_out`` an
     optional uint16 host array ``[4, P, D, Y, C]`` that also receives what :func:`metrics_host` returns (the samples cross PCIe
-    once for both).  Thresholds as for :func:`metrics_host` (host array, CUDA tensor, or a resident copy)."""
-    return _metric_pass_host(measure, thresholds, doy_map, defs, season_north, season_south, is_south, units, metrics_out, out, True)
+    once for both).  Thresholds as for :func:`metrics_host` (host array, CUDA tensor, or a resident copy); ``cold`` as for
+    :func:`intensity_array`."""
+    return _metric_pass_host(measure, thresholds, doy_map, defs, season_north, season_south, is_south, units, metrics_out, out, True,
+                             cold)
 
 
 def host_release() -> None:

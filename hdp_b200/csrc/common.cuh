@@ -101,7 +101,8 @@ int thresholds_launch(const float *d_temps, int64_t C, int64_t T_b, int64_t ld_t
                       void *d_workspace, size_t workspace_bytes, void *stream, int64_t carve_cells, bool tables_resident, int input_unit);
 
 // The whole of hdp_b200_metrics and hdp_b200_intensity (metric.cu): k_hot_words, then k_scan on its hot words when d_out is given
-// (u16 [4, P, D, Y, C]) and k_intensity when d_int is given (f32 [3, P, D, Y, C]).  carve_cells / tables_resident as above.
+// (u16 [4, P, D, Y, C]) and k_intensity when d_int is given (f32 [3, P, D, Y, C]).  carve_cells / tables_resident as above;
+// input_unit = unit code, OR-ed with HDP_B200_COLD for the cold-spell pass.
 int metric_pass(const float *d_measure, int64_t C, int64_t T, int64_t ld_t, int64_t ld_c,
                 const double *d_thr, int n_doy, int P, const int32_t *h_doy_map,
                 const int32_t *h_defs, int D,

@@ -13,6 +13,7 @@
 //                partial sum and maximum, which go to the season accumulators of the definitions that label it.  State machines
 //                and accumulators live in shared memory, [definition][lane] per warp; a season is flushed as float32 when it
 //                closes.  One open season per lane: the season tables of a hemisphere must be disjoint (intensity.h).
+//                k_intensity<true> (cold spells): the words hold cold-day bits and a day adds its deficit below the threshold.
 #include <algorithm>
 #include <vector>
 
@@ -32,6 +33,9 @@ constexpr int kIntBatch = 4;                 // days of a block whose sample and
 // bytes of shared memory one warp keeps: state machine + accumulator per (definition, lane)
 static size_t int_warp_bytes(int D) { return (size_t)D * 32 * (sizeof(IndexState) + sizeof(IntensityAcc)); }
 
+// COLD: the words hold cold-day bits and a day adds its deficit (a template parameter: as a run-time argument it cost the
+// heatwave instance 4 %)
+template <bool COLD>
 __global__ void __launch_bounds__(kIntWarpsMax * 32)
 k_intensity(const uint32_t *__restrict__ hot, const float *__restrict__ x, int64_t ld_t, const double *__restrict__ thr, int n_doy,
             int64_t C, int K, int T, const int4 *__restrict__ words, int P, int D, const __grid_constant__ IntensityDefs defs,
@@ -96,7 +100,7 @@ k_intensity(const uint32_t *__restrict__ hot, const float *__restrict__ x, int64
             }
 #pragma unroll
             for (int j = 0; j < kIntBatch; j++)
-                if (t0 + j < hi) intensity_day(r, m, intensity_excess(to_celsius_f(v[j], unit), th[j]));
+                if (t0 + j < hi) intensity_day(r, m, intensity_e(to_celsius_f(v[j], unit), th[j], COLD));
         }
     };
 
@@ -115,7 +119,7 @@ k_intensity(const uint32_t *__restrict__ hot, const float *__restrict__ x, int64
 
 int run_intensity(const Layout &L, const WordPlan &plan, const float *d_measure, int64_t C, int64_t T, int64_t ld_t, int64_t ld_c,
                   const double *d_thr, int n_doy, int P, const int32_t *h_defs, int D, const std::vector<int32_t> &seasons, int Y,
-                  const uint8_t *d_is_south, float *d_int, cudaStream_t st, bool tables_resident, int input_unit)
+                  const uint8_t *d_is_south, float *d_int, cudaStream_t st, bool tables_resident, int unit, bool cold)
 {
     const int K = (int)plan.words.size();
     const size_t words_bytes = ((size_t)K * sizeof(int2) + 15) & ~(size_t)15;
@@ -132,9 +136,10 @@ int run_intensity(const Layout &L, const WordPlan &plan, const float *d_measure,
     const int64_t n_warps = ((C + 31) / 32) * P;
     const unsigned grid = (unsigned)((n_warps + wpc - 1) / wpc);
     KernelTimer timer(kIntensity, st);
-    HDP_CUDA_TRY(cudaFuncSetAttribute(k_intensity, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    k_intensity<<<grid, wpc * 32, smem, st>>>(L.hot, x, x_ld_t, d_thr, n_doy, C, K, (int)T, L.words, P, D, defs,
-                                              L.int_seasons, Y, L.int_seasons + (Y + 1), Y, Y, d_is_south, input_unit, wpc, d_int);
+    const auto kernel = cold ? k_intensity<true> : k_intensity<false>;
+    HDP_CUDA_TRY(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    kernel<<<grid, wpc * 32, smem, st>>>(L.hot, x, x_ld_t, d_thr, n_doy, C, K, (int)T, L.words, P, D, defs,
+                                         L.int_seasons, Y, L.int_seasons + (Y + 1), Y, Y, d_is_south, unit, wpc, d_int);
     HDP_LAUNCH_CHECK();
     return HDP_B200_OK;
 }

@@ -10,6 +10,10 @@
 //   HWP  = max e_t over the set (0 when the set is empty)
 // each rounded once to float32.  A block is one labelled hot run clipped to the season: distinct runs are separated by at least
 // one cold day.
+//
+// Cold spells (CSC, CSI, CSP; HDP_B200_COLD): the same accounting over the runs of cold days ((double)x < thr) with the deficit
+// e_t = thr - (double)x in place of the exceedance (e_t > 0 on every day of the set again).  thr - x is bit for bit the
+// exceedance (-x) - (-thr): negation is exact and a - b is a + (-b), so the cold result equals the warm one on negated inputs.
 #pragma once
 
 #include <stdint.h>
@@ -25,6 +29,10 @@ struct IntensityAcc {
 };
 
 HDP_HD double intensity_excess(float x, double thr) { return (double)x - thr; }
+HDP_HD double intensity_deficit(float x, double thr) { return thr - (double)x; }
+
+// e_t of one day: the exceedance of a heatwave pass, the deficit of a cold-spell pass
+HDP_HD double intensity_e(float x, double thr, bool cold) { return cold ? intensity_deficit(x, thr) : intensity_excess(x, thr); }
 
 // one day of a block: r = r + e (time order), m = max(m, e)
 HDP_HD void intensity_day(double &r, double &m, double e)

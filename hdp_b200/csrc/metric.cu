@@ -13,7 +13,9 @@
 //                keeps that [32 doy][P][32 cell] threshold tile in shared memory (rounded DOWN to f32, which
 //                preserves the reference's double-precision `measure > threshold` exactly) and walks every
 //                year of the measure through it, so each threshold is fetched from HBM once and each
-//                measure sample once.  Output: one 32-bit word of hot-day bits per (percentile, word, cell).
+//                measure sample once.  Output: one 32-bit word of hot-day bits per (percentile, word, cell).  A cold-spell
+//                pass (HDP_B200_COLD) instantiates it with COLD: the tile is rounded UP and the bits mark `measure <
+//                threshold`; everything downstream works on the bits and does not know which direction made them.
 //   k_scan       one thread per (cell, percentile), lanes = cells (coalesced).  Walks the hot words in
 //                time order, pops hot runs with bit tricks and feeds each run to all definitions' state
 //                machines held in registers; season accumulators are flushed as u16 when a season closes.
@@ -44,7 +46,13 @@ __device__ __forceinline__ void or_if_gt(uint32_t &m, float v, float t, uint32_t
     asm("{\n\t.reg .pred p;\n\tsetp.gt.f32 p, %1, %2;\n\t@p or.b32 %0, %0, %3;\n\t}" : "+r"(m) : "f"(v), "f"(t), "r"(bit));
 }
 
-template <int PG, int J0, int UNIT>
+// the same with v < t: the cold-day bits of a cold-spell pass
+__device__ __forceinline__ void or_if_lt(uint32_t &m, float v, float t, uint32_t bit)
+{
+    asm("{\n\t.reg .pred p;\n\tsetp.lt.f32 p, %1, %2;\n\t@p or.b32 %0, %0, %3;\n\t}" : "+r"(m) : "f"(v), "f"(t), "r"(bit));
+}
+
+template <int PG, int J0, int UNIT, bool COLD>
 __device__ __forceinline__ void hot_half(uint32_t (&m)[kHotYears][PG], const float *const (&xp)[kHotYears], const int (&jo)[kHotYears],
                                          const int (&nb)[kHotYears], int64_t ld_t, const float *ts)
 {
@@ -68,11 +76,19 @@ __device__ __forceinline__ void hot_half(uint32_t (&m)[kHotYears][PG], const flo
 #pragma unroll
         for (int y = 0; y < kHotYears; y++)
 #pragma unroll
-            for (int q = 0; q < PG; q++) or_if_gt(m[y][q], v[y][j], t[q], 1u << (J0 + j));
+            for (int q = 0; q < PG; q++) {
+                if (COLD) or_if_lt(m[y][q], v[y][j], t[q], 1u << (J0 + j));
+                else or_if_gt(m[y][q], v[y][j], t[q], 1u << (J0 + j));
+            }
     }
 }
 
-template <int PG, int UNIT>
+// COLD: the bits mark days with (double)x < thr (cold spells) instead of (double)x > thr.  The tile is then rounded UP
+// (__double2float_ru), which keeps the double-precision `x < thr` exact for every float x: a thr that is a float is kept; else
+// ru(thr) is the smallest float above thr, so no float lies in [thr, ru(thr)) and x < thr <=> x < ru(thr).  At the ends: thr >
+// FLT_MAX becomes +inf, below which every finite float lies (all are < thr); thr < -FLT_MAX becomes -FLT_MAX, below which only
+// -inf lies (the only float < thr).  NaN stays NaN and compares false on either side; the padding is -inf, never cold.
+template <int PG, int UNIT, bool COLD>
 __global__ void __launch_bounds__(256, PG <= 10 ? 3 : 2)
 k_hot_words(const float *__restrict__ x, int64_t C, int64_t ld_t,
             const double *__restrict__ thr, int n_doy, int P,
@@ -88,10 +104,11 @@ k_hot_words(const float *__restrict__ x, int64_t C, int64_t ld_t,
 
     // Threshold tile.  Per cell the (doy, percentile) block of this tile is nd * P contiguous doubles in the reference's
     // [C, n_doy, P] order: a warp reads them with consecutive lanes, kFillLoads independent loads per lane in flight
-    // (the fill is pure HBM latency), and scatters them to [group][doy][PG][cell].  Padding percentiles / days: +inf.
+    // (the fill is pure HBM latency), and scatters them to [group][doy][PG][cell].  Padding percentiles / days: +inf (-inf
+    // for COLD), which no sample exceeds (falls below).
     const int n_el = nd * P;                               // doubles per cell
     if (nd < kTileDoy || Ppad != P)
-        for (int i = tid; i < (Ppad / PG) * kTileDoy * PG * kTilePad; i += 256) thr_s[i] = __int_as_float(0x7f800000);
+        for (int i = tid; i < (Ppad / PG) * kTileDoy * PG * kTilePad; i += 256) thr_s[i] = __int_as_float(COLD ? 0xff800000 : 0x7f800000);
     __syncthreads();
     const float inv_p = 1.0f / (float)P;                   // e / P for e < 1024, P <= 32: (e + 0.5) / P is >= 1 / 64 away from every
     for (int e0 = 0; e0 < n_el; e0 += 32 * kFillLoads) {   // integer, far more than the error of the float product
@@ -110,7 +127,7 @@ k_hot_words(const float *__restrict__ x, int64_t C, int64_t ld_t,
             for (int i = 0; i < kFillLoads; i++) v[i] = dst[i] >= 0 ? __ldg(src + 32 * i) : 0.0;
 #pragma unroll
             for (int i = 0; i < kFillLoads; i++)
-                if (dst[i] >= 0) thr_s[dst[i] + cell] = __double2float_rd(v[i]);
+                if (dst[i] >= 0) thr_s[dst[i] + cell] = COLD ? __double2float_ru(v[i]) : __double2float_rd(v[i]);
         }
     }
     __syncthreads();
@@ -147,8 +164,8 @@ k_hot_words(const float *__restrict__ x, int64_t C, int64_t ld_t,
             uint32_t *hp[kHotYears];                               // word kk[y] of percentile pg of this cell; percentile planes are K * C words apart
 #pragma unroll
             for (int y = 0; y < kHotYears; y++) hp[y] = hot + ((int64_t)pg * K + kk[y]) * C + c;
-            hot_half<PG, 0, UNIT>(m, xp, jo, nb, ld_t, ts);
-            if (j_hi > kHotDays) hot_half<PG, kHotDays, UNIT>(m, xp, jo, nb, ld_t, ts);      // warp-uniform
+            hot_half<PG, 0, UNIT, COLD>(m, xp, jo, nb, ld_t, ts);
+            if (j_hi > kHotDays) hot_half<PG, kHotDays, UNIT, COLD>(m, xp, jo, nb, ld_t, ts);      // warp-uniform
 #pragma unroll
             for (int y = 0; y < kHotYears; y++)
 #pragma unroll
@@ -618,13 +635,14 @@ size_t metric_pass_workspace_bytes(int64_t C, int64_t T, int64_t ld_c, int n_doy
 }
 
 // Runs k_hot_words (after the layout-normalising copy when ld_c != 1: the samples then live in L.xn, time-major, ld_t = C);
-// on success plan / L describe what lives in the workspace, and L.thr / L.n_doy the thresholds the kernels read.
+// on success plan / L describe what lives in the workspace, and L.thr / L.n_doy the thresholds the kernels read.  `unit` is a
+// plain unit code (0 - 2); `cold` makes the words cold-day bits.
 static int run_hot_words(const float *d_measure, int64_t C, int64_t T, int64_t ld_t, int64_t ld_c,
                          const double *d_thr, int n_doy, int P, const int32_t *h_doy_map,
                          int Y, void *ws, size_t ws_bytes, cudaStream_t st, WordPlan &plan, Layout &L,
-                         int64_t carve_cells = 0, bool tables_resident = false, int input_unit = 0, bool intensity = false)
+                         int64_t carve_cells = 0, bool tables_resident = false, int unit = 0, bool intensity = false, bool cold = false)
 {
-    if (input_unit < 0 || input_unit > 2) return HDP_B200_ERR_INVALID;
+    if (unit < 0 || unit > 2) return HDP_B200_ERR_INVALID;
     std::vector<int32_t> own_map;
     const int32_t *doy_map = nullptr;
     int rc = pass_doy_map(h_doy_map, T, n_doy, own_map, doy_map);
@@ -659,15 +677,20 @@ static int run_hot_words(const float *d_measure, int64_t C, int64_t T, int64_t l
     const size_t smem = (size_t)kTileDoy * Ppad * kTilePad * sizeof(float);
     dim3 grid((unsigned)((C + kTileCells - 1) / kTileCells), (unsigned)plan.n_blk);
     KernelTimer timer(kHotWords, st);
+#define HDP_LAUNCH_HOT_D(PG, U, CO)                                                                                \
+    do {                                                                                                           \
+        HDP_CUDA_TRY(cudaFuncSetAttribute(k_hot_words<PG, U, CO>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)); \
+        k_hot_words<PG, U, CO><<<grid, 256, smem, st>>>(x, C, ld_t, L.thr, L.n_doy, P, L.words, L.blk_start, L.blk_words, K, L.hot); \
+    } while (0)
 #define HDP_LAUNCH_HOT_U(PG, U)                                                                                    \
     do {                                                                                                           \
-        HDP_CUDA_TRY(cudaFuncSetAttribute(k_hot_words<PG, U>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)); \
-        k_hot_words<PG, U><<<grid, 256, smem, st>>>(x, C, ld_t, L.thr, L.n_doy, P, L.words, L.blk_start, L.blk_words, K, L.hot); \
+        if (cold) HDP_LAUNCH_HOT_D(PG, U, true);                                                                   \
+        else HDP_LAUNCH_HOT_D(PG, U, false);                                                                       \
     } while (0)
 #define HDP_LAUNCH_HOT(PG)                                                                                         \
     do {                                                                                                           \
-        if (input_unit == 0) HDP_LAUNCH_HOT_U(PG, 0);                                                              \
-        else if (input_unit == 1) HDP_LAUNCH_HOT_U(PG, 1);                                                         \
+        if (unit == 0) HDP_LAUNCH_HOT_U(PG, 0);                                                                    \
+        else if (unit == 1) HDP_LAUNCH_HOT_U(PG, 1);                                                               \
         else HDP_LAUNCH_HOT_U(PG, 2);                                                                              \
     } while (0)
     switch (pg) {
@@ -679,6 +702,7 @@ static int run_hot_words(const float *d_measure, int64_t C, int64_t T, int64_t l
     }
 #undef HDP_LAUNCH_HOT
 #undef HDP_LAUNCH_HOT_U
+#undef HDP_LAUNCH_HOT_D
     HDP_LAUNCH_CHECK();
     return HDP_B200_OK;
 }
@@ -857,6 +881,9 @@ int metric_pass(const float *d_measure, int64_t C, int64_t T, int64_t ld_t, int6
     if (C > 0 && T > 0 && (!d_measure || !d_thr)) return HDP_B200_ERR_INVALID;
     if (P > HDP_B200_MAX_PERCENTILES || D > HDP_B200_MAX_DEFINITIONS) return HDP_B200_ERR_UNSUPPORTED;
     cudaStream_t st = (cudaStream_t)stream;
+    // input_unit of the C ABI = unit code | HDP_B200_COLD; the kernels' launchers see the two as plain values
+    const bool cold = (input_unit & HDP_B200_COLD) != 0;
+    const int unit = input_unit & ~HDP_B200_COLD;
 
     // the season tables of both hemispheres, north then south (Y + 1 rows apart, as k_intensity reads them)
     std::vector<int32_t> seasons((size_t)8 * (Y + 1), 0);
@@ -874,7 +901,7 @@ int metric_pass(const float *d_measure, int64_t C, int64_t T, int64_t ld_t, int6
     WordPlan plan;
     Layout L;
     int rc = run_hot_words(d_measure, C, T, ld_t, ld_c, d_thr, n_doy, P, h_doy_map, Y, d_workspace, workspace_bytes, st, plan, L,
-                           carve_cells, tables_resident, input_unit, d_int != nullptr);
+                           carve_cells, tables_resident, unit, d_int != nullptr, cold);
     if (rc != HDP_B200_OK || C == 0 || Y == 0) return rc;
     if (d_out) {
         rc = run_scan(L, plan, C, T, P, h_defs, D, passes, Y, d_is_south, d_out, st, tables_resident);
@@ -882,7 +909,7 @@ int metric_pass(const float *d_measure, int64_t C, int64_t T, int64_t ld_t, int6
     }
     if (d_int)
         rc = run_intensity(L, plan, d_measure, C, T, ld_t, ld_c, L.thr, L.n_doy, P, h_defs, D, seasons, Y, d_is_south, d_int, st,
-                           tables_resident, input_unit);
+                           tables_resident, unit, cold);
     return rc;
 }
 

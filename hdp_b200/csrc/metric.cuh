@@ -33,9 +33,10 @@ struct Layout {
 size_t metric_pass_workspace_bytes(int64_t C, int64_t T, int64_t ld_c, int n_doy, int P, int Y, const int32_t *h_doy_map, bool intensity);
 
 // k_intensity over the hot words in L: the intensity metrics f32 [3, P, D, Y, C].  `seasons` i32 [2, Y + 1, 4]: the season tables
-// of both hemispheres as intensity_season_table (intensity.h) accepts them.
+// of both hemispheres as intensity_season_table (intensity.h) accepts them.  `unit`: a plain unit code (0 - 2); `cold`: the words
+// are cold-day bits and the intensity is the deficit below the threshold.
 int run_intensity(const Layout &L, const WordPlan &plan, const float *d_measure, int64_t C, int64_t T, int64_t ld_t, int64_t ld_c,
                   const double *d_thr, int n_doy, int P, const int32_t *h_defs, int D, const std::vector<int32_t> &seasons, int Y,
-                  const uint8_t *d_is_south, float *d_int, cudaStream_t st, bool tables_resident, int input_unit);
+                  const uint8_t *d_is_south, float *d_int, cudaStream_t st, bool tables_resident, int unit, bool cold);
 
 }  // namespace hdp

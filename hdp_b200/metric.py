@@ -34,6 +34,28 @@ INTENSITY_ATTRS = {
             "description": f"Largest {_EXCEEDANCE}; 0 without heatwave days"},
 }
 
+# The cold-spell variables (compute_individual_metrics(..., cold=True)): the same rules over the days below the threshold, in the
+# cold season (the other hemisphere's heatwave season).
+COLD_METRIC_ATTRS = {
+    "CSF": {"units": "cold spell days", "long_name": "Cold Spell Frequency",
+            "description": "Number of days that fall within a cold spell during a cold season"},
+    "CSD": {"units": "cold spell days", "long_name": "Cold Spell Duration",
+            "description": "Length of longest cold spell during a cold season"},
+    "CSN": {"units": "cold spell events", "long_name": "Cold Spell Number",
+            "description": "Number of distinct cold spells during a cold season"},
+    "CSA": {"units": "cold spell events", "long_name": "Cold Spell Average",
+            "description": "Average length of cold spells during a cold season"},
+}
+_DEFICIT = "deficit e = threshold - measure (float64) on the days that fall within a cold spell during a cold season"
+COLD_INTENSITY_ATTRS = {
+    "CSC": {"long_name": "Cold Spell Cumulative Intensity",
+            "description": f"Sum of the {_DEFICIT}, added cold spell by cold spell in time order; 0 without cold spell days"},
+    "CSI": {"long_name": "Cold Spell Mean Intensity",
+            "description": f"Cumulative intensity divided by the cold spell frequency: mean of the {_DEFICIT}; 0 without cold spell days"},
+    "CSP": {"long_name": "Cold Spell Peak Intensity",
+            "description": f"Largest {_DEFICIT}; 0 without cold spell days"},
+}
+
 
 # ----------------------------------------------------------------------------------------------
 # The building blocks under the reference's names (its unit tests import exactly these: hdp/tests/test_index_heatwaves.py,
@@ -174,11 +196,13 @@ def _widen_int64(a: np.ndarray) -> np.ndarray:
     return out
 
 
-def _metric_sweep(measure, threshold, hw_definitions, time_axis, doy_map=None, intensity=False):
+def _metric_sweep(measure, threshold, hw_definitions, time_axis, doy_map=None, intensity=False, cold=False):
     """The percentile x definition x cell sweep of compute_heatwave_metrics_wrapper (metric.py:344-369) as ONE library call:
     -> ((uint16 [4, P, D, Y, C], float32 [3, P, D, Y, C] or None), season tables, cell dims, cell shape, P, D).  With
-    ``intensity`` the call is the intensity pass, which also returns the intensity metrics."""
+    ``intensity`` the call is the intensity pass, which also returns the intensity metrics.  With ``cold`` it is the cold-spell
+    pass, and each hemisphere's season is the other one's heatwave season (north Nov 1 - Apr 1, south May 1 - Oct 1)."""
     st = _tables.hemisphere_ranges(time_axis)                       # compute_hemisphere_ranges, :410
+    north, south_tab = (st.south, st.north) if cold else (st.north, st.south)
     if doy_map is None:
         doy_map = _tables.doy_map(time_axis.dayofyr)                # build_doy_map, :413
     x, cell_dims, cell_shape = _layout.to_time_cells(xr.values_of(measure), tuple(measure.dims), require_float32=True)
@@ -199,9 +223,9 @@ def _metric_sweep(measure, threshold, hw_definitions, time_axis, doy_map=None, i
     defs = np.asarray(hw_definitions, dtype=np.int64).reshape(-1, 3)
     if intensity:
         out = np.empty((4, P, defs.shape[0], st.n_years, x.shape[1]), np.uint16)
-        heat = _core.intensity_host(x, thr_cdp, doy_map, defs, st.north, st.south, south, metrics_out=out)   # float32 [3, P, D, Y, C]
+        heat = _core.intensity_host(x, thr_cdp, doy_map, defs, north, south_tab, south, metrics_out=out, cold=cold)   # f32 [3, P, D, Y, C]
     else:
-        out, heat = _core.metrics_host(x, thr_cdp, doy_map, defs, st.north, st.south, south), None       # uint16 [4, P, D, Y, C]
+        out, heat = _core.metrics_host(x, thr_cdp, doy_map, defs, north, south_tab, south, cold=cold), None       # u16 [4, P, D, Y, C]
     return (out, heat), st, cell_dims, cell_shape, P, defs.shape[0]
 
 
@@ -217,10 +241,14 @@ def compute_heatwave_metrics_wrapper(measure, threshold, doy_map, hw_definitions
 
 
 def compute_individual_metrics(measure, threshold, hw_definitions: list, include_threshold: bool = True, check_variables: bool = True,
-                               *, intensity: bool = False):
+                               *, intensity: bool = False, cold: bool = False):
     """metric.py:372-506.  ``intensity=True`` adds three float32 variables to the four metrics (which stay identical): HWC, HWI
     and HWP, the cumulative, mean and peak exceedance ``measure - threshold`` over the heatwave days of every season, in the
-    measure's units (see hdp_b200_intensity in include/hdp_b200.h for the exact arithmetic).  Same dims and coords as HWF."""
+    measure's units (see hdp_b200_intensity in include/hdp_b200.h for the exact arithmetic).  Same dims and coords as HWF.
+
+    ``cold=True`` computes cold spells instead: CSF, CSN, CSD, CSA (and with ``intensity`` CSC, CSI, CSP, the deficit
+    ``threshold - measure``) by the same rules over the days with ``measure < threshold``, in each hemisphere's cold season (the
+    other hemisphere's heatwave season).  Use low percentiles for the threshold (e.g. 0.01 ... 0.10)."""
     time_axis = time_axis_of(measure)
     if check_variables:                                             # :393-398
         assert "hdp_type" in threshold.attrs
@@ -238,7 +266,10 @@ def compute_individual_metrics(measure, threshold, hw_definitions: list, include
             if entry != '':
                 combined_history += (f"(Threshold) {entry}\n")
 
-    (out, heat), st, cell_dims, cell_shape, P, D = _metric_sweep(measure, threshold, hw_definitions, time_axis, intensity=intensity)
+    (out, heat), st, cell_dims, cell_shape, P, D = _metric_sweep(measure, threshold, hw_definitions, time_axis, intensity=intensity,
+                                                                 cold=cold)
+    metric_names = _core.COLD_METRIC_NAMES if cold else _core.METRIC_NAMES
+    intensity_names = _core.COLD_INTENSITY_NAMES if cold else _core.INTENSITY_NAMES
     Y = st.n_years
 
     coords = dict(xr.non_time_coords(measure))
@@ -247,29 +278,31 @@ def compute_individual_metrics(measure, threshold, hw_definitions: list, include
     coords["time"] = _year_times(st.years, time_axis.calendar)
     dims = ["percentile", "definition", *cell_dims, "time"]
     data_vars = {}
-    for i, name in enumerate(_core.METRIC_NAMES):                   # HWF=0, HWN=1, HWD=2, HWA=3, :454-461
+    for i, name in enumerate(metric_names):                         # HWF=0, HWN=1, HWD=2, HWA=3, :454-461
         wide = out[i] if np.dtype(METRIC_DTYPE) == np.uint16 else _widen_int64(out[i]).astype(METRIC_DTYPE, copy=False)   # [P, D, Y, C]
         plane = wide.transpose(0, 1, 3, 2).reshape(P, D, *cell_shape, Y)                # view: no host transposition
         data_vars[name] = xr.DataArray(plane, dims=dims, coords=coords)
     if intensity:
-        for i, name in enumerate(_core.INTENSITY_NAMES):            # float32 [P, D, Y, C]
+        for i, name in enumerate(intensity_names):                  # float32 [P, D, Y, C]
             data_vars[name] = xr.DataArray(heat[i].transpose(0, 1, 3, 2).reshape(P, D, *cell_shape, Y), dims=dims, coords=coords)
     ds = xr.Dataset(data_vars)
+    kind = "Cold spell" if cold else "Heatwave"
     ds.attrs.update({
-        "description": f"Heatwave metric dataset generated by Heatwave Diagnostics Package (HDP v{get_version()})",
+        "description": f"{kind} metric dataset generated by Heatwave Diagnostics Package (HDP v{get_version()})",
         "hdp_version": get_version(),
         "hdp_type": "metric"
     })
-    for name, attrs in METRIC_ATTRS.items():
+    for name, attrs in (COLD_METRIC_ATTRS if cold else METRIC_ATTRS).items():
         ds[name].attrs.update(attrs)
     if intensity:
-        for name, attrs in INTENSITY_ATTRS.items():
+        for name, attrs in (COLD_INTENSITY_ATTRS if cold else INTENSITY_ATTRS).items():
             ds[name].attrs.update({"units": measure.attrs["units"], **attrs} if "units" in measure.attrs else attrs)
     xr.set_coord_attrs(ds, "percentile", {"range": "(0, 1)"})
+    days = "cold" if cold else "hot"
     xr.set_coord_attrs(ds, "definition", {
-        "first_number": "Minimum number of consecutively hot days",
+        "first_number": f"Minimum number of consecutively {days} days",
         "second_number": "Maximum number of break days after first wave",
-        "third_number": "Minimum number of consecutively hot days after the break"
+        "third_number": f"Minimum number of consecutively {days} days after the break"
     })
     for variable in ds:
         ds[variable].attrs["history"] = combined_history
@@ -278,9 +311,10 @@ def compute_individual_metrics(measure, threshold, hw_definitions: list, include
 
 
 def compute_group_metrics(measures, thresholds, hw_definitions: list, include_threshold: bool = False, check_variables: bool = True,
-                          *, intensity: bool = False):
+                          *, intensity: bool = False, cold: bool = False):
     """metric.py:509-523: every measure against every threshold of the same baseline variable.  ``intensity=True`` adds the
-    HWC / HWI / HWP variables of :func:`compute_individual_metrics` under the same ``{measure}.{threshold}.{metric}`` names."""
+    HWC / HWI / HWP variables of :func:`compute_individual_metrics` under the same ``{measure}.{threshold}.{metric}`` names;
+    ``cold=True`` gives the cold-spell variables (``{measure}.{threshold}.CSF`` ...) instead."""
     metric_sets = []
     for measure_name in list(measures.keys()):
         measure = measures[measure_name]
@@ -288,7 +322,7 @@ def compute_group_metrics(measures, thresholds, hw_definitions: list, include_th
             threshold = thresholds[threshold_name]
             if threshold.attrs["baseline_variable"] == measure.attrs["baseline_variable"]:
                 hw_metrics = compute_individual_metrics(measure, threshold, hw_definitions, include_threshold, check_variables,
-                                                        intensity=intensity)
+                                                        intensity=intensity, cold=cold)
                 var_renames = {name: f"{measure_name}.{threshold_name}.{name}" for name in list(hw_metrics.keys())}
                 metric_sets.append(hw_metrics.rename(var_renames))
     aggr_ds = xr.merge(metric_sets)

@@ -130,7 +130,18 @@ int hdp_b200_thresholds_host(const float *h_temps, int64_t C, int64_t T_b, int64
  *   d_out         u16 [4, P, D, Y, C]  metric-major: HWF, HWN, HWD, HWA (= HWF / HWN truncated, metric.py:336-340);
  *                 the reference's int64 (percentile, definition, <cells>, metric, year) array is
  *                 out[m][p][d][y][c] widened.  Every value is <= the longest season, which must be < 65536.
+ *   input_unit    as for hdp_b200_thresholds, optionally OR-ed with HDP_B200_COLD (here and in hdp_b200_metrics_host,
+ *                 hdp_b200_intensity and hdp_b200_intensity_host).
+ *
+ * Cold spells (HDP_B200_COLD): a day counts when (double)x(t) < thr[c, doy_map[t], p] instead of x(t) > thr (NaN on either side:
+ * never; a -inf sample is cold unless thr is -inf), and the planes are CSF, CSN, CSD, CSA: exactly the rules of HWF, HWN, HWD,
+ * HWA applied to the cold days, in the same layout.  The cold result equals the heatwave result for -x and -thr bit for bit.
+ * The season tables are used as given: the cold season of a hemisphere is usually the other hemisphere's warm season.
+ * Libraries of ABI version 6 without cold spells reject the flag with HDP_B200_ERR_INVALID.  The threshold entry points take
+ * no direction and reject it too.
  * ------------------------------------------------------------------------------------------------- */
+#define HDP_B200_COLD 0x100
+
 /* h_doy_map may be NULL: the size is then an upper bound for regular daily calendars. */
 size_t hdp_b200_metrics_workspace_bytes(int64_t C, int64_t T, int64_t ld_t, int64_t ld_c,
                                         int n_doy, int P, int D, int Y, const int32_t *h_doy_map);
@@ -181,6 +192,10 @@ int hdp_b200_metrics_host(const float *h_measure, int64_t C, int64_t T, int64_t 
  *                 pass over the samples
  * The non-empty seasons of each hemisphere's table must be pairwise disjoint after slice clamping (every table built by
  * compute_hemisphere_ranges / get_range_indices is); other tables return HDP_B200_ERR_UNSUPPORTED.
+ *
+ * With HDP_B200_COLD in input_unit: CSC, CSI, CSP over the cold-spell days (see Path 2 above), with the deficit
+ * e_t = thr[c, doy_map[t], p] - (double)x_c(t) > 0 in place of the exceedance, in the same order and layout (a -inf sample
+ * gives inf); d_out then receives CSF, CSN, CSD, CSA.
  * ------------------------------------------------------------------------------------------------- */
 /* h_doy_map may be NULL: the size is then an upper bound for regular daily calendars. */
 size_t hdp_b200_intensity_workspace_bytes(int64_t C, int64_t T, int64_t ld_t, int64_t ld_c,
