@@ -207,6 +207,20 @@ constexpr int kScanWarps = 8;
 constexpr int kScanQ = 16;                                       // queued words per lane (power of two)
 constexpr int kScanQueueWords = 3 * kScanQ * 32;                  // u32 per warp: run starts, run ends, first day of the word
 
+// p + bytes as one 64-bit add the compiler keeps: written as `p += n`, the flush's pointers were turned back into element indices
+// and every store rebuilt its address from them
+__device__ __forceinline__ uint16_t *add_ptr(uint16_t *p, int64_t bytes)
+{
+    uint16_t *r;
+    asm("add.s64 %0, %1, %2;" : "=l"(r) : "l"(p), "l"(bytes));
+    return r;
+}
+
+__device__ __forceinline__ void stg_u16(uint16_t *p, uint32_t v)
+{
+    asm volatile("st.global.u16 [%0], %1;" ::"l"(p), "h"((unsigned short)v) : "memory");
+}
+
 // k_scan.  One warp per (32 neighbouring cells, percentile), one lane per cell.  Two alternating phases:
 //
 //  A (warp-synchronous over the hot words, in time order): the lanes read word k of their cells (one coalesced
@@ -256,7 +270,10 @@ k_scan(const uint32_t *__restrict__ hot, int64_t C, int K, int T, const int4 *__
     // [K + 1] per hot word {first day, days, unknown days of the NEXT word (they count as hot), unknown days after that};
     // word K is a virtual cold day at T that closes a run still open at the end of the series
     int4 *word_meta = (int4 *)(smem_scan + ((kScanWarps * kScanQueueWords + tabs.ge_len + tabs.brk_len + 3) & ~3));
+    uint32_t *hwa_rcp = (uint32_t *)(word_meta + K + 1);         // [256] 8-bit lanes only: the HWA divisors' reciprocals
     const int tid = threadIdx.x, nthreads = kScanWarps * 32;
+    if (kBytes)
+        for (int i = tid; i < 256; i += nthreads) hwa_rcp[i] = scan_hwa_rcp(i);
     for (int i = tid; i < tabs.ge_len; i += nthreads) ge_s[i] = ge_tab[i];
     for (int i = tid; i < tabs.brk_len; i += nthreads) brk_s[i] = brk_tab[i];
     for (int i = tid; i <= K; i += nthreads) {
@@ -305,37 +322,46 @@ k_scan(const uint32_t *__restrict__ hot, int64_t C, int K, int T, const int4 *__
 #pragma unroll
     for (int j = 0; j < NG; j++) { cntg[j] = 0u; hwfg[j] = 0u; hwng[j] = 0u; hwdg[j] = 0u; }
 
-    const int64_t plane = (int64_t)P * D * Y * C;                 // one metric
+    // metric m of definition d, season row r of this lane's cell: out_pc[m * P * D * Y * C + d * Y * C + r * C]
+    uint16_t *const out_pc = out + (int64_t)p * D * Y * C + c;
+    auto lane_of = [](uint32_t v, int h) -> uint32_t {            // accumulator lane h of a register, zero-extended (one PRMT)
+        return kBytes ? __byte_perm(v, 0u, 0x4440 + h) : (v >> (BITS * h)) & LANE_MASK;
+    };
     auto flush = [&]() {                                          // close season `ys`
+        if (alive) {
+            const int64_t dstride_b = (int64_t)Y * C * sizeof(uint16_t), plane_b = P * D * dstride_b;
+            uint16_t *o = out_pc + (int64_t)row_cur * C;
 #pragma unroll
-        for (int j = 0; j < NG; j++) {
+            for (int j = 0; j < NG; j++) {
 #pragma unroll
-            for (int h = 0; h < PER; h++) {
-                const int d = PER * j + h;
-                if (d < D && alive) {
-                    const uint32_t f = (hwfg[j] >> (BITS * h)) & LANE_MASK, nn = (hwng[j] >> (BITS * h)) & LANE_MASK;
-                    const int64_t o = (((int64_t)p * D + d) * Y + row_cur) * C + c;
-                    out[o] = (uint16_t)f;
-                    out[o + plane] = (uint16_t)nn;
-                    out[o + 2 * plane] = (uint16_t)((hwdg[j] >> (BITS * h)) & LANE_MASK);
-                    // trunc(mean) = f / nn in integers, metric.py:340.  f, nn < 65536, so (f + 0.5) / nn is at least 0.5 / nn
-                    // away from every integer - orders of magnitude more than the error of the fast float division
-                    out[o + 3 * plane] = (uint16_t)(nn ? __float2uint_rz(__fdividef((float)f + 0.5f, (float)nn)) : 0u);
+                for (int h = 0; h < PER; h++) {
+                    if (PER * j + h < D) {                        // warp-uniform
+                        const uint32_t f = lane_of(hwfg[j], h), nn = lane_of(hwng[j], h);
+                        uint16_t *const o1 = add_ptr(o, plane_b), *const o2 = add_ptr(o1, plane_b), *const o3 = add_ptr(o2, plane_b);
+                        stg_u16(o, f);
+                        stg_u16(o1, nn);
+                        stg_u16(o2, lane_of(hwdg[j], h));
+                        // trunc(mean) = f / nn in integers, metric.py:340; 8-bit lanes: f * ceil(2^16 / nn) >> 16, exact for
+                        // f, nn < 256 (scan_hwa_rcp)
+                        stg_u16(o3, kBytes ? (f * hwa_rcp[nn]) >> 16 : nn ? f / nn : 0u);
+                    }
+                    o = add_ptr(o, dstride_b);
                 }
             }
-            cntg[j] = 0u; hwfg[j] = 0u; hwng[j] = 0u; hwdg[j] = 0u;
         }
+#pragma unroll
+        for (int j = 0; j < NG; j++) { cntg[j] = 0u; hwfg[j] = 0u; hwng[j] = 0u; hwdg[j] = 0u; }
         fresh = 0xffffffffu;
         ys++;
         if (ys < n_seasons) { const int4 s4 = seas[ys]; a_cur = s4.x; b_cur = s4.y; row_cur = s4.z; }
         else { a_cur = INT_MAX; b_cur = INT_MAX; }
     };
 
-    // definition bits -> one 0/1 per accumulator lane
+    // definition bits -> one 0/1 per accumulator lane.  The bits are those of definitions < D <= PER * NG (labels are made from
+    // the definition tables), so the last group needs no mask.
     auto spread = [](uint32_t bits, int j) -> uint32_t {
-        if (kBytes) return (((bits >> (4 * j)) & 0xfu) * 0x00204081u) & 0x01010101u;
-        const uint32_t t = bits >> (2 * j);
-        return (t & 1u) | ((t & 2u) << 15);
+        const uint32_t t = bits >> (PER * j), g = j == NG - 1 ? t : t & ((1u << PER) - 1u);
+        return kBytes ? (g * 0x00204081u) & 0x01010101u : (g * 0x00008001u) & 0x00010001u;
     };
     // accounting of `days` heatwave days of the definitions in `lab` to the open season (HWF/HWN/HWD, metric.py:63-137)
     auto account = [&](uint32_t lab, uint32_t days) {
@@ -800,8 +826,9 @@ static int run_scan(const Layout &L, const WordPlan &plan, int64_t C, int64_t T,
     const ScanTables &tabs = cfg.tabs;
     if (!tables_resident) HDP_CUDA_TRY(cudaMemcpyAsync(L.lut, cfg.lut.data(), sizeof(uint32_t) * cfg.lut.size(), cudaMemcpyHostToDevice, st));
     const uint32_t *ge_tab = L.lut, *brk_tab = L.lut + tabs.ge_len;
-    const size_t scan_smem = (((size_t)kScanWarps * kScanQueueWords + cfg.lut.size() + 3) & ~(size_t)3) * sizeof(uint32_t) + ((size_t)K + 1) * sizeof(int4);
+    size_t scan_smem = (((size_t)kScanWarps * kScanQueueWords + cfg.lut.size() + 3) & ~(size_t)3) * sizeof(uint32_t) + ((size_t)K + 1) * sizeof(int4);
     if (scan_smem > 200 * 1024) return HDP_B200_ERR_UNSUPPORTED;             // > ~9 000 hot words (~800 years of daily data)
+    if (cfg.bytes) scan_smem += 256 * sizeof(uint32_t);                      // k_scan's hwa_rcp
     const int64_t n_warps = ((C + 31) / 32) * P;                             // one warp per (32 cells, percentile)
     const unsigned scan_grid = (unsigned)((n_warps + kScanWarps - 1) / kScanWarps);
 

@@ -1,7 +1,8 @@
 // seams.h - the per-run and per-season logic of the reference's path-2 BUILDING BLOCKS, as plain functions that compile for
 // the device (seams.cu) and for the host (tests/seams_host.cpp, which replays the kernels' lane loops on the CPU against the
 // oracle: the logic below is checked without a GPU, the kernels add only the warp plumbing around it).  It also holds the two
-// rules of the fused pass that its host replay (tests/intensity_host.cpp) shares: the season table and the cut into hot-day words.
+// rules of the fused pass that its host replay (tests/intensity_host.cpp) shares: the season table and the cut into hot-day words,
+// and the integer HWA division of k_scan's 8-bit accumulator lanes.
 //
 // Reference = AgentOxygen/HDP v1.0.2:
 //   index_heatwaves      hdp/metric.py:11-60
@@ -154,5 +155,11 @@ HDP_HD double season_average(const SeasonAcc &a, int64_t n, bool multi)
     if (n <= 0) return 0.0;
     return (double)a.sum / (double)(multi ? a.uniq - 1 : 1);
 }
+
+// ---- the fused pass's HWA (k_scan, metric.cu) -----------------------------------------------------------------------------
+// trunc(HWF / HWN) of an 8-bit accumulator lane as (f * scan_hwa_rcp(nn)) >> 16, exact for every f, nn < 256: ceil(2^16 / nn) =
+// (2^16 + e) / nn with 0 <= e < nn, so the product exceeds f / nn by f e / (nn 2^16) < 1 / nn, less than the distance from f / nn
+// up to the next integer.  nn = 0 (a season without heatwaves, f = 0 too) gives 0.  tests/test_scan_hwa.py checks all pairs.
+HDP_HD uint32_t scan_hwa_rcp(uint32_t nn) { return nn ? (0x10000u + nn - 1u) / nn : 0u; }
 
 }  // namespace hdp
