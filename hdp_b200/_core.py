@@ -11,6 +11,8 @@ These are the two seams of the reference that the CUDA library replaces:
   heatwave days of a season), which the reference does not have; optionally with the four metrics from the same pass
 * ``cold=True`` on the metric and intensity calls: cold spells (CSF ... CSA, CSC ... CSP), the same sweep over the days below the
   threshold, which the reference does not have either
+* :func:`compound_metrics_array`, :func:`compound_intensity_array`: compound (day-night) heatwaves, the same sweep over the days on
+  which two measures (e.g. tmax and tmin) both exceed their own thresholds
 * :func:`index_heatwaves_array`, :func:`season_metrics_array` <- ``index_heatwaves`` and ``heatwave_frequency`` / ``number`` /
   ``duration`` / ``average`` (reference hdp/metric.py:11-172), the building blocks the hot path never materialises
 
@@ -212,6 +214,99 @@ def intensity_array(measure, thresholds, doy_map, defs, season_north, season_sou
     be disjoint (every table compute_hemisphere_ranges builds is).  ``cold=True``: CSC, CSI, CSP - the deficit
     ``threshold - measure`` over the cold-spell days (and CSF ... CSA in ``metrics_out``), see :func:`metrics_array`."""
     return _metric_pass(measure, thresholds, doy_map, defs, season_north, season_south, is_south, units, metrics_out, out, True, cold)
+
+
+def _compound_pass(measure_a, thresholds_a, measure_b, thresholds_b, doy_map, defs, season_north, season_south, is_south, units, met,
+                   heat, intensity, cold):
+    """hdp_b200_compound on CUDA tensors: the metrics (``met``) and / or, with ``intensity``, both measures' intensity blocks
+    (``heat``, float32 ``[2, 3, P, D, Y, C]``).  Returns the intensity output of an intensity pass, else the metrics."""
+    torch = _torch()
+    unit = _unit_code(units) | (COLD if cold else 0)
+    _check_measure(measure_a, "measure_a")
+    _check_measure(measure_b, "measure_b")
+    if tuple(measure_a.shape) != tuple(measure_b.shape) or measure_a.device != measure_b.device:
+        raise ValueError("measure_a and measure_b must have the same shape [T, C] and device")
+    T, C = measure_a.shape
+    _check_thr(thresholds_a, C)
+    _check_thr(thresholds_b, C)
+    if tuple(thresholds_a.shape) != tuple(thresholds_b.shape):
+        raise ValueError("thresholds_a and thresholds_b must have the same shape [C, n_doy, P]")
+    n_doy, P = int(thresholds_a.shape[1]), int(thresholds_a.shape[2])
+    dm, df, sn, ss = _metric_tables(doy_map, defs, season_north, season_south)
+    if dm.size != T:
+        raise ValueError("doy_map must have one entry per time step")
+    L = _lib.lib()
+    D, Y = int(df.shape[0]), int(sn.shape[0])
+    dev = measure_a.device
+    south_t = _south_tensor(is_south, C, dev)
+    if intensity:
+        heat = _device_out(heat, torch.float32, (2, 3, P, D, Y, C), dev, "out must be a contiguous float32 CUDA tensor [2, 3, P, D, Y, C]")
+    if met is not None or not intensity:
+        met = _device_out(met, torch.uint16, (4, P, D, Y, C), dev,
+                          f"{'metrics_out' if intensity else 'out'} must be a contiguous uint16 CUDA tensor [4, P, D, Y, C]")
+    (ld_ta, ld_ca), (ld_tb, ld_cb) = _strides(measure_a), _strides(measure_b)
+    with torch.cuda.device(dev):
+        nbytes = L.hdp_b200_compound_workspace_bytes(C, T, ld_ca, ld_cb, n_doy, P, D, Y, _hp(dm))
+        ws = _workspace(dev, nbytes)
+        rc = L.hdp_b200_compound(measure_a.data_ptr(), ld_ta, ld_ca, measure_b.data_ptr(), ld_tb, ld_cb, C, T, thresholds_a.data_ptr(),
+                                 thresholds_b.data_ptr(), n_doy, P, _hp(dm), _hp(df), D, _hp(sn), _hp(ss), Y,
+                                 south_t.data_ptr() if south_t is not None else None, met.data_ptr() if met is not None else None,
+                                 heat.data_ptr() if intensity else None, ws.data_ptr(), ws.numel(), torch.cuda.current_stream().cuda_stream,
+                                 unit)
+    _lib.check(rc, "hdp_b200_compound")
+    return heat if intensity else met
+
+
+def compound_metrics_array(measure_a, thresholds_a, measure_b, thresholds_b, doy_map, defs, season_north, season_south, is_south=None,
+                           out=None, units=None, *, cold=False):
+    """Compound heatwaves: :func:`metrics_array` over the days on which BOTH ``measure_a > thresholds_a`` and
+    ``measure_b > thresholds_b`` (e.g. tmax and tmin: hot days and hot nights) -> uint16 ``[4, P, D, Y, C]``.  The two measures are
+    f32 ``[T, C]`` CUDA tensors (any strides each), the two thresholds f64 ``[C, n_doy, P]`` of the same shape: percentile p of A is
+    paired with percentile p of B.  ``units`` applies to both measures; ``cold=True``: days on which both are below their
+    thresholds (CSF ... CSA)."""
+    return _compound_pass(measure_a, thresholds_a, measure_b, thresholds_b, doy_map, defs, season_north, season_south, is_south, units,
+                          out, None, False, cold)
+
+
+def compound_intensity_array(measure_a, thresholds_a, measure_b, thresholds_b, doy_map, defs, season_north, season_south, is_south=None,
+                             out=None, metrics_out=None, units=None, *, cold=False):
+    """Intensity of the compound heatwaves of :func:`compound_metrics_array`: float32 ``[2, 3, P, D, Y, C]``, block 0 = HWC, HWI, HWP
+    of measure A (its exceedance ``measure_a - thresholds_a`` over the compound heatwave days, as :func:`intensity_array` computes
+    it), block 1 = the same for measure B.  ``metrics_out``: an optional uint16 CUDA tensor ``[4, P, D, Y, C]`` that also receives
+    what :func:`compound_metrics_array` returns, from the same pass.  ``cold``: the deficits over the compound cold spells."""
+    return _compound_pass(measure_a, thresholds_a, measure_b, thresholds_b, doy_map, defs, season_north, season_south, is_south, units,
+                          metrics_out, out, True, cold)
+
+
+def compound_hot_days_array(measure_a, thresholds_a, measure_b, thresholds_b, doy_map, units=None, *, cold=False):
+    """The compound mask of every percentile: uint8 ``[P, T, C]``, 1 where both measures exceed their thresholds (``cold``: are
+    below them)."""
+    torch = _torch()
+    _check_measure(measure_a, "measure_a")
+    _check_measure(measure_b, "measure_b")
+    if tuple(measure_a.shape) != tuple(measure_b.shape) or measure_a.device != measure_b.device:
+        raise ValueError("measure_a and measure_b must have the same shape [T, C] and device")
+    T, C = measure_a.shape
+    _check_thr(thresholds_a, C)
+    _check_thr(thresholds_b, C)
+    if tuple(thresholds_a.shape) != tuple(thresholds_b.shape):
+        raise ValueError("thresholds_a and thresholds_b must have the same shape [C, n_doy, P]")
+    n_doy, P = int(thresholds_a.shape[1]), int(thresholds_a.shape[2])
+    dm = _i32(doy_map).ravel()
+    if dm.size != T:
+        raise ValueError("doy_map must have one entry per time step")
+    L = _lib.lib()
+    out = torch.empty((P, T, C), dtype=torch.uint8, device=measure_a.device)
+    (ld_ta, ld_ca), (ld_tb, ld_cb) = _strides(measure_a), _strides(measure_b)
+    with torch.cuda.device(measure_a.device):
+        nbytes = L.hdp_b200_compound_workspace_bytes(C, T, ld_ca, ld_cb, n_doy, P, 1, 0, _hp(dm))
+        ws = _workspace(measure_a.device, nbytes)
+        rc = L.hdp_b200_compound_hot_days(measure_a.data_ptr(), ld_ta, ld_ca, measure_b.data_ptr(), ld_tb, ld_cb, C, T,
+                                          thresholds_a.data_ptr(), thresholds_b.data_ptr(), n_doy, P, _hp(dm), out.data_ptr(),
+                                          ws.data_ptr(), ws.numel(), torch.cuda.current_stream().cuda_stream,
+                                          _unit_code(units) | (COLD if cold else 0))
+    _lib.check(rc, "hdp_b200_compound_hot_days")
+    return out
 
 
 def hot_days_array(measure, thresholds, doy_map):
@@ -497,6 +592,67 @@ def _metric_pass_host(measure, thresholds, doy_map, defs, season_north, season_s
     return heat if intensity else met
 
 
+def _host_thresholds(thresholds, C):
+    """(host array or None, device tensor or None) of one threshold argument of a host call: a CUDA tensor is used where it is, a
+    host array that :func:`thresholds_host` returned with ``keep=True`` through its device copy."""
+    torch = _torch()
+    if isinstance(thresholds, torch.Tensor):
+        _check_thr(thresholds, C)
+        return None, thresholds
+    thr = np.ascontiguousarray(thresholds, dtype=np.float64)
+    if thr.ndim != 3 or thr.shape[0] != C:
+        raise TypeError("thresholds must be float64 [C, n_doy, P]")
+    return thr, resident_thresholds(thr)
+
+
+def _compound_pass_host(measure_a, thresholds_a, measure_b, thresholds_b, doy_map, defs, season_north, season_south, is_south, units,
+                        met, heat, intensity, cold):
+    """:func:`_compound_pass` with host arrays (hdp_b200_compound_host); each threshold as for :func:`metrics_host`."""
+    a, ld_ta, ld_ca = _host_measure(measure_a, "measure_a")
+    b, ld_tb, ld_cb = _host_measure(measure_b, "measure_b")
+    if a.shape != b.shape:
+        raise ValueError("measure_a and measure_b must have the same shape [T, C]")
+    T, C = a.shape
+    (h_a, d_a), (h_b, d_b) = _host_thresholds(thresholds_a, C), _host_thresholds(thresholds_b, C)
+    shape_a = tuple((d_a if h_a is None else h_a).shape)
+    if shape_a != tuple((d_b if h_b is None else h_b).shape):
+        raise ValueError("thresholds_a and thresholds_b must have the same shape [C, n_doy, P]")
+    n_doy, P = int(shape_a[1]), int(shape_a[2])
+    dm, df, sn, ss = _metric_tables(doy_map, defs, season_north, season_south)
+    if dm.size != T:
+        raise ValueError("doy_map must have one entry per time step")
+    south = None if is_south is None else np.ascontiguousarray(is_south, dtype=np.uint8)
+    D, Y = df.shape[0], sn.shape[0]
+    if intensity:
+        heat = _host_out(heat, np.float32, (2, 3, P, D, Y, C), "out must be a C-contiguous float32 array [2, 3, P, D, Y, C]")
+    if met is not None or not intensity:
+        met = _host_out(met, np.uint16, (4, P, D, Y, C),
+                        f"{'metrics_out' if intensity else 'out'} must be a C-contiguous uint16 array [4, P, D, Y, C]")
+    hp = lambda h: _hp(h) if h is not None else None                # noqa: E731
+    dp = lambda d: d.data_ptr() if d is not None else None          # noqa: E731
+    rc = _lib.lib().hdp_b200_compound_host(_hp(a), ld_ta, ld_ca, _hp(b), ld_tb, ld_cb, C, T, hp(h_a), dp(d_a), hp(h_b), dp(d_b), n_doy, P,
+                                           _hp(dm), _hp(df), D, _hp(sn), _hp(ss), Y, hp(south), hp(met), hp(heat),
+                                           _unit_code(units) | (COLD if cold else 0))
+    _lib.check(rc, "hdp_b200_compound_host")
+    return heat if intensity else met
+
+
+def compound_metrics_host(measure_a: np.ndarray, thresholds_a, measure_b: np.ndarray, thresholds_b, doy_map, defs, season_north,
+                          season_south, is_south=None, out: Optional[np.ndarray] = None, units=None, *, cold=False) -> np.ndarray:
+    """Host-array counterpart of :func:`compound_metrics_array` (both measures' cells of a chunk cross PCIe once).  Each threshold
+    as for :func:`metrics_host`: a host array, a CUDA tensor, or a resident copy."""
+    return _compound_pass_host(measure_a, thresholds_a, measure_b, thresholds_b, doy_map, defs, season_north, season_south, is_south,
+                               units, out, None, False, cold)
+
+
+def compound_intensity_host(measure_a: np.ndarray, thresholds_a, measure_b: np.ndarray, thresholds_b, doy_map, defs, season_north,
+                            season_south, is_south=None, out: Optional[np.ndarray] = None, metrics_out: Optional[np.ndarray] = None,
+                            units=None, *, cold=False) -> np.ndarray:
+    """Host-array counterpart of :func:`compound_intensity_array`: float32 ``[2, 3, P, D, Y, C]``."""
+    return _compound_pass_host(measure_a, thresholds_a, measure_b, thresholds_b, doy_map, defs, season_north, season_south, is_south,
+                               units, metrics_out, out, True, cold)
+
+
 def metrics_host(measure: np.ndarray, thresholds, doy_map, defs, season_north, season_south,
                  is_south=None, out: Optional[np.ndarray] = None, units=None, *, cold=False) -> np.ndarray:
     """``thresholds``: float64 ``[C, n_doy, P]`` as a host array, or as a CUDA tensor (device-resident: no upload).  A host
@@ -528,7 +684,7 @@ def launch_count() -> int:
 
 KERNEL_NAMES = {1: "normalize", 2: "k_thr_generic", 3: "k_hot_words", 4: "k_scan", 5: "k_unpack_mask",
                 6: "k_thr_seg", 7: "k_thr_ranked", 8: "k_measure", 9: "k_thr_cand", 10: "k_thr_net", 11: "k_seam",
-                12: "k_intensity"}
+                12: "k_intensity", 13: "k_hot_pair"}
 
 
 def timing_enable(on: bool) -> None:

@@ -33,6 +33,13 @@ SIGNATURES = {
     "hdp_b200_intensity_workspace_bytes": (_sz, [_i64, _i64, _i64, _i64, _int, _int, _int, _int, _p]),
     "hdp_b200_intensity": (_int, [_p, _i64, _i64, _i64, _i64, _p, _int, _int, _p, _p, _int, _p, _p, _int, _p, _p, _p, _p, _sz, _p, _int]),
     "hdp_b200_intensity_host": (_int, [_p, _i64, _i64, _i64, _i64, _p, _p, _int, _int, _p, _p, _int, _p, _p, _int, _p, _p, _p, _int]),
+    "hdp_b200_compound_workspace_bytes": (_sz, [_i64, _i64, _i64, _i64, _int, _int, _int, _int, _p]),
+    "hdp_b200_compound": (_int, [_p, _i64, _i64, _p, _i64, _i64, _i64, _i64, _p, _p, _int, _int, _p, _p, _int, _p, _p, _int, _p, _p, _p,
+                                 _p, _sz, _p, _int]),
+    "hdp_b200_compound_host": (_int, [_p, _i64, _i64, _p, _i64, _i64, _i64, _i64, _p, _p, _p, _p, _int, _int, _p, _p, _int, _p, _p, _int,
+                                      _p, _p, _p, _int]),
+    "hdp_b200_compound_hot_days": (_int, [_p, _i64, _i64, _p, _i64, _i64, _i64, _i64, _p, _p, _int, _int, _p, _p, _p, _sz, _p, _int]),
+    "hdp_b200_compound_plan": (_int, [_int, _p]),
     "hdp_b200_host_release": (None, []),
     "hdp_b200_metrics_run_filter": (None, [_int]),
     "hdp_b200_metrics_kernel_choice": (_int, [_p, _int, _p, _p, _int, _i64, _p]),

@@ -16,7 +16,7 @@ ROOT = os.path.dirname(HERE)
 CSRC = os.path.join(HERE, "csrc")
 INCLUDE = os.path.join(ROOT, "include")
 LIB = os.path.join(HERE, "libhdp_b200.so")
-SOURCES = ["abi.cu", "threshold.cu", "thr_net.cu", "metric.cu", "intensity.cu", "seams.cu", "measure.cu", "host.cu"]
+SOURCES = ["abi.cu", "threshold.cu", "thr_net.cu", "metric.cu", "compound.cu", "intensity.cu", "seams.cu", "measure.cu", "host.cu"]
 HEADERS = ["common.cuh", "thr_net.cuh", "thr_net_gen.cuh", "seams.h", "metric.cuh", "intensity.h"]
 OBJ = os.path.join(HERE, "_obj")
 

@@ -30,7 +30,7 @@ inline int cuda_status(cudaError_t e) { return e == cudaSuccess ? HDP_B200_OK : 
     } while (0)
 
 // Optional per-kernel CUDA-event timing (hdp_b200_timing_enable / hdp_b200_timing_read).
-enum KernelId { kNormalize = 1, kThrGeneric = 2, kHotWords = 3, kScan = 4, kUnpackMask = 5, kThrSeg = 6, kThrRanked = 7, kMeasure = 8, kThrCand = 9, kThrNet = 10, kSeam = 11, kIntensity = 12 };
+enum KernelId { kNormalize = 1, kThrGeneric = 2, kHotWords = 3, kScan = 4, kUnpackMask = 5, kThrSeg = 6, kThrRanked = 7, kMeasure = 8, kThrCand = 9, kThrNet = 10, kSeam = 11, kIntensity = 12, kHotPair = 13 };
 struct KernelTimer {
     bool on;
     cudaStream_t st;
@@ -100,14 +100,23 @@ int thresholds_launch(const float *d_temps, int64_t C, int64_t T_b, int64_t ld_t
                       const double *h_q, int P, double *d_out,
                       void *d_workspace, size_t workspace_bytes, void *stream, int64_t carve_cells, bool tables_resident, int input_unit);
 
-// The whole of hdp_b200_metrics and hdp_b200_intensity (metric.cu): k_hot_words, then k_scan on its hot words when d_out is given
-// (u16 [4, P, D, Y, C]) and k_intensity when d_int is given (f32 [3, P, D, Y, C]).  carve_cells / tables_resident as above;
-// input_unit = unit code, OR-ed with HDP_B200_COLD for the cold-spell pass.
+// The second measure of a compound pass (hdp_b200_compound): a day counts only where both measures pass their own thresholds.
+struct SecondMeasure {
+    const float *x = nullptr;       // nullptr: a single-measure pass
+    int64_t ld_t = 0, ld_c = 1;
+    const double *thr = nullptr;    // [C, n_doy, P], the n_doy and P of the first measure's thresholds
+};
+
+// The whole of hdp_b200_metrics, hdp_b200_intensity and hdp_b200_compound (metric.cu): k_hot_words (k_hot_pair when b.x is given),
+// then k_scan on its hot words when d_out is given (u16 [4, P, D, Y, C]) and k_intensity when d_int is given (f32 [3, P, D, Y, C];
+// for a compound pass [2, 3, P, D, Y, C], one block per measure).  carve_cells / tables_resident as above; input_unit = unit code,
+// OR-ed with HDP_B200_COLD for the cold-spell pass.
 int metric_pass(const float *d_measure, int64_t C, int64_t T, int64_t ld_t, int64_t ld_c,
                 const double *d_thr, int n_doy, int P, const int32_t *h_doy_map,
                 const int32_t *h_defs, int D,
                 const int32_t *h_season_north, const int32_t *h_season_south, int Y,
                 const uint8_t *d_is_south, uint16_t *d_out, float *d_int,
-                void *d_workspace, size_t workspace_bytes, void *stream, int64_t carve_cells, bool tables_resident, int input_unit);
+                void *d_workspace, size_t workspace_bytes, void *stream, int64_t carve_cells, bool tables_resident, int input_unit,
+                const SecondMeasure &b = SecondMeasure());
 
 }  // namespace hdp

@@ -153,6 +153,7 @@ struct HostCtx {
     cudaStream_t s_in = nullptr, s_k = nullptr, s_out = nullptr;
     cudaEvent_t in_ready[kSlots] = {}, k_done[kSlots] = {}, out_done[kSlots] = {};
     DeviceBuf x[kSlots], aux[kSlots], south[kSlots], out[kSlots], out_f[kSlots], ws;
+    DeviceBuf x_b[kSlots], aux_b[kSlots];            // the second measure of a compound pass and its thresholds
     PinnedRing ring_in, ring_out;                    // staging for pageable sources / destinations (allocated on first use)
     std::deque<PendingOut> pending;                  // D2H blocks on their way through ring_out
 
@@ -258,7 +259,10 @@ struct HostCtx {
             for (int i = 0; i < kSlots; i++) { cudaEventDestroy(in_ready[i]); cudaEventDestroy(k_done[i]); cudaEventDestroy(out_done[i]); }
             ready = false;
         }
-        for (int i = 0; i < kSlots; i++) { x[i].release(); aux[i].release(); south[i].release(); out[i].release(); out_f[i].release(); }
+        for (int i = 0; i < kSlots; i++) {
+            x[i].release(); aux[i].release(); south[i].release(); out[i].release(); out_f[i].release();
+            x_b[i].release(); aux_b[i].release();
+        }
         ws.release();
         ring_in.release(); ring_out.release();
     }
@@ -320,19 +324,31 @@ using namespace hdp;
     } while (0)
 #define HDP_HOST_CUDA(expr) HDP_HOST_TRY(cuda_status(expr))
 
-// hdp_b200_metrics_host and hdp_b200_intensity_host: metric_pass chunk by chunk; the u16 planes (h_out) and the f32 planes (h_int),
-// whichever are given, go back to the host.
+// The second measure of hdp_b200_compound_host: host samples, thresholds from the host (h_thr) or the device (d_thr).
+struct HostSecond {
+    const float *h = nullptr;       // nullptr: a single-measure pass
+    int64_t ld_t = 0, ld_c = 1;
+    const double *h_thr = nullptr, *d_thr = nullptr;
+};
+
+// hdp_b200_metrics_host, hdp_b200_intensity_host and hdp_b200_compound_host: metric_pass chunk by chunk; the u16 planes (h_out) and
+// the f32 planes (h_int), whichever are given, go back to the host.  With a second measure both measures' cells of a chunk go up
+// together.
 static int metric_pass_host(const float *h_measure, int64_t C, int64_t T, int64_t ld_t, int64_t ld_c,
                             const double *h_thr, const double *d_thr, int n_doy, int P, const int32_t *h_doy_map,
                             const int32_t *h_defs, int D,
                             const int32_t *h_season_north, const int32_t *h_season_south, int Y,
-                            const uint8_t *h_is_south, float *h_int, uint16_t *h_out, int input_unit)
+                            const uint8_t *h_is_south, float *h_int, uint16_t *h_out, int input_unit, const HostSecond &m2 = HostSecond())
 {
     if (C < 0 || T <= 0 || n_doy <= 0 || P <= 0 || D <= 0 || Y < 0 || !h_doy_map) return HDP_B200_ERR_INVALID;
     if (C == 0 || Y == 0) return HDP_B200_OK;
     if (!h_measure || (!h_thr && !d_thr)) return HDP_B200_ERR_INVALID;
     if (ld_t <= 0 || ld_c <= 0) return HDP_B200_ERR_INVALID;
     if (ld_c != 1 && ld_t != 1) return HDP_B200_ERR_UNSUPPORTED;
+    const bool pair = m2.h != nullptr;
+    if (pair && (!m2.h_thr && !m2.d_thr)) return HDP_B200_ERR_INVALID;
+    if (pair && (m2.ld_t <= 0 || m2.ld_c <= 0)) return HDP_B200_ERR_INVALID;
+    if (pair && m2.ld_c != 1 && m2.ld_t != 1) return HDP_B200_ERR_UNSUPPORTED;
     HostCtx *ctx = nullptr;
     int rc = current_ctx(&ctx);
     if (rc) return rc;
@@ -341,15 +357,19 @@ static int metric_pass_host(const float *h_measure, int64_t C, int64_t T, int64_
 
     const size_t thr_per_cell = (size_t)n_doy * P * sizeof(double);
     const size_t rows = (size_t)4 * P * D * Y;                                 // output rows of C cells each
-    const size_t rows_f = (size_t)3 * P * D * Y;
-    const int64_t chunk = pick_chunk(C, (size_t)T * sizeof(float) + thr_per_cell, (size_t)320 << 20);
+    const size_t rows_f = (size_t)(pair ? 6 : 3) * P * D * Y;
+    const int64_t chunk = pick_chunk(C, (pair ? 2 : 1) * ((size_t)T * sizeof(float) + thr_per_cell), (size_t)320 << 20);
     const int64_t dl_t = ld_c == 1 ? chunk : 1, dl_c = ld_c == 1 ? 1 : T;
-    const size_t ws_bytes = h_int ? hdp_b200_intensity_workspace_bytes(chunk, T, dl_t, dl_c, n_doy, P, D, Y, h_doy_map)
-                                  : hdp_b200_metrics_workspace_bytes(chunk, T, dl_t, dl_c, n_doy, P, D, Y, h_doy_map);
+    const int64_t dl_c_b = m2.ld_c == 1 ? 1 : T;
+    const size_t ws_bytes = pair ? hdp_b200_compound_workspace_bytes(chunk, T, dl_c, dl_c_b, n_doy, P, D, Y, h_doy_map)
+                            : h_int ? hdp_b200_intensity_workspace_bytes(chunk, T, dl_t, dl_c, n_doy, P, D, Y, h_doy_map)
+                                    : hdp_b200_metrics_workspace_bytes(chunk, T, dl_t, dl_c, n_doy, P, D, Y, h_doy_map);
     if ((rc = ctx->ws.reserve(ws_bytes))) return rc;
     for (int i = 0; i < kSlots; i++) {
         if ((rc = ctx->x[i].reserve((size_t)chunk * T * sizeof(float)))) return rc;
         if (!d_thr && (rc = ctx->aux[i].reserve((size_t)chunk * thr_per_cell))) return rc;
+        if (pair && (rc = ctx->x_b[i].reserve((size_t)chunk * T * sizeof(float)))) return rc;
+        if (pair && !m2.d_thr && (rc = ctx->aux_b[i].reserve((size_t)chunk * thr_per_cell))) return rc;
         if ((rc = ctx->south[i].reserve((size_t)chunk))) return rc;
         if (h_out && (rc = ctx->out[i].reserve(rows * chunk * sizeof(uint16_t)))) return rc;
         if (h_int && (rc = ctx->out_f[i].reserve(rows_f * chunk * sizeof(float)))) return rc;
@@ -357,6 +377,7 @@ static int metric_pass_host(const float *h_measure, int64_t C, int64_t T, int64_
     const bool page_x = is_pageable(h_measure), page_thr = !d_thr && is_pageable(h_thr), page_out = h_out && is_pageable(h_out);
     const bool page_int = h_int && is_pageable(h_int);
     const bool page_south = h_is_south && is_pageable(h_is_south);
+    const bool page_xb = pair && is_pageable(m2.h), page_thr_b = pair && !m2.d_thr && is_pageable(m2.h_thr);
     int64_t i = 0;
     for (int64_t c0 = 0; c0 < C; c0 += chunk, i++) {
         const int slot = (int)(i % kSlots);
@@ -367,6 +388,15 @@ static int metric_pass_host(const float *h_measure, int64_t C, int64_t T, int64_
         if (!d_thr)                                                            // device-resident thresholds never cross PCIe again
             HDP_HOST_TRY(ctx->h2d((char *)ctx->aux[slot].p, 0, (const char *)(h_thr + (size_t)c0 * n_doy * P), 0, (size_t)nc * thr_per_cell, 1,
                                   page_thr, ctx->s_in));
+        SecondMeasure sb;
+        if (pair) {
+            HDP_HOST_TRY(upload_cells(ctx, m2.h, page_xb, T, m2.ld_t, m2.ld_c, c0, nc, (float *)ctx->x_b[slot].p, &sb.ld_t, &sb.ld_c, ctx->s_in));
+            if (!m2.d_thr)
+                HDP_HOST_TRY(ctx->h2d((char *)ctx->aux_b[slot].p, 0, (const char *)(m2.h_thr + (size_t)c0 * n_doy * P), 0,
+                                      (size_t)nc * thr_per_cell, 1, page_thr_b, ctx->s_in));
+            sb.x = (const float *)ctx->x_b[slot].p;
+            sb.thr = m2.d_thr ? m2.d_thr + (size_t)c0 * n_doy * P : (const double *)ctx->aux_b[slot].p;
+        }
         if (h_is_south)
             HDP_HOST_TRY(ctx->h2d((char *)ctx->south[slot].p, 0, (const char *)(h_is_south + c0), 0, (size_t)nc, 1, page_south, ctx->s_in));
         HDP_HOST_CUDA(cudaEventRecord(ctx->in_ready[slot], ctx->s_in));
@@ -377,7 +407,7 @@ static int metric_pass_host(const float *h_measure, int64_t C, int64_t T, int64_
         const uint8_t *south_chunk = h_is_south ? (const uint8_t *)ctx->south[slot].p : nullptr;
         HDP_HOST_TRY(metric_pass((const float *)ctx->x[slot].p, nc, T, a, b, thr_chunk, n_doy, P, h_doy_map, h_defs, D,
                                  h_season_north, h_season_south, Y, south_chunk, h_out ? (uint16_t *)ctx->out[slot].p : nullptr,
-                                 h_int ? (float *)ctx->out_f[slot].p : nullptr, ctx->ws.p, ws_bytes, ctx->s_k, chunk, i > 0, input_unit));
+                                 h_int ? (float *)ctx->out_f[slot].p : nullptr, ctx->ws.p, ws_bytes, ctx->s_k, chunk, i > 0, input_unit, sb));
         HDP_HOST_CUDA(cudaEventRecord(ctx->k_done[slot], ctx->s_k));
 
         // device chunk is [rows, nc]; host array is [rows, C]
@@ -475,6 +505,20 @@ int hdp_b200_intensity_host(const float *h_measure, int64_t C, int64_t T, int64_
     if (!h_int && C > 0 && Y > 0) return HDP_B200_ERR_INVALID;
     return metric_pass_host(h_measure, C, T, ld_t, ld_c, h_thr, d_thr, n_doy, P, h_doy_map, h_defs, D, h_season_north, h_season_south, Y,
                             h_is_south, h_int, h_out, input_unit);
+}
+
+int hdp_b200_compound_host(const float *h_a, int64_t ld_t_a, int64_t ld_c_a, const float *h_b, int64_t ld_t_b, int64_t ld_c_b,
+                           int64_t C, int64_t T, const double *h_thr_a, const double *d_thr_a, const double *h_thr_b, const double *d_thr_b,
+                           int n_doy, int P, const int32_t *h_doy_map, const int32_t *h_defs, int D,
+                           const int32_t *h_season_north, const int32_t *h_season_south, int Y,
+                           const uint8_t *h_is_south, uint16_t *h_out, float *h_int, int input_unit)
+{
+    if (C > 0 && Y > 0 && !h_out && !h_int) return HDP_B200_ERR_INVALID;
+    if (C > 0 && !h_b) return HDP_B200_ERR_INVALID;
+    HostSecond b;
+    b.h = h_b; b.ld_t = ld_t_b; b.ld_c = ld_c_b; b.h_thr = h_thr_b; b.d_thr = d_thr_b;
+    return metric_pass_host(h_a, C, T, ld_t_a, ld_c_a, h_thr_a, d_thr_a, n_doy, P, h_doy_map, h_defs, D, h_season_north, h_season_south, Y,
+                            h_is_south, h_int, h_out, input_unit, b);
 }
 
 }  // extern "C"

@@ -117,7 +117,7 @@ k_intensity(const uint32_t *__restrict__ hot, const float *__restrict__ x, int64
     while (L.open()) { flush(); L.next(); }
 }
 
-int run_intensity(const Layout &L, const WordPlan &plan, const float *d_measure, int64_t C, int64_t T, int64_t ld_t, int64_t ld_c,
+int run_intensity(const Layout &L, const WordPlan &plan, const float *x, int64_t x_ld_t, int64_t C, int64_t T,
                   const double *d_thr, int n_doy, int P, const int32_t *h_defs, int D, const std::vector<int32_t> &seasons, int Y,
                   const uint8_t *d_is_south, float *d_int, cudaStream_t st, bool tables_resident, int unit, bool cold)
 {
@@ -131,8 +131,6 @@ int run_intensity(const Layout &L, const WordPlan &plan, const float *d_measure,
     for (int i = 0; i < 3 * HDP_B200_MAX_DEFINITIONS; i++) defs.v[i] = i < 3 * D ? h_defs[i] : 0;
     if (!tables_resident)
         HDP_CUDA_TRY(cudaMemcpyAsync(L.int_seasons, seasons.data(), sizeof(int32_t) * seasons.size(), cudaMemcpyHostToDevice, st));
-    const float *x = ld_c != 1 ? L.xn : d_measure;                  // run_hot_words normalised other layouts into L.xn
-    const int64_t x_ld_t = ld_c != 1 ? C : ld_t;
     const int64_t n_warps = ((C + 31) / 32) * P;
     const unsigned grid = (unsigned)((n_warps + wpc - 1) / wpc);
     KernelTimer timer(kIntensity, st);

@@ -33,24 +33,7 @@ namespace hdp {
 // ----------------------------------------------------------------------------------------------------
 // k_hot_words
 // ----------------------------------------------------------------------------------------------------
-constexpr int kTileCells = 32;
-constexpr int kTileDoy = 32;
-constexpr int kHotYears = 2;  // words (years) a warp compares against one register copy of the day's thresholds
-constexpr int kFillLoads = 5;  // doubles of the threshold tile a lane has in flight
-constexpr int kHotDays = 16;  // days of each of them whose samples are in flight together
-constexpr int kTilePad = 33;   // [.. ][33]: conflict-free both for the e-major fill and the lane-major reads
-
-// m |= bit where v > t (false when either side is NaN): one compare and one predicated OR with an immediate
-__device__ __forceinline__ void or_if_gt(uint32_t &m, float v, float t, uint32_t bit)
-{
-    asm("{\n\t.reg .pred p;\n\tsetp.gt.f32 p, %1, %2;\n\t@p or.b32 %0, %0, %3;\n\t}" : "+r"(m) : "f"(v), "f"(t), "r"(bit));
-}
-
-// the same with v < t: the cold-day bits of a cold-spell pass
-__device__ __forceinline__ void or_if_lt(uint32_t &m, float v, float t, uint32_t bit)
-{
-    asm("{\n\t.reg .pred p;\n\tsetp.lt.f32 p, %1, %2;\n\t@p or.b32 %0, %0, %3;\n\t}" : "+r"(m) : "f"(v), "f"(t), "r"(bit));
-}
+constexpr int kHotDays = 16;  // days of each of kHotYears words whose samples are in flight together
 
 template <int PG, int J0, int UNIT, bool COLD>
 __device__ __forceinline__ void hot_half(uint32_t (&m)[kHotYears][PG], const float *const (&xp)[kHotYears], const int (&jo)[kHotYears],
@@ -619,7 +602,7 @@ static int replicate_rows(const double *thr, int64_t C, int P, double *rep, cuda
     return HDP_B200_OK;
 }
 
-static int pick_pg(int P)
+int pick_pg(int P)
 {
     const int cand[] = {4, 8, 10, 16, 20};
     int best = 4, best_waste = INT_MAX;
@@ -630,8 +613,10 @@ static int pick_pg(int P)
     return best;
 }
 
-// Workspace layout; `intensity` appends the intensity pass's season tables behind what the metric pass uses.
-static Layout carve(void *ws, size_t ws_bytes, int64_t C, int64_t T, bool need_norm, int64_t K, int n_doy, int P, int Y, bool intensity)
+// Workspace layout; `intensity` appends the intensity pass's season tables behind what the metric pass uses, `pair` the second
+// measure's normalised copy (need_norm_b) and replicated thresholds of a compound pass.
+static Layout carve(void *ws, size_t ws_bytes, int64_t C, int64_t T, bool need_norm, int64_t K, int n_doy, int P, int Y, bool intensity,
+                    bool pair = false, bool need_norm_b = false)
 {
     Layout L;
     Carver cv(ws, ws_bytes);
@@ -644,6 +629,8 @@ static Layout carve(void *ws, size_t ws_bytes, int64_t C, int64_t T, bool need_n
     L.hot = cv.take<uint32_t>((size_t)P * K * C);
     if (intensity) L.int_seasons = cv.take<int4>((size_t)2 * (Y + 1));
     if (n_doy == 1) L.thr_rep = cv.take<double>((size_t)C * kTileDoy * P);
+    if (pair && need_norm_b) L.xn_b = cv.take<float>((size_t)C * T);
+    if (pair && n_doy == 1) L.thr_rep_b = cv.take<double>((size_t)C * kTileDoy * P);
     L.total = cv.off;
     return L;
 }
@@ -653,20 +640,24 @@ static bool bad_dims(int64_t C, int64_t T, int n_doy, int P)
     return C < 0 || T < 0 || n_doy <= 0 || P <= 0 || T > 0x3fffffff;
 }
 
-size_t metric_pass_workspace_bytes(int64_t C, int64_t T, int64_t ld_c, int n_doy, int P, int Y, const int32_t *h_doy_map, bool intensity)
+size_t metric_pass_workspace_bytes(int64_t C, int64_t T, int64_t ld_c, int n_doy, int P, int Y, const int32_t *h_doy_map, bool intensity,
+                                   bool pair, int64_t ld_c_b)
 {
     if (bad_dims(C, T, n_doy, P) || Y < 0) return 0;
     const int64_t K = n_doy == 1 ? (T + kTileDoy - 1) / kTileDoy : h_doy_map ? count_words(h_doy_map, T) : words_upper_bound(T, n_doy);
-    return carve(nullptr, 0, C, T, ld_c != 1, K, n_doy, P, Y, intensity).total;
+    return carve(nullptr, 0, C, T, ld_c != 1, K, n_doy, P, Y, intensity, pair, ld_c_b != 1).total;
 }
 
 // Runs k_hot_words (after the layout-normalising copy when ld_c != 1: the samples then live in L.xn, time-major, ld_t = C);
-// on success plan / L describe what lives in the workspace, and L.thr / L.n_doy the thresholds the kernels read.  `unit` is a
-// plain unit code (0 - 2); `cold` makes the words cold-day bits.
+// on success plan / L describe what lives in the workspace, L.thr / L.n_doy the thresholds and L.x / L.ld_t the samples the
+// kernels read.  `unit` is a plain unit code (0 - 2); `cold` makes the words cold-day bits.  With a second measure (b.x) it
+// prepares that one the same way (L.x_b, L.thr_b) and runs k_hot_pair instead: the words then mark the days on which both
+// measures pass their thresholds.
 static int run_hot_words(const float *d_measure, int64_t C, int64_t T, int64_t ld_t, int64_t ld_c,
                          const double *d_thr, int n_doy, int P, const int32_t *h_doy_map,
                          int Y, void *ws, size_t ws_bytes, cudaStream_t st, WordPlan &plan, Layout &L,
-                         int64_t carve_cells = 0, bool tables_resident = false, int unit = 0, bool intensity = false, bool cold = false)
+                         int64_t carve_cells = 0, bool tables_resident = false, int unit = 0, bool intensity = false, bool cold = false,
+                         const SecondMeasure &b = SecondMeasure())
 {
     if (unit < 0 || unit > 2) return HDP_B200_ERR_INVALID;
     std::vector<int32_t> own_map;
@@ -676,11 +667,16 @@ static int run_hot_words(const float *d_measure, int64_t C, int64_t T, int64_t l
     rc = build_words(doy_map, T, pass_n_doy(n_doy), plan);
     if (rc != HDP_B200_OK) return rc;
     const int K = (int)plan.words.size();
-    const bool need_norm = ld_c != 1;
-    L = carve(ws, ws_bytes, std::max(C, carve_cells), T, need_norm, K, n_doy, P, Y, intensity);
+    const bool need_norm = ld_c != 1, pair = b.x != nullptr;
+    L = carve(ws, ws_bytes, std::max(C, carve_cells), T, need_norm, K, n_doy, P, Y, intensity, pair, b.ld_c != 1);
     if (ws == nullptr || L.total > ws_bytes) return HDP_B200_ERR_WORKSPACE;
     L.thr = d_thr;
     L.n_doy = pass_n_doy(n_doy);
+    L.x = d_measure;
+    L.ld_t = ld_t;
+    L.thr_b = b.thr;
+    L.x_b = b.x;
+    L.ld_t_b = b.ld_t;
     if (C == 0 || T == 0) return HDP_B200_OK;
     if (L.thr_rep) {
         rc = replicate_rows(d_thr, C, P, L.thr_rep, st);
@@ -694,9 +690,23 @@ static int run_hot_words(const float *d_measure, int64_t C, int64_t T, int64_t l
         x = L.xn;
         ld_t = C;
     }
+    L.x = x;
+    L.ld_t = ld_t;
+    if (pair && L.thr_rep_b) {
+        rc = replicate_rows(b.thr, C, P, L.thr_rep_b, st);
+        if (rc != HDP_B200_OK) return rc;
+        L.thr_b = L.thr_rep_b;
+    }
+    if (pair && L.xn_b) {
+        rc = normalize_layout(b.x, C, T, b.ld_t, b.ld_c, L.xn_b, st);
+        if (rc != HDP_B200_OK) return rc;
+        L.x_b = L.xn_b;
+        L.ld_t_b = C;
+    }
     if (!tables_resident) HDP_CUDA_TRY(cudaMemcpyAsync(L.words, plan.words.data(), sizeof(int4) * K, cudaMemcpyHostToDevice, st));
     if (!tables_resident) HDP_CUDA_TRY(cudaMemcpyAsync(L.blk_start, plan.blk_start.data(), sizeof(int) * plan.blk_start.size(), cudaMemcpyHostToDevice, st));
     if (!tables_resident) HDP_CUDA_TRY(cudaMemcpyAsync(L.blk_words, plan.blk_words.data(), sizeof(int) * K, cudaMemcpyHostToDevice, st));
+    if (pair) return run_hot_pair(L, plan, C, P, st, unit, cold);
 
     const int pg = pick_pg(P);
     const int Ppad = (P + pg - 1) / pg * pg;
@@ -901,11 +911,12 @@ int metric_pass(const float *d_measure, int64_t C, int64_t T, int64_t ld_t, int6
                 const int32_t *h_defs, int D,
                 const int32_t *h_season_north, const int32_t *h_season_south, int Y,
                 const uint8_t *d_is_south, uint16_t *d_out, float *d_int,
-                void *d_workspace, size_t workspace_bytes, void *stream, int64_t carve_cells, bool tables_resident, int input_unit)
+                void *d_workspace, size_t workspace_bytes, void *stream, int64_t carve_cells, bool tables_resident, int input_unit,
+                const SecondMeasure &b)
 {
     if (bad_dims(C, T, n_doy, P) || D <= 0 || Y < 0) return HDP_B200_ERR_INVALID;
     if ((T > 0 && !h_doy_map) || !h_defs || (Y > 0 && (!h_season_north || !h_season_south))) return HDP_B200_ERR_INVALID;
-    if (C > 0 && T > 0 && (!d_measure || !d_thr)) return HDP_B200_ERR_INVALID;
+    if (C > 0 && T > 0 && (!d_measure || !d_thr || (b.x && !b.thr))) return HDP_B200_ERR_INVALID;
     if (P > HDP_B200_MAX_PERCENTILES || D > HDP_B200_MAX_DEFINITIONS) return HDP_B200_ERR_UNSUPPORTED;
     cudaStream_t st = (cudaStream_t)stream;
     // input_unit of the C ABI = unit code | HDP_B200_COLD; the kernels' launchers see the two as plain values
@@ -928,16 +939,42 @@ int metric_pass(const float *d_measure, int64_t C, int64_t T, int64_t ld_t, int6
     WordPlan plan;
     Layout L;
     int rc = run_hot_words(d_measure, C, T, ld_t, ld_c, d_thr, n_doy, P, h_doy_map, Y, d_workspace, workspace_bytes, st, plan, L,
-                           carve_cells, tables_resident, unit, d_int != nullptr, cold);
+                           carve_cells, tables_resident, unit, d_int != nullptr, cold, b);
     if (rc != HDP_B200_OK || C == 0 || Y == 0) return rc;
     if (d_out) {
         rc = run_scan(L, plan, C, T, P, h_defs, D, passes, Y, d_is_south, d_out, st, tables_resident);
         if (rc != HDP_B200_OK) return rc;
     }
     if (d_int)
-        rc = run_intensity(L, plan, d_measure, C, T, ld_t, ld_c, L.thr, L.n_doy, P, h_defs, D, seasons, Y, d_is_south, d_int, st,
+        rc = run_intensity(L, plan, L.x, L.ld_t, C, T, L.thr, L.n_doy, P, h_defs, D, seasons, Y, d_is_south, d_int, st,
                            tables_resident, unit, cold);
+    if (d_int && b.x && rc == HDP_B200_OK)                                  // the second measure's block, on the same words
+        rc = run_intensity(L, plan, L.x_b, L.ld_t_b, C, T, L.thr_b, L.n_doy, P, h_defs, D, seasons, Y, d_is_south,
+                           d_int + (size_t)3 * P * D * Y * C, st, true, unit, cold);
     return rc;
+}
+
+// hdp_b200_hot_days and hdp_b200_compound_hot_days: the hot words, unpacked to u8 [P, T, C]
+static int hot_days_pass(const float *d_measure, int64_t C, int64_t T, int64_t ld_t, int64_t ld_c,
+                         const double *d_thr, int n_doy, int P, const int32_t *h_doy_map,
+                         uint8_t *d_mask, void *d_workspace, size_t workspace_bytes, void *stream, int unit, bool cold, const SecondMeasure &b)
+{
+    if (bad_dims(C, T, n_doy, P) || !h_doy_map && T > 0) return HDP_B200_ERR_INVALID;
+    if (C > 0 && T > 0 && (!d_measure || !d_thr || !d_mask || (b.x && !b.thr))) return HDP_B200_ERR_INVALID;
+    if (P > HDP_B200_MAX_PERCENTILES) return HDP_B200_ERR_UNSUPPORTED;
+    cudaStream_t st = (cudaStream_t)stream;
+    WordPlan plan;
+    Layout L;
+    int rc = run_hot_words(d_measure, C, T, ld_t, ld_c, d_thr, n_doy, P, h_doy_map, 0, d_workspace, workspace_bytes, st, plan, L,
+                           0, false, unit, false, cold, b);
+    if (rc != HDP_B200_OK || C == 0 || T == 0) return rc;
+    const int K = (int)plan.words.size();
+    dim3 grid((unsigned)((C + 255) / 256), (unsigned)K);
+    if (K > 65535) return HDP_B200_ERR_UNSUPPORTED;
+    KernelTimer timer(kUnpackMask, st);
+    k_unpack_mask<<<grid, 256, 0, st>>>(L.hot, C, T, P, K, L.words, d_mask);
+    HDP_LAUNCH_CHECK();
+    return HDP_B200_OK;
 }
 
 }  // namespace hdp
@@ -980,21 +1017,20 @@ int hdp_b200_hot_days(const float *d_measure, int64_t C, int64_t T, int64_t ld_t
                       const double *d_thr, int n_doy, int P, const int32_t *h_doy_map,
                       uint8_t *d_mask, void *d_workspace, size_t workspace_bytes, void *stream)
 {
-    if (bad_dims(C, T, n_doy, P) || !h_doy_map && T > 0) return HDP_B200_ERR_INVALID;
-    if (C > 0 && T > 0 && (!d_measure || !d_thr || !d_mask)) return HDP_B200_ERR_INVALID;
-    if (P > HDP_B200_MAX_PERCENTILES) return HDP_B200_ERR_UNSUPPORTED;
-    cudaStream_t st = (cudaStream_t)stream;
-    WordPlan plan;
-    Layout L;
-    int rc = run_hot_words(d_measure, C, T, ld_t, ld_c, d_thr, n_doy, P, h_doy_map, 0, d_workspace, workspace_bytes, st, plan, L);
-    if (rc != HDP_B200_OK || C == 0 || T == 0) return rc;
-    const int K = (int)plan.words.size();
-    dim3 grid((unsigned)((C + 255) / 256), (unsigned)K);
-    if (K > 65535) return HDP_B200_ERR_UNSUPPORTED;
-    KernelTimer timer(kUnpackMask, st);
-    k_unpack_mask<<<grid, 256, 0, st>>>(L.hot, C, T, P, K, L.words, d_mask);
-    HDP_LAUNCH_CHECK();
-    return HDP_B200_OK;
+    return hot_days_pass(d_measure, C, T, ld_t, ld_c, d_thr, n_doy, P, h_doy_map, d_mask, d_workspace, workspace_bytes, stream, 0, false,
+                         SecondMeasure());
+}
+
+int hdp_b200_compound_hot_days(const float *d_a, int64_t ld_t_a, int64_t ld_c_a, const float *d_b, int64_t ld_t_b, int64_t ld_c_b,
+                               int64_t C, int64_t T, const double *d_thr_a, const double *d_thr_b, int n_doy, int P,
+                               const int32_t *h_doy_map, uint8_t *d_mask, void *d_workspace, size_t workspace_bytes, void *stream,
+                               int input_unit)
+{
+    if (C > 0 && T > 0 && !d_b) return HDP_B200_ERR_INVALID;
+    SecondMeasure b;
+    b.x = d_b; b.ld_t = ld_t_b; b.ld_c = ld_c_b; b.thr = d_thr_b;
+    return hot_days_pass(d_a, C, T, ld_t_a, ld_c_a, d_thr_a, n_doy, P, h_doy_map, d_mask, d_workspace, workspace_bytes, stream,
+                         input_unit & ~HDP_B200_COLD, (input_unit & HDP_B200_COLD) != 0, b);
 }
 
 int hdp_b200_metrics(const float *d_measure, int64_t C, int64_t T, int64_t ld_t, int64_t ld_c,

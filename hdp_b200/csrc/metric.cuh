@@ -8,6 +8,27 @@
 
 namespace hdp {
 
+// The hot-word tiles of k_hot_words (metric.cu) and k_hot_pair (compound.cu)
+constexpr int kTileCells = 32;
+constexpr int kTileDoy = 32;
+constexpr int kHotYears = 2;  // words (years) a warp compares against one register copy of the day's thresholds
+constexpr int kFillLoads = 5;  // doubles of the threshold tile a lane has in flight
+constexpr int kTilePad = 33;   // [.. ][33]: conflict-free both for the e-major fill and the lane-major reads
+
+#ifdef __CUDACC__
+// m |= bit where v > t (false when either side is NaN): one compare and one predicated OR with an immediate
+__device__ __forceinline__ void or_if_gt(uint32_t &m, float v, float t, uint32_t bit)
+{
+    asm("{\n\t.reg .pred p;\n\tsetp.gt.f32 p, %1, %2;\n\t@p or.b32 %0, %0, %3;\n\t}" : "+r"(m) : "f"(v), "f"(t), "r"(bit));
+}
+
+// the same with v < t: the cold-day bits of a cold-spell pass
+__device__ __forceinline__ void or_if_lt(uint32_t &m, float v, float t, uint32_t bit)
+{
+    asm("{\n\t.reg .pred p;\n\tsetp.lt.f32 p, %1, %2;\n\t@p or.b32 %0, %0, %3;\n\t}" : "+r"(m) : "f"(v), "f"(t), "r"(bit));
+}
+#endif
+
 struct WordPlan {
     std::vector<int4> words;        // {t0, nbits, doy of bit 0, 0}
     std::vector<int> blk_start;     // [n_blk + 1]
@@ -27,15 +48,36 @@ struct Layout {
     double *thr_rep = nullptr;      // n_doy = 1 only: the thresholds replicated to kTileDoy rows (metric.cu, pass_n_doy)
     const double *thr = nullptr;    // the thresholds the kernels read, [C, n_doy, P]: the caller's, or thr_rep
     int n_doy = 0;
+    const float *x = nullptr;       // the samples the kernels read, cell-contiguous, ld_t apart: the caller's, or xn
+    int64_t ld_t = 0;
+    // compound pass only (compound.cu): the same for the second measure
+    float *xn_b = nullptr;
+    double *thr_rep_b = nullptr;
+    const double *thr_b = nullptr;
+    const float *x_b = nullptr;
+    int64_t ld_t_b = 0;
 };
 
-// Workspace of metric_pass; `intensity` appends the intensity pass's season tables behind what the metric pass uses.
-size_t metric_pass_workspace_bytes(int64_t C, int64_t T, int64_t ld_c, int n_doy, int P, int Y, const int32_t *h_doy_map, bool intensity);
+// Workspace of metric_pass; `intensity` appends the intensity pass's season tables behind what the metric pass uses.  `pair`: a
+// compound pass, whose second measure has stride ld_c_b.
+size_t metric_pass_workspace_bytes(int64_t C, int64_t T, int64_t ld_c, int n_doy, int P, int Y, const int32_t *h_doy_map, bool intensity,
+                                   bool pair = false, int64_t ld_c_b = 1);
 
-// k_intensity over the hot words in L: the intensity metrics f32 [3, P, D, Y, C].  `seasons` i32 [2, Y + 1, 4]: the season tables
-// of both hemispheres as intensity_season_table (intensity.h) accepts them.  `unit`: a plain unit code (0 - 2); `cold`: the words
-// are cold-day bits and the intensity is the deficit below the threshold.
-int run_intensity(const Layout &L, const WordPlan &plan, const float *d_measure, int64_t C, int64_t T, int64_t ld_t, int64_t ld_c,
+// pick_pg: the percentiles per group of the hot-word kernels (PG of k_hot_words and k_hot_pair) for P percentiles
+int pick_pg(int P);
+
+// k_hot_pair (compound.cu): percentile groups per CTA, CTAs per (cells, day-of-year block) and shared-memory bytes per CTA for P
+// percentiles; false when P is outside 1 .. HDP_B200_MAX_PERCENTILES
+bool hot_pair_plan(int P, int &pg, int &slices, int &groups_per_slice, size_t &smem);
+
+// k_hot_pair over the samples and thresholds in L (L.x / L.thr and L.x_b / L.thr_b): the compound hot-day words in L.hot
+int run_hot_pair(const Layout &L, const WordPlan &plan, int64_t C, int P, cudaStream_t st, int unit, bool cold);
+
+// k_intensity over the hot words in L: the intensity metrics f32 [3, P, D, Y, C] of the samples x (cell-contiguous, x_ld_t apart)
+// against d_thr.  `seasons` i32 [2, Y + 1, 4]: the season tables of both hemispheres as intensity_season_table (intensity.h)
+// accepts them.  `unit`: a plain unit code (0 - 2); `cold`: the words are cold-day bits and the intensity is the deficit below
+// the threshold.
+int run_intensity(const Layout &L, const WordPlan &plan, const float *x, int64_t x_ld_t, int64_t C, int64_t T,
                   const double *d_thr, int n_doy, int P, const int32_t *h_defs, int D, const std::vector<int32_t> &seasons, int Y,
                   const uint8_t *d_is_south, float *d_int, cudaStream_t st, bool tables_resident, int unit, bool cold);
 

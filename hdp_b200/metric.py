@@ -196,19 +196,8 @@ def _widen_int64(a: np.ndarray) -> np.ndarray:
     return out
 
 
-def _metric_sweep(measure, threshold, hw_definitions, time_axis, doy_map=None, intensity=False, cold=False):
-    """The percentile x definition x cell sweep of compute_heatwave_metrics_wrapper (metric.py:344-369) as ONE library call:
-    -> ((uint16 [4, P, D, Y, C], float32 [3, P, D, Y, C] or None), season tables, cell dims, cell shape, P, D).  With
-    ``intensity`` the call is the intensity pass, which also returns the intensity metrics.  With ``cold`` it is the cold-spell
-    pass, and each hemisphere's season is the other one's heatwave season (north Nov 1 - Apr 1, south May 1 - Oct 1)."""
-    st = _tables.hemisphere_ranges(time_axis)                       # compute_hemisphere_ranges, :410
-    north, south_tab = (st.south, st.north) if cold else (st.north, st.south)
-    if doy_map is None:
-        doy_map = _tables.doy_map(time_axis.dayofyr)                # build_doy_map, :413
-    x, cell_dims, cell_shape = _layout.to_time_cells(xr.values_of(measure), tuple(measure.dims), require_float32=True)
-    south = _tables.is_south(_layout.cell_latitudes(xr.coord_values(measure, "lat"), cell_dims, cell_shape))
-
-    # thresholds [<cells in the measure's order>, doy, percentile] -> [C, n_doy, P]; exact coordinate join like apply_ufunc
+def _threshold_cdp(threshold, measure, cell_dims):
+    """thresholds [<cells in the measure's order>, doy, percentile] -> [C, n_doy, P]; exact coordinate join like apply_ufunc"""
     thr_dims = tuple(threshold.dims)
     want = [*cell_dims, "doy", "percentile"]
     if sorted(thr_dims) != sorted(want):
@@ -218,9 +207,39 @@ def _metric_sweep(measure, threshold, hw_definitions, time_axis, doy_map=None, i
             raise ValueError(f"cannot align measure and threshold exactly along '{d}'")
     thr_vals = np.transpose(xr.values_of(threshold), [thr_dims.index(d) for d in want]).astype(np.float64, copy=False)
     n_doy, P = thr_vals.shape[-2], thr_vals.shape[-1]
-    thr_cdp = np.ascontiguousarray(thr_vals).reshape(-1, n_doy, P)
+    return np.ascontiguousarray(thr_vals).reshape(-1, n_doy, P)
+
+
+def _metric_sweep(measure, threshold, hw_definitions, time_axis, doy_map=None, intensity=False, cold=False, second=None):
+    """The percentile x definition x cell sweep of compute_heatwave_metrics_wrapper (metric.py:344-369) as ONE library call:
+    -> ((uint16 [4, P, D, Y, C], float32 [3, P, D, Y, C] or None), season tables, cell dims, cell shape, P, D).  With
+    ``intensity`` the call is the intensity pass, which also returns the intensity metrics.  With ``cold`` it is the cold-spell
+    pass, and each hemisphere's season is the other one's heatwave season (north Nov 1 - Apr 1, south May 1 - Oct 1).
+    ``second``: (measure B, threshold B) of a compound pass (:func:`compute_compound_metrics`), whose intensity output is float32
+    [2, 3, P, D, Y, C]."""
+    st = _tables.hemisphere_ranges(time_axis)                       # compute_hemisphere_ranges, :410
+    north, south_tab = (st.south, st.north) if cold else (st.north, st.south)
+    if doy_map is None:
+        doy_map = _tables.doy_map(time_axis.dayofyr)                # build_doy_map, :413
+    x, cell_dims, cell_shape = _layout.to_time_cells(xr.values_of(measure), tuple(measure.dims), require_float32=True)
+    south = _tables.is_south(_layout.cell_latitudes(xr.coord_values(measure, "lat"), cell_dims, cell_shape))
+    thr_cdp = _threshold_cdp(threshold, measure, cell_dims)
+    n_doy, P = thr_cdp.shape[1], thr_cdp.shape[2]
 
     defs = np.asarray(hw_definitions, dtype=np.int64).reshape(-1, 3)
+    if second is not None:
+        measure_b, threshold_b = second
+        x_b, cell_dims_b, _ = _layout.to_time_cells(xr.values_of(measure_b), tuple(measure_b.dims), require_float32=True)
+        if cell_dims_b != cell_dims or x_b.shape != x.shape:
+            raise ValueError("the two measures must have the same dims and shape")
+        thr_b = _threshold_cdp(threshold_b, measure, cell_dims)
+        args = (x, thr_cdp, x_b, thr_b, doy_map, defs, north, south_tab, south)
+        if intensity:
+            out = np.empty((4, P, defs.shape[0], st.n_years, x.shape[1]), np.uint16)
+            heat = _core.compound_intensity_host(*args, metrics_out=out, cold=cold)          # f32 [2, 3, P, D, Y, C]
+        else:
+            out, heat = _core.compound_metrics_host(*args, cold=cold), None
+        return (out, heat), st, cell_dims, cell_shape, P, defs.shape[0]
     if intensity:
         out = np.empty((4, P, defs.shape[0], st.n_years, x.shape[1]), np.uint16)
         heat = _core.intensity_host(x, thr_cdp, doy_map, defs, north, south_tab, south, metrics_out=out, cold=cold)   # f32 [3, P, D, Y, C]
@@ -307,6 +326,99 @@ def compute_individual_metrics(measure, threshold, hw_definitions: list, include
     for variable in ds:
         ds[variable].attrs["history"] = combined_history
         add_history(ds[variable], f"Heatwave metrics generated by HDP v{get_version()}")
+    return ds
+
+
+COMPOUND_LONG_NAMES = {"HWF": "Compound Heatwave Frequency", "HWN": "Compound Heatwave Number", "HWD": "Compound Heatwave Duration",
+                       "HWA": "Compound Heatwave Average", "HWC": "Compound Heatwave Cumulative Intensity",
+                       "HWI": "Compound Heatwave Mean Intensity", "HWP": "Compound Heatwave Peak Intensity",
+                       "CSF": "Compound Cold Spell Frequency", "CSN": "Compound Cold Spell Number", "CSD": "Compound Cold Spell Duration",
+                       "CSA": "Compound Cold Spell Average", "CSC": "Compound Cold Spell Cumulative Intensity",
+                       "CSI": "Compound Cold Spell Mean Intensity", "CSP": "Compound Cold Spell Peak Intensity"}
+
+
+def _measure_name(measure, fallback):
+    return str(getattr(measure, "name", None) or measure.attrs.get("baseline_variable") or fallback)
+
+
+def compute_compound_metrics(measure_a, threshold_a, measure_b, threshold_b, hw_definitions: list, check_variables: bool = True, *,
+                             intensity: bool = False, cold: bool = False):
+    """Compound (day-night) heatwaves: the metrics of :func:`compute_individual_metrics` over the days on which BOTH measures exceed
+    their own thresholds (e.g. tmax and tmin: hot days and hot nights), percentile p of ``threshold_a`` paired with percentile p of
+    ``threshold_b``.  The measures must have the same cell dims, coordinates and time axis, the thresholds identical
+    ``percentile`` coordinates and the same day-of-year axis length; else ``ValueError``.
+
+    Returns HWF, HWN, HWD, HWA with the dims and coords of :func:`compute_individual_metrics`; with ``intensity`` also HWC, HWI and
+    HWP with a leading ``measure`` dim (coordinate ``[<a>, <b>]``): each measure's exceedance over the compound heatwave days.
+    ``cold=True``: days on which both are below their thresholds (CSF ... CSP, the deficits), in the cold season."""
+    time_axis = time_axis_of(measure_a)
+    time_b = time_axis_of(measure_b)
+    if time_axis.calendar != time_b.calendar or any(
+            not np.array_equal(getattr(time_axis, f), getattr(time_b, f)) for f in ("year", "month", "day", "dayofyr")):
+        raise ValueError("measure_a and measure_b must have the same time axis")
+    if tuple(measure_a.dims) != tuple(measure_b.dims):
+        raise ValueError(f"measure dims {tuple(measure_a.dims)} and {tuple(measure_b.dims)} differ")
+    for d in measure_a.dims:
+        if d != "time" and not np.array_equal(np.asarray(xr.coord_values(measure_a, d)), np.asarray(xr.coord_values(measure_b, d))):
+            raise ValueError(f"measure_a and measure_b differ along '{d}'")
+    pa, pb = np.asarray(xr.coord_values(threshold_a, "percentile")), np.asarray(xr.coord_values(threshold_b, "percentile"))
+    if pa.shape != pb.shape or not np.array_equal(pa, pb):
+        raise ValueError("threshold_a and threshold_b must have identical percentile coordinates")
+    if threshold_a.shape[tuple(threshold_a.dims).index("doy")] != threshold_b.shape[tuple(threshold_b.dims).index("doy")]:
+        raise ValueError("threshold_a and threshold_b must have the same number of days of year")
+    if check_variables:                                             # as compute_individual_metrics, each pair on its own
+        for m, t in ((measure_a, threshold_a), (measure_b, threshold_b)):
+            assert "hdp_type" in t.attrs
+            assert t.attrs["hdp_type"] == "threshold"
+            assert t.attrs["baseline_variable"] == m.attrs["baseline_variable"]
+            assert t.attrs["baseline_calendar"] == time_axis.calendar
+
+    (out, heat), st, cell_dims, cell_shape, P, D = _metric_sweep(measure_a, threshold_a, hw_definitions, time_axis, intensity=intensity,
+                                                                 cold=cold, second=(measure_b, threshold_b))
+    metric_names = _core.COLD_METRIC_NAMES if cold else _core.METRIC_NAMES
+    intensity_names = _core.COLD_INTENSITY_NAMES if cold else _core.INTENSITY_NAMES
+    Y = st.n_years
+    name_a, name_b = _measure_name(measure_a, "measure_a"), _measure_name(measure_b, "measure_b")
+
+    coords = dict(xr.non_time_coords(measure_a))
+    coords["definition"] = [f"{hw_def[0]}-{hw_def[1]}-{hw_def[2]}" for hw_def in hw_definitions]
+    coords["percentile"] = pa
+    coords["time"] = _year_times(st.years, time_axis.calendar)
+    dims = ["percentile", "definition", *cell_dims, "time"]
+    data_vars = {}
+    for i, name in enumerate(metric_names):
+        wide = out[i] if np.dtype(METRIC_DTYPE) == np.uint16 else _widen_int64(out[i]).astype(METRIC_DTYPE, copy=False)
+        data_vars[name] = xr.DataArray(wide.transpose(0, 1, 3, 2).reshape(P, D, *cell_shape, Y), dims=dims, coords=coords)
+    if intensity:
+        coords_m = {**coords, "measure": [name_a, name_b]}
+        for i, name in enumerate(intensity_names):                  # float32 [2, P, D, Y, C]
+            data_vars[name] = xr.DataArray(heat[:, i].transpose(0, 1, 2, 4, 3).reshape(2, P, D, *cell_shape, Y), dims=["measure", *dims],
+                                           coords=coords_m)
+    ds = xr.Dataset(data_vars)
+    kind = "Compound cold spell" if cold else "Compound heatwave"
+    ds.attrs.update({
+        "description": f"{kind} metric dataset generated by Heatwave Diagnostics Package (HDP v{get_version()})",
+        "hdp_version": get_version(),
+        "hdp_type": "metric",
+        "compound_measures": f"{name_a} & {name_b}",
+    })
+    both = f"days on which both {name_a} and {name_b} are {'below' if cold else 'above'} their thresholds"
+    for name, attrs in (COLD_METRIC_ATTRS if cold else METRIC_ATTRS).items():
+        ds[name].attrs.update({**attrs, "long_name": COMPOUND_LONG_NAMES[name], "description": f"{attrs['description']}; {both}"})
+    if intensity:
+        for name, attrs in (COLD_INTENSITY_ATTRS if cold else INTENSITY_ATTRS).items():
+            units = {"units": measure_a.attrs["units"]} if "units" in measure_a.attrs else {}
+            ds[name].attrs.update({**units, **attrs, "long_name": COMPOUND_LONG_NAMES[name],
+                                   "description": f"{attrs['description']}, of each measure; {both}"})
+    xr.set_coord_attrs(ds, "percentile", {"range": "(0, 1)"})
+    days = "cold" if cold else "hot"
+    xr.set_coord_attrs(ds, "definition", {
+        "first_number": f"Minimum number of consecutively {days} days",
+        "second_number": "Maximum number of break days after first wave",
+        "third_number": f"Minimum number of consecutively {days} days after the break"
+    })
+    for variable in ds:
+        add_history(ds[variable], f"Compound heatwave metrics of {name_a} & {name_b} generated by HDP v{get_version()}")
     return ds
 
 

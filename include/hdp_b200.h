@@ -220,6 +220,58 @@ int hdp_b200_intensity_host(const float *h_measure, int64_t C, int64_t T, int64_
                             const uint8_t *h_is_south,
                             float *h_int, uint16_t *h_out, int input_unit);
 
+/* ---------------------------------------------------------------------------------------------------
+ * Path 2 - compound heatwaves (opt-in): the sweep over the days on which TWO measures of one grid, e.g. tmax and tmin (hot days
+ * and hot nights), both exceed their own thresholds.  Measure A (d_a) and measure B (d_b) share C, T, doy_map, the season
+ * tables and input_unit (which applies to both); each has its own strides and its own thresholds, f64 [C, n_doy, P] with the
+ * same n_doy and P: percentile p of A is paired with percentile p of B.
+ *
+ *   compound hot day   (double)x_a(t) > thr_a[c, doy_map[t], p]  and  (double)x_b(t) > thr_b[c, doy_map[t], p]  (NaN on either
+ *                      side of either comparison: not hot).  With HDP_B200_COLD both comparisons are < (cold days and cold
+ *                      nights); the season tables are used as given.
+ *   d_out              optional u16 [4, P, D, Y, C]: HWF, HWN, HWD, HWA (CSF ... CSA with HDP_B200_COLD) by exactly the rules of
+ *                      hdp_b200_metrics, applied to the compound days
+ *   d_int              optional f32 [2, 3, P, D, Y, C]: block 0 = HWC, HWI, HWP of measure A (its exceedance x_a - thr_a over the
+ *                      compound heatwave days), block 1 = the same for measure B; each block has the arithmetic and order of
+ *                      hdp_b200_intensity (the deficit with HDP_B200_COLD), and the season tables must be disjoint as there
+ * At least one of d_out and d_int must be given.  The result at percentile p equals hdp_b200_metrics / hdp_b200_intensity of
+ * where(M_p, x_a, NaN) against thr_a (block 1: where(M_p, x_b, NaN) against thr_b), M_p being the compound mask.
+ * ------------------------------------------------------------------------------------------------- */
+/* h_doy_map may be NULL: the size is then an upper bound for regular daily calendars.  Serves hdp_b200_compound and
+ * hdp_b200_compound_hot_days. */
+size_t hdp_b200_compound_workspace_bytes(int64_t C, int64_t T, int64_t ld_c_a, int64_t ld_c_b, int n_doy, int P, int D, int Y,
+                                         const int32_t *h_doy_map);
+
+int hdp_b200_compound(const float *d_a, int64_t ld_t_a, int64_t ld_c_a, const float *d_b, int64_t ld_t_b, int64_t ld_c_b,
+                      int64_t C, int64_t T, const double *d_thr_a, const double *d_thr_b, int n_doy, int P,
+                      const int32_t *h_doy_map,
+                      const int32_t *h_defs, int D,
+                      const int32_t *h_season_north, const int32_t *h_season_south, int Y,
+                      const uint8_t *d_is_south,
+                      uint16_t *d_out, float *d_int,
+                      void *d_workspace, size_t workspace_bytes, void *stream, int input_unit);
+
+/* Host-buffer variant (the pipeline of hdp_b200_metrics_host; both measures' cells of a chunk cross PCIe once).  Each threshold
+ * array comes from the host (h_thr_*) unless its DEVICE copy (d_thr_*) is given. */
+int hdp_b200_compound_host(const float *h_a, int64_t ld_t_a, int64_t ld_c_a, const float *h_b, int64_t ld_t_b, int64_t ld_c_b,
+                           int64_t C, int64_t T, const double *h_thr_a, const double *d_thr_a, const double *h_thr_b, const double *d_thr_b,
+                           int n_doy, int P, const int32_t *h_doy_map,
+                           const int32_t *h_defs, int D,
+                           const int32_t *h_season_north, const int32_t *h_season_south, int Y,
+                           const uint8_t *h_is_south,
+                           uint16_t *h_out, float *h_int, int input_unit);
+
+/* Compound mask only (parity checks): d_mask u8 [P, T, C], 1 on the compound hot (with HDP_B200_COLD: cold) days. */
+int hdp_b200_compound_hot_days(const float *d_a, int64_t ld_t_a, int64_t ld_c_a, const float *d_b, int64_t ld_t_b, int64_t ld_c_b,
+                               int64_t C, int64_t T, const double *d_thr_a, const double *d_thr_b, int n_doy, int P,
+                               const int32_t *h_doy_map, uint8_t *d_mask,
+                               void *d_workspace, size_t workspace_bytes, void *stream, int input_unit);
+
+/* How the compound hot-day kernel k_hot_pair splits P percentiles (host logic only: no device needed): info[0..2] = {percentiles
+ * per group PG, CTAs per (32 cells, day-of-year block) - slices of whole groups, each with both measures' threshold tiles -,
+ * shared-memory bytes per CTA}. */
+int hdp_b200_compound_plan(int P, int *info);
+
 /* The *_host variants keep their streams, events and device buffers (grown on demand) in a per-device context between
  * calls; this frees them.  Safe to call at any time no *_host call is running. */
 void hdp_b200_host_release(void);
@@ -290,6 +342,7 @@ int64_t hdp_b200_launch_count(void);
 #define HDP_B200_KERNEL_THR_NET     10   /* k_thr_net / k_thr_net_tm / k_thr_net_irr */
 #define HDP_B200_KERNEL_SEAM        11   /* k_index_heatwaves, k_season_metrics */
 #define HDP_B200_KERNEL_INTENSITY   12   /* k_intensity */
+#define HDP_B200_KERNEL_HOT_PAIR    13   /* k_hot_pair */
 void hdp_b200_timing_enable(int on);
 int  hdp_b200_timing_read(int *ids, float *ms, int cap);
 
