@@ -124,12 +124,14 @@ def thresholds_array(temps, tables: WindowTables, percentiles: Sequence[float], 
     return out
 
 
-def _metric_tables(doy_map, defs, season_north, season_south):
+def _metric_tables(doy_map, defs, season_north, season_south, T):
     dm = _i32(doy_map).ravel()
     df = _i32(defs).reshape(-1, 3)
     sn, ss = _i32(season_north).reshape(-1, 2), _i32(season_south).reshape(-1, 2)
     if sn.shape != ss.shape:
         raise ValueError("northern and southern season tables must have the same number of rows")
+    if dm.size != T:
+        raise ValueError("doy_map must have one entry per time step")
     return dm, df, sn, ss
 
 
@@ -160,37 +162,68 @@ def _device_out(out, dtype, shape, device, message):
     return out
 
 
-def _metric_pass(measure, thresholds, doy_map, defs, season_north, season_south, is_south, units, met, heat, intensity, cold):
-    """hdp_b200_metrics, or with ``intensity`` hdp_b200_intensity, on CUDA tensors.  ``met`` / ``heat``: the uint16 metrics /
-    float32 intensity output or None; the metrics are allocated unless the intensity pass runs without them.  Returns the
-    intensity output of the intensity pass, else the metrics.  ``cold``: the cold-spell pass."""
+def _names(pairs, name):
+    return (name,) if len(pairs) == 1 else (f"{name}_a", f"{name}_b")
+
+
+def _check_pairs(pairs):
+    """(T, C, n_doy, P) of one (measure, thresholds) pair of CUDA tensors, or of the two of a compound call: f32 ``[T, C]`` measures
+    of one shape and device, f64 ``[C, n_doy, P]`` thresholds of one shape."""
+    for (x, _), name in zip(pairs, _names(pairs, "measure")):
+        _check_measure(x, name)
+    x0, t0 = pairs[0]
+    if any(tuple(x.shape) != tuple(x0.shape) or x.device != x0.device for x, _ in pairs[1:]):
+        raise ValueError("measure_a and measure_b must have the same shape [T, C] and device")
+    T, C = x0.shape
+    for _, thr in pairs:
+        _check_thr(thr, C)
+    if any(tuple(thr.shape) != tuple(t0.shape) for _, thr in pairs[1:]):
+        raise ValueError("thresholds_a and thresholds_b must have the same shape [C, n_doy, P]")
+    return T, C, int(t0.shape[1]), int(t0.shape[2])
+
+
+def _ptr(t):
+    return t.data_ptr() if t is not None else None
+
+
+def _metric_pass(pairs, doy_map, defs, season_north, season_south, is_south, units, met, heat, intensity, cold):
+    """hdp_b200_metrics, or with ``intensity`` hdp_b200_intensity, on one (measure, thresholds) pair of CUDA tensors; hdp_b200_compound
+    on two.  ``met`` / ``heat``: the uint16 metrics / float32 intensity output (``[2, 3, P, D, Y, C]`` for two pairs) or None; the
+    metrics are allocated unless the intensity pass runs without them.  Returns the intensity output of the intensity pass, else the
+    metrics.  ``cold``: the cold-spell pass."""
     torch = _torch()
     unit = _unit_code(units) | (COLD if cold else 0)
-    _check_measure(measure, "measure")
-    T, C = measure.shape
-    _check_thr(thresholds, C)
-    n_doy, P = int(thresholds.shape[1]), int(thresholds.shape[2])
-    dm, df, sn, ss = _metric_tables(doy_map, defs, season_north, season_south)
-    if dm.size != T:
-        raise ValueError("doy_map must have one entry per time step")
+    T, C, n_doy, P = _check_pairs(pairs)
+    dm, df, sn, ss = _metric_tables(doy_map, defs, season_north, season_south, T)
     L = _lib.lib()
     D, Y = int(df.shape[0]), int(sn.shape[0])
-    south_t = _south_tensor(is_south, C, measure.device)
+    dev = pairs[0][0].device
+    south_t = _south_tensor(is_south, C, dev)
+    compound = len(pairs) == 2
     if intensity:
-        heat = _device_out(heat, torch.float32, (3, P, D, Y, C), measure.device,
-                           "out must be a contiguous float32 CUDA tensor [3, P, D, Y, C]")
+        heat = _device_out(heat, torch.float32, (2, 3, P, D, Y, C) if compound else (3, P, D, Y, C), dev,
+                           f"out must be a contiguous float32 CUDA tensor [{'2, ' if compound else ''}3, P, D, Y, C]")
     if met is not None or not intensity:
-        met = _device_out(met, torch.uint16, (4, P, D, Y, C), measure.device,
+        met = _device_out(met, torch.uint16, (4, P, D, Y, C), dev,
                           f"{'metrics_out' if intensity else 'out'} must be a contiguous uint16 CUDA tensor [4, P, D, Y, C]")
-    outs = (heat.data_ptr(), met.data_ptr() if met is not None else None) if intensity else (met.data_ptr(),)
-    name = "hdp_b200_intensity" if intensity else "hdp_b200_metrics"
-    ld_t, ld_c = _strides(measure)
-    with torch.cuda.device(measure.device):
-        nbytes = getattr(L, name + "_workspace_bytes")(C, T, ld_t, ld_c, n_doy, P, D, Y, _hp(dm))
-        ws = _workspace(measure.device, nbytes)
-        rc = getattr(L, name)(measure.data_ptr(), C, T, ld_t, ld_c, thresholds.data_ptr(), n_doy, P, _hp(dm),
-                              _hp(df), D, _hp(sn), _hp(ss), Y, south_t.data_ptr() if south_t is not None else None,
-                              *outs, ws.data_ptr(), ws.numel(), torch.cuda.current_stream().cuda_stream, unit)
+    tables = (_hp(dm), _hp(df), D, _hp(sn), _hp(ss), Y, _ptr(south_t))
+    with torch.cuda.device(dev):
+        stream = torch.cuda.current_stream().cuda_stream
+        if compound:
+            name = "hdp_b200_compound"
+            (xa, ta), (xb, tb) = pairs
+            (ld_ta, ld_ca), (ld_tb, ld_cb) = _strides(xa), _strides(xb)
+            ws = _workspace(dev, L.hdp_b200_compound_workspace_bytes(C, T, ld_ca, ld_cb, n_doy, P, D, Y, _hp(dm)))
+            rc = L.hdp_b200_compound(xa.data_ptr(), ld_ta, ld_ca, xb.data_ptr(), ld_tb, ld_cb, C, T, ta.data_ptr(), tb.data_ptr(), n_doy,
+                                     P, *tables, _ptr(met), _ptr(heat), ws.data_ptr(), ws.numel(), stream, unit)
+        else:
+            name = "hdp_b200_intensity" if intensity else "hdp_b200_metrics"
+            (x, thr), = pairs
+            ld_t, ld_c = _strides(x)
+            outs = (heat.data_ptr(), _ptr(met)) if intensity else (met.data_ptr(),)
+            ws = _workspace(dev, getattr(L, name + "_workspace_bytes")(C, T, ld_t, ld_c, n_doy, P, D, Y, _hp(dm)))
+            rc = getattr(L, name)(x.data_ptr(), C, T, ld_t, ld_c, thr.data_ptr(), n_doy, P, *tables, *outs, ws.data_ptr(), ws.numel(),
+                                  stream, unit)
     _lib.check(rc, name)
     return heat if intensity else met
 
@@ -202,7 +235,7 @@ def metrics_array(measure, thresholds, doy_map, defs, season_north, season_south
     ``units`` of the measure's samples as for :func:`thresholds_array`.  ``cold=True``: cold spells - the same rules over the
     days with ``measure < threshold``, planes CSF, CSN, CSD, CSA (the season tables are used as given; the cold season of a
     hemisphere is usually the other one's warm season)."""
-    return _metric_pass(measure, thresholds, doy_map, defs, season_north, season_south, is_south, units, out, None, False, cold)
+    return _metric_pass([(measure, thresholds)], doy_map, defs, season_north, season_south, is_south, units, out, None, False, cold)
 
 
 def intensity_array(measure, thresholds, doy_map, defs, season_north, season_south, is_south=None, out=None, metrics_out=None,
@@ -213,48 +246,8 @@ def intensity_array(measure, thresholds, doy_map, defs, season_north, season_sou
     receives exactly what :func:`metrics_array` returns, from the same pass.  The non-empty seasons of each hemisphere's table must
     be disjoint (every table compute_hemisphere_ranges builds is).  ``cold=True``: CSC, CSI, CSP - the deficit
     ``threshold - measure`` over the cold-spell days (and CSF ... CSA in ``metrics_out``), see :func:`metrics_array`."""
-    return _metric_pass(measure, thresholds, doy_map, defs, season_north, season_south, is_south, units, metrics_out, out, True, cold)
-
-
-def _compound_pass(measure_a, thresholds_a, measure_b, thresholds_b, doy_map, defs, season_north, season_south, is_south, units, met,
-                   heat, intensity, cold):
-    """hdp_b200_compound on CUDA tensors: the metrics (``met``) and / or, with ``intensity``, both measures' intensity blocks
-    (``heat``, float32 ``[2, 3, P, D, Y, C]``).  Returns the intensity output of an intensity pass, else the metrics."""
-    torch = _torch()
-    unit = _unit_code(units) | (COLD if cold else 0)
-    _check_measure(measure_a, "measure_a")
-    _check_measure(measure_b, "measure_b")
-    if tuple(measure_a.shape) != tuple(measure_b.shape) or measure_a.device != measure_b.device:
-        raise ValueError("measure_a and measure_b must have the same shape [T, C] and device")
-    T, C = measure_a.shape
-    _check_thr(thresholds_a, C)
-    _check_thr(thresholds_b, C)
-    if tuple(thresholds_a.shape) != tuple(thresholds_b.shape):
-        raise ValueError("thresholds_a and thresholds_b must have the same shape [C, n_doy, P]")
-    n_doy, P = int(thresholds_a.shape[1]), int(thresholds_a.shape[2])
-    dm, df, sn, ss = _metric_tables(doy_map, defs, season_north, season_south)
-    if dm.size != T:
-        raise ValueError("doy_map must have one entry per time step")
-    L = _lib.lib()
-    D, Y = int(df.shape[0]), int(sn.shape[0])
-    dev = measure_a.device
-    south_t = _south_tensor(is_south, C, dev)
-    if intensity:
-        heat = _device_out(heat, torch.float32, (2, 3, P, D, Y, C), dev, "out must be a contiguous float32 CUDA tensor [2, 3, P, D, Y, C]")
-    if met is not None or not intensity:
-        met = _device_out(met, torch.uint16, (4, P, D, Y, C), dev,
-                          f"{'metrics_out' if intensity else 'out'} must be a contiguous uint16 CUDA tensor [4, P, D, Y, C]")
-    (ld_ta, ld_ca), (ld_tb, ld_cb) = _strides(measure_a), _strides(measure_b)
-    with torch.cuda.device(dev):
-        nbytes = L.hdp_b200_compound_workspace_bytes(C, T, ld_ca, ld_cb, n_doy, P, D, Y, _hp(dm))
-        ws = _workspace(dev, nbytes)
-        rc = L.hdp_b200_compound(measure_a.data_ptr(), ld_ta, ld_ca, measure_b.data_ptr(), ld_tb, ld_cb, C, T, thresholds_a.data_ptr(),
-                                 thresholds_b.data_ptr(), n_doy, P, _hp(dm), _hp(df), D, _hp(sn), _hp(ss), Y,
-                                 south_t.data_ptr() if south_t is not None else None, met.data_ptr() if met is not None else None,
-                                 heat.data_ptr() if intensity else None, ws.data_ptr(), ws.numel(), torch.cuda.current_stream().cuda_stream,
-                                 unit)
-    _lib.check(rc, "hdp_b200_compound")
-    return heat if intensity else met
+    return _metric_pass([(measure, thresholds)], doy_map, defs, season_north, season_south, is_south, units, metrics_out, out, True,
+                        cold)
 
 
 def compound_metrics_array(measure_a, thresholds_a, measure_b, thresholds_b, doy_map, defs, season_north, season_south, is_south=None,
@@ -264,8 +257,8 @@ def compound_metrics_array(measure_a, thresholds_a, measure_b, thresholds_b, doy
     f32 ``[T, C]`` CUDA tensors (any strides each), the two thresholds f64 ``[C, n_doy, P]`` of the same shape: percentile p of A is
     paired with percentile p of B.  ``units`` applies to both measures; ``cold=True``: days on which both are below their
     thresholds (CSF ... CSA)."""
-    return _compound_pass(measure_a, thresholds_a, measure_b, thresholds_b, doy_map, defs, season_north, season_south, is_south, units,
-                          out, None, False, cold)
+    return _metric_pass([(measure_a, thresholds_a), (measure_b, thresholds_b)], doy_map, defs, season_north, season_south, is_south,
+                        units, out, None, False, cold)
 
 
 def compound_intensity_array(measure_a, thresholds_a, measure_b, thresholds_b, doy_map, defs, season_north, season_south, is_south=None,
@@ -274,61 +267,51 @@ def compound_intensity_array(measure_a, thresholds_a, measure_b, thresholds_b, d
     of measure A (its exceedance ``measure_a - thresholds_a`` over the compound heatwave days, as :func:`intensity_array` computes
     it), block 1 = the same for measure B.  ``metrics_out``: an optional uint16 CUDA tensor ``[4, P, D, Y, C]`` that also receives
     what :func:`compound_metrics_array` returns, from the same pass.  ``cold``: the deficits over the compound cold spells."""
-    return _compound_pass(measure_a, thresholds_a, measure_b, thresholds_b, doy_map, defs, season_north, season_south, is_south, units,
-                          metrics_out, out, True, cold)
+    return _metric_pass([(measure_a, thresholds_a), (measure_b, thresholds_b)], doy_map, defs, season_north, season_south, is_south,
+                        units, metrics_out, out, True, cold)
+
+
+def _hot_days(pairs, doy_map, units=None, cold=False):
+    """The hot-day mask uint8 ``[P, T, C]`` of one (measure, thresholds) pair (hdp_b200_hot_days) or the compound mask of two
+    (hdp_b200_compound_hot_days)."""
+    torch = _torch()
+    T, C, n_doy, P = _check_pairs(pairs)
+    dm = _i32(doy_map).ravel()
+    if dm.size != T:
+        raise ValueError("doy_map must have one entry per time step")
+    L = _lib.lib()
+    dev = pairs[0][0].device
+    out = torch.empty((P, T, C), dtype=torch.uint8, device=dev)
+    with torch.cuda.device(dev):
+        stream = torch.cuda.current_stream().cuda_stream
+        if len(pairs) == 2:
+            name = "hdp_b200_compound_hot_days"
+            (xa, ta), (xb, tb) = pairs
+            (ld_ta, ld_ca), (ld_tb, ld_cb) = _strides(xa), _strides(xb)
+            ws = _workspace(dev, L.hdp_b200_compound_workspace_bytes(C, T, ld_ca, ld_cb, n_doy, P, 1, 0, _hp(dm)))
+            rc = L.hdp_b200_compound_hot_days(xa.data_ptr(), ld_ta, ld_ca, xb.data_ptr(), ld_tb, ld_cb, C, T, ta.data_ptr(), tb.data_ptr(),
+                                              n_doy, P, _hp(dm), out.data_ptr(), ws.data_ptr(), ws.numel(), stream,
+                                              _unit_code(units) | (COLD if cold else 0))
+        else:
+            name = "hdp_b200_hot_days"
+            (x, thr), = pairs
+            ld_t, ld_c = _strides(x)
+            ws = _workspace(dev, L.hdp_b200_metrics_workspace_bytes(C, T, ld_t, ld_c, n_doy, P, 1, 0, _hp(dm)))
+            rc = L.hdp_b200_hot_days(x.data_ptr(), C, T, ld_t, ld_c, thr.data_ptr(), n_doy, P, _hp(dm), out.data_ptr(), ws.data_ptr(),
+                                     ws.numel(), stream)
+    _lib.check(rc, name)
+    return out
 
 
 def compound_hot_days_array(measure_a, thresholds_a, measure_b, thresholds_b, doy_map, units=None, *, cold=False):
     """The compound mask of every percentile: uint8 ``[P, T, C]``, 1 where both measures exceed their thresholds (``cold``: are
     below them)."""
-    torch = _torch()
-    _check_measure(measure_a, "measure_a")
-    _check_measure(measure_b, "measure_b")
-    if tuple(measure_a.shape) != tuple(measure_b.shape) or measure_a.device != measure_b.device:
-        raise ValueError("measure_a and measure_b must have the same shape [T, C] and device")
-    T, C = measure_a.shape
-    _check_thr(thresholds_a, C)
-    _check_thr(thresholds_b, C)
-    if tuple(thresholds_a.shape) != tuple(thresholds_b.shape):
-        raise ValueError("thresholds_a and thresholds_b must have the same shape [C, n_doy, P]")
-    n_doy, P = int(thresholds_a.shape[1]), int(thresholds_a.shape[2])
-    dm = _i32(doy_map).ravel()
-    if dm.size != T:
-        raise ValueError("doy_map must have one entry per time step")
-    L = _lib.lib()
-    out = torch.empty((P, T, C), dtype=torch.uint8, device=measure_a.device)
-    (ld_ta, ld_ca), (ld_tb, ld_cb) = _strides(measure_a), _strides(measure_b)
-    with torch.cuda.device(measure_a.device):
-        nbytes = L.hdp_b200_compound_workspace_bytes(C, T, ld_ca, ld_cb, n_doy, P, 1, 0, _hp(dm))
-        ws = _workspace(measure_a.device, nbytes)
-        rc = L.hdp_b200_compound_hot_days(measure_a.data_ptr(), ld_ta, ld_ca, measure_b.data_ptr(), ld_tb, ld_cb, C, T,
-                                          thresholds_a.data_ptr(), thresholds_b.data_ptr(), n_doy, P, _hp(dm), out.data_ptr(),
-                                          ws.data_ptr(), ws.numel(), torch.cuda.current_stream().cuda_stream,
-                                          _unit_code(units) | (COLD if cold else 0))
-    _lib.check(rc, "hdp_b200_compound_hot_days")
-    return out
+    return _hot_days([(measure_a, thresholds_a), (measure_b, thresholds_b)], doy_map, units, cold)
 
 
 def hot_days_array(measure, thresholds, doy_map):
     """``indicate_hot_days`` for every percentile: uint8 ``[P, T, C]``."""
-    torch = _torch()
-    _check_measure(measure, "measure")
-    T, C = measure.shape
-    _check_thr(thresholds, C)
-    L = _lib.lib()
-    n_doy, P = int(thresholds.shape[1]), int(thresholds.shape[2])
-    dm = _i32(doy_map).ravel()
-    if dm.size != T:
-        raise ValueError("doy_map must have one entry per time step")
-    out = torch.empty((P, T, C), dtype=torch.uint8, device=measure.device)
-    ld_t, ld_c = _strides(measure)
-    with torch.cuda.device(measure.device):
-        nbytes = L.hdp_b200_metrics_workspace_bytes(C, T, ld_t, ld_c, n_doy, P, 1, 0, _hp(dm))
-        ws = _workspace(measure.device, nbytes)
-        rc = L.hdp_b200_hot_days(measure.data_ptr(), C, T, ld_t, ld_c, thresholds.data_ptr(), n_doy, P, _hp(dm),
-                                 out.data_ptr(), ws.data_ptr(), ws.numel(), torch.cuda.current_stream().cuda_stream)
-    _lib.check(rc, "hdp_b200_hot_days")
-    return out
+    return _hot_days([(measure, thresholds)], doy_map)
 
 
 # ----------------------------------------------------------------------------------------------
@@ -557,41 +540,6 @@ def _host_out(out, dtype, shape, message):
     return out
 
 
-def _metric_pass_host(measure, thresholds, doy_map, defs, season_north, season_south, is_south, units, met, heat, intensity, cold):
-    """:func:`_metric_pass` with host arrays: hdp_b200_metrics_host, or with ``intensity`` hdp_b200_intensity_host."""
-    torch = _torch()
-    measure, ld_t, ld_c = _host_measure(measure, "measure")
-    T, C = measure.shape
-    d_thr = None
-    if isinstance(thresholds, torch.Tensor):
-        _check_thr(thresholds, C)
-        d_thr, thr = thresholds, None
-        n_doy, P = int(d_thr.shape[1]), int(d_thr.shape[2])
-    else:
-        thr = np.ascontiguousarray(thresholds, dtype=np.float64)
-        if thr.ndim != 3 or thr.shape[0] != C:
-            raise TypeError("thresholds must be float64 [C, n_doy, P]")
-        n_doy, P = thr.shape[1], thr.shape[2]
-        d_thr = resident_thresholds(thr)
-    dm, df, sn, ss = _metric_tables(doy_map, defs, season_north, season_south)
-    if dm.size != T:
-        raise ValueError("doy_map must have one entry per time step")
-    south = None if is_south is None else np.ascontiguousarray(is_south, dtype=np.uint8)
-    D, Y = df.shape[0], sn.shape[0]
-    if intensity:
-        heat = _host_out(heat, np.float32, (3, P, D, Y, C), "out must be a C-contiguous float32 array [3, P, D, Y, C]")
-    if met is not None or not intensity:
-        met = _host_out(met, np.uint16, (4, P, D, Y, C),
-                        f"{'metrics_out' if intensity else 'out'} must be a C-contiguous uint16 array [4, P, D, Y, C]")
-    outs = (_hp(heat), _hp(met) if met is not None else None) if intensity else (_hp(met),)
-    name = "hdp_b200_intensity_host" if intensity else "hdp_b200_metrics_host"
-    rc = getattr(_lib.lib(), name)(_hp(measure), C, T, ld_t, ld_c, _hp(thr) if thr is not None else None,
-                                   d_thr.data_ptr() if d_thr is not None else None, n_doy, P, _hp(dm), _hp(df), D, _hp(sn), _hp(ss), Y,
-                                   _hp(south) if south is not None else None, *outs, _unit_code(units) | (COLD if cold else 0))
-    _lib.check(rc, name)
-    return heat if intensity else met
-
-
 def _host_thresholds(thresholds, C):
     """(host array or None, device tensor or None) of one threshold argument of a host call: a CUDA tensor is used where it is, a
     host array that :func:`thresholds_host` returned with ``keep=True`` through its device copy."""
@@ -605,35 +553,43 @@ def _host_thresholds(thresholds, C):
     return thr, resident_thresholds(thr)
 
 
-def _compound_pass_host(measure_a, thresholds_a, measure_b, thresholds_b, doy_map, defs, season_north, season_south, is_south, units,
-                        met, heat, intensity, cold):
-    """:func:`_compound_pass` with host arrays (hdp_b200_compound_host); each threshold as for :func:`metrics_host`."""
-    a, ld_ta, ld_ca = _host_measure(measure_a, "measure_a")
-    b, ld_tb, ld_cb = _host_measure(measure_b, "measure_b")
-    if a.shape != b.shape:
+def _metric_pass_host(pairs, doy_map, defs, season_north, season_south, is_south, units, met, heat, intensity, cold):
+    """:func:`_metric_pass` with host arrays: hdp_b200_metrics_host or hdp_b200_intensity_host on one (measure, thresholds) pair,
+    hdp_b200_compound_host on two; each threshold as for :func:`metrics_host`."""
+    _torch()
+    xs = [_host_measure(x, name) for (x, _), name in zip(pairs, _names(pairs, "measure"))]      # (samples, ld_t, ld_c)
+    if any(x.shape != xs[0][0].shape for x, _, _ in xs[1:]):
         raise ValueError("measure_a and measure_b must have the same shape [T, C]")
-    T, C = a.shape
-    (h_a, d_a), (h_b, d_b) = _host_thresholds(thresholds_a, C), _host_thresholds(thresholds_b, C)
-    shape_a = tuple((d_a if h_a is None else h_a).shape)
-    if shape_a != tuple((d_b if h_b is None else h_b).shape):
+    T, C = xs[0][0].shape
+    thrs = [_host_thresholds(thr, C) for _, thr in pairs]                                       # (host, device)
+    shapes = [tuple((d if h is None else h).shape) for h, d in thrs]
+    if any(shape != shapes[0] for shape in shapes[1:]):
         raise ValueError("thresholds_a and thresholds_b must have the same shape [C, n_doy, P]")
-    n_doy, P = int(shape_a[1]), int(shape_a[2])
-    dm, df, sn, ss = _metric_tables(doy_map, defs, season_north, season_south)
-    if dm.size != T:
-        raise ValueError("doy_map must have one entry per time step")
+    n_doy, P = int(shapes[0][1]), int(shapes[0][2])
+    dm, df, sn, ss = _metric_tables(doy_map, defs, season_north, season_south, T)
     south = None if is_south is None else np.ascontiguousarray(is_south, dtype=np.uint8)
     D, Y = df.shape[0], sn.shape[0]
+    compound = len(pairs) == 2
     if intensity:
-        heat = _host_out(heat, np.float32, (2, 3, P, D, Y, C), "out must be a C-contiguous float32 array [2, 3, P, D, Y, C]")
+        heat = _host_out(heat, np.float32, (2, 3, P, D, Y, C) if compound else (3, P, D, Y, C),
+                         f"out must be a C-contiguous float32 array [{'2, ' if compound else ''}3, P, D, Y, C]")
     if met is not None or not intensity:
         met = _host_out(met, np.uint16, (4, P, D, Y, C),
                         f"{'metrics_out' if intensity else 'out'} must be a C-contiguous uint16 array [4, P, D, Y, C]")
     hp = lambda h: _hp(h) if h is not None else None                # noqa: E731
-    dp = lambda d: d.data_ptr() if d is not None else None          # noqa: E731
-    rc = _lib.lib().hdp_b200_compound_host(_hp(a), ld_ta, ld_ca, _hp(b), ld_tb, ld_cb, C, T, hp(h_a), dp(d_a), hp(h_b), dp(d_b), n_doy, P,
-                                           _hp(dm), _hp(df), D, _hp(sn), _hp(ss), Y, hp(south), hp(met), hp(heat),
-                                           _unit_code(units) | (COLD if cold else 0))
-    _lib.check(rc, "hdp_b200_compound_host")
+    tables = (_hp(dm), _hp(df), D, _hp(sn), _hp(ss), Y, hp(south))
+    if compound:
+        name = "hdp_b200_compound_host"
+        ((a, ld_ta, ld_ca), (b, ld_tb, ld_cb)), ((h_a, d_a), (h_b, d_b)) = xs, thrs
+        rc = _lib.lib().hdp_b200_compound_host(_hp(a), ld_ta, ld_ca, _hp(b), ld_tb, ld_cb, C, T, hp(h_a), _ptr(d_a), hp(h_b), _ptr(d_b),
+                                               n_doy, P, *tables, hp(met), hp(heat), _unit_code(units) | (COLD if cold else 0))
+    else:
+        name = "hdp_b200_intensity_host" if intensity else "hdp_b200_metrics_host"
+        ((x, ld_t, ld_c),), ((h_thr, d_thr),) = xs, thrs
+        outs = (_hp(heat), hp(met)) if intensity else (_hp(met),)
+        rc = getattr(_lib.lib(), name)(_hp(x), C, T, ld_t, ld_c, hp(h_thr), _ptr(d_thr), n_doy, P, *tables, *outs,
+                                       _unit_code(units) | (COLD if cold else 0))
+    _lib.check(rc, name)
     return heat if intensity else met
 
 
@@ -641,16 +597,16 @@ def compound_metrics_host(measure_a: np.ndarray, thresholds_a, measure_b: np.nda
                           season_south, is_south=None, out: Optional[np.ndarray] = None, units=None, *, cold=False) -> np.ndarray:
     """Host-array counterpart of :func:`compound_metrics_array` (both measures' cells of a chunk cross PCIe once).  Each threshold
     as for :func:`metrics_host`: a host array, a CUDA tensor, or a resident copy."""
-    return _compound_pass_host(measure_a, thresholds_a, measure_b, thresholds_b, doy_map, defs, season_north, season_south, is_south,
-                               units, out, None, False, cold)
+    return _metric_pass_host([(measure_a, thresholds_a), (measure_b, thresholds_b)], doy_map, defs, season_north, season_south, is_south,
+                             units, out, None, False, cold)
 
 
 def compound_intensity_host(measure_a: np.ndarray, thresholds_a, measure_b: np.ndarray, thresholds_b, doy_map, defs, season_north,
                             season_south, is_south=None, out: Optional[np.ndarray] = None, metrics_out: Optional[np.ndarray] = None,
                             units=None, *, cold=False) -> np.ndarray:
     """Host-array counterpart of :func:`compound_intensity_array`: float32 ``[2, 3, P, D, Y, C]``."""
-    return _compound_pass_host(measure_a, thresholds_a, measure_b, thresholds_b, doy_map, defs, season_north, season_south, is_south,
-                               units, metrics_out, out, True, cold)
+    return _metric_pass_host([(measure_a, thresholds_a), (measure_b, thresholds_b)], doy_map, defs, season_north, season_south, is_south,
+                             units, metrics_out, out, True, cold)
 
 
 def metrics_host(measure: np.ndarray, thresholds, doy_map, defs, season_north, season_south,
@@ -658,7 +614,7 @@ def metrics_host(measure: np.ndarray, thresholds, doy_map, defs, season_north, s
     """``thresholds``: float64 ``[C, n_doy, P]`` as a host array, or as a CUDA tensor (device-resident: no upload).  A host
     array that :func:`thresholds_host` returned with ``keep=True`` is recognised and its device copy used.  ``cold`` as for
     :func:`metrics_array`."""
-    return _metric_pass_host(measure, thresholds, doy_map, defs, season_north, season_south, is_south, units, out, None, False, cold)
+    return _metric_pass_host([(measure, thresholds)], doy_map, defs, season_north, season_south, is_south, units, out, None, False, cold)
 
 
 def intensity_host(measure: np.ndarray, thresholds, doy_map, defs, season_north, season_south, is_south=None,
@@ -668,7 +624,7 @@ def intensity_host(measure: np.ndarray, thresholds, doy_map, defs, season_north,
     optional uint16 host array ``[4, P, D, Y, C]`` that also receives what :func:`metrics_host` returns (the samples cross PCIe
     once for both).  Thresholds as for :func:`metrics_host` (host array, CUDA tensor, or a resident copy); ``cold`` as for
     :func:`intensity_array`."""
-    return _metric_pass_host(measure, thresholds, doy_map, defs, season_north, season_south, is_south, units, metrics_out, out, True,
+    return _metric_pass_host([(measure, thresholds)], doy_map, defs, season_north, season_south, is_south, units, metrics_out, out, True,
                              cold)
 
 

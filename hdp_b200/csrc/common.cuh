@@ -100,23 +100,23 @@ int thresholds_launch(const float *d_temps, int64_t C, int64_t T_b, int64_t ld_t
                       const double *h_q, int P, double *d_out,
                       void *d_workspace, size_t workspace_bytes, void *stream, int64_t carve_cells, bool tables_resident, int input_unit);
 
-// The second measure of a compound pass (hdp_b200_compound): a day counts only where both measures pass their own thresholds.
-struct SecondMeasure {
-    const float *x = nullptr;       // nullptr: a single-measure pass
-    int64_t ld_t = 0, ld_c = 1;
-    const double *thr = nullptr;    // [C, n_doy, P], the n_doy and P of the first measure's thresholds
+// One measure of a metric pass: samples [T, C] (day t of cell c at x[t * ld_t + c * ld_c]) and their thresholds [C, n_doy, P].
+// A pass takes one or two; with two (hdp_b200_compound) a day counts only where both measures pass their own thresholds, and both
+// threshold tables have the same n_doy and P.
+struct Measure {
+    const float *x;
+    int64_t ld_t, ld_c;
+    const double *thr;
 };
 
-// The whole of hdp_b200_metrics, hdp_b200_intensity and hdp_b200_compound (metric.cu): k_hot_words (k_hot_pair when b.x is given),
-// then k_scan on its hot words when d_out is given (u16 [4, P, D, Y, C]) and k_intensity when d_int is given (f32 [3, P, D, Y, C];
-// for a compound pass [2, 3, P, D, Y, C], one block per measure).  carve_cells / tables_resident as above; input_unit = unit code,
-// OR-ed with HDP_B200_COLD for the cold-spell pass.
-int metric_pass(const float *d_measure, int64_t C, int64_t T, int64_t ld_t, int64_t ld_c,
-                const double *d_thr, int n_doy, int P, const int32_t *h_doy_map,
+// The whole of hdp_b200_metrics, hdp_b200_intensity and hdp_b200_compound (metric.cu) over n_measures (1 or 2) measures:
+// k_hot_words (k_hot_pair for two), then k_scan on its hot words when d_out is given (u16 [4, P, D, Y, C]) and k_intensity when
+// d_int is given (f32 [n_measures, 3, P, D, Y, C], one block per measure).  carve_cells / tables_resident as above; input_unit =
+// unit code, OR-ed with HDP_B200_COLD for the cold-spell pass.
+int metric_pass(const Measure *ms, int n_measures, int64_t C, int64_t T, int n_doy, int P, const int32_t *h_doy_map,
                 const int32_t *h_defs, int D,
                 const int32_t *h_season_north, const int32_t *h_season_south, int Y,
                 const uint8_t *d_is_south, uint16_t *d_out, float *d_int,
-                void *d_workspace, size_t workspace_bytes, void *stream, int64_t carve_cells, bool tables_resident, int input_unit,
-                const SecondMeasure &b = SecondMeasure());
+                void *d_workspace, size_t workspace_bytes, void *stream, int64_t carve_cells, bool tables_resident, int input_unit);
 
 }  // namespace hdp

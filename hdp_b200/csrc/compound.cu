@@ -189,34 +189,13 @@ int run_hot_pair(const Layout &L, const WordPlan &plan, int64_t C, int P, cudaSt
     size_t smem;
     if (!hot_pair_plan(P, pg, slices, gps, smem)) return HDP_B200_ERR_UNSUPPORTED;
     dim3 grid((unsigned)((C + kTileCells - 1) / kTileCells), (unsigned)plan.n_blk, (unsigned)slices);
+    const auto kernel = hot_kernel(pg, unit, cold, [](auto PG, auto U, auto CO) {
+        return k_hot_pair<decltype(PG)::value, decltype(U)::value, decltype(CO)::value>;
+    });
     KernelTimer timer(kHotPair, st);
-#define HDP_LAUNCH_PAIR_D(PG, U, CO)                                                                               \
-    do {                                                                                                           \
-        HDP_CUDA_TRY(cudaFuncSetAttribute(k_hot_pair<PG, U, CO>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)); \
-        k_hot_pair<PG, U, CO><<<grid, 256, smem, st>>>(L.x, L.ld_t, L.x_b, L.ld_t_b, C, L.thr, L.thr_b, L.n_doy, P, gps, L.words, \
-                                                       L.blk_start, L.blk_words, K, L.hot);                        \
-    } while (0)
-#define HDP_LAUNCH_PAIR_U(PG, U)                                                                                   \
-    do {                                                                                                           \
-        if (cold) HDP_LAUNCH_PAIR_D(PG, U, true);                                                                  \
-        else HDP_LAUNCH_PAIR_D(PG, U, false);                                                                      \
-    } while (0)
-#define HDP_LAUNCH_PAIR(PG)                                                                                        \
-    do {                                                                                                           \
-        if (unit == 0) HDP_LAUNCH_PAIR_U(PG, 0);                                                                   \
-        else if (unit == 1) HDP_LAUNCH_PAIR_U(PG, 1);                                                              \
-        else HDP_LAUNCH_PAIR_U(PG, 2);                                                                             \
-    } while (0)
-    switch (pg) {
-    case 4: HDP_LAUNCH_PAIR(4); break;
-    case 8: HDP_LAUNCH_PAIR(8); break;
-    case 10: HDP_LAUNCH_PAIR(10); break;
-    case 16: HDP_LAUNCH_PAIR(16); break;
-    default: HDP_LAUNCH_PAIR(20); break;
-    }
-#undef HDP_LAUNCH_PAIR
-#undef HDP_LAUNCH_PAIR_U
-#undef HDP_LAUNCH_PAIR_D
+    HDP_CUDA_TRY(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    kernel<<<grid, 256, smem, st>>>(L.x[0], L.ld_t[0], L.x[1], L.ld_t[1], C, L.thr[0], L.thr[1], L.n_doy, P, gps, L.words, L.blk_start,
+                                    L.blk_words, K, L.hot);
     HDP_LAUNCH_CHECK();
     return HDP_B200_OK;
 }
@@ -231,7 +210,8 @@ size_t hdp_b200_compound_workspace_bytes(int64_t C, int64_t T, int64_t ld_c_a, i
                                          const int32_t *h_doy_map)
 {
     (void)D;
-    return metric_pass_workspace_bytes(C, T, ld_c_a, n_doy, P, Y, h_doy_map, true, true, ld_c_b);
+    const int64_t ld_c[2] = {ld_c_a, ld_c_b};
+    return metric_pass_workspace_bytes(C, T, ld_c, 2, n_doy, P, Y, h_doy_map, true);
 }
 
 int hdp_b200_compound(const float *d_a, int64_t ld_t_a, int64_t ld_c_a, const float *d_b, int64_t ld_t_b, int64_t ld_c_b,
@@ -242,11 +222,9 @@ int hdp_b200_compound(const float *d_a, int64_t ld_t_a, int64_t ld_c_a, const fl
                       void *d_workspace, size_t workspace_bytes, void *stream, int input_unit)
 {
     if (C > 0 && Y > 0 && !d_out && !d_int) return HDP_B200_ERR_INVALID;
-    if (C > 0 && T > 0 && !d_b) return HDP_B200_ERR_INVALID;
-    SecondMeasure b;
-    b.x = d_b; b.ld_t = ld_t_b; b.ld_c = ld_c_b; b.thr = d_thr_b;
-    return metric_pass(d_a, C, T, ld_t_a, ld_c_a, d_thr_a, n_doy, P, h_doy_map, h_defs, D, h_season_north, h_season_south, Y,
-                       d_is_south, d_out, d_int, d_workspace, workspace_bytes, stream, C, false, input_unit, b);
+    const Measure ms[2] = {{d_a, ld_t_a, ld_c_a, d_thr_a}, {d_b, ld_t_b, ld_c_b, d_thr_b}};
+    return metric_pass(ms, 2, C, T, n_doy, P, h_doy_map, h_defs, D, h_season_north, h_season_south, Y, d_is_south, d_out, d_int,
+                       d_workspace, workspace_bytes, stream, C, false, input_unit);
 }
 
 int hdp_b200_compound_plan(int P, int *info)

@@ -152,8 +152,8 @@ struct HostCtx {
     bool ready = false;
     cudaStream_t s_in = nullptr, s_k = nullptr, s_out = nullptr;
     cudaEvent_t in_ready[kSlots] = {}, k_done[kSlots] = {}, out_done[kSlots] = {};
-    DeviceBuf x[kSlots], aux[kSlots], south[kSlots], out[kSlots], out_f[kSlots], ws;
-    DeviceBuf x_b[kSlots], aux_b[kSlots];            // the second measure of a compound pass and its thresholds
+    DeviceBuf x[2][kSlots], thr[2][kSlots];          // per measure (two for a compound pass): samples, thresholds from the host
+    DeviceBuf south[kSlots], out[kSlots], out_f[kSlots], ws;
     PinnedRing ring_in, ring_out;                    // staging for pageable sources / destinations (allocated on first use)
     std::deque<PendingOut> pending;                  // D2H blocks on their way through ring_out
 
@@ -260,8 +260,8 @@ struct HostCtx {
             ready = false;
         }
         for (int i = 0; i < kSlots; i++) {
-            x[i].release(); aux[i].release(); south[i].release(); out[i].release(); out_f[i].release();
-            x_b[i].release(); aux_b[i].release();
+            for (int m = 0; m < 2; m++) { x[m][i].release(); thr[m][i].release(); }
+            south[i].release(); out[i].release(); out_f[i].release();
         }
         ws.release();
         ring_in.release(); ring_out.release();
@@ -324,31 +324,28 @@ using namespace hdp;
     } while (0)
 #define HDP_HOST_CUDA(expr) HDP_HOST_TRY(cuda_status(expr))
 
-// The second measure of hdp_b200_compound_host: host samples, thresholds from the host (h_thr) or the device (d_thr).
-struct HostSecond {
-    const float *h = nullptr;       // nullptr: a single-measure pass
-    int64_t ld_t = 0, ld_c = 1;
-    const double *h_thr = nullptr, *d_thr = nullptr;
+// One measure of a host call: host samples [T, C] (strides ld_t, ld_c), thresholds from the host (h_thr) or the device (d_thr).
+struct HostMeasure {
+    const float *x;
+    int64_t ld_t, ld_c;
+    const double *h_thr, *d_thr;
 };
 
-// hdp_b200_metrics_host, hdp_b200_intensity_host and hdp_b200_compound_host: metric_pass chunk by chunk; the u16 planes (h_out) and
-// the f32 planes (h_int), whichever are given, go back to the host.  With a second measure both measures' cells of a chunk go up
-// together.
-static int metric_pass_host(const float *h_measure, int64_t C, int64_t T, int64_t ld_t, int64_t ld_c,
-                            const double *h_thr, const double *d_thr, int n_doy, int P, const int32_t *h_doy_map,
+// hdp_b200_metrics_host, hdp_b200_intensity_host and hdp_b200_compound_host: metric_pass over n_measures (1 or 2) measures chunk by
+// chunk; the u16 planes (h_out) and the f32 planes (h_int), whichever are given, go back to the host.  Every measure's cells of a
+// chunk go up together.
+static int metric_pass_host(const HostMeasure *hm, int n_measures, int64_t C, int64_t T, int n_doy, int P, const int32_t *h_doy_map,
                             const int32_t *h_defs, int D,
                             const int32_t *h_season_north, const int32_t *h_season_south, int Y,
-                            const uint8_t *h_is_south, float *h_int, uint16_t *h_out, int input_unit, const HostSecond &m2 = HostSecond())
+                            const uint8_t *h_is_south, float *h_int, uint16_t *h_out, int input_unit)
 {
     if (C < 0 || T <= 0 || n_doy <= 0 || P <= 0 || D <= 0 || Y < 0 || !h_doy_map) return HDP_B200_ERR_INVALID;
     if (C == 0 || Y == 0) return HDP_B200_OK;
-    if (!h_measure || (!h_thr && !d_thr)) return HDP_B200_ERR_INVALID;
-    if (ld_t <= 0 || ld_c <= 0) return HDP_B200_ERR_INVALID;
-    if (ld_c != 1 && ld_t != 1) return HDP_B200_ERR_UNSUPPORTED;
-    const bool pair = m2.h != nullptr;
-    if (pair && (!m2.h_thr && !m2.d_thr)) return HDP_B200_ERR_INVALID;
-    if (pair && (m2.ld_t <= 0 || m2.ld_c <= 0)) return HDP_B200_ERR_INVALID;
-    if (pair && m2.ld_c != 1 && m2.ld_t != 1) return HDP_B200_ERR_UNSUPPORTED;
+    for (int m = 0; m < n_measures; m++) {
+        if (!hm[m].x || (!hm[m].h_thr && !hm[m].d_thr)) return HDP_B200_ERR_INVALID;
+        if (hm[m].ld_t <= 0 || hm[m].ld_c <= 0) return HDP_B200_ERR_INVALID;
+        if (hm[m].ld_c != 1 && hm[m].ld_t != 1) return HDP_B200_ERR_UNSUPPORTED;
+    }
     HostCtx *ctx = nullptr;
     int rc = current_ctx(&ctx);
     if (rc) return rc;
@@ -357,45 +354,46 @@ static int metric_pass_host(const float *h_measure, int64_t C, int64_t T, int64_
 
     const size_t thr_per_cell = (size_t)n_doy * P * sizeof(double);
     const size_t rows = (size_t)4 * P * D * Y;                                 // output rows of C cells each
-    const size_t rows_f = (size_t)(pair ? 6 : 3) * P * D * Y;
-    const int64_t chunk = pick_chunk(C, (pair ? 2 : 1) * ((size_t)T * sizeof(float) + thr_per_cell), (size_t)320 << 20);
-    const int64_t dl_t = ld_c == 1 ? chunk : 1, dl_c = ld_c == 1 ? 1 : T;
-    const int64_t dl_c_b = m2.ld_c == 1 ? 1 : T;
-    const size_t ws_bytes = pair ? hdp_b200_compound_workspace_bytes(chunk, T, dl_c, dl_c_b, n_doy, P, D, Y, h_doy_map)
-                            : h_int ? hdp_b200_intensity_workspace_bytes(chunk, T, dl_t, dl_c, n_doy, P, D, Y, h_doy_map)
-                                    : hdp_b200_metrics_workspace_bytes(chunk, T, dl_t, dl_c, n_doy, P, D, Y, h_doy_map);
+    const size_t rows_f = (size_t)n_measures * 3 * P * D * Y;
+    const int64_t chunk = pick_chunk(C, n_measures * ((size_t)T * sizeof(float) + thr_per_cell), (size_t)320 << 20);
+    int64_t dl_c[2] = {};                                                      // cell strides of the device copies (upload_cells)
+    for (int m = 0; m < n_measures; m++) dl_c[m] = hm[m].ld_c == 1 ? 1 : T;
+    const int64_t dl_t = dl_c[0] == 1 ? chunk : 1;
+    const size_t ws_bytes = n_measures == 2 ? hdp_b200_compound_workspace_bytes(chunk, T, dl_c[0], dl_c[1], n_doy, P, D, Y, h_doy_map)
+                            : h_int ? hdp_b200_intensity_workspace_bytes(chunk, T, dl_t, dl_c[0], n_doy, P, D, Y, h_doy_map)
+                                    : hdp_b200_metrics_workspace_bytes(chunk, T, dl_t, dl_c[0], n_doy, P, D, Y, h_doy_map);
     if ((rc = ctx->ws.reserve(ws_bytes))) return rc;
     for (int i = 0; i < kSlots; i++) {
-        if ((rc = ctx->x[i].reserve((size_t)chunk * T * sizeof(float)))) return rc;
-        if (!d_thr && (rc = ctx->aux[i].reserve((size_t)chunk * thr_per_cell))) return rc;
-        if (pair && (rc = ctx->x_b[i].reserve((size_t)chunk * T * sizeof(float)))) return rc;
-        if (pair && !m2.d_thr && (rc = ctx->aux_b[i].reserve((size_t)chunk * thr_per_cell))) return rc;
+        for (int m = 0; m < n_measures; m++) {
+            if ((rc = ctx->x[m][i].reserve((size_t)chunk * T * sizeof(float)))) return rc;
+            if (!hm[m].d_thr && (rc = ctx->thr[m][i].reserve((size_t)chunk * thr_per_cell))) return rc;
+        }
         if ((rc = ctx->south[i].reserve((size_t)chunk))) return rc;
         if (h_out && (rc = ctx->out[i].reserve(rows * chunk * sizeof(uint16_t)))) return rc;
         if (h_int && (rc = ctx->out_f[i].reserve(rows_f * chunk * sizeof(float)))) return rc;
     }
-    const bool page_x = is_pageable(h_measure), page_thr = !d_thr && is_pageable(h_thr), page_out = h_out && is_pageable(h_out);
-    const bool page_int = h_int && is_pageable(h_int);
+    bool page_x[2] = {}, page_thr[2] = {};
+    for (int m = 0; m < n_measures; m++) {
+        page_x[m] = is_pageable(hm[m].x);
+        page_thr[m] = !hm[m].d_thr && is_pageable(hm[m].h_thr);
+    }
+    const bool page_out = h_out && is_pageable(h_out), page_int = h_int && is_pageable(h_int);
     const bool page_south = h_is_south && is_pageable(h_is_south);
-    const bool page_xb = pair && is_pageable(m2.h), page_thr_b = pair && !m2.d_thr && is_pageable(m2.h_thr);
     int64_t i = 0;
     for (int64_t c0 = 0; c0 < C; c0 += chunk, i++) {
         const int slot = (int)(i % kSlots);
         const int64_t nc = std::min(chunk, C - c0);
-        int64_t a, b;
+        const size_t thr_off = (size_t)c0 * n_doy * P;
+        Measure dm[2];                                                         // the chunk's measures on the device
         HDP_HOST_CUDA(cudaStreamWaitEvent(ctx->s_in, ctx->k_done[slot], 0));
-        HDP_HOST_TRY(upload_cells(ctx, h_measure, page_x, T, ld_t, ld_c, c0, nc, (float *)ctx->x[slot].p, &a, &b, ctx->s_in));
-        if (!d_thr)                                                            // device-resident thresholds never cross PCIe again
-            HDP_HOST_TRY(ctx->h2d((char *)ctx->aux[slot].p, 0, (const char *)(h_thr + (size_t)c0 * n_doy * P), 0, (size_t)nc * thr_per_cell, 1,
-                                  page_thr, ctx->s_in));
-        SecondMeasure sb;
-        if (pair) {
-            HDP_HOST_TRY(upload_cells(ctx, m2.h, page_xb, T, m2.ld_t, m2.ld_c, c0, nc, (float *)ctx->x_b[slot].p, &sb.ld_t, &sb.ld_c, ctx->s_in));
-            if (!m2.d_thr)
-                HDP_HOST_TRY(ctx->h2d((char *)ctx->aux_b[slot].p, 0, (const char *)(m2.h_thr + (size_t)c0 * n_doy * P), 0,
-                                      (size_t)nc * thr_per_cell, 1, page_thr_b, ctx->s_in));
-            sb.x = (const float *)ctx->x_b[slot].p;
-            sb.thr = m2.d_thr ? m2.d_thr + (size_t)c0 * n_doy * P : (const double *)ctx->aux_b[slot].p;
+        for (int m = 0; m < n_measures; m++) {
+            dm[m].x = (const float *)ctx->x[m][slot].p;
+            HDP_HOST_TRY(upload_cells(ctx, hm[m].x, page_x[m], T, hm[m].ld_t, hm[m].ld_c, c0, nc, (float *)ctx->x[m][slot].p, &dm[m].ld_t,
+                                      &dm[m].ld_c, ctx->s_in));
+            if (!hm[m].d_thr)                                                  // device-resident thresholds never cross PCIe again
+                HDP_HOST_TRY(ctx->h2d((char *)ctx->thr[m][slot].p, 0, (const char *)(hm[m].h_thr + thr_off), 0, (size_t)nc * thr_per_cell, 1,
+                                      page_thr[m], ctx->s_in));
+            dm[m].thr = hm[m].d_thr ? hm[m].d_thr + thr_off : (const double *)ctx->thr[m][slot].p;
         }
         if (h_is_south)
             HDP_HOST_TRY(ctx->h2d((char *)ctx->south[slot].p, 0, (const char *)(h_is_south + c0), 0, (size_t)nc, 1, page_south, ctx->s_in));
@@ -403,11 +401,10 @@ static int metric_pass_host(const float *h_measure, int64_t C, int64_t T, int64_
 
         HDP_HOST_CUDA(cudaStreamWaitEvent(ctx->s_k, ctx->in_ready[slot], 0));
         HDP_HOST_CUDA(cudaStreamWaitEvent(ctx->s_k, ctx->out_done[slot], 0));
-        const double *thr_chunk = d_thr ? d_thr + (size_t)c0 * n_doy * P : (const double *)ctx->aux[slot].p;
         const uint8_t *south_chunk = h_is_south ? (const uint8_t *)ctx->south[slot].p : nullptr;
-        HDP_HOST_TRY(metric_pass((const float *)ctx->x[slot].p, nc, T, a, b, thr_chunk, n_doy, P, h_doy_map, h_defs, D,
-                                 h_season_north, h_season_south, Y, south_chunk, h_out ? (uint16_t *)ctx->out[slot].p : nullptr,
-                                 h_int ? (float *)ctx->out_f[slot].p : nullptr, ctx->ws.p, ws_bytes, ctx->s_k, chunk, i > 0, input_unit, sb));
+        HDP_HOST_TRY(metric_pass(dm, n_measures, nc, T, n_doy, P, h_doy_map, h_defs, D, h_season_north, h_season_south, Y, south_chunk,
+                                 h_out ? (uint16_t *)ctx->out[slot].p : nullptr, h_int ? (float *)ctx->out_f[slot].p : nullptr,
+                                 ctx->ws.p, ws_bytes, ctx->s_k, chunk, i > 0, input_unit));
         HDP_HOST_CUDA(cudaEventRecord(ctx->k_done[slot], ctx->s_k));
 
         // device chunk is [rows, nc]; host array is [rows, C]
@@ -429,7 +426,7 @@ void hdp_b200_host_release(void)
 {
     for (HostCtx &c : g_ctx) {
         std::lock_guard<std::mutex> lock(c.mu);
-        if (c.ready || c.ws.p || c.x[0].p) c.release();
+        if (c.ready || c.ws.p || c.x[0][0].p) c.release();
     }
 }
 
@@ -454,7 +451,7 @@ int hdp_b200_thresholds_host(const float *h_temps, int64_t C, int64_t T_b, int64
     const size_t ws_bytes = hdp_b200_thresholds_workspace_bytes(chunk, T_b, dl_t, dl_c, n_doy, n_y, W, P, input_unit);
     if ((rc = ctx->ws.reserve(ws_bytes))) return rc;
     for (int i = 0; i < kSlots; i++) {
-        if ((rc = ctx->x[i].reserve((size_t)chunk * T_b * sizeof(float)))) return rc;
+        if ((rc = ctx->x[0][i].reserve((size_t)chunk * T_b * sizeof(float)))) return rc;
         if (!d_keep && (rc = ctx->out[i].reserve((size_t)chunk * out_per_cell))) return rc;
     }
     const bool page_in = is_pageable(h_temps), page_out = is_pageable(h_out);
@@ -465,7 +462,7 @@ int hdp_b200_thresholds_host(const float *h_temps, int64_t C, int64_t T_b, int64
         int64_t a, b;
         // stage 1: samples of this chunk (the slot's previous user must have been consumed by its kernels)
         HDP_HOST_CUDA(cudaStreamWaitEvent(ctx->s_in, ctx->k_done[slot], 0));
-        HDP_HOST_TRY(upload_cells(ctx, h_temps, page_in, T_b, ld_t, ld_c, c0, nc, (float *)ctx->x[slot].p, &a, &b, ctx->s_in));
+        HDP_HOST_TRY(upload_cells(ctx, h_temps, page_in, T_b, ld_t, ld_c, c0, nc, (float *)ctx->x[0][slot].p, &a, &b, ctx->s_in));
         HDP_HOST_CUDA(cudaEventRecord(ctx->in_ready[slot], ctx->s_in));
         // stage 2: kernels (the slot's previous results must have left for the host)
         // with d_keep the kernels write the chunk straight into its place in the caller's device-resident copy (which then feeds
@@ -473,7 +470,7 @@ int hdp_b200_thresholds_host(const float *h_temps, int64_t C, int64_t T_b, int64
         double *d_chunk_out = d_keep ? d_keep + (size_t)c0 * n_doy * P : (double *)ctx->out[slot].p;
         HDP_HOST_CUDA(cudaStreamWaitEvent(ctx->s_k, ctx->in_ready[slot], 0));
         if (!d_keep) HDP_HOST_CUDA(cudaStreamWaitEvent(ctx->s_k, ctx->out_done[slot], 0));
-        HDP_HOST_TRY(thresholds_launch((const float *)ctx->x[slot].p, nc, T_b, a, b, h_time_index, h_win_rows, n_doy, n_y, W, h_q, P,
+        HDP_HOST_TRY(thresholds_launch((const float *)ctx->x[0][slot].p, nc, T_b, a, b, h_time_index, h_win_rows, n_doy, n_y, W, h_q, P,
                                        d_chunk_out, ctx->ws.p, ws_bytes, ctx->s_k, chunk, i > 0, input_unit));
         HDP_HOST_CUDA(cudaEventRecord(ctx->k_done[slot], ctx->s_k));
         // stage 3: results
@@ -492,8 +489,9 @@ int hdp_b200_metrics_host(const float *h_measure, int64_t C, int64_t T, int64_t 
                           const uint8_t *h_is_south, uint16_t *h_out, int input_unit)
 {
     if (!h_out && C > 0 && Y > 0) return HDP_B200_ERR_INVALID;
-    return metric_pass_host(h_measure, C, T, ld_t, ld_c, h_thr, d_thr, n_doy, P, h_doy_map, h_defs, D, h_season_north, h_season_south, Y,
-                            h_is_south, nullptr, h_out, input_unit);
+    const HostMeasure m = {h_measure, ld_t, ld_c, h_thr, d_thr};
+    return metric_pass_host(&m, 1, C, T, n_doy, P, h_doy_map, h_defs, D, h_season_north, h_season_south, Y, h_is_south, nullptr, h_out,
+                            input_unit);
 }
 
 int hdp_b200_intensity_host(const float *h_measure, int64_t C, int64_t T, int64_t ld_t, int64_t ld_c,
@@ -503,8 +501,9 @@ int hdp_b200_intensity_host(const float *h_measure, int64_t C, int64_t T, int64_
                             const uint8_t *h_is_south, float *h_int, uint16_t *h_out, int input_unit)
 {
     if (!h_int && C > 0 && Y > 0) return HDP_B200_ERR_INVALID;
-    return metric_pass_host(h_measure, C, T, ld_t, ld_c, h_thr, d_thr, n_doy, P, h_doy_map, h_defs, D, h_season_north, h_season_south, Y,
-                            h_is_south, h_int, h_out, input_unit);
+    const HostMeasure m = {h_measure, ld_t, ld_c, h_thr, d_thr};
+    return metric_pass_host(&m, 1, C, T, n_doy, P, h_doy_map, h_defs, D, h_season_north, h_season_south, Y, h_is_south, h_int, h_out,
+                            input_unit);
 }
 
 int hdp_b200_compound_host(const float *h_a, int64_t ld_t_a, int64_t ld_c_a, const float *h_b, int64_t ld_t_b, int64_t ld_c_b,
@@ -514,11 +513,10 @@ int hdp_b200_compound_host(const float *h_a, int64_t ld_t_a, int64_t ld_c_a, con
                            const uint8_t *h_is_south, uint16_t *h_out, float *h_int, int input_unit)
 {
     if (C > 0 && Y > 0 && !h_out && !h_int) return HDP_B200_ERR_INVALID;
-    if (C > 0 && !h_b) return HDP_B200_ERR_INVALID;
-    HostSecond b;
-    b.h = h_b; b.ld_t = ld_t_b; b.ld_c = ld_c_b; b.h_thr = h_thr_b; b.d_thr = d_thr_b;
-    return metric_pass_host(h_a, C, T, ld_t_a, ld_c_a, h_thr_a, d_thr_a, n_doy, P, h_doy_map, h_defs, D, h_season_north, h_season_south, Y,
-                            h_is_south, h_int, h_out, input_unit, b);
+    if (C > 0 && !h_b) return HDP_B200_ERR_INVALID;                       // (also when metric_pass_host has nothing to do)
+    const HostMeasure ms[2] = {{h_a, ld_t_a, ld_c_a, h_thr_a, d_thr_a}, {h_b, ld_t_b, ld_c_b, h_thr_b, d_thr_b}};
+    return metric_pass_host(ms, 2, C, T, n_doy, P, h_doy_map, h_defs, D, h_season_north, h_season_south, Y, h_is_south, h_int, h_out,
+                            input_unit);
 }
 
 }  // extern "C"

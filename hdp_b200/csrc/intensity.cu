@@ -117,9 +117,9 @@ k_intensity(const uint32_t *__restrict__ hot, const float *__restrict__ x, int64
     while (L.open()) { flush(); L.next(); }
 }
 
-int run_intensity(const Layout &L, const WordPlan &plan, const float *x, int64_t x_ld_t, int64_t C, int64_t T,
-                  const double *d_thr, int n_doy, int P, const int32_t *h_defs, int D, const std::vector<int32_t> &seasons, int Y,
-                  const uint8_t *d_is_south, float *d_int, cudaStream_t st, bool tables_resident, int unit, bool cold)
+int run_intensity(const Layout &L, const WordPlan &plan, int m, int64_t C, int64_t T, int P, const int32_t *h_defs, int D,
+                  const std::vector<int32_t> &seasons, int Y, const uint8_t *d_is_south, float *d_int, cudaStream_t st,
+                  bool tables_resident, int unit, bool cold)
 {
     const int K = (int)plan.words.size();
     const size_t words_bytes = ((size_t)K * sizeof(int2) + 15) & ~(size_t)15;
@@ -136,7 +136,7 @@ int run_intensity(const Layout &L, const WordPlan &plan, const float *x, int64_t
     KernelTimer timer(kIntensity, st);
     const auto kernel = cold ? k_intensity<true> : k_intensity<false>;
     HDP_CUDA_TRY(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    kernel<<<grid, wpc * 32, smem, st>>>(L.hot, x, x_ld_t, d_thr, n_doy, C, K, (int)T, L.words, P, D, defs,
+    kernel<<<grid, wpc * 32, smem, st>>>(L.hot, L.x[m], L.ld_t[m], L.thr[m], L.n_doy, C, K, (int)T, L.words, P, D, defs,
                                          L.int_seasons, Y, L.int_seasons + (Y + 1), Y, Y, d_is_south, unit, wpc, d_int);
     HDP_LAUNCH_CHECK();
     return HDP_B200_OK;
@@ -152,7 +152,7 @@ size_t hdp_b200_intensity_workspace_bytes(int64_t C, int64_t T, int64_t ld_t, in
                                           int n_doy, int P, int D, int Y, const int32_t *h_doy_map)
 {
     (void)ld_t; (void)D;
-    return metric_pass_workspace_bytes(C, T, ld_c, n_doy, P, Y, h_doy_map, true);
+    return metric_pass_workspace_bytes(C, T, &ld_c, 1, n_doy, P, Y, h_doy_map, true);
 }
 
 int hdp_b200_intensity(const float *d_measure, int64_t C, int64_t T, int64_t ld_t, int64_t ld_c,
@@ -163,8 +163,9 @@ int hdp_b200_intensity(const float *d_measure, int64_t C, int64_t T, int64_t ld_
                        void *d_workspace, size_t workspace_bytes, void *stream, int input_unit)
 {
     if (C > 0 && Y > 0 && !d_int) return HDP_B200_ERR_INVALID;
-    return metric_pass(d_measure, C, T, ld_t, ld_c, d_thr, n_doy, P, h_doy_map, h_defs, D, h_season_north, h_season_south, Y,
-                       d_is_south, d_out, d_int, d_workspace, workspace_bytes, stream, C, false, input_unit);
+    const Measure m = {d_measure, ld_t, ld_c, d_thr};
+    return metric_pass(&m, 1, C, T, n_doy, P, h_doy_map, h_defs, D, h_season_north, h_season_south, Y, d_is_south, d_out, d_int,
+                       d_workspace, workspace_bytes, stream, C, false, input_unit);
 }
 
 }  // extern "C"

@@ -613,14 +613,13 @@ int pick_pg(int P)
     return best;
 }
 
-// Workspace layout; `intensity` appends the intensity pass's season tables behind what the metric pass uses, `pair` the second
-// measure's normalised copy (need_norm_b) and replicated thresholds of a compound pass.
-static Layout carve(void *ws, size_t ws_bytes, int64_t C, int64_t T, bool need_norm, int64_t K, int n_doy, int P, int Y, bool intensity,
-                    bool pair = false, bool need_norm_b = false)
+// Workspace layout; `intensity` appends the intensity pass's season tables behind what the metric pass uses, then each of the
+// n_measures measures its normalised copy (need_norm[m]) and, for n_doy = 1, its replicated thresholds.
+static Layout carve(void *ws, size_t ws_bytes, int64_t C, int64_t T, int n_measures, const bool *need_norm, int64_t K, int n_doy, int P,
+                    int Y, bool intensity)
 {
     Layout L;
     Carver cv(ws, ws_bytes);
-    if (need_norm) L.xn = cv.take<float>((size_t)C * T);
     L.words = cv.take<int4>((size_t)K + 1);
     L.blk_start = cv.take<int>((size_t)(pass_n_doy(n_doy) + kTileDoy - 1) / kTileDoy + 1);
     L.blk_words = cv.take<int>((size_t)K + 1);
@@ -628,9 +627,10 @@ static Layout carve(void *ws, size_t ws_bytes, int64_t C, int64_t T, bool need_n
     L.lut = cv.take<uint32_t>((size_t)2 * 8192);
     L.hot = cv.take<uint32_t>((size_t)P * K * C);
     if (intensity) L.int_seasons = cv.take<int4>((size_t)2 * (Y + 1));
-    if (n_doy == 1) L.thr_rep = cv.take<double>((size_t)C * kTileDoy * P);
-    if (pair && need_norm_b) L.xn_b = cv.take<float>((size_t)C * T);
-    if (pair && n_doy == 1) L.thr_rep_b = cv.take<double>((size_t)C * kTileDoy * P);
+    for (int m = 0; m < n_measures; m++) {
+        if (need_norm[m]) L.xn[m] = cv.take<float>((size_t)C * T);
+        if (n_doy == 1) L.thr_rep[m] = cv.take<double>((size_t)C * kTileDoy * P);
+    }
     L.total = cv.off;
     return L;
 }
@@ -640,24 +640,23 @@ static bool bad_dims(int64_t C, int64_t T, int n_doy, int P)
     return C < 0 || T < 0 || n_doy <= 0 || P <= 0 || T > 0x3fffffff;
 }
 
-size_t metric_pass_workspace_bytes(int64_t C, int64_t T, int64_t ld_c, int n_doy, int P, int Y, const int32_t *h_doy_map, bool intensity,
-                                   bool pair, int64_t ld_c_b)
+size_t metric_pass_workspace_bytes(int64_t C, int64_t T, const int64_t *ld_c, int n_measures, int n_doy, int P, int Y,
+                                   const int32_t *h_doy_map, bool intensity)
 {
     if (bad_dims(C, T, n_doy, P) || Y < 0) return 0;
     const int64_t K = n_doy == 1 ? (T + kTileDoy - 1) / kTileDoy : h_doy_map ? count_words(h_doy_map, T) : words_upper_bound(T, n_doy);
-    return carve(nullptr, 0, C, T, ld_c != 1, K, n_doy, P, Y, intensity, pair, ld_c_b != 1).total;
+    bool need_norm[2] = {};
+    for (int m = 0; m < n_measures; m++) need_norm[m] = ld_c[m] != 1;
+    return carve(nullptr, 0, C, T, n_measures, need_norm, K, n_doy, P, Y, intensity).total;
 }
 
-// Runs k_hot_words (after the layout-normalising copy when ld_c != 1: the samples then live in L.xn, time-major, ld_t = C);
-// on success plan / L describe what lives in the workspace, L.thr / L.n_doy the thresholds and L.x / L.ld_t the samples the
-// kernels read.  `unit` is a plain unit code (0 - 2); `cold` makes the words cold-day bits.  With a second measure (b.x) it
-// prepares that one the same way (L.x_b, L.thr_b) and runs k_hot_pair instead: the words then mark the days on which both
-// measures pass their thresholds.
-static int run_hot_words(const float *d_measure, int64_t C, int64_t T, int64_t ld_t, int64_t ld_c,
-                         const double *d_thr, int n_doy, int P, const int32_t *h_doy_map,
+// Prepares each of the n_measures measures (its thresholds replicated for n_doy = 1, its samples copied to time-major L.xn[m], ld_t
+// = C, when ld_c != 1) and runs k_hot_words on one measure, k_hot_pair on two: the words then mark the days on which both measures
+// pass their thresholds.  On success plan / L describe what lives in the workspace, L.thr / L.n_doy the thresholds and L.x / L.ld_t
+// the samples the kernels read.  `unit` is a plain unit code (0 - 2); `cold` makes the words cold-day bits.
+static int run_hot_words(const Measure *ms, int n_measures, int64_t C, int64_t T, int n_doy, int P, const int32_t *h_doy_map,
                          int Y, void *ws, size_t ws_bytes, cudaStream_t st, WordPlan &plan, Layout &L,
-                         int64_t carve_cells = 0, bool tables_resident = false, int unit = 0, bool intensity = false, bool cold = false,
-                         const SecondMeasure &b = SecondMeasure())
+                         int64_t carve_cells = 0, bool tables_resident = false, int unit = 0, bool intensity = false, bool cold = false)
 {
     if (unit < 0 || unit > 2) return HDP_B200_ERR_INVALID;
     std::vector<int32_t> own_map;
@@ -667,78 +666,45 @@ static int run_hot_words(const float *d_measure, int64_t C, int64_t T, int64_t l
     rc = build_words(doy_map, T, pass_n_doy(n_doy), plan);
     if (rc != HDP_B200_OK) return rc;
     const int K = (int)plan.words.size();
-    const bool need_norm = ld_c != 1, pair = b.x != nullptr;
-    L = carve(ws, ws_bytes, std::max(C, carve_cells), T, need_norm, K, n_doy, P, Y, intensity, pair, b.ld_c != 1);
+    bool need_norm[2] = {};
+    for (int m = 0; m < n_measures; m++) need_norm[m] = ms[m].ld_c != 1;
+    L = carve(ws, ws_bytes, std::max(C, carve_cells), T, n_measures, need_norm, K, n_doy, P, Y, intensity);
     if (ws == nullptr || L.total > ws_bytes) return HDP_B200_ERR_WORKSPACE;
-    L.thr = d_thr;
     L.n_doy = pass_n_doy(n_doy);
-    L.x = d_measure;
-    L.ld_t = ld_t;
-    L.thr_b = b.thr;
-    L.x_b = b.x;
-    L.ld_t_b = b.ld_t;
+    for (int m = 0; m < n_measures; m++) {
+        L.thr[m] = ms[m].thr;
+        L.x[m] = ms[m].x;
+        L.ld_t[m] = ms[m].ld_t;
+    }
     if (C == 0 || T == 0) return HDP_B200_OK;
-    if (L.thr_rep) {
-        rc = replicate_rows(d_thr, C, P, L.thr_rep, st);
-        if (rc != HDP_B200_OK) return rc;
-        L.thr = L.thr_rep;
-    }
-    const float *x = d_measure;
-    if (need_norm) {
-        rc = normalize_layout(d_measure, C, T, ld_t, ld_c, L.xn, st);
-        if (rc != HDP_B200_OK) return rc;
-        x = L.xn;
-        ld_t = C;
-    }
-    L.x = x;
-    L.ld_t = ld_t;
-    if (pair && L.thr_rep_b) {
-        rc = replicate_rows(b.thr, C, P, L.thr_rep_b, st);
-        if (rc != HDP_B200_OK) return rc;
-        L.thr_b = L.thr_rep_b;
-    }
-    if (pair && L.xn_b) {
-        rc = normalize_layout(b.x, C, T, b.ld_t, b.ld_c, L.xn_b, st);
-        if (rc != HDP_B200_OK) return rc;
-        L.x_b = L.xn_b;
-        L.ld_t_b = C;
+    for (int m = 0; m < n_measures; m++) {
+        if (L.thr_rep[m]) {
+            rc = replicate_rows(ms[m].thr, C, P, L.thr_rep[m], st);
+            if (rc != HDP_B200_OK) return rc;
+            L.thr[m] = L.thr_rep[m];
+        }
+        if (L.xn[m]) {
+            rc = normalize_layout(ms[m].x, C, T, ms[m].ld_t, ms[m].ld_c, L.xn[m], st);
+            if (rc != HDP_B200_OK) return rc;
+            L.x[m] = L.xn[m];
+            L.ld_t[m] = C;
+        }
     }
     if (!tables_resident) HDP_CUDA_TRY(cudaMemcpyAsync(L.words, plan.words.data(), sizeof(int4) * K, cudaMemcpyHostToDevice, st));
     if (!tables_resident) HDP_CUDA_TRY(cudaMemcpyAsync(L.blk_start, plan.blk_start.data(), sizeof(int) * plan.blk_start.size(), cudaMemcpyHostToDevice, st));
     if (!tables_resident) HDP_CUDA_TRY(cudaMemcpyAsync(L.blk_words, plan.blk_words.data(), sizeof(int) * K, cudaMemcpyHostToDevice, st));
-    if (pair) return run_hot_pair(L, plan, C, P, st, unit, cold);
+    if (n_measures == 2) return run_hot_pair(L, plan, C, P, st, unit, cold);
 
     const int pg = pick_pg(P);
     const int Ppad = (P + pg - 1) / pg * pg;
     const size_t smem = (size_t)kTileDoy * Ppad * kTilePad * sizeof(float);
     dim3 grid((unsigned)((C + kTileCells - 1) / kTileCells), (unsigned)plan.n_blk);
+    const auto kernel = hot_kernel(pg, unit, cold, [](auto PG, auto U, auto CO) {
+        return k_hot_words<decltype(PG)::value, decltype(U)::value, decltype(CO)::value>;
+    });
     KernelTimer timer(kHotWords, st);
-#define HDP_LAUNCH_HOT_D(PG, U, CO)                                                                                \
-    do {                                                                                                           \
-        HDP_CUDA_TRY(cudaFuncSetAttribute(k_hot_words<PG, U, CO>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)); \
-        k_hot_words<PG, U, CO><<<grid, 256, smem, st>>>(x, C, ld_t, L.thr, L.n_doy, P, L.words, L.blk_start, L.blk_words, K, L.hot); \
-    } while (0)
-#define HDP_LAUNCH_HOT_U(PG, U)                                                                                    \
-    do {                                                                                                           \
-        if (cold) HDP_LAUNCH_HOT_D(PG, U, true);                                                                   \
-        else HDP_LAUNCH_HOT_D(PG, U, false);                                                                       \
-    } while (0)
-#define HDP_LAUNCH_HOT(PG)                                                                                         \
-    do {                                                                                                           \
-        if (unit == 0) HDP_LAUNCH_HOT_U(PG, 0);                                                                    \
-        else if (unit == 1) HDP_LAUNCH_HOT_U(PG, 1);                                                               \
-        else HDP_LAUNCH_HOT_U(PG, 2);                                                                              \
-    } while (0)
-    switch (pg) {
-    case 4: HDP_LAUNCH_HOT(4); break;
-    case 8: HDP_LAUNCH_HOT(8); break;
-    case 10: HDP_LAUNCH_HOT(10); break;
-    case 16: HDP_LAUNCH_HOT(16); break;
-    default: HDP_LAUNCH_HOT(20); break;
-    }
-#undef HDP_LAUNCH_HOT
-#undef HDP_LAUNCH_HOT_U
-#undef HDP_LAUNCH_HOT_D
+    HDP_CUDA_TRY(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    kernel<<<grid, 256, smem, st>>>(L.x[0], C, L.ld_t[0], L.thr[0], L.n_doy, P, L.words, L.blk_start, L.blk_words, K, L.hot);
     HDP_LAUNCH_CHECK();
     return HDP_B200_OK;
 }
@@ -906,17 +872,23 @@ static int run_scan(const Layout &L, const WordPlan &plan, int64_t C, int64_t T,
     return HDP_B200_OK;
 }
 
-int metric_pass(const float *d_measure, int64_t C, int64_t T, int64_t ld_t, int64_t ld_c,
-                const double *d_thr, int n_doy, int P, const int32_t *h_doy_map,
+// Every measure of a pass must have samples and thresholds once there is work
+static bool missing_measure(const Measure *ms, int n_measures, int64_t C, int64_t T)
+{
+    for (int m = 0; m < n_measures; m++)
+        if (C > 0 && T > 0 && (!ms[m].x || !ms[m].thr)) return true;
+    return false;
+}
+
+int metric_pass(const Measure *ms, int n_measures, int64_t C, int64_t T, int n_doy, int P, const int32_t *h_doy_map,
                 const int32_t *h_defs, int D,
                 const int32_t *h_season_north, const int32_t *h_season_south, int Y,
                 const uint8_t *d_is_south, uint16_t *d_out, float *d_int,
-                void *d_workspace, size_t workspace_bytes, void *stream, int64_t carve_cells, bool tables_resident, int input_unit,
-                const SecondMeasure &b)
+                void *d_workspace, size_t workspace_bytes, void *stream, int64_t carve_cells, bool tables_resident, int input_unit)
 {
     if (bad_dims(C, T, n_doy, P) || D <= 0 || Y < 0) return HDP_B200_ERR_INVALID;
     if ((T > 0 && !h_doy_map) || !h_defs || (Y > 0 && (!h_season_north || !h_season_south))) return HDP_B200_ERR_INVALID;
-    if (C > 0 && T > 0 && (!d_measure || !d_thr || (b.x && !b.thr))) return HDP_B200_ERR_INVALID;
+    if (missing_measure(ms, n_measures, C, T)) return HDP_B200_ERR_INVALID;
     if (P > HDP_B200_MAX_PERCENTILES || D > HDP_B200_MAX_DEFINITIONS) return HDP_B200_ERR_UNSUPPORTED;
     cudaStream_t st = (cudaStream_t)stream;
     // input_unit of the C ABI = unit code | HDP_B200_COLD; the kernels' launchers see the two as plain values
@@ -938,35 +910,31 @@ int metric_pass(const float *d_measure, int64_t C, int64_t T, int64_t ld_t, int6
 
     WordPlan plan;
     Layout L;
-    int rc = run_hot_words(d_measure, C, T, ld_t, ld_c, d_thr, n_doy, P, h_doy_map, Y, d_workspace, workspace_bytes, st, plan, L,
-                           carve_cells, tables_resident, unit, d_int != nullptr, cold, b);
+    int rc = run_hot_words(ms, n_measures, C, T, n_doy, P, h_doy_map, Y, d_workspace, workspace_bytes, st, plan, L,
+                           carve_cells, tables_resident, unit, d_int != nullptr, cold);
     if (rc != HDP_B200_OK || C == 0 || Y == 0) return rc;
     if (d_out) {
         rc = run_scan(L, plan, C, T, P, h_defs, D, passes, Y, d_is_south, d_out, st, tables_resident);
         if (rc != HDP_B200_OK) return rc;
     }
-    if (d_int)
-        rc = run_intensity(L, plan, L.x, L.ld_t, C, T, L.thr, L.n_doy, P, h_defs, D, seasons, Y, d_is_south, d_int, st,
-                           tables_resident, unit, cold);
-    if (d_int && b.x && rc == HDP_B200_OK)                                  // the second measure's block, on the same words
-        rc = run_intensity(L, plan, L.x_b, L.ld_t_b, C, T, L.thr_b, L.n_doy, P, h_defs, D, seasons, Y, d_is_south,
-                           d_int + (size_t)3 * P * D * Y * C, st, true, unit, cold);
+    for (int m = 0; d_int && m < n_measures && rc == HDP_B200_OK; m++)     // one block per measure, on the same words
+        rc = run_intensity(L, plan, m, C, T, P, h_defs, D, seasons, Y, d_is_south, d_int + (size_t)m * 3 * P * D * Y * C, st,
+                           tables_resident || m > 0, unit, cold);
     return rc;
 }
 
 // hdp_b200_hot_days and hdp_b200_compound_hot_days: the hot words, unpacked to u8 [P, T, C]
-static int hot_days_pass(const float *d_measure, int64_t C, int64_t T, int64_t ld_t, int64_t ld_c,
-                         const double *d_thr, int n_doy, int P, const int32_t *h_doy_map,
-                         uint8_t *d_mask, void *d_workspace, size_t workspace_bytes, void *stream, int unit, bool cold, const SecondMeasure &b)
+static int hot_days_pass(const Measure *ms, int n_measures, int64_t C, int64_t T, int n_doy, int P, const int32_t *h_doy_map,
+                         uint8_t *d_mask, void *d_workspace, size_t workspace_bytes, void *stream, int unit, bool cold)
 {
     if (bad_dims(C, T, n_doy, P) || !h_doy_map && T > 0) return HDP_B200_ERR_INVALID;
-    if (C > 0 && T > 0 && (!d_measure || !d_thr || !d_mask || (b.x && !b.thr))) return HDP_B200_ERR_INVALID;
+    if (missing_measure(ms, n_measures, C, T) || (C > 0 && T > 0 && !d_mask)) return HDP_B200_ERR_INVALID;
     if (P > HDP_B200_MAX_PERCENTILES) return HDP_B200_ERR_UNSUPPORTED;
     cudaStream_t st = (cudaStream_t)stream;
     WordPlan plan;
     Layout L;
-    int rc = run_hot_words(d_measure, C, T, ld_t, ld_c, d_thr, n_doy, P, h_doy_map, 0, d_workspace, workspace_bytes, st, plan, L,
-                           0, false, unit, false, cold, b);
+    int rc = run_hot_words(ms, n_measures, C, T, n_doy, P, h_doy_map, 0, d_workspace, workspace_bytes, st, plan, L,
+                           0, false, unit, false, cold);
     if (rc != HDP_B200_OK || C == 0 || T == 0) return rc;
     const int K = (int)plan.words.size();
     dim3 grid((unsigned)((C + 255) / 256), (unsigned)K);
@@ -987,7 +955,7 @@ size_t hdp_b200_metrics_workspace_bytes(int64_t C, int64_t T, int64_t ld_t, int6
                                         int n_doy, int P, int D, int Y, const int32_t *h_doy_map)
 {
     (void)ld_t; (void)D;
-    return metric_pass_workspace_bytes(C, T, ld_c, n_doy, P, Y, h_doy_map, false);
+    return metric_pass_workspace_bytes(C, T, &ld_c, 1, n_doy, P, Y, h_doy_map, false);
 }
 
 void hdp_b200_metrics_run_filter(int on) { g_scan_filter = on != 0; }
@@ -1017,8 +985,8 @@ int hdp_b200_hot_days(const float *d_measure, int64_t C, int64_t T, int64_t ld_t
                       const double *d_thr, int n_doy, int P, const int32_t *h_doy_map,
                       uint8_t *d_mask, void *d_workspace, size_t workspace_bytes, void *stream)
 {
-    return hot_days_pass(d_measure, C, T, ld_t, ld_c, d_thr, n_doy, P, h_doy_map, d_mask, d_workspace, workspace_bytes, stream, 0, false,
-                         SecondMeasure());
+    const Measure m = {d_measure, ld_t, ld_c, d_thr};
+    return hot_days_pass(&m, 1, C, T, n_doy, P, h_doy_map, d_mask, d_workspace, workspace_bytes, stream, 0, false);
 }
 
 int hdp_b200_compound_hot_days(const float *d_a, int64_t ld_t_a, int64_t ld_c_a, const float *d_b, int64_t ld_t_b, int64_t ld_c_b,
@@ -1026,11 +994,9 @@ int hdp_b200_compound_hot_days(const float *d_a, int64_t ld_t_a, int64_t ld_c_a,
                                const int32_t *h_doy_map, uint8_t *d_mask, void *d_workspace, size_t workspace_bytes, void *stream,
                                int input_unit)
 {
-    if (C > 0 && T > 0 && !d_b) return HDP_B200_ERR_INVALID;
-    SecondMeasure b;
-    b.x = d_b; b.ld_t = ld_t_b; b.ld_c = ld_c_b; b.thr = d_thr_b;
-    return hot_days_pass(d_a, C, T, ld_t_a, ld_c_a, d_thr_a, n_doy, P, h_doy_map, d_mask, d_workspace, workspace_bytes, stream,
-                         input_unit & ~HDP_B200_COLD, (input_unit & HDP_B200_COLD) != 0, b);
+    const Measure ms[2] = {{d_a, ld_t_a, ld_c_a, d_thr_a}, {d_b, ld_t_b, ld_c_b, d_thr_b}};
+    return hot_days_pass(ms, 2, C, T, n_doy, P, h_doy_map, d_mask, d_workspace, workspace_bytes, stream, input_unit & ~HDP_B200_COLD,
+                         (input_unit & HDP_B200_COLD) != 0);
 }
 
 int hdp_b200_metrics(const float *d_measure, int64_t C, int64_t T, int64_t ld_t, int64_t ld_c,
@@ -1041,8 +1007,9 @@ int hdp_b200_metrics(const float *d_measure, int64_t C, int64_t T, int64_t ld_t,
                      void *d_workspace, size_t workspace_bytes, void *stream, int input_unit)
 {
     if (C > 0 && Y > 0 && !d_out) return HDP_B200_ERR_INVALID;
-    return metric_pass(d_measure, C, T, ld_t, ld_c, d_thr, n_doy, P, h_doy_map, h_defs, D, h_season_north, h_season_south, Y,
-                       d_is_south, d_out, nullptr, d_workspace, workspace_bytes, stream, C, false, input_unit);
+    const Measure m = {d_measure, ld_t, ld_c, d_thr};
+    return metric_pass(&m, 1, C, T, n_doy, P, h_doy_map, h_defs, D, h_season_north, h_season_south, Y, d_is_south, d_out, nullptr,
+                       d_workspace, workspace_bytes, stream, C, false, input_unit);
 }
 
 }  // extern "C"

@@ -1,7 +1,9 @@
-// metric.cuh - what the intensity kernel (intensity.cu) shares with the fused metric pass (metric.cu, metric_pass): the hot-day
-// words of k_hot_words and the workspace layout they live in.
+// metric.cuh - what the hot-word kernels (k_hot_words in metric.cu, k_hot_pair in compound.cu) and the intensity kernel
+// (intensity.cu) share with the fused metric pass (metric.cu, metric_pass): the tile constants, the instance dispatch, the hot-day
+// words and the workspace layout they live in.
 #pragma once
 
+#include <type_traits>
 #include <vector>
 
 #include "common.cuh"
@@ -29,6 +31,26 @@ __device__ __forceinline__ void or_if_lt(uint32_t &m, float v, float t, uint32_t
 }
 #endif
 
+// The instance of a hot-word kernel template <PG, UNIT, COLD> (k_hot_words, k_hot_pair) for percentile group size pg (pick_pg),
+// plain unit code `unit` (0 - 2) and direction `cold`: inst(PG, UNIT, COLD), called with std::integral_constant arguments, names it.
+template <class Inst>
+auto hot_kernel(int pg, int unit, bool cold, Inst inst)
+{
+    using std::integral_constant;
+    auto dir = [&](auto pg_c, auto unit_c) { return cold ? inst(pg_c, unit_c, std::true_type()) : inst(pg_c, unit_c, std::false_type()); };
+    auto by_unit = [&](auto pg_c) {
+        return unit == 0 ? dir(pg_c, integral_constant<int, 0>()) : unit == 1 ? dir(pg_c, integral_constant<int, 1>())
+                                                                              : dir(pg_c, integral_constant<int, 2>());
+    };
+    switch (pg) {
+    case 4: return by_unit(integral_constant<int, 4>());
+    case 8: return by_unit(integral_constant<int, 8>());
+    case 10: return by_unit(integral_constant<int, 10>());
+    case 16: return by_unit(integral_constant<int, 16>());
+    default: return by_unit(integral_constant<int, 20>());
+    }
+}
+
 struct WordPlan {
     std::vector<int4> words;        // {t0, nbits, doy of bit 0, 0}
     std::vector<int> blk_start;     // [n_blk + 1]
@@ -38,30 +60,25 @@ struct WordPlan {
 
 struct Layout {
     size_t total = 0;
-    float *xn = nullptr;
     int4 *words = nullptr;
     int *blk_start = nullptr, *blk_words = nullptr;
     int4 *seasons = nullptr;
     uint32_t *lut = nullptr;
     uint32_t *hot = nullptr;
     int4 *int_seasons = nullptr;    // intensity pass only: its season tables (north, then south)
-    double *thr_rep = nullptr;      // n_doy = 1 only: the thresholds replicated to kTileDoy rows (metric.cu, pass_n_doy)
-    const double *thr = nullptr;    // the thresholds the kernels read, [C, n_doy, P]: the caller's, or thr_rep
     int n_doy = 0;
-    const float *x = nullptr;       // the samples the kernels read, cell-contiguous, ld_t apart: the caller's, or xn
-    int64_t ld_t = 0;
-    // compound pass only (compound.cu): the same for the second measure
-    float *xn_b = nullptr;
-    double *thr_rep_b = nullptr;
-    const double *thr_b = nullptr;
-    const float *x_b = nullptr;
-    int64_t ld_t_b = 0;
+    // per measure of the pass (one, or two for a compound pass):
+    float *xn[2] = {};              // ld_c != 1 only: the samples normalised to cell-contiguous [T, C]
+    double *thr_rep[2] = {};        // n_doy = 1 only: the thresholds replicated to kTileDoy rows (metric.cu, pass_n_doy)
+    const double *thr[2] = {};      // the thresholds the kernels read, [C, n_doy, P]: the caller's, or thr_rep
+    const float *x[2] = {};         // the samples the kernels read, cell-contiguous, ld_t apart: the caller's, or xn
+    int64_t ld_t[2] = {};
 };
 
-// Workspace of metric_pass; `intensity` appends the intensity pass's season tables behind what the metric pass uses.  `pair`: a
-// compound pass, whose second measure has stride ld_c_b.
-size_t metric_pass_workspace_bytes(int64_t C, int64_t T, int64_t ld_c, int n_doy, int P, int Y, const int32_t *h_doy_map, bool intensity,
-                                   bool pair = false, int64_t ld_c_b = 1);
+// Workspace of metric_pass over n_measures measures with cell strides ld_c[]; `intensity` appends the intensity pass's season tables
+// behind what the metric pass uses.
+size_t metric_pass_workspace_bytes(int64_t C, int64_t T, const int64_t *ld_c, int n_measures, int n_doy, int P, int Y,
+                                   const int32_t *h_doy_map, bool intensity);
 
 // pick_pg: the percentiles per group of the hot-word kernels (PG of k_hot_words and k_hot_pair) for P percentiles
 int pick_pg(int P);
@@ -70,15 +87,14 @@ int pick_pg(int P);
 // percentiles; false when P is outside 1 .. HDP_B200_MAX_PERCENTILES
 bool hot_pair_plan(int P, int &pg, int &slices, int &groups_per_slice, size_t &smem);
 
-// k_hot_pair over the samples and thresholds in L (L.x / L.thr and L.x_b / L.thr_b): the compound hot-day words in L.hot
+// k_hot_pair over both measures' samples and thresholds in L: the compound hot-day words in L.hot
 int run_hot_pair(const Layout &L, const WordPlan &plan, int64_t C, int P, cudaStream_t st, int unit, bool cold);
 
-// k_intensity over the hot words in L: the intensity metrics f32 [3, P, D, Y, C] of the samples x (cell-contiguous, x_ld_t apart)
-// against d_thr.  `seasons` i32 [2, Y + 1, 4]: the season tables of both hemispheres as intensity_season_table (intensity.h)
-// accepts them.  `unit`: a plain unit code (0 - 2); `cold`: the words are cold-day bits and the intensity is the deficit below
-// the threshold.
-int run_intensity(const Layout &L, const WordPlan &plan, const float *x, int64_t x_ld_t, int64_t C, int64_t T,
-                  const double *d_thr, int n_doy, int P, const int32_t *h_defs, int D, const std::vector<int32_t> &seasons, int Y,
-                  const uint8_t *d_is_south, float *d_int, cudaStream_t st, bool tables_resident, int unit, bool cold);
+// k_intensity over the hot words in L: the intensity metrics f32 [3, P, D, Y, C] of measure m of L (its samples and thresholds).
+// `seasons` i32 [2, Y + 1, 4]: the season tables of both hemispheres as intensity_season_table (intensity.h) accepts them.  `unit`:
+// a plain unit code (0 - 2); `cold`: the words are cold-day bits and the intensity is the deficit below the threshold.
+int run_intensity(const Layout &L, const WordPlan &plan, int m, int64_t C, int64_t T, int P, const int32_t *h_defs, int D,
+                  const std::vector<int32_t> &seasons, int Y, const uint8_t *d_is_south, float *d_int, cudaStream_t st,
+                  bool tables_resident, int unit, bool cold);
 
 }  // namespace hdp

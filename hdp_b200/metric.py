@@ -210,41 +210,34 @@ def _threshold_cdp(threshold, measure, cell_dims):
     return np.ascontiguousarray(thr_vals).reshape(-1, n_doy, P)
 
 
-def _metric_sweep(measure, threshold, hw_definitions, time_axis, doy_map=None, intensity=False, cold=False, second=None):
-    """The percentile x definition x cell sweep of compute_heatwave_metrics_wrapper (metric.py:344-369) as ONE library call:
-    -> ((uint16 [4, P, D, Y, C], float32 [3, P, D, Y, C] or None), season tables, cell dims, cell shape, P, D).  With
-    ``intensity`` the call is the intensity pass, which also returns the intensity metrics.  With ``cold`` it is the cold-spell
-    pass, and each hemisphere's season is the other one's heatwave season (north Nov 1 - Apr 1, south May 1 - Oct 1).
-    ``second``: (measure B, threshold B) of a compound pass (:func:`compute_compound_metrics`), whose intensity output is float32
-    [2, 3, P, D, Y, C]."""
+def _metric_sweep(pairs, hw_definitions, time_axis, doy_map=None, intensity=False, cold=False):
+    """The percentile x definition x cell sweep of compute_heatwave_metrics_wrapper (metric.py:344-369) as ONE library call on one
+    (measure, threshold) pair, or on the two of a compound pass (:func:`compute_compound_metrics`):
+    -> ((uint16 [4, P, D, Y, C], float32 [3, P, D, Y, C] ([2, 3, P, D, Y, C] for two pairs) or None), season tables, cell dims, cell
+    shape, P, D).  With ``intensity`` the call is the intensity pass, which also returns the intensity metrics.  With ``cold`` it is
+    the cold-spell pass, and each hemisphere's season is the other one's heatwave season (north Nov 1 - Apr 1, south May 1 - Oct 1)."""
     st = _tables.hemisphere_ranges(time_axis)                       # compute_hemisphere_ranges, :410
     north, south_tab = (st.south, st.north) if cold else (st.north, st.south)
     if doy_map is None:
         doy_map = _tables.doy_map(time_axis.dayofyr)                # build_doy_map, :413
+    measure, threshold = pairs[0]
     x, cell_dims, cell_shape = _layout.to_time_cells(xr.values_of(measure), tuple(measure.dims), require_float32=True)
     south = _tables.is_south(_layout.cell_latitudes(xr.coord_values(measure, "lat"), cell_dims, cell_shape))
-    thr_cdp = _threshold_cdp(threshold, measure, cell_dims)
-    n_doy, P = thr_cdp.shape[1], thr_cdp.shape[2]
-
+    arrays = [x, _threshold_cdp(threshold, measure, cell_dims)]     # samples, thresholds of each pair
+    P = arrays[1].shape[2]
     defs = np.asarray(hw_definitions, dtype=np.int64).reshape(-1, 3)
-    if second is not None:
-        measure_b, threshold_b = second
+    for measure_b, threshold_b in pairs[1:]:
         x_b, cell_dims_b, _ = _layout.to_time_cells(xr.values_of(measure_b), tuple(measure_b.dims), require_float32=True)
         if cell_dims_b != cell_dims or x_b.shape != x.shape:
             raise ValueError("the two measures must have the same dims and shape")
-        thr_b = _threshold_cdp(threshold_b, measure, cell_dims)
-        args = (x, thr_cdp, x_b, thr_b, doy_map, defs, north, south_tab, south)
-        if intensity:
-            out = np.empty((4, P, defs.shape[0], st.n_years, x.shape[1]), np.uint16)
-            heat = _core.compound_intensity_host(*args, metrics_out=out, cold=cold)          # f32 [2, 3, P, D, Y, C]
-        else:
-            out, heat = _core.compound_metrics_host(*args, cold=cold), None
-        return (out, heat), st, cell_dims, cell_shape, P, defs.shape[0]
+        arrays += [x_b, _threshold_cdp(threshold_b, measure, cell_dims)]
+    args = (*arrays, doy_map, defs, north, south_tab, south)
+    one = len(pairs) == 1
     if intensity:
         out = np.empty((4, P, defs.shape[0], st.n_years, x.shape[1]), np.uint16)
-        heat = _core.intensity_host(x, thr_cdp, doy_map, defs, north, south_tab, south, metrics_out=out, cold=cold)   # f32 [3, P, D, Y, C]
+        heat = (_core.intensity_host if one else _core.compound_intensity_host)(*args, metrics_out=out, cold=cold)
     else:
-        out, heat = _core.metrics_host(x, thr_cdp, doy_map, defs, north, south_tab, south, cold=cold), None       # u16 [4, P, D, Y, C]
+        out, heat = (_core.metrics_host if one else _core.compound_metrics_host)(*args, cold=cold), None
     return (out, heat), st, cell_dims, cell_shape, P, defs.shape[0]
 
 
@@ -252,11 +245,38 @@ def compute_heatwave_metrics_wrapper(measure, threshold, doy_map, hw_definitions
     """metric.py:344-369: the four metrics of every cell for every percentile and definition as one int64 array with dims
     ``(percentile, definition, <cells>, metric, year)``; ``metric`` = HWF, HWN, HWD, HWA in this order (:336-340)."""
     dm = None if doy_map is None else np.asarray(getattr(doy_map, "values", doy_map))
-    (out, _), st, cell_dims, cell_shape, P, D = _metric_sweep(measure, threshold, hw_definitions, time_axis_of(measure), dm)
+    (out, _), st, cell_dims, cell_shape, P, D = _metric_sweep([(measure, threshold)], hw_definitions, time_axis_of(measure), dm)
     data = out.astype(np.int64).transpose(1, 2, 4, 0, 3).reshape(P, D, *cell_shape, 4, st.n_years)
     coords = {"definition": [f"{hw_def[0]}-{hw_def[1]}-{hw_def[2]}" for hw_def in hw_definitions],      # :347-350
               "percentile": np.asarray(xr.coord_values(threshold, "percentile"))}
     return xr.DataArray(data, dims=["percentile", "definition", *cell_dims, "metric", "year"], coords=coords)
+
+
+def _metric_dataset(out, intensity_vars, st, calendar, cell_dims, cell_shape, P, D, measure, threshold, hw_definitions, cold):
+    """What individual and compound metric datasets share: the coordinates, the four metric planes of ``out`` (uint16 [4, P, D, Y, C],
+    as METRIC_DTYPE) and the percentile / definition coordinate attributes.  ``intensity_vars(coords, dims)``: the intensity variables
+    the caller adds ({name: DataArray})."""
+    Y = st.n_years
+    coords = dict(xr.non_time_coords(measure))
+    coords["definition"] = [f"{hw_def[0]}-{hw_def[1]}-{hw_def[2]}" for hw_def in hw_definitions]   # :432
+    coords["percentile"] = np.asarray(xr.coord_values(threshold, "percentile"))
+    coords["time"] = _year_times(st.years, calendar)
+    dims = ["percentile", "definition", *cell_dims, "time"]
+    data_vars = {}
+    for i, name in enumerate(_core.COLD_METRIC_NAMES if cold else _core.METRIC_NAMES):   # HWF=0, HWN=1, HWD=2, HWA=3, :454-461
+        wide = out[i] if np.dtype(METRIC_DTYPE) == np.uint16 else _widen_int64(out[i]).astype(METRIC_DTYPE, copy=False)   # [P, D, Y, C]
+        plane = wide.transpose(0, 1, 3, 2).reshape(P, D, *cell_shape, Y)                # view: no host transposition
+        data_vars[name] = xr.DataArray(plane, dims=dims, coords=coords)
+    data_vars.update(intensity_vars(coords, dims))
+    ds = xr.Dataset(data_vars)
+    xr.set_coord_attrs(ds, "percentile", {"range": "(0, 1)"})
+    days = "cold" if cold else "hot"
+    xr.set_coord_attrs(ds, "definition", {
+        "first_number": f"Minimum number of consecutively {days} days",
+        "second_number": "Maximum number of break days after first wave",
+        "third_number": f"Minimum number of consecutively {days} days after the break"
+    })
+    return ds
 
 
 def compute_individual_metrics(measure, threshold, hw_definitions: list, include_threshold: bool = True, check_variables: bool = True,
@@ -285,26 +305,15 @@ def compute_individual_metrics(measure, threshold, hw_definitions: list, include
             if entry != '':
                 combined_history += (f"(Threshold) {entry}\n")
 
-    (out, heat), st, cell_dims, cell_shape, P, D = _metric_sweep(measure, threshold, hw_definitions, time_axis, intensity=intensity,
+    (out, heat), st, cell_dims, cell_shape, P, D = _metric_sweep([(measure, threshold)], hw_definitions, time_axis, intensity=intensity,
                                                                  cold=cold)
-    metric_names = _core.COLD_METRIC_NAMES if cold else _core.METRIC_NAMES
     intensity_names = _core.COLD_INTENSITY_NAMES if cold else _core.INTENSITY_NAMES
-    Y = st.n_years
 
-    coords = dict(xr.non_time_coords(measure))
-    coords["definition"] = [f"{hw_def[0]}-{hw_def[1]}-{hw_def[2]}" for hw_def in hw_definitions]   # :432
-    coords["percentile"] = np.asarray(xr.coord_values(threshold, "percentile"))
-    coords["time"] = _year_times(st.years, time_axis.calendar)
-    dims = ["percentile", "definition", *cell_dims, "time"]
-    data_vars = {}
-    for i, name in enumerate(metric_names):                         # HWF=0, HWN=1, HWD=2, HWA=3, :454-461
-        wide = out[i] if np.dtype(METRIC_DTYPE) == np.uint16 else _widen_int64(out[i]).astype(METRIC_DTYPE, copy=False)   # [P, D, Y, C]
-        plane = wide.transpose(0, 1, 3, 2).reshape(P, D, *cell_shape, Y)                # view: no host transposition
-        data_vars[name] = xr.DataArray(plane, dims=dims, coords=coords)
-    if intensity:
-        for i, name in enumerate(intensity_names):                  # float32 [P, D, Y, C]
-            data_vars[name] = xr.DataArray(heat[i].transpose(0, 1, 3, 2).reshape(P, D, *cell_shape, Y), dims=dims, coords=coords)
-    ds = xr.Dataset(data_vars)
+    def intensity_vars(coords, dims):                               # float32 [P, D, Y, C] each
+        return {name: xr.DataArray(heat[i].transpose(0, 1, 3, 2).reshape(P, D, *cell_shape, st.n_years), dims=dims, coords=coords)
+                for i, name in enumerate(intensity_names)} if intensity else {}
+    ds = _metric_dataset(out, intensity_vars, st, time_axis.calendar, cell_dims, cell_shape, P, D, measure, threshold, hw_definitions,
+                         cold)
     kind = "Cold spell" if cold else "Heatwave"
     ds.attrs.update({
         "description": f"{kind} metric dataset generated by Heatwave Diagnostics Package (HDP v{get_version()})",
@@ -316,13 +325,6 @@ def compute_individual_metrics(measure, threshold, hw_definitions: list, include
     if intensity:
         for name, attrs in (COLD_INTENSITY_ATTRS if cold else INTENSITY_ATTRS).items():
             ds[name].attrs.update({"units": measure.attrs["units"], **attrs} if "units" in measure.attrs else attrs)
-    xr.set_coord_attrs(ds, "percentile", {"range": "(0, 1)"})
-    days = "cold" if cold else "hot"
-    xr.set_coord_attrs(ds, "definition", {
-        "first_number": f"Minimum number of consecutively {days} days",
-        "second_number": "Maximum number of break days after first wave",
-        "third_number": f"Minimum number of consecutively {days} days after the break"
-    })
     for variable in ds:
         ds[variable].attrs["history"] = combined_history
         add_history(ds[variable], f"Heatwave metrics generated by HDP v{get_version()}")
@@ -373,28 +375,17 @@ def compute_compound_metrics(measure_a, threshold_a, measure_b, threshold_b, hw_
             assert t.attrs["baseline_variable"] == m.attrs["baseline_variable"]
             assert t.attrs["baseline_calendar"] == time_axis.calendar
 
-    (out, heat), st, cell_dims, cell_shape, P, D = _metric_sweep(measure_a, threshold_a, hw_definitions, time_axis, intensity=intensity,
-                                                                 cold=cold, second=(measure_b, threshold_b))
-    metric_names = _core.COLD_METRIC_NAMES if cold else _core.METRIC_NAMES
+    (out, heat), st, cell_dims, cell_shape, P, D = _metric_sweep([(measure_a, threshold_a), (measure_b, threshold_b)], hw_definitions,
+                                                                 time_axis, intensity=intensity, cold=cold)
     intensity_names = _core.COLD_INTENSITY_NAMES if cold else _core.INTENSITY_NAMES
-    Y = st.n_years
     name_a, name_b = _measure_name(measure_a, "measure_a"), _measure_name(measure_b, "measure_b")
 
-    coords = dict(xr.non_time_coords(measure_a))
-    coords["definition"] = [f"{hw_def[0]}-{hw_def[1]}-{hw_def[2]}" for hw_def in hw_definitions]
-    coords["percentile"] = pa
-    coords["time"] = _year_times(st.years, time_axis.calendar)
-    dims = ["percentile", "definition", *cell_dims, "time"]
-    data_vars = {}
-    for i, name in enumerate(metric_names):
-        wide = out[i] if np.dtype(METRIC_DTYPE) == np.uint16 else _widen_int64(out[i]).astype(METRIC_DTYPE, copy=False)
-        data_vars[name] = xr.DataArray(wide.transpose(0, 1, 3, 2).reshape(P, D, *cell_shape, Y), dims=dims, coords=coords)
-    if intensity:
+    def intensity_vars(coords, dims):                               # float32 [2, P, D, Y, C] each
         coords_m = {**coords, "measure": [name_a, name_b]}
-        for i, name in enumerate(intensity_names):                  # float32 [2, P, D, Y, C]
-            data_vars[name] = xr.DataArray(heat[:, i].transpose(0, 1, 2, 4, 3).reshape(2, P, D, *cell_shape, Y), dims=["measure", *dims],
-                                           coords=coords_m)
-    ds = xr.Dataset(data_vars)
+        return {name: xr.DataArray(heat[:, i].transpose(0, 1, 2, 4, 3).reshape(2, P, D, *cell_shape, st.n_years), dims=["measure", *dims],
+                                   coords=coords_m) for i, name in enumerate(intensity_names)} if intensity else {}
+    ds = _metric_dataset(out, intensity_vars, st, time_axis.calendar, cell_dims, cell_shape, P, D, measure_a, threshold_a,
+                         hw_definitions, cold)
     kind = "Compound cold spell" if cold else "Compound heatwave"
     ds.attrs.update({
         "description": f"{kind} metric dataset generated by Heatwave Diagnostics Package (HDP v{get_version()})",
@@ -410,13 +401,6 @@ def compute_compound_metrics(measure_a, threshold_a, measure_b, threshold_b, hw_
             units = {"units": measure_a.attrs["units"]} if "units" in measure_a.attrs else {}
             ds[name].attrs.update({**units, **attrs, "long_name": COMPOUND_LONG_NAMES[name],
                                    "description": f"{attrs['description']}, of each measure; {both}"})
-    xr.set_coord_attrs(ds, "percentile", {"range": "(0, 1)"})
-    days = "cold" if cold else "hot"
-    xr.set_coord_attrs(ds, "definition", {
-        "first_number": f"Minimum number of consecutively {days} days",
-        "second_number": "Maximum number of break days after first wave",
-        "third_number": f"Minimum number of consecutively {days} days after the break"
-    })
     for variable in ds:
         add_history(ds[variable], f"Compound heatwave metrics of {name_a} & {name_b} generated by HDP v{get_version()}")
     return ds
