@@ -13,6 +13,8 @@ These are the two seams of the reference that the CUDA library replaces:
   threshold, which the reference does not have either
 * :func:`compound_metrics_array`, :func:`compound_intensity_array`: compound (day-night) heatwaves, the same sweep over the days on
   which two measures (e.g. tmax and tmin) both exceed their own thresholds
+* ``onset=True`` on the metric, intensity and compound calls: two more uint16 planes, HWO and HWE, the day of the season of its first
+  and last heatwave day (0xFFFF without one)
 * :func:`index_heatwaves_array`, :func:`season_metrics_array` <- ``index_heatwaves`` and ``heatwave_frequency`` / ``number`` /
   ``duration`` / ``average`` (reference hdp/metric.py:11-172), the building blocks the hot path never materialises
 
@@ -35,6 +37,10 @@ INTENSITY_NAMES = ("HWC", "HWI", "HWP")          # plane order of the intensity 
 COLD_METRIC_NAMES = ("CSF", "CSN", "CSD", "CSA")  # the same planes of a cold-spell pass (cold=True)
 COLD_INTENSITY_NAMES = ("CSC", "CSI", "CSP")
 COLD = 0x100                                      # HDP_B200_COLD, OR-ed into the unit code of the metric entry points
+ONSET_NAMES = ("HWO", "HWE")                      # planes 4 and 5 of the metric output with onset=True
+COLD_ONSET_NAMES = ("CSO", "CSE")
+ONSET = 0x200                                     # HDP_B200_ONSET, OR-ed in the same way
+NO_DAY = 0xFFFF                                   # HWO / HWE of a season without heatwave days
 
 _workspaces = {}
 
@@ -186,13 +192,24 @@ def _ptr(t):
     return t.data_ptr() if t is not None else None
 
 
-def _metric_pass(pairs, doy_map, defs, season_north, season_south, is_south, units, met, heat, intensity, cold):
+def _flags(units, cold, onset):
+    return _unit_code(units) | (COLD if cold else 0) | (ONSET if onset else 0)
+
+
+def _check_onset(met, intensity, onset):
+    if onset and intensity and met is None:
+        raise ValueError("onset=True needs metrics_out: HWO and HWE are planes of the uint16 metric output")
+
+
+def _metric_pass(pairs, doy_map, defs, season_north, season_south, is_south, units, met, heat, intensity, cold, onset=False):
     """hdp_b200_metrics, or with ``intensity`` hdp_b200_intensity, on one (measure, thresholds) pair of CUDA tensors; hdp_b200_compound
     on two.  ``met`` / ``heat``: the uint16 metrics / float32 intensity output (``[2, 3, P, D, Y, C]`` for two pairs) or None; the
     metrics are allocated unless the intensity pass runs without them.  Returns the intensity output of the intensity pass, else the
-    metrics.  ``cold``: the cold-spell pass."""
+    metrics.  ``cold``: the cold-spell pass; ``onset``: the metrics have six planes, HWO and HWE behind the four."""
     torch = _torch()
-    unit = _unit_code(units) | (COLD if cold else 0)
+    _check_onset(met, intensity, onset)
+    unit = _flags(units, cold, onset)
+    planes = 6 if onset else 4
     T, C, n_doy, P = _check_pairs(pairs)
     dm, df, sn, ss = _metric_tables(doy_map, defs, season_north, season_south, T)
     L = _lib.lib()
@@ -204,8 +221,8 @@ def _metric_pass(pairs, doy_map, defs, season_north, season_south, is_south, uni
         heat = _device_out(heat, torch.float32, (2, 3, P, D, Y, C) if compound else (3, P, D, Y, C), dev,
                            f"out must be a contiguous float32 CUDA tensor [{'2, ' if compound else ''}3, P, D, Y, C]")
     if met is not None or not intensity:
-        met = _device_out(met, torch.uint16, (4, P, D, Y, C), dev,
-                          f"{'metrics_out' if intensity else 'out'} must be a contiguous uint16 CUDA tensor [4, P, D, Y, C]")
+        met = _device_out(met, torch.uint16, (planes, P, D, Y, C), dev,
+                          f"{'metrics_out' if intensity else 'out'} must be a contiguous uint16 CUDA tensor [{planes}, P, D, Y, C]")
     tables = (_hp(dm), _hp(df), D, _hp(sn), _hp(ss), Y, _ptr(south_t))
     with torch.cuda.device(dev):
         stream = torch.cuda.current_stream().cuda_stream
@@ -229,46 +246,50 @@ def _metric_pass(pairs, doy_map, defs, season_north, season_south, is_south, uni
 
 
 def metrics_array(measure, thresholds, doy_map, defs, season_north, season_south, is_south=None, out=None, units=None, *,
-                  cold=False):
+                  cold=False, onset=False):
     """``measure`` f32 ``[T, C]``, ``thresholds`` f64 ``[C, n_doy, P]`` -> uint16 ``[4, P, D, Y, C]``
     (planes HWF, HWN, HWD, HWA; the reference's int64 ``[P, D, C, 4, Y]`` is ``out.permute(1, 2, 4, 0, 3)`` widened).
     ``units`` of the measure's samples as for :func:`thresholds_array`.  ``cold=True``: cold spells - the same rules over the
     days with ``measure < threshold``, planes CSF, CSN, CSD, CSA (the season tables are used as given; the cold season of a
-    hemisphere is usually the other one's warm season)."""
-    return _metric_pass([(measure, thresholds)], doy_map, defs, season_north, season_south, is_south, units, out, None, False, cold)
+    hemisphere is usually the other one's warm season).  ``onset=True``: uint16 ``[6, P, D, Y, C]``, planes 4 and 5 HWO and HWE
+    (CSO, CSE): the day of the season (0 = its first day) of its first and last heatwave day, :data:`NO_DAY` where HWF is 0."""
+    return _metric_pass([(measure, thresholds)], doy_map, defs, season_north, season_south, is_south, units, out, None, False, cold,
+                        onset)
 
 
 def intensity_array(measure, thresholds, doy_map, defs, season_north, season_south, is_south=None, out=None, metrics_out=None,
-                    units=None, *, cold=False):
+                    units=None, *, cold=False, onset=False):
     """Heatwave intensity: ``measure`` f32 ``[T, C]``, ``thresholds`` f64 ``[C, n_doy, P]`` -> float32 ``[3, P, D, Y, C]``, planes
     HWC (cumulative), HWI (mean) and HWP (peak) exceedance ``measure - threshold`` over the heatwave days of every season (the
     days HWF counts; 0 where there are none).  ``metrics_out``: an optional uint16 CUDA tensor ``[4, P, D, Y, C]`` that also
     receives exactly what :func:`metrics_array` returns, from the same pass.  The non-empty seasons of each hemisphere's table must
     be disjoint (every table compute_hemisphere_ranges builds is).  ``cold=True``: CSC, CSI, CSP - the deficit
-    ``threshold - measure`` over the cold-spell days (and CSF ... CSA in ``metrics_out``), see :func:`metrics_array`."""
+    ``threshold - measure`` over the cold-spell days (and CSF ... CSA in ``metrics_out``), see :func:`metrics_array`.  ``onset=True``:
+    ``metrics_out`` (required) is ``[6, P, D, Y, C]`` with HWO and HWE, as for :func:`metrics_array`."""
     return _metric_pass([(measure, thresholds)], doy_map, defs, season_north, season_south, is_south, units, metrics_out, out, True,
-                        cold)
+                        cold, onset)
 
 
 def compound_metrics_array(measure_a, thresholds_a, measure_b, thresholds_b, doy_map, defs, season_north, season_south, is_south=None,
-                           out=None, units=None, *, cold=False):
+                           out=None, units=None, *, cold=False, onset=False):
     """Compound heatwaves: :func:`metrics_array` over the days on which BOTH ``measure_a > thresholds_a`` and
     ``measure_b > thresholds_b`` (e.g. tmax and tmin: hot days and hot nights) -> uint16 ``[4, P, D, Y, C]``.  The two measures are
     f32 ``[T, C]`` CUDA tensors (any strides each), the two thresholds f64 ``[C, n_doy, P]`` of the same shape: percentile p of A is
     paired with percentile p of B.  ``units`` applies to both measures; ``cold=True``: days on which both are below their
-    thresholds (CSF ... CSA)."""
+    thresholds (CSF ... CSA); ``onset=True``: ``[6, P, D, Y, C]`` with HWO and HWE of the compound days."""
     return _metric_pass([(measure_a, thresholds_a), (measure_b, thresholds_b)], doy_map, defs, season_north, season_south, is_south,
-                        units, out, None, False, cold)
+                        units, out, None, False, cold, onset)
 
 
 def compound_intensity_array(measure_a, thresholds_a, measure_b, thresholds_b, doy_map, defs, season_north, season_south, is_south=None,
-                             out=None, metrics_out=None, units=None, *, cold=False):
+                             out=None, metrics_out=None, units=None, *, cold=False, onset=False):
     """Intensity of the compound heatwaves of :func:`compound_metrics_array`: float32 ``[2, 3, P, D, Y, C]``, block 0 = HWC, HWI, HWP
     of measure A (its exceedance ``measure_a - thresholds_a`` over the compound heatwave days, as :func:`intensity_array` computes
     it), block 1 = the same for measure B.  ``metrics_out``: an optional uint16 CUDA tensor ``[4, P, D, Y, C]`` that also receives
-    what :func:`compound_metrics_array` returns, from the same pass.  ``cold``: the deficits over the compound cold spells."""
+    what :func:`compound_metrics_array` returns, from the same pass.  ``cold``: the deficits over the compound cold spells.
+    ``onset=True``: ``metrics_out`` (required) is ``[6, P, D, Y, C]``."""
     return _metric_pass([(measure_a, thresholds_a), (measure_b, thresholds_b)], doy_map, defs, season_north, season_south, is_south,
-                        units, metrics_out, out, True, cold)
+                        units, metrics_out, out, True, cold, onset)
 
 
 def _hot_days(pairs, doy_map, units=None, cold=False):
@@ -553,10 +574,12 @@ def _host_thresholds(thresholds, C):
     return thr, resident_thresholds(thr)
 
 
-def _metric_pass_host(pairs, doy_map, defs, season_north, season_south, is_south, units, met, heat, intensity, cold):
+def _metric_pass_host(pairs, doy_map, defs, season_north, season_south, is_south, units, met, heat, intensity, cold, onset=False):
     """:func:`_metric_pass` with host arrays: hdp_b200_metrics_host or hdp_b200_intensity_host on one (measure, thresholds) pair,
     hdp_b200_compound_host on two; each threshold as for :func:`metrics_host`."""
     _torch()
+    _check_onset(met, intensity, onset)
+    planes = 6 if onset else 4
     xs = [_host_measure(x, name) for (x, _), name in zip(pairs, _names(pairs, "measure"))]      # (samples, ld_t, ld_c)
     if any(x.shape != xs[0][0].shape for x, _, _ in xs[1:]):
         raise ValueError("measure_a and measure_b must have the same shape [T, C]")
@@ -574,58 +597,60 @@ def _metric_pass_host(pairs, doy_map, defs, season_north, season_south, is_south
         heat = _host_out(heat, np.float32, (2, 3, P, D, Y, C) if compound else (3, P, D, Y, C),
                          f"out must be a C-contiguous float32 array [{'2, ' if compound else ''}3, P, D, Y, C]")
     if met is not None or not intensity:
-        met = _host_out(met, np.uint16, (4, P, D, Y, C),
-                        f"{'metrics_out' if intensity else 'out'} must be a C-contiguous uint16 array [4, P, D, Y, C]")
+        met = _host_out(met, np.uint16, (planes, P, D, Y, C),
+                        f"{'metrics_out' if intensity else 'out'} must be a C-contiguous uint16 array [{planes}, P, D, Y, C]")
     hp = lambda h: _hp(h) if h is not None else None                # noqa: E731
     tables = (_hp(dm), _hp(df), D, _hp(sn), _hp(ss), Y, hp(south))
     if compound:
         name = "hdp_b200_compound_host"
         ((a, ld_ta, ld_ca), (b, ld_tb, ld_cb)), ((h_a, d_a), (h_b, d_b)) = xs, thrs
         rc = _lib.lib().hdp_b200_compound_host(_hp(a), ld_ta, ld_ca, _hp(b), ld_tb, ld_cb, C, T, hp(h_a), _ptr(d_a), hp(h_b), _ptr(d_b),
-                                               n_doy, P, *tables, hp(met), hp(heat), _unit_code(units) | (COLD if cold else 0))
+                                               n_doy, P, *tables, hp(met), hp(heat), _flags(units, cold, onset))
     else:
         name = "hdp_b200_intensity_host" if intensity else "hdp_b200_metrics_host"
         ((x, ld_t, ld_c),), ((h_thr, d_thr),) = xs, thrs
         outs = (_hp(heat), hp(met)) if intensity else (_hp(met),)
         rc = getattr(_lib.lib(), name)(_hp(x), C, T, ld_t, ld_c, hp(h_thr), _ptr(d_thr), n_doy, P, *tables, *outs,
-                                       _unit_code(units) | (COLD if cold else 0))
+                                       _flags(units, cold, onset))
     _lib.check(rc, name)
     return heat if intensity else met
 
 
 def compound_metrics_host(measure_a: np.ndarray, thresholds_a, measure_b: np.ndarray, thresholds_b, doy_map, defs, season_north,
-                          season_south, is_south=None, out: Optional[np.ndarray] = None, units=None, *, cold=False) -> np.ndarray:
+                          season_south, is_south=None, out: Optional[np.ndarray] = None, units=None, *, cold=False,
+                          onset=False) -> np.ndarray:
     """Host-array counterpart of :func:`compound_metrics_array` (both measures' cells of a chunk cross PCIe once).  Each threshold
     as for :func:`metrics_host`: a host array, a CUDA tensor, or a resident copy."""
     return _metric_pass_host([(measure_a, thresholds_a), (measure_b, thresholds_b)], doy_map, defs, season_north, season_south, is_south,
-                             units, out, None, False, cold)
+                             units, out, None, False, cold, onset)
 
 
 def compound_intensity_host(measure_a: np.ndarray, thresholds_a, measure_b: np.ndarray, thresholds_b, doy_map, defs, season_north,
                             season_south, is_south=None, out: Optional[np.ndarray] = None, metrics_out: Optional[np.ndarray] = None,
-                            units=None, *, cold=False) -> np.ndarray:
+                            units=None, *, cold=False, onset=False) -> np.ndarray:
     """Host-array counterpart of :func:`compound_intensity_array`: float32 ``[2, 3, P, D, Y, C]``."""
     return _metric_pass_host([(measure_a, thresholds_a), (measure_b, thresholds_b)], doy_map, defs, season_north, season_south, is_south,
-                             units, metrics_out, out, True, cold)
+                             units, metrics_out, out, True, cold, onset)
 
 
 def metrics_host(measure: np.ndarray, thresholds, doy_map, defs, season_north, season_south,
-                 is_south=None, out: Optional[np.ndarray] = None, units=None, *, cold=False) -> np.ndarray:
+                 is_south=None, out: Optional[np.ndarray] = None, units=None, *, cold=False, onset=False) -> np.ndarray:
     """``thresholds``: float64 ``[C, n_doy, P]`` as a host array, or as a CUDA tensor (device-resident: no upload).  A host
-    array that :func:`thresholds_host` returned with ``keep=True`` is recognised and its device copy used.  ``cold`` as for
-    :func:`metrics_array`."""
-    return _metric_pass_host([(measure, thresholds)], doy_map, defs, season_north, season_south, is_south, units, out, None, False, cold)
+    array that :func:`thresholds_host` returned with ``keep=True`` is recognised and its device copy used.  ``cold`` and ``onset`` as
+    for :func:`metrics_array`."""
+    return _metric_pass_host([(measure, thresholds)], doy_map, defs, season_north, season_south, is_south, units, out, None, False, cold,
+                             onset)
 
 
 def intensity_host(measure: np.ndarray, thresholds, doy_map, defs, season_north, season_south, is_south=None,
                    out: Optional[np.ndarray] = None, metrics_out: Optional[np.ndarray] = None, units=None, *,
-                   cold=False) -> np.ndarray:
+                   cold=False, onset=False) -> np.ndarray:
     """Host-array counterpart of :func:`intensity_array`: float32 ``[3, P, D, Y, C]`` (HWC, HWI, HWP); ``metrics_out`` an
     optional uint16 host array ``[4, P, D, Y, C]`` that also receives what :func:`metrics_host` returns (the samples cross PCIe
-    once for both).  Thresholds as for :func:`metrics_host` (host array, CUDA tensor, or a resident copy); ``cold`` as for
-    :func:`intensity_array`."""
+    once for both).  Thresholds as for :func:`metrics_host` (host array, CUDA tensor, or a resident copy); ``cold`` and ``onset``
+    as for :func:`intensity_array`."""
     return _metric_pass_host([(measure, thresholds)], doy_map, defs, season_north, season_south, is_south, units, metrics_out, out, True,
-                             cold)
+                             cold, onset)
 
 
 def host_release() -> None:

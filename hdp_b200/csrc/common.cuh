@@ -110,9 +110,10 @@ struct Measure {
 };
 
 // The whole of hdp_b200_metrics, hdp_b200_intensity and hdp_b200_compound (metric.cu) over n_measures (1 or 2) measures:
-// k_hot_words (k_hot_pair for two), then k_scan on its hot words when d_out is given (u16 [4, P, D, Y, C]) and k_intensity when
-// d_int is given (f32 [n_measures, 3, P, D, Y, C], one block per measure).  carve_cells / tables_resident as above; input_unit =
-// unit code, OR-ed with HDP_B200_COLD for the cold-spell pass.
+// k_hot_words (k_hot_pair for two), then k_scan on its hot words when d_out is given (u16 [4, P, D, Y, C], [6, ...] with HWO and
+// HWE for HDP_B200_ONSET) and k_intensity when d_int is given (f32 [n_measures, 3, P, D, Y, C], one block per measure).
+// carve_cells / tables_resident as above; input_unit = unit code, OR-ed with HDP_B200_COLD for the cold-spell pass and with
+// HDP_B200_ONSET for the onset planes.
 int metric_pass(const Measure *ms, int n_measures, int64_t C, int64_t T, int n_doy, int P, const int32_t *h_doy_map,
                 const int32_t *h_defs, int D,
                 const int32_t *h_season_north, const int32_t *h_season_south, int Y,

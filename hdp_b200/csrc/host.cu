@@ -332,7 +332,7 @@ struct HostMeasure {
 };
 
 // hdp_b200_metrics_host, hdp_b200_intensity_host and hdp_b200_compound_host: metric_pass over n_measures (1 or 2) measures chunk by
-// chunk; the u16 planes (h_out) and the f32 planes (h_int), whichever are given, go back to the host.  Every measure's cells of a
+// chunk; the u16 planes (h_out: 4, or 6 with HDP_B200_ONSET) and the f32 planes (h_int), whichever are given, go back to the host.  Every measure's cells of a
 // chunk go up together.
 static int metric_pass_host(const HostMeasure *hm, int n_measures, int64_t C, int64_t T, int n_doy, int P, const int32_t *h_doy_map,
                             const int32_t *h_defs, int D,
@@ -340,6 +340,8 @@ static int metric_pass_host(const HostMeasure *hm, int n_measures, int64_t C, in
                             const uint8_t *h_is_south, float *h_int, uint16_t *h_out, int input_unit)
 {
     if (C < 0 || T <= 0 || n_doy <= 0 || P <= 0 || D <= 0 || Y < 0 || !h_doy_map) return HDP_B200_ERR_INVALID;
+    const bool onset = (input_unit & HDP_B200_ONSET) != 0;
+    if (onset && !h_out) return HDP_B200_ERR_INVALID;                          // HWO / HWE are planes of the u16 output
     if (C == 0 || Y == 0) return HDP_B200_OK;
     for (int m = 0; m < n_measures; m++) {
         if (!hm[m].x || (!hm[m].h_thr && !hm[m].d_thr)) return HDP_B200_ERR_INVALID;
@@ -353,7 +355,7 @@ static int metric_pass_host(const HostMeasure *hm, int n_measures, int64_t C, in
     if ((rc = ctx->init())) return rc;
 
     const size_t thr_per_cell = (size_t)n_doy * P * sizeof(double);
-    const size_t rows = (size_t)4 * P * D * Y;                                 // output rows of C cells each
+    const size_t rows = (size_t)(onset ? 6 : 4) * P * D * Y;                  // output rows of C cells each
     const size_t rows_f = (size_t)n_measures * 3 * P * D * Y;
     const int64_t chunk = pick_chunk(C, n_measures * ((size_t)T * sizeof(float) + thr_per_cell), (size_t)320 << 20);
     int64_t dl_c[2] = {};                                                      // cell strides of the device copies (upload_cells)

@@ -186,6 +186,23 @@ struct ScanTables {
     int f_on, f_lmin, f_bmax;        // run filter: on/off, min over definitions of min_dur, max over definitions of max_break
 };
 
+// k_scan's ONSET state: per accumulator register the packed onset and end lanes (day of the season of the first / last in-season
+// heatwave day, the packing of HWF), and `seen`, bit i = definition i has had an in-season block.  Empty without ONSET.
+template <bool ONSET, int NG>
+struct ScanOnset {
+    uint32_t ons[NG], end[NG], seen;
+    __device__ __forceinline__ void reset()
+    {
+#pragma unroll
+        for (int j = 0; j < NG; j++) { ons[j] = 0u; end[j] = 0u; }
+        seen = 0u;
+    }
+};
+template <int NG>
+struct ScanOnset<false, NG> {
+    __device__ __forceinline__ void reset() {}
+};
+
 constexpr int kScanWarps = 8;
 constexpr int kScanQ = 16;                                       // queued words per lane (power of two)
 constexpr int kScanQueueWords = 3 * kScanQ * 32;                  // u32 per warp: run starts, run ends, first day of the word
@@ -234,10 +251,13 @@ __device__ __forceinline__ void stg_u16(uint16_t *p, uint32_t v)
 // (Three CTAs per SM for every accumulator-group count: with 24 definitions the 80-register build spills 100 - 400 bytes per
 // thread, but two CTAs with 128 registers and no spills measured SLOWER - 34.0 against 32.1 ms on wide_sweep: the kernel needs
 // the warps more than the registers.)
+// ONSET: also HWO and HWE, the first and last heatwave day of every season (planes 4 and 5 of u16 [6, P, D, Y, C]), from two more
+// packed accumulators per register: the onset of the first in-season block of a labelled run and the end of the last one.  The run
+// filter drops only runs that get no label, so it cannot drop a block.
 // LMIN / BMAX > = 0: the run filter's two constants (smallest min_duration, largest max_break of the definition set) at compile
 // time, which unrolls its shift loops completely - 12 % of the kernel on the reference's documented definitions (README.md:51:
 // min duration 3 .. 5, at most one break day: LMIN = 3, BMAX = 1).  LMIN = 0: run-time values (any definition set).
-template <int NG, int KS, bool kBytes, int LMIN = 0, int BMAX = 0>
+template <int NG, int KS, bool kBytes, int LMIN = 0, int BMAX = 0, bool ONSET = false>
 __global__ void __launch_bounds__(kScanWarps * 32, 3)
 k_scan(const uint32_t *__restrict__ hot, int64_t C, int K, int T, const int4 *__restrict__ words,
        int P, int D, const __grid_constant__ ScanTables tabs, const uint32_t *__restrict__ ge_tab, const uint32_t *__restrict__ brk_tab,
@@ -304,6 +324,8 @@ k_scan(const uint32_t *__restrict__ hot, int64_t C, int K, int T, const int4 *__
     uint32_t cntg[NG], hwfg[NG], hwng[NG], hwdg[NG];              // definitions PER * j .. PER * j + PER - 1
 #pragma unroll
     for (int j = 0; j < NG; j++) { cntg[j] = 0u; hwfg[j] = 0u; hwng[j] = 0u; hwdg[j] = 0u; }
+    ScanOnset<ONSET, NG> on;
+    on.reset();
 
     // metric m of definition d, season row r of this lane's cell: out_pc[m * P * D * Y * C + d * Y * C + r * C]
     uint16_t *const out_pc = out + (int64_t)p * D * Y * C + c;
@@ -327,6 +349,11 @@ k_scan(const uint32_t *__restrict__ hot, int64_t C, int K, int T, const int4 *__
                         // trunc(mean) = f / nn in integers, metric.py:340; 8-bit lanes: f * ceil(2^16 / nn) >> 16, exact for
                         // f, nn < 256 (scan_hwa_rcp)
                         stg_u16(o3, kBytes ? (f * hwa_rcp[nn]) >> 16 : nn ? f / nn : 0u);
+                        if constexpr (ONSET) {
+                            uint16_t *const o4 = add_ptr(o3, plane_b), *const o5 = add_ptr(o4, plane_b);
+                            stg_u16(o4, scan_onset_value(f, lane_of(on.ons[j], h)));
+                            stg_u16(o5, scan_onset_value(f, lane_of(on.end[j], h)));
+                        }
                     }
                     o = add_ptr(o, dstride_b);
                 }
@@ -334,6 +361,7 @@ k_scan(const uint32_t *__restrict__ hot, int64_t C, int K, int T, const int4 *__
         }
 #pragma unroll
         for (int j = 0; j < NG; j++) { cntg[j] = 0u; hwfg[j] = 0u; hwng[j] = 0u; hwdg[j] = 0u; }
+        on.reset();
         fresh = 0xffffffffu;
         ys++;
         if (ys < n_seasons) { const int4 s4 = seas[ys]; a_cur = s4.x; b_cur = s4.y; row_cur = s4.z; }
@@ -346,8 +374,9 @@ k_scan(const uint32_t *__restrict__ hot, int64_t C, int K, int T, const int4 *__
         const uint32_t t = bits >> (PER * j), g = j == NG - 1 ? t : t & ((1u << PER) - 1u);
         return kBytes ? (g * 0x00204081u) & 0x01010101u : (g * 0x00008001u) & 0x00010001u;
     };
-    // accounting of `days` heatwave days of the definitions in `lab` to the open season (HWF/HWN/HWD, metric.py:63-137)
-    auto account = [&](uint32_t lab, uint32_t days) {
+    // accounting of `days` heatwave days of the definitions in `lab` to the open season (HWF/HWN/HWD, metric.py:63-137): the
+    // in-season block [max(s, a_cur), max(s, a_cur) + days) of a labelled run that starts on day s
+    auto account = [&](uint32_t lab, uint32_t days, int s) {
         const uint32_t newly = lab & fresh;                       // first labelled run of an id inside this season
         fresh &= ~lab;
 #pragma unroll
@@ -357,6 +386,12 @@ k_scan(const uint32_t *__restrict__ hot, int64_t C, int K, int T, const int4 *__
             hwfg[j] += add;
             hwng[j] += neu;
             hwdg[j] = kBytes ? __vmaxu4(hwdg[j], cntg[j]) : __vmaxu2(hwdg[j], cntg[j]);
+        }
+        if constexpr (ONSET) {
+            const uint32_t first = lab & ~on.seen, off = (uint32_t)(max(s, a_cur) - a_cur);     // the block's first day of the season
+#pragma unroll
+            for (int j = 0; j < NG; j++) scan_onset_update(on.ons[j], on.end[j], spread(first, j), spread(lab, j), off, off + days - 1u, LANE_MASK);
+            on.seen |= lab;
         }
     };
 
@@ -469,7 +504,7 @@ k_scan(const uint32_t *__restrict__ hot, int64_t C, int K, int T, const int4 *__
         if (!open) qr = qw;                                       // a lane without seasons left drops what it has queued
         if (open && pend_lab) {
             const int days = min(pend_e, b_cur) - max(pend_s, a_cur);
-            if (days > 0) account(pend_lab, (uint32_t)days);
+            if (days > 0) account(pend_lab, (uint32_t)days, pend_s);
             if (pend_e <= b_cur) pend_lab = 0u; else state = 1;
         }
         for (;;) {
@@ -517,7 +552,7 @@ k_scan(const uint32_t *__restrict__ hot, int64_t C, int K, int T, const int4 *__
                             sublt |= rem[q];
                         }
                         const int days = min(e, b_cur) - max(s, a_cur);
-                        if (lab != 0u && days > 0) account(lab, (uint32_t)days);
+                        if (lab != 0u && days > 0) account(lab, (uint32_t)days, s);
                         if (lab != 0u && e > b_cur) { pend_lab = lab; pend_s = s; pend_e = e; state = 1; }
                     }
                 }
@@ -791,9 +826,11 @@ static int scan_config(const int32_t *h_defs, int D, int64_t T, const ScanPasses
     return HDP_B200_OK;
 }
 
-// k_scan over the hot words in L (one launch per pass): the integer metrics u16 [4, P, D, Y, C].
+// k_scan over the hot words in L (one launch per pass): the integer metrics u16 [4, P, D, Y, C], with `onset` u16 [6, P, D, Y, C]
+// (HWO, HWE behind them, from the ONSET twin of the same instantiation).
 static int run_scan(const Layout &L, const WordPlan &plan, int64_t C, int64_t T, int P, const int32_t *h_defs, int D,
-                    const ScanPasses (&passes)[2], int Y, const uint8_t *d_is_south, uint16_t *d_out, cudaStream_t st, bool tables_resident)
+                    const ScanPasses (&passes)[2], int Y, const uint8_t *d_is_south, uint16_t *d_out, cudaStream_t st, bool tables_resident,
+                    bool onset)
 {
     const int K = (int)plan.words.size();
     ScanConfig cfg;
@@ -823,50 +860,57 @@ static int run_scan(const Layout &L, const WordPlan &plan, int64_t C, int64_t T,
         const int nn = ip < passes[0].size() ? (int)passes[0][ip].size() : 0;
         const int ns = ip < passes[1].size() ? (int)passes[1][ip].size() : 0;
         KernelTimer timer(kScan, st);
+        // the instantiation, with ONSET = ON
+        auto launch = [&](auto on) -> int {
+            constexpr bool ON = decltype(on)::value;
 #define HDP_LAUNCH_SCAN(NG, KS, BY)                                                                                      \
-        do {                                                                                                             \
-            HDP_CUDA_TRY(cudaFuncSetAttribute(k_scan<NG, KS, BY>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)scan_smem)); \
-            k_scan<NG, KS, BY><<<scan_grid, kScanWarps * 32, scan_smem, st>>>(L.hot, C, K, (int)T, L.words, P, D, tabs, ge_tab, brk_tab, \
-                                                                              sn, nn, ss, ns, Y, d_is_south, d_out);     \
-        } while (0)
+            do {                                                                                                             \
+                HDP_CUDA_TRY(cudaFuncSetAttribute(k_scan<NG, KS, BY, 0, 0, ON>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)scan_smem)); \
+                k_scan<NG, KS, BY, 0, 0, ON><<<scan_grid, kScanWarps * 32, scan_smem, st>>>(L.hot, C, K, (int)T, L.words, P, D, tabs, ge_tab, brk_tab, \
+                                                                                  sn, nn, ss, ns, Y, d_is_south, d_out);     \
+            } while (0)
 #define HDP_LAUNCH_SCAN_F(NG, BY, LM, BM)                                                                                \
-        do {                                                                                                             \
-            HDP_CUDA_TRY(cudaFuncSetAttribute(k_scan<NG, 1, BY, LM, BM>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)scan_smem)); \
-            k_scan<NG, 1, BY, LM, BM><<<scan_grid, kScanWarps * 32, scan_smem, st>>>(L.hot, C, K, (int)T, L.words, P, D, tabs, ge_tab, \
-                                                                                     brk_tab, sn, nn, ss, ns, Y, d_is_south, d_out); \
-        } while (0)
+            do {                                                                                                             \
+                HDP_CUDA_TRY(cudaFuncSetAttribute(k_scan<NG, 1, BY, LM, BM, ON>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)scan_smem)); \
+                k_scan<NG, 1, BY, LM, BM, ON><<<scan_grid, kScanWarps * 32, scan_smem, st>>>(L.hot, C, K, (int)T, L.words, P, D, tabs, ge_tab, \
+                                                                                         brk_tab, sn, nn, ss, ns, Y, d_is_south, d_out); \
+            } while (0)
 #define HDP_SCAN_KS(NG, BY)                                                \
-        switch (cfg.ks) {                                                  \
-        case 1:                                                            \
-            if (BY && cfg.lmin == 3 && cfg.bmax == 1) HDP_LAUNCH_SCAN_F(NG, true, 3, 1);                          \
-            else if (BY && cfg.lmin == 3 && cfg.bmax == 2) HDP_LAUNCH_SCAN_F(NG, true, 3, 2);                     \
-            else HDP_LAUNCH_SCAN(NG, 1, BY);                               \
-            break;                                                         \
-        case 2: HDP_LAUNCH_SCAN(NG, 2, BY); break;                         \
-        default: HDP_LAUNCH_SCAN(NG, 32, BY); break;                       \
-        }
-        if (cfg.bytes) {
-            switch (cfg.ng) {                                                  // D <= 32: at most 8 registers of 4
-            case 2: HDP_SCAN_KS(2, true); break;
-            case 3: HDP_SCAN_KS(3, true); break;
-            case 4: HDP_SCAN_KS(4, true); break;
-            case 6: HDP_SCAN_KS(6, true); break;
-            default: HDP_SCAN_KS(8, true); break;
+            switch (cfg.ks) {                                                  \
+            case 1:                                                            \
+                if (BY && cfg.lmin == 3 && cfg.bmax == 1) HDP_LAUNCH_SCAN_F(NG, true, 3, 1);                          \
+                else if (BY && cfg.lmin == 3 && cfg.bmax == 2) HDP_LAUNCH_SCAN_F(NG, true, 3, 2);                     \
+                else HDP_LAUNCH_SCAN(NG, 1, BY);                               \
+                break;                                                         \
+            case 2: HDP_LAUNCH_SCAN(NG, 2, BY); break;                         \
+            default: HDP_LAUNCH_SCAN(NG, 32, BY); break;                       \
             }
-        } else {
-            switch (cfg.ng) {
-            case 2: HDP_SCAN_KS(2, false); break;
-            case 3: HDP_SCAN_KS(3, false); break;
-            case 4: HDP_SCAN_KS(4, false); break;
-            case 6: HDP_SCAN_KS(6, false); break;
-            case 8: HDP_SCAN_KS(8, false); break;
-            case 12: HDP_SCAN_KS(12, false); break;
-            default: HDP_SCAN_KS(16, false); break;
+            if (cfg.bytes) {
+                switch (cfg.ng) {                                                  // D <= 32: at most 8 registers of 4
+                case 2: HDP_SCAN_KS(2, true); break;
+                case 3: HDP_SCAN_KS(3, true); break;
+                case 4: HDP_SCAN_KS(4, true); break;
+                case 6: HDP_SCAN_KS(6, true); break;
+                default: HDP_SCAN_KS(8, true); break;
+                }
+            } else {
+                switch (cfg.ng) {
+                case 2: HDP_SCAN_KS(2, false); break;
+                case 3: HDP_SCAN_KS(3, false); break;
+                case 4: HDP_SCAN_KS(4, false); break;
+                case 6: HDP_SCAN_KS(6, false); break;
+                case 8: HDP_SCAN_KS(8, false); break;
+                case 12: HDP_SCAN_KS(12, false); break;
+                default: HDP_SCAN_KS(16, false); break;
+                }
             }
-        }
 #undef HDP_SCAN_KS
 #undef HDP_LAUNCH_SCAN_F
 #undef HDP_LAUNCH_SCAN
+            return HDP_B200_OK;
+        };
+        const int lrc = onset ? launch(std::true_type()) : launch(std::false_type());
+        if (lrc != HDP_B200_OK) return lrc;
         HDP_LAUNCH_CHECK();
     }
     return HDP_B200_OK;
@@ -891,9 +935,10 @@ int metric_pass(const Measure *ms, int n_measures, int64_t C, int64_t T, int n_d
     if (missing_measure(ms, n_measures, C, T)) return HDP_B200_ERR_INVALID;
     if (P > HDP_B200_MAX_PERCENTILES || D > HDP_B200_MAX_DEFINITIONS) return HDP_B200_ERR_UNSUPPORTED;
     cudaStream_t st = (cudaStream_t)stream;
-    // input_unit of the C ABI = unit code | HDP_B200_COLD; the kernels' launchers see the two as plain values
-    const bool cold = (input_unit & HDP_B200_COLD) != 0;
-    const int unit = input_unit & ~HDP_B200_COLD;
+    // input_unit of the C ABI = unit code | HDP_B200_COLD | HDP_B200_ONSET; the kernels' launchers see them as plain values
+    const bool cold = (input_unit & HDP_B200_COLD) != 0, onset = (input_unit & HDP_B200_ONSET) != 0;
+    const int unit = input_unit & ~(HDP_B200_COLD | HDP_B200_ONSET);
+    if (onset && !d_out) return HDP_B200_ERR_INVALID;                                   // HWO / HWE are planes of the u16 output
 
     // the season tables of both hemispheres, north then south (Y + 1 rows apart, as k_intensity reads them)
     std::vector<int32_t> seasons((size_t)8 * (Y + 1), 0);
@@ -914,7 +959,7 @@ int metric_pass(const Measure *ms, int n_measures, int64_t C, int64_t T, int n_d
                            carve_cells, tables_resident, unit, d_int != nullptr, cold);
     if (rc != HDP_B200_OK || C == 0 || Y == 0) return rc;
     if (d_out) {
-        rc = run_scan(L, plan, C, T, P, h_defs, D, passes, Y, d_is_south, d_out, st, tables_resident);
+        rc = run_scan(L, plan, C, T, P, h_defs, D, passes, Y, d_is_south, d_out, st, tables_resident, onset);
         if (rc != HDP_B200_OK) return rc;
     }
     for (int m = 0; d_int && m < n_measures && rc == HDP_B200_OK; m++)     // one block per measure, on the same words

@@ -162,4 +162,20 @@ HDP_HD double season_average(const SeasonAcc &a, int64_t n, bool multi)
 // up to the next integer.  nn = 0 (a season without heatwaves, f = 0 too) gives 0.  tests/test_scan_hwa.py checks all pairs.
 HDP_HD uint32_t scan_hwa_rcp(uint32_t nn) { return nn ? (0x10000u + nn - 1u) / nn : 0u; }
 
+// ---- the fused pass's HWO / HWE (k_scan with ONSET, metric.cu) ------------------------------------------------------------
+// One in-season block of a labelled run, days lo .. last of the season (offsets from its first day), fed to the packed onset and
+// end accumulators of one register.  `first` and `sel` are already spread to one 0/1 per lane (lane_mask = 0xff or 0xffff):
+// `sel` = the definitions that label the run, `first` = those of them without an earlier block in the season, whose onset lane is
+// still 0.  The onset of a first block is its lo; the end of every block overwrites the last one's (the blocks come in time order).
+// Offsets stay below the lane's maximum (< 255 in 8-bit lanes, which hold seasons of at most 255 days), so nothing carries.
+// tests/test_onset_host.py checks the packed form lane by lane.
+HDP_HD void scan_onset_update(uint32_t &ons, uint32_t &end, uint32_t first, uint32_t sel, uint32_t lo, uint32_t last, uint32_t lane_mask)
+{
+    ons += first * lo;
+    end = (end & ~(sel * lane_mask)) | (sel * last);
+}
+
+// HWO / HWE as stored: the day of the season, or 0xFFFF where the season has no heatwave day (hwf = 0)
+HDP_HD uint32_t scan_onset_value(uint32_t hwf, uint32_t v) { return hwf ? v : 0xffffu; }
+
 }  // namespace hdp

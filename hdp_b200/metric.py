@@ -56,6 +56,24 @@ COLD_INTENSITY_ATTRS = {
             "description": f"Largest {_DEFICIT}; 0 without cold spell days"},
 }
 
+# The onset variables (onset=True): day of the season of its first and last heatwave (cold spell) day, NaN without one.  The season
+# starts are those of compute_hemisphere_ranges: heatwave season north May 1, south Nov 1; cold season north Nov 1, south May 1.
+# The onset variables (onset=True): the day of the season of its first and last heatwave (cold spell) day, NaN without one.  The
+# season starts are those of compute_hemisphere_ranges.
+def _onset_attrs(prefix, kind, days, season, starts):
+    where = f"counted from 0 on the season's first day ({starts}); NaN without {days}"
+    return {
+        f"{prefix}O": {"units": "days", "long_name": f"{kind} Onset",
+                       "description": f"Day of the season of the first day that falls within a {kind.lower()} during a {season}, {where}.  "
+                                      f"{prefix}E - {prefix}O + 1 is the length of the season's {kind.lower()} period"},
+        f"{prefix}E": {"units": "days", "long_name": f"{kind} End",
+                       "description": f"Day of the season of the last day that falls within a {kind.lower()} during a {season}, {where}"},
+    }
+
+
+ONSET_ATTRS = _onset_attrs("HW", "Heatwave", "heatwave days", "heatwave season", "north May 1, south Nov 1")
+COLD_ONSET_ATTRS = _onset_attrs("CS", "Cold Spell", "cold spell days", "cold season", "north Nov 1, south May 1")
+
 
 # ----------------------------------------------------------------------------------------------
 # The building blocks under the reference's names (its unit tests import exactly these: hdp/tests/test_index_heatwaves.py,
@@ -210,12 +228,13 @@ def _threshold_cdp(threshold, measure, cell_dims):
     return np.ascontiguousarray(thr_vals).reshape(-1, n_doy, P)
 
 
-def _metric_sweep(pairs, hw_definitions, time_axis, doy_map=None, intensity=False, cold=False):
+def _metric_sweep(pairs, hw_definitions, time_axis, doy_map=None, intensity=False, cold=False, onset=False):
     """The percentile x definition x cell sweep of compute_heatwave_metrics_wrapper (metric.py:344-369) as ONE library call on one
     (measure, threshold) pair, or on the two of a compound pass (:func:`compute_compound_metrics`):
     -> ((uint16 [4, P, D, Y, C], float32 [3, P, D, Y, C] ([2, 3, P, D, Y, C] for two pairs) or None), season tables, cell dims, cell
     shape, P, D).  With ``intensity`` the call is the intensity pass, which also returns the intensity metrics.  With ``cold`` it is
-    the cold-spell pass, and each hemisphere's season is the other one's heatwave season (north Nov 1 - Apr 1, south May 1 - Oct 1)."""
+    the cold-spell pass, and each hemisphere's season is the other one's heatwave season (north Nov 1 - Apr 1, south May 1 - Oct 1).
+    With ``onset`` the metrics are uint16 [6, P, D, Y, C], HWO and HWE behind the four."""
     st = _tables.hemisphere_ranges(time_axis)                       # compute_hemisphere_ranges, :410
     north, south_tab = (st.south, st.north) if cold else (st.north, st.south)
     if doy_map is None:
@@ -232,12 +251,13 @@ def _metric_sweep(pairs, hw_definitions, time_axis, doy_map=None, intensity=Fals
             raise ValueError("the two measures must have the same dims and shape")
         arrays += [x_b, _threshold_cdp(threshold_b, measure, cell_dims)]
     args = (*arrays, doy_map, defs, north, south_tab, south)
+    flags = {"onset": True} if onset else {}                        # without onset, the call the metric layer always made
     one = len(pairs) == 1
     if intensity:
-        out = np.empty((4, P, defs.shape[0], st.n_years, x.shape[1]), np.uint16)
-        heat = (_core.intensity_host if one else _core.compound_intensity_host)(*args, metrics_out=out, cold=cold)
+        out = np.empty((6 if onset else 4, P, defs.shape[0], st.n_years, x.shape[1]), np.uint16)
+        heat = (_core.intensity_host if one else _core.compound_intensity_host)(*args, metrics_out=out, cold=cold, **flags)
     else:
-        out, heat = (_core.metrics_host if one else _core.compound_metrics_host)(*args, cold=cold), None
+        out, heat = (_core.metrics_host if one else _core.compound_metrics_host)(*args, cold=cold, **flags), None
     return (out, heat), st, cell_dims, cell_shape, P, defs.shape[0]
 
 
@@ -254,8 +274,8 @@ def compute_heatwave_metrics_wrapper(measure, threshold, doy_map, hw_definitions
 
 def _metric_dataset(out, intensity_vars, st, calendar, cell_dims, cell_shape, P, D, measure, threshold, hw_definitions, cold):
     """What individual and compound metric datasets share: the coordinates, the four metric planes of ``out`` (uint16 [4, P, D, Y, C],
-    as METRIC_DTYPE) and the percentile / definition coordinate attributes.  ``intensity_vars(coords, dims)``: the intensity variables
-    the caller adds ({name: DataArray})."""
+    as METRIC_DTYPE), the onset planes 4 and 5 when ``out`` has six (float32, NaN for NO_DAY) and the percentile / definition
+    coordinate attributes.  ``intensity_vars(coords, dims)``: the intensity variables the caller adds ({name: DataArray})."""
     Y = st.n_years
     coords = dict(xr.non_time_coords(measure))
     coords["definition"] = [f"{hw_def[0]}-{hw_def[1]}-{hw_def[2]}" for hw_def in hw_definitions]   # :432
@@ -267,6 +287,10 @@ def _metric_dataset(out, intensity_vars, st, calendar, cell_dims, cell_shape, P,
         wide = out[i] if np.dtype(METRIC_DTYPE) == np.uint16 else _widen_int64(out[i]).astype(METRIC_DTYPE, copy=False)   # [P, D, Y, C]
         plane = wide.transpose(0, 1, 3, 2).reshape(P, D, *cell_shape, Y)                # view: no host transposition
         data_vars[name] = xr.DataArray(plane, dims=dims, coords=coords)
+    for i, name in enumerate(_core.COLD_ONSET_NAMES if cold else _core.ONSET_NAMES, 4):
+        if i < out.shape[0]:
+            day = np.where(out[i] == _core.NO_DAY, np.float32(np.nan), out[i].astype(np.float32))          # [P, D, Y, C]
+            data_vars[name] = xr.DataArray(day.transpose(0, 1, 3, 2).reshape(P, D, *cell_shape, Y), dims=dims, coords=coords)
     data_vars.update(intensity_vars(coords, dims))
     ds = xr.Dataset(data_vars)
     xr.set_coord_attrs(ds, "percentile", {"range": "(0, 1)"})
@@ -280,14 +304,18 @@ def _metric_dataset(out, intensity_vars, st, calendar, cell_dims, cell_shape, P,
 
 
 def compute_individual_metrics(measure, threshold, hw_definitions: list, include_threshold: bool = True, check_variables: bool = True,
-                               *, intensity: bool = False, cold: bool = False):
+                               *, intensity: bool = False, cold: bool = False, onset: bool = False):
     """metric.py:372-506.  ``intensity=True`` adds three float32 variables to the four metrics (which stay identical): HWC, HWI
     and HWP, the cumulative, mean and peak exceedance ``measure - threshold`` over the heatwave days of every season, in the
     measure's units (see hdp_b200_intensity in include/hdp_b200.h for the exact arithmetic).  Same dims and coords as HWF.
 
     ``cold=True`` computes cold spells instead: CSF, CSN, CSD, CSA (and with ``intensity`` CSC, CSI, CSP, the deficit
     ``threshold - measure``) by the same rules over the days with ``measure < threshold``, in each hemisphere's cold season (the
-    other hemisphere's heatwave season).  Use low percentiles for the threshold (e.g. 0.01 ... 0.10)."""
+    other hemisphere's heatwave season).  Use low percentiles for the threshold (e.g. 0.01 ... 0.10).
+
+    ``onset=True`` adds two float32 variables with HWF's dims and coords: HWO and HWE (CSO and CSE when ``cold``), the day of the
+    season (0 = its first day: north May 1, south Nov 1 for heatwaves) of its first and last heatwave day, NaN in a season without
+    heatwave days.  HWE - HWO + 1 is the length of the season's heatwave period.  The four metrics stay identical."""
     time_axis = time_axis_of(measure)
     if check_variables:                                             # :393-398
         assert "hdp_type" in threshold.attrs
@@ -306,7 +334,7 @@ def compute_individual_metrics(measure, threshold, hw_definitions: list, include
                 combined_history += (f"(Threshold) {entry}\n")
 
     (out, heat), st, cell_dims, cell_shape, P, D = _metric_sweep([(measure, threshold)], hw_definitions, time_axis, intensity=intensity,
-                                                                 cold=cold)
+                                                                 cold=cold, onset=onset)
     intensity_names = _core.COLD_INTENSITY_NAMES if cold else _core.INTENSITY_NAMES
 
     def intensity_vars(coords, dims):                               # float32 [P, D, Y, C] each
@@ -322,6 +350,9 @@ def compute_individual_metrics(measure, threshold, hw_definitions: list, include
     })
     for name, attrs in (COLD_METRIC_ATTRS if cold else METRIC_ATTRS).items():
         ds[name].attrs.update(attrs)
+    if onset:
+        for name, attrs in (COLD_ONSET_ATTRS if cold else ONSET_ATTRS).items():
+            ds[name].attrs.update(attrs)
     if intensity:
         for name, attrs in (COLD_INTENSITY_ATTRS if cold else INTENSITY_ATTRS).items():
             ds[name].attrs.update({"units": measure.attrs["units"], **attrs} if "units" in measure.attrs else attrs)
@@ -336,7 +367,9 @@ COMPOUND_LONG_NAMES = {"HWF": "Compound Heatwave Frequency", "HWN": "Compound He
                        "HWI": "Compound Heatwave Mean Intensity", "HWP": "Compound Heatwave Peak Intensity",
                        "CSF": "Compound Cold Spell Frequency", "CSN": "Compound Cold Spell Number", "CSD": "Compound Cold Spell Duration",
                        "CSA": "Compound Cold Spell Average", "CSC": "Compound Cold Spell Cumulative Intensity",
-                       "CSI": "Compound Cold Spell Mean Intensity", "CSP": "Compound Cold Spell Peak Intensity"}
+                       "CSI": "Compound Cold Spell Mean Intensity", "CSP": "Compound Cold Spell Peak Intensity",
+                       "HWO": "Compound Heatwave Onset", "HWE": "Compound Heatwave End", "CSO": "Compound Cold Spell Onset",
+                       "CSE": "Compound Cold Spell End"}
 
 
 def _measure_name(measure, fallback):
@@ -344,7 +377,7 @@ def _measure_name(measure, fallback):
 
 
 def compute_compound_metrics(measure_a, threshold_a, measure_b, threshold_b, hw_definitions: list, check_variables: bool = True, *,
-                             intensity: bool = False, cold: bool = False):
+                             intensity: bool = False, cold: bool = False, onset: bool = False):
     """Compound (day-night) heatwaves: the metrics of :func:`compute_individual_metrics` over the days on which BOTH measures exceed
     their own thresholds (e.g. tmax and tmin: hot days and hot nights), percentile p of ``threshold_a`` paired with percentile p of
     ``threshold_b``.  The measures must have the same cell dims, coordinates and time axis, the thresholds identical
@@ -352,7 +385,8 @@ def compute_compound_metrics(measure_a, threshold_a, measure_b, threshold_b, hw_
 
     Returns HWF, HWN, HWD, HWA with the dims and coords of :func:`compute_individual_metrics`; with ``intensity`` also HWC, HWI and
     HWP with a leading ``measure`` dim (coordinate ``[<a>, <b>]``): each measure's exceedance over the compound heatwave days.
-    ``cold=True``: days on which both are below their thresholds (CSF ... CSP, the deficits), in the cold season."""
+    ``cold=True``: days on which both are below their thresholds (CSF ... CSP, the deficits), in the cold season.  ``onset=True`` adds
+    HWO and HWE (CSO, CSE) of :func:`compute_individual_metrics` over the compound days, without a ``measure`` dim."""
     time_axis = time_axis_of(measure_a)
     time_b = time_axis_of(measure_b)
     if time_axis.calendar != time_b.calendar or any(
@@ -376,7 +410,7 @@ def compute_compound_metrics(measure_a, threshold_a, measure_b, threshold_b, hw_
             assert t.attrs["baseline_calendar"] == time_axis.calendar
 
     (out, heat), st, cell_dims, cell_shape, P, D = _metric_sweep([(measure_a, threshold_a), (measure_b, threshold_b)], hw_definitions,
-                                                                 time_axis, intensity=intensity, cold=cold)
+                                                                 time_axis, intensity=intensity, cold=cold, onset=onset)
     intensity_names = _core.COLD_INTENSITY_NAMES if cold else _core.INTENSITY_NAMES
     name_a, name_b = _measure_name(measure_a, "measure_a"), _measure_name(measure_b, "measure_b")
 
@@ -394,7 +428,8 @@ def compute_compound_metrics(measure_a, threshold_a, measure_b, threshold_b, hw_
         "compound_measures": f"{name_a} & {name_b}",
     })
     both = f"days on which both {name_a} and {name_b} are {'below' if cold else 'above'} their thresholds"
-    for name, attrs in (COLD_METRIC_ATTRS if cold else METRIC_ATTRS).items():
+    metric_attrs = {**(COLD_METRIC_ATTRS if cold else METRIC_ATTRS), **((COLD_ONSET_ATTRS if cold else ONSET_ATTRS) if onset else {})}
+    for name, attrs in metric_attrs.items():
         ds[name].attrs.update({**attrs, "long_name": COMPOUND_LONG_NAMES[name], "description": f"{attrs['description']}; {both}"})
     if intensity:
         for name, attrs in (COLD_INTENSITY_ATTRS if cold else INTENSITY_ATTRS).items():
@@ -407,10 +442,11 @@ def compute_compound_metrics(measure_a, threshold_a, measure_b, threshold_b, hw_
 
 
 def compute_group_metrics(measures, thresholds, hw_definitions: list, include_threshold: bool = False, check_variables: bool = True,
-                          *, intensity: bool = False, cold: bool = False):
+                          *, intensity: bool = False, cold: bool = False, onset: bool = False):
     """metric.py:509-523: every measure against every threshold of the same baseline variable.  ``intensity=True`` adds the
     HWC / HWI / HWP variables of :func:`compute_individual_metrics` under the same ``{measure}.{threshold}.{metric}`` names;
-    ``cold=True`` gives the cold-spell variables (``{measure}.{threshold}.CSF`` ...) instead."""
+    ``cold=True`` gives the cold-spell variables (``{measure}.{threshold}.CSF`` ...) instead; ``onset=True`` adds HWO and HWE
+    (CSO, CSE)."""
     metric_sets = []
     for measure_name in list(measures.keys()):
         measure = measures[measure_name]
@@ -418,7 +454,7 @@ def compute_group_metrics(measures, thresholds, hw_definitions: list, include_th
             threshold = thresholds[threshold_name]
             if threshold.attrs["baseline_variable"] == measure.attrs["baseline_variable"]:
                 hw_metrics = compute_individual_metrics(measure, threshold, hw_definitions, include_threshold, check_variables,
-                                                        intensity=intensity, cold=cold)
+                                                        intensity=intensity, cold=cold, onset=onset)
                 var_renames = {name: f"{measure_name}.{threshold_name}.{name}" for name in list(hw_metrics.keys())}
                 metric_sets.append(hw_metrics.rename(var_renames))
     aggr_ds = xr.merge(metric_sets)

@@ -131,7 +131,7 @@ int hdp_b200_thresholds_host(const float *h_temps, int64_t C, int64_t T_b, int64
  *                 the reference's int64 (percentile, definition, <cells>, metric, year) array is
  *                 out[m][p][d][y][c] widened.  Every value is <= the longest season, which must be < 65536.
  *   input_unit    as for hdp_b200_thresholds, optionally OR-ed with HDP_B200_COLD (here and in hdp_b200_metrics_host,
- *                 hdp_b200_intensity and hdp_b200_intensity_host).
+ *                 hdp_b200_intensity and hdp_b200_intensity_host) and with HDP_B200_ONSET (below: d_out gets 6 planes).
  *
  * Cold spells (HDP_B200_COLD): a day counts when (double)x(t) < thr[c, doy_map[t], p] instead of x(t) > thr (NaN on either side:
  * never; a -inf sample is cold unless thr is -inf), and the planes are CSF, CSN, CSD, CSA: exactly the rules of HWF, HWN, HWD,
@@ -141,6 +141,21 @@ int hdp_b200_thresholds_host(const float *h_temps, int64_t C, int64_t T_b, int64
  * no direction and reject it too.
  * ------------------------------------------------------------------------------------------------- */
 #define HDP_B200_COLD 0x100
+
+/* Heatwave onset and end (HDP_B200_ONSET, OR-ed into input_unit of hdp_b200_metrics, hdp_b200_intensity, hdp_b200_compound and
+ * their _host variants, with or without HDP_B200_COLD): the u16 output (d_out / h_out) is then [6, P, D, Y, C], planes 0 - 3
+ * exactly the result without the flag and
+ *   plane 4  HWO  min(H) - lo: the day of the season (0 = its first day) of its first heatwave day
+ *   plane 5  HWE  max(H) - lo: the day of the season of its last heatwave day
+ * where [lo, hi) is the season slice after the slice semantics above and H the days t in [lo, hi) whose heatwave id is > 0 (the
+ * days HWF counts).  Both are 0xFFFF where H is empty (HWF = 0, also for an empty season); a value is < hi - lo <= 65 535, so the
+ * sentinel is never a day.  HWO = 0xFFFF <=> HWE = 0xFFFF <=> HWF = 0; otherwise HWO <= HWE and HWE - HWO + 1 >= HWF >= HWD.  A
+ * heatwave that began before the season gives HWO = 0, one that continues past its end HWE = hi - lo - 1 (the clipping of HWF).
+ * With HDP_B200_COLD: CSO, CSE over the cold-spell days; compound: over the compound days.  Without a u16 output (the intensity
+ * and compound calls) the flag returns HDP_B200_ERR_INVALID; workspace sizes do not depend on it.  Libraries of ABI version 6
+ * without onset reject the flag with HDP_B200_ERR_INVALID, and so do the threshold and hot-day entry points.
+ * ------------------------------------------------------------------------------------------------- */
+#define HDP_B200_ONSET 0x200
 
 /* h_doy_map may be NULL: the size is then an upper bound for regular daily calendars. */
 size_t hdp_b200_metrics_workspace_bytes(int64_t C, int64_t T, int64_t ld_t, int64_t ld_c,
@@ -188,8 +203,8 @@ int hdp_b200_metrics_host(const float *h_measure, int64_t C, int64_t T, int64_t 
  *
  *   d_int         f32 [3, P, D, Y, C]  planes HWC, HWI, HWP, each rounded once from float64 (the canonical order above makes
  *                 the result reproducible bit for bit)
- *   d_out         optional u16 [4, P, D, Y, C]: when given, also exactly what hdp_b200_metrics writes, from the same hot-day
- *                 pass over the samples
+ *   d_out         optional u16 [4, P, D, Y, C] ([6, ...] with HDP_B200_ONSET, which needs it): when given, also exactly what
+ *                 hdp_b200_metrics writes, from the same hot-day pass over the samples
  * The non-empty seasons of each hemisphere's table must be pairwise disjoint after slice clamping (every table built by
  * compute_hemisphere_ranges / get_range_indices is); other tables return HDP_B200_ERR_UNSUPPORTED.
  *
@@ -230,7 +245,7 @@ int hdp_b200_intensity_host(const float *h_measure, int64_t C, int64_t T, int64_
  *                      side of either comparison: not hot).  With HDP_B200_COLD both comparisons are < (cold days and cold
  *                      nights); the season tables are used as given.
  *   d_out              optional u16 [4, P, D, Y, C]: HWF, HWN, HWD, HWA (CSF ... CSA with HDP_B200_COLD) by exactly the rules of
- *                      hdp_b200_metrics, applied to the compound days
+ *                      hdp_b200_metrics, applied to the compound days; [6, ...] with HWO, HWE with HDP_B200_ONSET (which needs it)
  *   d_int              optional f32 [2, 3, P, D, Y, C]: block 0 = HWC, HWI, HWP of measure A (its exceedance x_a - thr_a over the
  *                      compound heatwave days), block 1 = the same for measure B; each block has the arithmetic and order of
  *                      hdp_b200_intensity (the deficit with HDP_B200_COLD), and the season tables must be disjoint as there
