@@ -15,6 +15,8 @@ These are the two seams of the reference that the CUDA library replaces:
   which two measures (e.g. tmax and tmin) both exceed their own thresholds
 * ``onset=True`` on the metric, intensity and compound calls: two more uint16 planes, HWO and HWE, the day of the season of its first
   and last heatwave day (0xFFFF without one)
+* :func:`trend_array`: Theil-Sen slope, its confidence interval and the Mann-Kendall test of every season series of a metric or
+  intensity output (or any ``[..., Y, C]`` array)
 * :func:`index_heatwaves_array`, :func:`season_metrics_array` <- ``index_heatwaves`` and ``heatwave_frequency`` / ``number`` /
   ``duration`` / ``average`` (reference hdp/metric.py:11-172), the building blocks the hot path never materialises
 
@@ -659,13 +661,82 @@ def host_release() -> None:
     _lib.lib().hdp_b200_host_release()
 
 
+# ----------------------------------------------------------------------------------------------
+# trend statistics of season series (csrc/trend.cu)
+# ----------------------------------------------------------------------------------------------
+
+TREND_NAMES = ("slope", "intercept", "slope_low", "slope_high", "mk_s", "mk_var", "mk_p", "n")   # plane order of the trend output
+DTYPE_U16, DTYPE_F32 = 1, 2                                      # HDP_B200_DTYPE_U16, HDP_B200_DTYPE_F32
+TREND_MAX_Y = 512
+
+
+def _trend_args(dtype_name: str, shape, missing, alpha):
+    """(dtype code, rows, Y, C, missing code, zq) of a trend call on ``[..., Y, C]`` values."""
+    if len(shape) < 2:
+        raise ValueError("values must be [..., Y, C]")
+    if dtype_name == "uint16":
+        if missing is not None and not (0 <= int(missing) <= 0xFFFF):
+            raise ValueError("missing must be a uint16 value or None")
+        code, miss = DTYPE_U16, -1 if missing is None else int(missing)
+    elif dtype_name == "float32":
+        if missing is not None:
+            raise ValueError("missing applies to uint16 values; in float32 values every non-finite value is missing")
+        code, miss = DTYPE_F32, -1
+    else:
+        raise TypeError("values must be uint16 or float32")
+    if not 0.0 < alpha < 1.0:
+        raise ValueError("alpha must be in (0, 1)")
+    from statistics import NormalDist
+    zq = NormalDist().inv_cdf(alpha / 2)
+    Y, C = int(shape[-2]), int(shape[-1])
+    rows = int(np.prod(shape[:-2], dtype=np.int64))
+    return code, rows, Y, C, miss, zq
+
+
+def trend_array(values, *, missing=None, alpha=0.05):
+    """Trend of every season series of ``values``, a contiguous uint16 or float32 CUDA tensor ``[..., Y, C]`` (e.g. the metric output
+    ``[M, P, D, Y, C]``): float64 ``[8, ..., C]``, planes :data:`TREND_NAMES` - the Theil-Sen slope per season, its intercept at season
+    0, the bounds of its Sen (1968) ``1 - alpha`` confidence interval, and the Mann-Kendall S, variance (tie-corrected) and two-sided
+    p-value, and the number of valid seasons.  ``missing``: the uint16 value of a missing season (:data:`NO_DAY` for HWO / HWE), or
+    None; in float32 values every non-finite value is missing.  Y <= 512.  The exact rules are those of hdp_b200_trend in
+    include/hdp_b200.h."""
+    torch = _torch()
+    if not (isinstance(values, torch.Tensor) and values.is_cuda and values.is_contiguous()):
+        raise TypeError("values must be a contiguous uint16 or float32 CUDA tensor [..., Y, C]")
+    code, rows, Y, C, miss, zq = _trend_args(str(values.dtype).replace("torch.", ""), tuple(values.shape), missing, alpha)
+    out = torch.empty((8, *values.shape[:-2], C), dtype=torch.float64, device=values.device)
+    with torch.cuda.device(values.device):
+        rc = _lib.lib().hdp_b200_trend(values.data_ptr(), code, rows, Y, C, miss, zq, out.data_ptr(),
+                                       torch.cuda.current_stream().cuda_stream)
+    _lib.check(rc, "hdp_b200_trend")
+    return out
+
+
+TREND_CHUNK_BYTES = 1 << 28
+
+
+def trend_host(values: np.ndarray, *, missing=None, alpha=0.05) -> np.ndarray:
+    """:func:`trend_array` on a host array ``[..., Y, C]`` (uint16 or float32): uploaded in chunks of whole rows (about
+    :data:`TREND_CHUNK_BYTES` each), float64 ``[8, ..., C]`` NumPy out."""
+    torch = _torch()
+    x = np.ascontiguousarray(values)
+    code, rows, Y, C, miss, zq = _trend_args(str(x.dtype), x.shape, missing, alpha)
+    out = np.empty((8, rows, C), np.float64)
+    flat = x.reshape(rows, Y, C)
+    step = max(1, TREND_CHUNK_BYTES // max(1, Y * C * x.itemsize))
+    for r0 in range(0, rows, step):
+        dev = torch.as_tensor(flat[r0:r0 + step]).cuda()
+        out[:, r0:r0 + dev.shape[0]] = trend_array(dev, missing=missing, alpha=alpha).cpu().numpy()
+    return out.reshape(8, *x.shape[:-2], C)
+
+
 def launch_count() -> int:
     return int(_lib.lib().hdp_b200_launch_count())
 
 
 KERNEL_NAMES = {1: "normalize", 2: "k_thr_generic", 3: "k_hot_words", 4: "k_scan", 5: "k_unpack_mask",
                 6: "k_thr_seg", 7: "k_thr_ranked", 8: "k_measure", 9: "k_thr_cand", 10: "k_thr_net", 11: "k_seam",
-                12: "k_intensity", 13: "k_hot_pair"}
+                12: "k_intensity", 13: "k_hot_pair", 14: "k_trend"}
 
 
 def timing_enable(on: bool) -> None:

@@ -47,6 +47,7 @@ SIGNATURES = {
     "hdp_b200_heat_index_measure": (_int, [_p, _p, _i64, _int, _p, _p]),
     "hdp_b200_to_celsius": (_int, [_p, _i64, _int, _p, _p]),
     "hdp_b200_weighted_mean": (_int, [_p, _i64, _i64, _p, ctypes.c_double, _p, _p]),
+    "hdp_b200_trend": (_int, [_p, _int, _i64, _int, _i64, _i64, ctypes.c_double, _p, _p]),
     "hdp_b200_timing_enable": (None, [_int]),
     "hdp_b200_timing_read": (_int, [_p, _p, _int]),
     "hdp_b200_hot_days": (_int, [_p, _i64, _i64, _i64, _i64, _p, _int, _int, _p, _p, _p, _sz, _p]),

@@ -463,6 +463,68 @@ def compute_group_metrics(measures, thresholds, hw_definitions: list, include_th
     return aggr_ds
 
 
+_TREND_LEAD_DIMS = ("measure", "percentile", "definition")      # dims of a metric variable that are neither cells nor time
+TREND_METHOD = ("Theil-Sen slope per year with the Sen (1968) confidence interval; intercept median(y) - slope * median(x) at the "
+                "first season; two-sided Mann-Kendall test with tie-corrected variance and continuity correction")
+
+
+def _trend_attrs(name, units, alpha):
+    level = f"{100 * (1 - alpha):g} %"
+    per_year = {"units": f"{units} per year"} if units else {}
+    return {
+        "slope": {**per_year, "long_name": f"Theil-Sen slope of {name}"},
+        "intercept": {**({"units": units} if units else {}), "long_name": f"Theil-Sen intercept of {name} at the first season"},
+        "slope_low": {**per_year, "long_name": f"Lower bound of the {level} confidence interval of the slope of {name}"},
+        "slope_high": {**per_year, "long_name": f"Upper bound of the {level} confidence interval of the slope of {name}"},
+        "mk_s": {"long_name": f"Mann-Kendall S of {name}"},
+        "mk_var": {"long_name": f"Tie-corrected variance of the Mann-Kendall S of {name}"},
+        "mk_p": {"long_name": f"Two-sided Mann-Kendall p-value of {name}"},
+        "n": {"long_name": f"Number of seasons with a value of {name}"},
+    }
+
+
+def compute_metric_trends(ds, variables=None, alpha: float = 0.05):
+    """Trends over the seasons of a dataset from :func:`compute_individual_metrics`, :func:`compute_group_metrics` or
+    :func:`compute_compound_metrics`: for every variable with a ``time`` dim (or the ones named in ``variables``), ``{name}_slope``,
+    ``_intercept``, ``_slope_low``, ``_slope_high`` (Theil-Sen slope per year, its intercept at the first season and its Sen (1968)
+    ``1 - alpha`` confidence interval), ``_mk_s``, ``_mk_var``, ``_mk_p`` (Mann-Kendall S, tie-corrected variance, two-sided p-value)
+    and ``_n`` (seasons used), float64 with the variable's dims and coords without ``time``.
+
+    Integer variables (HWF ... HWA) are used as they are; in float variables a non-finite value is a missing season (HWO / HWE without a
+    heatwave day are NaN, an intensity can be inf).  The arithmetic is that of hdp_b200_trend (include/hdp_b200.h), on the device."""
+    names = [v for v in ds if "time" in ds[v].dims] if variables is None else list(variables)
+    out = {}
+    for name in names:
+        da = ds[name]
+        dims = tuple(da.dims)
+        if "time" not in dims:
+            raise ValueError(f"'{name}' has no time dim")
+        lead = [d for d in dims if d in _TREND_LEAD_DIMS]
+        cells = [d for d in dims if d not in _TREND_LEAD_DIMS and d != "time"]
+        order = [dims.index(d) for d in (*lead, "time", *cells)]
+        values = np.asarray(da.values).transpose(order)              # [*lead, Y, *cells]: a view of the [P, D, Y, C] planes
+        Y = values.shape[len(lead)]
+        shape = values.shape[:len(lead)] + values.shape[len(lead) + 1:]
+        if np.issubdtype(values.dtype, np.integer):
+            if values.size and (values.min() < 0 or values.max() > 0xFFFF):
+                raise ValueError(f"'{name}' has values outside uint16")
+            x = values.astype(np.uint16, copy=False)
+        elif np.issubdtype(values.dtype, np.floating):
+            x = values.astype(np.float32, copy=False)
+        else:
+            raise TypeError(f"'{name}' is neither an integer nor a float variable")
+        x = x.reshape(*values.shape[:len(lead)], Y, -1)
+        planes = _core.trend_host(x, alpha=alpha).reshape(8, *shape)
+        coords = xr.non_time_coords(da)
+        attrs = _trend_attrs(name, da.attrs.get("units"), alpha)
+        for i, stat in enumerate(_core.TREND_NAMES):
+            out[f"{name}_{stat}"] = xr.DataArray(planes[i], dims=[*lead, *cells], coords=coords, attrs=attrs[stat])
+    trends = xr.Dataset(out)
+    trends.attrs.update({"alpha": alpha, "trend_method": TREND_METHOD,
+                         "description": f"Trends over the seasons of a metric dataset, by HDP v{get_version()}"})
+    return trends
+
+
 def compute_metrics_io(output_path: str, measure_path: str, measure_var: str, threshold_path: str, hw_definitions: list,
                        include_threshold: bool = False, override_threshold_var: str = None, overwrite: bool = False) -> None:
     """hdp/metric.py:526-590: metrics from netCDF files / zarr stores, written back to disk.  The reference's wrapper does not run

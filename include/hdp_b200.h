@@ -17,6 +17,8 @@
  *                         threshold over the heatwave days of every season, optionally with the metrics in the same pass
  *   hdp_b200_index_heatwaves   replaces  index_heatwaves                  hdp/metric.py:11-60     (the building blocks under
  *   hdp_b200_season_metrics    replaces  heatwave_frequency / number / duration / average  hdp/metric.py:63-172   their own names)
+ *   hdp_b200_trend        (no reference counterpart) Theil-Sen slope, its confidence interval and the Mann-Kendall test of every
+ *                         season series of a metric or intensity output
  *   *_host variants       the same calls with HOST buffers (cell chunks pipelined H2D -> kernels -> D2H on three streams).
  *
  * Conventions
@@ -338,6 +340,37 @@ int hdp_b200_to_celsius(const float *d_temp, int64_t n, int unit, float *d_out_c
  * reduction of the reference's figure deck (hdp/graphics/figure.py:14-15 compute_weighted_spatial_mean). */
 int hdp_b200_weighted_mean(const uint16_t *d_x, int64_t rows, int64_t C, const double *d_w, double w_sum, double *d_out, void *stream);
 
+/* ---------------------------------------------------------------------------------------------------
+ * Trend statistics of season series: Theil-Sen slope with its Sen (1968) confidence interval, and the Mann-Kendall test.
+ *
+ *   d_x      [rows, Y, C], cell-contiguous: series (r, c) is d_x[(r * Y + y) * C + c], y = 0 .. Y-1.  The metric output
+ *            u16 [M, P, D, Y, C] is this layout with rows = M * P * D, the intensity output f32 [3, P, D, Y, C] likewise.
+ *   dtype    HDP_B200_DTYPE_U16 or HDP_B200_DTYPE_F32
+ *   missing  u16: the sentinel of a missing season (0xFFFF for the HWO / HWE / CSO / CSE planes), or -1 for none; ignored for f32,
+ *            where every non-finite value (NaN, +-inf) is missing
+ *   zq       Phi^-1(alpha / 2) < 0, the normal quantile of the two-sided (1 - alpha) confidence interval
+ *   d_out    f64 [8, rows, C], planes slope, intercept, slope_low, slope_high, mk_s, mk_var, mk_p, n
+ *
+ * For one series, x = the season index (0 = first season: slopes are per season), n = the number of valid seasons, and only the
+ * pairs i < j of valid seasons are used; values are widened to f64 before any arithmetic.
+ *   slopes      s_ij = (y_j - y_i) / (double)(j - i): one f64 subtraction and one correctly rounded f64 division, N = n(n-1)/2 of them
+ *   median      sorted ascending (-0.0 before +0.0): a[N/2] for odd N, (a[N/2-1] + a[N/2]) * 0.5 for even N; the same rule for y and x
+ *   slope       the median of the slopes
+ *   intercept   median(y_valid) - slope * median(x_valid) (Conover's "separate" form, as scipy.stats.theilslopes by default)
+ *   mk_s        S = sum of sign(y_j - y_i) over the pairs
+ *   mk_var      (n(n-1)(2n+5) - sum_i (t_i - 1)(2 t_i + 5)) / 18, t_i = #{valid k: y_k == y_i}; the numerator exact in int64
+ *   mk_p        two-sided, continuity-corrected: z = (S - sgn S) / sqrt(var) when var > 0, else 0; p = erfc(|z| / sqrt(2))
+ *   slope_low   a[Rl], Rl = max(rint((N + zq sigma) / 2) - 1, 0)     sigma = sqrt(max(var, 0)), rint rounds half to even
+ *   slope_high  a[Ru], Ru = min(rint((N - zq sigma) / 2), N - 1)
+ *   n           n
+ * With n < 2: slope, intercept, slope_low, slope_high and mk_p are NaN, mk_s = mk_var = 0.  Every plane but mk_p is exact to the
+ * bit; mk_p goes through the device's erfc.  Y up to 512; a longer series returns HDP_B200_ERR_UNSUPPORTED.  No workspace.
+ * ------------------------------------------------------------------------------------------------- */
+#define HDP_B200_DTYPE_U16 1
+#define HDP_B200_DTYPE_F32 2
+
+int hdp_b200_trend(const void *d_x, int dtype, int64_t rows, int Y, int64_t C, int64_t missing, double zq, double *d_out, void *stream);
+
 /* Last kernel-launch counters (for bench.py's gpu_launches claim): number of kernels this library has
  * launched since it was loaded. */
 int64_t hdp_b200_launch_count(void);
@@ -358,6 +391,7 @@ int64_t hdp_b200_launch_count(void);
 #define HDP_B200_KERNEL_SEAM        11   /* k_index_heatwaves, k_season_metrics */
 #define HDP_B200_KERNEL_INTENSITY   12   /* k_intensity */
 #define HDP_B200_KERNEL_HOT_PAIR    13   /* k_hot_pair */
+#define HDP_B200_KERNEL_TREND       14   /* k_trend */
 void hdp_b200_timing_enable(int on);
 int  hdp_b200_timing_read(int *ids, float *ms, int cap);
 
