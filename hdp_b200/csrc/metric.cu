@@ -572,7 +572,10 @@ k_scan(const uint32_t *__restrict__ hot, int64_t C, int K, int T, const int4 *__
 // ----------------------------------------------------------------------------------------------------
 static_assert(kTileDoy == 32, "word_length (seams.h) cuts words at 32-day blocks of the day-of-year axis");
 
-// Cuts the time axis into hot-day words (word_length) and groups them by day-of-year block.
+// Cuts the time axis into hot-day words (word_length) and groups them by day-of-year block.  A word holds consecutive days of
+// year d0 .. d0 + nb - 1, so checking its first and last day checks every map entry: an entry >= n_doy inside a word (noleap
+// thresholds with a standard-calendar run: 31 December of a leap year maps to 365 in the word that starts at 352) would otherwise
+// meet k_hot_words' +inf tile padding and be silently never hot.
 static int build_words(const int32_t *doy_map, int64_t T, int n_doy, WordPlan &plan)
 {
     plan.n_blk = (n_doy + kTileDoy - 1) / kTileDoy;
@@ -580,6 +583,7 @@ static int build_words(const int32_t *doy_map, int64_t T, int n_doy, WordPlan &p
         const int d0 = doy_map[t];
         if (d0 < 0 || d0 >= n_doy) return HDP_B200_ERR_INVALID;
         const int nb = word_length(doy_map, t, T);
+        if (d0 + nb - 1 >= n_doy) return HDP_B200_ERR_INVALID;
         plan.words.push_back(make_int4((int)t, nb, d0, 0));
         t += nb;
     }

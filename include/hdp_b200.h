@@ -125,6 +125,7 @@ int hdp_b200_thresholds_host(const float *h_temps, int64_t C, int64_t T_b, int64
  *   d_measure     f32 series, element (t, c) at [t*ld_t + c*ld_c], t < T, c < C
  *   d_thr         f64 [C, n_doy, P]   thresholds, exactly what path 1 writes
  *   h_doy_map     i32 [T]             day-of-year row of every time step (metric.py:265-277), 0 <= v < n_doy
+ *                                     (HDP_B200_ERR_INVALID for any other entry, before anything is written)
  *   h_defs        i32 [D, 3]          [min_duration, max_break, max_subs] per definition (metric.py:11)
  *   h_season_north / h_season_south   i32 [Y, 2] season [start, end) time indices per hemisphere
  *                 (metric.py:175-262); Python slice semantics are applied to negative / out-of-range values
@@ -159,7 +160,8 @@ int hdp_b200_thresholds_host(const float *h_temps, int64_t C, int64_t T_b, int64
  * ------------------------------------------------------------------------------------------------- */
 #define HDP_B200_ONSET 0x200
 
-/* h_doy_map may be NULL: the size is then an upper bound for regular daily calendars. */
+/* h_doy_map may be NULL: the size is then an upper bound for regular daily calendars (gap-free daily series); a series with missing
+ * days or a seasonal subset cuts into more hot-day words and then gets HDP_B200_ERR_WORKSPACE from that size. */
 size_t hdp_b200_metrics_workspace_bytes(int64_t C, int64_t T, int64_t ld_t, int64_t ld_c,
                                         int n_doy, int P, int D, int Y, const int32_t *h_doy_map);
 
