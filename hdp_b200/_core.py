@@ -15,6 +15,7 @@ These are the two seams of the reference that the CUDA library replaces:
   which two measures (e.g. tmax and tmin) both exceed their own thresholds
 * ``onset=True`` on the metric, intensity and compound calls: two more uint16 planes, HWO and HWE, the day of the season of its first
   and last heatwave day (0xFFFF without one)
+* :func:`extent_array`: the heatwave spatial extent, the daily weighted number of cells of each region on a heatwave day
 * :func:`trend_array`: Theil-Sen slope, its confidence interval and the Mann-Kendall test of every season series of a metric or
   intensity output (or any ``[..., Y, C]`` array)
 * :func:`index_heatwaves_array`, :func:`season_metrics_array` <- ``index_heatwaves`` and ``heatwave_frequency`` / ``number`` /
@@ -43,6 +44,7 @@ ONSET_NAMES = ("HWO", "HWE")                      # planes 4 and 5 of the metric
 COLD_ONSET_NAMES = ("CSO", "CSE")
 ONSET = 0x200                                     # HDP_B200_ONSET, OR-ed in the same way
 NO_DAY = 0xFFFF                                   # HWO / HWE of a season without heatwave days
+MAX_REGIONS = 256                                 # HDP_B200_MAX_REGIONS: regions of the extent calls
 
 _workspaces = {}
 
@@ -655,6 +657,91 @@ def intensity_host(measure: np.ndarray, thresholds, doy_map, defs, season_north,
                              cold, onset)
 
 
+def _extent_cells(weights, regions, n_regions, C):
+    """uint32 weights and int32 regions of C cells as contiguous NumPy arrays (None stays None), and the region count."""
+    R = int(n_regions)
+    if not 1 <= R <= MAX_REGIONS:
+        raise ValueError(f"n_regions must be in 1 .. {MAX_REGIONS}")
+    w = r = None
+    if weights is not None:
+        w = np.asarray(weights.cpu() if hasattr(weights, "cpu") else weights).ravel()
+        if w.size != C:
+            raise ValueError("weights must have one entry per cell")
+        if not np.issubdtype(w.dtype, np.integer) or (w.size and (w.min() < 0 or w.max() > 0xFFFFFFFF)):
+            raise ValueError("weights must be integers in 0 .. 2**32 - 1")
+        w = np.ascontiguousarray(w, dtype=np.uint32)
+    if regions is not None:
+        r = np.asarray(regions.cpu() if hasattr(regions, "cpu") else regions).ravel()
+        if r.size != C:
+            raise ValueError("regions must have one entry per cell")
+        if not np.issubdtype(r.dtype, np.integer):
+            raise ValueError("regions must be integers")
+        r = np.ascontiguousarray(np.where((r < 0) | (r >= R), -1, r), dtype=np.int32)     # outside [0, R): in no region
+    return w, r, R
+
+
+def extent_array(measure, thresholds, doy_map, defs, season_north, season_south, is_south=None, weights=None, regions=None, n_regions=1,
+                 out=None, metrics_out=None, units=None, *, cold=False):
+    """Heatwave spatial extent: ``measure`` f32 ``[T, C]``, ``thresholds`` f64 ``[C, n_doy, P]`` -> int64 ``[R, P, D, T]``, the sum of
+    the weights of the cells of region r for which day t is a heatwave day that HWF counts (inside the cell's season, heatwave id >
+    0).  ``weights``: integer weights ``[C]`` (uint32; None = 1 each, a cell count); ``regions``: integer region ``[C]`` of every cell
+    (None = all in region 0; a value outside ``[0, n_regions)`` = in no region).  The result is ADDED to ``out`` when it is given (a
+    contiguous int64 CUDA tensor ``[R, P, D, T]``): the sums are exact, so a loop over cell ranges into one ``out`` gives the result of
+    one call.  ``metrics_out``: an optional uint16 CUDA tensor ``[4, P, D, Y, C]`` that also receives what :func:`metrics_array`
+    returns, from the same pass.  The non-empty seasons of each hemisphere's table must be disjoint.  ``cold=True``: the cold-spell
+    days."""
+    torch = _torch()
+    unit = _flags(units, cold, False)
+    T, C, n_doy, P = _check_pairs([(measure, thresholds)])
+    dm, df, sn, ss = _metric_tables(doy_map, defs, season_north, season_south, T)
+    D, Y = int(df.shape[0]), int(sn.shape[0])
+    w, r, R = _extent_cells(weights, regions, n_regions, C)
+    dev = measure.device
+    south_t = _south_tensor(is_south, C, dev)
+    w_t = None if w is None else torch.from_numpy(w.view(np.int32)).to(dev)      # (bits of the uint32 weights)
+    r_t = None if r is None else torch.from_numpy(r).to(dev)
+    if out is None:
+        out = torch.zeros((R, P, D, T), dtype=torch.int64, device=dev)
+    elif not (out.is_cuda and out.dtype == torch.int64 and out.is_contiguous() and tuple(out.shape) == (R, P, D, T)):
+        raise TypeError("out must be a contiguous int64 CUDA tensor [R, P, D, T]")
+    if metrics_out is not None:
+        metrics_out = _device_out(metrics_out, torch.uint16, (4, P, D, Y, C), dev, "metrics_out must be a contiguous uint16 CUDA tensor "
+                                  "[4, P, D, Y, C]")
+    L = _lib.lib()
+    ld_t, ld_c = _strides(measure)
+    with torch.cuda.device(dev):
+        ws = _workspace(dev, L.hdp_b200_extent_workspace_bytes(C, T, ld_t, ld_c, n_doy, P, D, Y, R, _hp(dm)))
+        rc = L.hdp_b200_extent(measure.data_ptr(), C, T, ld_t, ld_c, thresholds.data_ptr(), n_doy, P, _hp(dm), _hp(df), D, _hp(sn), _hp(ss),
+                               Y, _ptr(south_t), _ptr(w_t), _ptr(r_t), R, out.data_ptr(), _ptr(metrics_out), ws.data_ptr(), ws.numel(),
+                               torch.cuda.current_stream().cuda_stream, unit)
+    _lib.check(rc, "hdp_b200_extent")
+    return out
+
+
+def extent_host(measure: np.ndarray, thresholds, doy_map, defs, season_north, season_south, is_south=None, weights=None, regions=None,
+                n_regions=1, out: Optional[np.ndarray] = None, metrics_out: Optional[np.ndarray] = None, units=None, *,
+                cold=False) -> np.ndarray:
+    """Host-array counterpart of :func:`extent_array` (the pipeline of :func:`metrics_host`): int64 ``[R, P, D, T]`` NumPy out.  ``out``
+    is OVERWRITTEN here, not added to.  Thresholds as for :func:`metrics_host` (host array, CUDA tensor, or a resident copy)."""
+    _torch()
+    x, ld_t, ld_c = _host_measure(measure, "measure")
+    T, C = x.shape
+    h_thr, d_thr = _host_thresholds(thresholds, C)
+    n_doy, P = int((d_thr if h_thr is None else h_thr).shape[1]), int((d_thr if h_thr is None else h_thr).shape[2])
+    dm, df, sn, ss = _metric_tables(doy_map, defs, season_north, season_south, T)
+    D, Y = int(df.shape[0]), int(sn.shape[0])
+    w, r, R = _extent_cells(weights, regions, n_regions, C)
+    south = None if is_south is None else np.ascontiguousarray(is_south, dtype=np.uint8)
+    out = _host_out(out, np.int64, (R, P, D, T), "out must be a C-contiguous int64 array [R, P, D, T]")
+    if metrics_out is not None:
+        metrics_out = _host_out(metrics_out, np.uint16, (4, P, D, Y, C), "metrics_out must be a C-contiguous uint16 array [4, P, D, Y, C]")
+    hp = lambda h: _hp(h) if h is not None else None                # noqa: E731
+    rc = _lib.lib().hdp_b200_extent_host(_hp(x), C, T, ld_t, ld_c, hp(h_thr), _ptr(d_thr), n_doy, P, _hp(dm), _hp(df), D, _hp(sn), _hp(ss),
+                                         Y, hp(south), hp(w), hp(r), R, _hp(out), hp(metrics_out), _flags(units, cold, False))
+    _lib.check(rc, "hdp_b200_extent_host")
+    return out
+
+
 def host_release() -> None:
     """Free the streams and device buffers the ``*_host`` entry points keep between calls."""
     release_resident()
@@ -736,7 +823,7 @@ def launch_count() -> int:
 
 KERNEL_NAMES = {1: "normalize", 2: "k_thr_generic", 3: "k_hot_words", 4: "k_scan", 5: "k_unpack_mask",
                 6: "k_thr_seg", 7: "k_thr_ranked", 8: "k_measure", 9: "k_thr_cand", 10: "k_thr_net", 11: "k_seam",
-                12: "k_intensity", 13: "k_hot_pair", 14: "k_trend"}
+                12: "k_intensity", 13: "k_hot_pair", 14: "k_trend", 15: "k_extent_prefix"}
 
 
 def timing_enable(on: bool) -> None:

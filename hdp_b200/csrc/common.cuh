@@ -30,7 +30,7 @@ inline int cuda_status(cudaError_t e) { return e == cudaSuccess ? HDP_B200_OK : 
     } while (0)
 
 // Optional per-kernel CUDA-event timing (hdp_b200_timing_enable / hdp_b200_timing_read).
-enum KernelId { kNormalize = 1, kThrGeneric = 2, kHotWords = 3, kScan = 4, kUnpackMask = 5, kThrSeg = 6, kThrRanked = 7, kMeasure = 8, kThrCand = 9, kThrNet = 10, kSeam = 11, kIntensity = 12, kHotPair = 13, kTrend = 14 };
+enum KernelId { kNormalize = 1, kThrGeneric = 2, kHotWords = 3, kScan = 4, kUnpackMask = 5, kThrSeg = 6, kThrRanked = 7, kMeasure = 8, kThrCand = 9, kThrNet = 10, kSeam = 11, kIntensity = 12, kHotPair = 13, kTrend = 14, kExtent = 15 };
 struct KernelTimer {
     bool on;
     cudaStream_t st;
@@ -109,15 +109,34 @@ struct Measure {
     const double *thr;
 };
 
+// The heatwave spatial extent of a metric pass (hdp_b200_extent): the arguments of k_scan's EXTENT twins (scan.cuh), one trailing
+// kernel parameter, so that the parameters of the other instances keep their offsets.
+// diff i64 [R, P, D, T + 1], the difference array of the daily weighted heatwave-day sums; weight u32 [C] (NULL = 1 each); region
+// i32 [C] (NULL = 0 each; a cell outside [0, R) is in no region).
+struct ScanExtent {
+    int64_t *diff = nullptr;
+    const uint32_t *weight = nullptr;
+    const int32_t *region = nullptr;
+    int R = 0;
+};
+
 // The whole of hdp_b200_metrics, hdp_b200_intensity and hdp_b200_compound (metric.cu) over n_measures (1 or 2) measures:
 // k_hot_words (k_hot_pair for two), then k_scan on its hot words when d_out is given (u16 [4, P, D, Y, C], [6, ...] with HWO and
 // HWE for HDP_B200_ONSET) and k_intensity when d_int is given (f32 [n_measures, 3, P, D, Y, C], one block per measure).
 // carve_cells / tables_resident as above; input_unit = unit code, OR-ed with HDP_B200_COLD for the cold-spell pass and with
-// HDP_B200_ONSET for the onset planes.
+// HDP_B200_ONSET for the onset planes.  With `ext` (one measure, disjoint season tables, no onset) k_scan's EXTENT twin also adds the
+// pass's heatwave days to ext->diff, and d_out may be NULL.
 int metric_pass(const Measure *ms, int n_measures, int64_t C, int64_t T, int n_doy, int P, const int32_t *h_doy_map,
                 const int32_t *h_defs, int D,
                 const int32_t *h_season_north, const int32_t *h_season_south, int Y,
                 const uint8_t *d_is_south, uint16_t *d_out, float *d_int,
-                void *d_workspace, size_t workspace_bytes, void *stream, int64_t carve_cells, bool tables_resident, int input_unit);
+                void *d_workspace, size_t workspace_bytes, void *stream, int64_t carve_cells, bool tables_resident, int input_unit,
+                const ScanExtent *ext = nullptr);
+
+// extent.cu: the bytes of the difference array i64 [rows, T + 1] (rows = R * P * D); ext i64 [rows, T] += the prefix sums of its rows
+// (k_extent_prefix); the checks of the region count R, the output and the flags that hdp_b200_extent and _extent_host share.
+size_t extent_diff_bytes(int64_t rows, int64_t T);
+int extent_prefix_launch(const int64_t *diff, int64_t rows, int64_t T, int64_t *ext, cudaStream_t st);
+int extent_args(int R, const void *ext, int64_t T, int input_unit);
 
 }  // namespace hdp

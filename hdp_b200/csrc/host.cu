@@ -154,6 +154,7 @@ struct HostCtx {
     cudaEvent_t in_ready[kSlots] = {}, k_done[kSlots] = {}, out_done[kSlots] = {};
     DeviceBuf x[2][kSlots], thr[2][kSlots];          // per measure (two for a compound pass): samples, thresholds from the host
     DeviceBuf south[kSlots], out[kSlots], out_f[kSlots], ws;
+    DeviceBuf ext_cells, ext_diff, ext_out;         // extent: the weights and regions of all cells, the difference array, the result
     PinnedRing ring_in, ring_out;                    // staging for pageable sources / destinations (allocated on first use)
     std::deque<PendingOut> pending;                  // D2H blocks on their way through ring_out
 
@@ -264,6 +265,7 @@ struct HostCtx {
             south[i].release(); out[i].release(); out_f[i].release();
         }
         ws.release();
+        ext_cells.release(); ext_diff.release(); ext_out.release();
         ring_in.release(); ring_out.release();
     }
 };
@@ -331,18 +333,31 @@ struct HostMeasure {
     const double *h_thr, *d_thr;
 };
 
-// hdp_b200_metrics_host, hdp_b200_intensity_host and hdp_b200_compound_host: metric_pass over n_measures (1 or 2) measures chunk by
-// chunk; the u16 planes (h_out: 4, or 6 with HDP_B200_ONSET) and the f32 planes (h_int), whichever are given, go back to the host.  Every measure's cells of a
-// chunk go up together.
+// The extent of a host call: host weights and regions of all cells (either may be NULL), R regions, the result i64 [R, P, D, T].
+struct HostExtent {
+    const uint32_t *weight;
+    const int32_t *region;
+    int R;
+    int64_t *ext;
+};
+
+// hdp_b200_metrics_host, hdp_b200_intensity_host, hdp_b200_compound_host and hdp_b200_extent_host: metric_pass over n_measures (1 or
+// 2) measures chunk by chunk; the u16 planes (h_out: 4, or 6 with HDP_B200_ONSET) and the f32 planes (h_int), whichever are given,
+// go back to the host.  Every measure's cells of a chunk go up together.  With `he` every chunk adds to one difference array on the
+// device, whose prefix sums go to he->ext at the end.
 static int metric_pass_host(const HostMeasure *hm, int n_measures, int64_t C, int64_t T, int n_doy, int P, const int32_t *h_doy_map,
                             const int32_t *h_defs, int D,
                             const int32_t *h_season_north, const int32_t *h_season_south, int Y,
-                            const uint8_t *h_is_south, float *h_int, uint16_t *h_out, int input_unit)
+                            const uint8_t *h_is_south, float *h_int, uint16_t *h_out, int input_unit, const HostExtent *he = nullptr)
 {
     if (C < 0 || T <= 0 || n_doy <= 0 || P <= 0 || D <= 0 || Y < 0 || !h_doy_map) return HDP_B200_ERR_INVALID;
     const bool onset = (input_unit & HDP_B200_ONSET) != 0;
     if (onset && !h_out) return HDP_B200_ERR_INVALID;                          // HWO / HWE are planes of the u16 output
-    if (C == 0 || Y == 0) return HDP_B200_OK;
+    const int64_t ext_rows = he ? (int64_t)he->R * P * D : 0;
+    if (C == 0 || Y == 0) {                                                    // no heatwave day anywhere
+        if (he) std::memset(he->ext, 0, (size_t)ext_rows * T * sizeof(int64_t));
+        return HDP_B200_OK;
+    }
     for (int m = 0; m < n_measures; m++) {
         if (!hm[m].x || (!hm[m].h_thr && !hm[m].d_thr)) return HDP_B200_ERR_INVALID;
         if (hm[m].ld_t <= 0 || hm[m].ld_c <= 0) return HDP_B200_ERR_INVALID;
@@ -381,6 +396,24 @@ static int metric_pass_host(const HostMeasure *hm, int n_measures, int64_t C, in
     }
     const bool page_out = h_out && is_pageable(h_out), page_int = h_int && is_pageable(h_int);
     const bool page_south = h_is_south && is_pageable(h_is_south);
+    ScanExtent ext;
+    const size_t ext_bytes = (size_t)ext_rows * T * sizeof(int64_t);
+    if (he) {                                                                  // weights and regions of all cells, then a zero diff
+        const size_t diff_bytes = extent_diff_bytes(ext_rows, T);
+        if ((rc = ctx->ext_cells.reserve((size_t)C * (sizeof(uint32_t) + sizeof(int32_t))))) return rc;
+        if ((rc = ctx->ext_diff.reserve(diff_bytes)) || (rc = ctx->ext_out.reserve(ext_bytes))) return rc;
+        uint32_t *d_w = (uint32_t *)ctx->ext_cells.p;
+        int32_t *d_r = (int32_t *)(d_w + C);
+        if (he->weight)
+            HDP_HOST_TRY(ctx->h2d((char *)d_w, 0, (const char *)he->weight, 0, (size_t)C * sizeof(uint32_t), 1, is_pageable(he->weight), ctx->s_k));
+        if (he->region)
+            HDP_HOST_TRY(ctx->h2d((char *)d_r, 0, (const char *)he->region, 0, (size_t)C * sizeof(int32_t), 1, is_pageable(he->region), ctx->s_k));
+        HDP_HOST_CUDA(cudaMemsetAsync(ctx->ext_diff.p, 0, diff_bytes, ctx->s_k));
+        ext.diff = (int64_t *)ctx->ext_diff.p;
+        ext.weight = he->weight ? d_w : nullptr;
+        ext.region = he->region ? d_r : nullptr;
+        ext.R = he->R;
+    }
     int64_t i = 0;
     for (int64_t c0 = 0; c0 < C; c0 += chunk, i++) {
         const int slot = (int)(i % kSlots);
@@ -404,9 +437,12 @@ static int metric_pass_host(const HostMeasure *hm, int n_measures, int64_t C, in
         HDP_HOST_CUDA(cudaStreamWaitEvent(ctx->s_k, ctx->in_ready[slot], 0));
         HDP_HOST_CUDA(cudaStreamWaitEvent(ctx->s_k, ctx->out_done[slot], 0));
         const uint8_t *south_chunk = h_is_south ? (const uint8_t *)ctx->south[slot].p : nullptr;
+        ScanExtent ext_chunk = ext;                                            // the chunk's cells
+        if (ext_chunk.weight) ext_chunk.weight += c0;
+        if (ext_chunk.region) ext_chunk.region += c0;
         HDP_HOST_TRY(metric_pass(dm, n_measures, nc, T, n_doy, P, h_doy_map, h_defs, D, h_season_north, h_season_south, Y, south_chunk,
                                  h_out ? (uint16_t *)ctx->out[slot].p : nullptr, h_int ? (float *)ctx->out_f[slot].p : nullptr,
-                                 ctx->ws.p, ws_bytes, ctx->s_k, chunk, i > 0, input_unit));
+                                 ctx->ws.p, ws_bytes, ctx->s_k, chunk, i > 0, input_unit, he ? &ext_chunk : nullptr));
         HDP_HOST_CUDA(cudaEventRecord(ctx->k_done[slot], ctx->s_k));
 
         // device chunk is [rows, nc]; host array is [rows, C]
@@ -418,6 +454,11 @@ static int metric_pass_host(const HostMeasure *hm, int n_measures, int64_t C, in
             HDP_HOST_TRY(ctx->d2h((char *)(h_int + c0), (size_t)C * sizeof(float), (const char *)ctx->out_f[slot].p, (size_t)nc * sizeof(float),
                                   (size_t)nc * sizeof(float), rows_f, page_int, ctx->s_out));
         HDP_HOST_CUDA(cudaEventRecord(ctx->out_done[slot], ctx->s_out));
+    }
+    if (he) {                                                                  // after the last chunk's k_scan, on the same stream
+        HDP_HOST_CUDA(cudaMemsetAsync(ctx->ext_out.p, 0, ext_bytes, ctx->s_k));
+        HDP_HOST_TRY(extent_prefix_launch(ext.diff, ext_rows, T, (int64_t *)ctx->ext_out.p, ctx->s_k));
+        HDP_HOST_TRY(ctx->d2h((char *)he->ext, 0, (const char *)ctx->ext_out.p, 0, ext_bytes, 1, is_pageable(he->ext), ctx->s_k));
     }
     return ctx->drain();
 }
@@ -506,6 +547,22 @@ int hdp_b200_intensity_host(const float *h_measure, int64_t C, int64_t T, int64_
     const HostMeasure m = {h_measure, ld_t, ld_c, h_thr, d_thr};
     return metric_pass_host(&m, 1, C, T, n_doy, P, h_doy_map, h_defs, D, h_season_north, h_season_south, Y, h_is_south, h_int, h_out,
                             input_unit);
+}
+
+int hdp_b200_extent_host(const float *h_measure, int64_t C, int64_t T, int64_t ld_t, int64_t ld_c,
+                         const double *h_thr, const double *d_thr, int n_doy, int P, const int32_t *h_doy_map,
+                         const int32_t *h_defs, int D,
+                         const int32_t *h_season_north, const int32_t *h_season_south, int Y,
+                         const uint8_t *h_is_south, const uint32_t *h_weight, const int32_t *h_region, int R,
+                         int64_t *h_ext, uint16_t *h_out, int input_unit)
+{
+    const int rc = extent_args(R, h_ext, T, input_unit);
+    if (rc != HDP_B200_OK) return rc;
+    if (P > HDP_B200_MAX_PERCENTILES || D > HDP_B200_MAX_DEFINITIONS) return HDP_B200_ERR_UNSUPPORTED;
+    const HostMeasure m = {h_measure, ld_t, ld_c, h_thr, d_thr};
+    const HostExtent he = {h_weight, h_region, R, h_ext};
+    return metric_pass_host(&m, 1, C, T, n_doy, P, h_doy_map, h_defs, D, h_season_north, h_season_south, Y, h_is_south, nullptr, h_out,
+                            input_unit, &he);
 }
 
 int hdp_b200_compound_host(const float *h_a, int64_t ld_t_a, int64_t ld_c_a, const float *h_b, int64_t ld_t_b, int64_t ld_c_b,

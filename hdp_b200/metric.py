@@ -463,6 +463,136 @@ def compute_group_metrics(measures, thresholds, hw_definitions: list, include_th
     return aggr_ds
 
 
+EXTENT_ATTRS = {
+    "HWS": {"units": "1", "long_name": "Heatwave Spatial Extent",
+            "description": "Share of the region's total cell weight (cos(latitude) by default) whose cells are on a day that falls "
+                           "within a heatwave during their heatwave season, for every day"},
+    "CSS": {"units": "1", "long_name": "Cold Spell Spatial Extent",
+            "description": "Share of the region's total cell weight (cos(latitude) by default) whose cells are on a day that falls "
+                           "within a cold spell during their cold season, for every day"},
+}
+EXTENT_WEIGHT_MAX = 1 << 30         # the largest quantized weight
+EXTENT_TOTAL_LIMIT = 1 << 53        # every region's total of quantized weights stays below this: its int64 sums are exact in float64
+
+
+def quantize_weights(weights, regions, n_regions: int) -> np.ndarray:
+    """uint32 cell weights for the extent kernel: ``weights`` (finite, >= 0) scaled so that the largest becomes
+    :data:`EXTENT_WEIGHT_MAX`, or less where needed to keep the total of every region (cells with ``regions`` in ``[0, n_regions)``)
+    below :data:`EXTENT_TOTAL_LIMIT`, then rounded to the nearest integer.  Every sum of them is then exact in int64 and in float64,
+    so the extent share is reproducible to the bit.  Negative or non-finite weights raise ``ValueError``; all-zero weights stay 0."""
+    w = np.asarray(weights, dtype=np.float64).ravel()
+    if not np.all(np.isfinite(w)):
+        raise ValueError("weights must be finite")
+    if np.any(w < 0):
+        raise ValueError("weights must not be negative")
+    r = np.asarray(regions).ravel()
+    inside = (r >= 0) & (r < n_regions)
+    w_max = float(w.max()) if w.size else 0.0
+    if w_max == 0.0:
+        return np.zeros(w.size, np.uint32)
+    totals = np.bincount(r[inside].astype(np.int64), weights=w[inside], minlength=n_regions) if inside.any() else np.zeros(1)
+    scale = EXTENT_WEIGHT_MAX / w_max
+    # rint(w * scale) <= w * scale + 1/2: a region's total stays below scale * sum(w) + C / 2
+    limit = (EXTENT_TOTAL_LIMIT - w.size) / float(totals.max()) if totals.max() > 0 else scale
+    scale = min(scale, limit)
+    return np.minimum(np.rint(w * scale), EXTENT_WEIGHT_MAX).astype(np.uint32)
+
+
+def extent_share(ext: np.ndarray, weights_q: np.ndarray, regions: np.ndarray, n_regions: int) -> np.ndarray:
+    """int64 [R, P, D, T] weighted cell sums -> float64 shares: ``ext / total_r`` (one float64 division; both sides exact below
+    2^53), NaN for a region with total weight 0."""
+    r = np.asarray(regions).ravel()
+    inside = (r >= 0) & (r < n_regions)
+    totals = np.zeros(n_regions, np.int64)
+    np.add.at(totals, r[inside].astype(np.int64), weights_q[inside].astype(np.int64))
+    with np.errstate(invalid="ignore", divide="ignore"):
+        share = ext.astype(np.float64) / totals.astype(np.float64)[:, None, None, None]
+    return np.where(totals[:, None, None, None] > 0, share, np.nan)
+
+
+def compute_heatwave_extent(measure, threshold, hw_definitions: list, *, weights=None, regions=None, region_names=None, cold: bool = False,
+                            check_variables: bool = True):
+    """Heatwave spatial extent: for every region, percentile, definition and DAY of the measure, the share of the region's total cell
+    weight whose cells are on a heatwave day that HWF counts (inside the cell's heatwave season, heatwave id > 0).  Returns a Dataset
+    with one float64 variable, HWS (CSS with ``cold=True``, over the cold spells in the cold season), dims ``(region, percentile,
+    definition, time)``, with the measure's daily time coordinate.  Values lie in [0, 1]; NaN for a region of total weight 0.
+
+    ``weights``: a non-negative array with the measure's cell dims (default: cos(latitude) of every cell, the weights of
+    :func:`hdp_b200._core.weighted_spatial_mean`), quantized by :func:`quantize_weights`, so the share is exact to the bit whatever the
+    cell order.  ``regions``: an integer array with the measure's cell dims, -1 (or any value outside ``0 .. R-1``) for cells in no
+    region; default: one region.  ``region_names``: the names of regions 0 .. R-1, which also sets R (default: ``"all"`` for one region,
+    else ``0 .. max(regions)``).  At most 256 regions.  The
+    maximum extent of a season or the days above an area are one reduction of the result."""
+    time_axis = time_axis_of(measure)
+    if check_variables:                                             # as compute_individual_metrics
+        assert "hdp_type" in threshold.attrs
+        assert threshold.attrs["hdp_type"] == "threshold"
+        assert threshold.attrs["baseline_variable"] == measure.attrs["baseline_variable"]
+        assert threshold.attrs["baseline_calendar"] == time_axis.calendar
+
+    combined_history = ""
+    if "history" in measure.attrs:
+        for entry in measure.attrs["history"].split("\n"):
+            if entry != '':
+                combined_history += (f"(Measure) {entry}\n")
+    if "history" in threshold.attrs:
+        for entry in threshold.attrs["history"].split("\n"):
+            if entry != '':
+                combined_history += (f"(Threshold) {entry}\n")
+
+    st = _tables.hemisphere_ranges(time_axis)
+    north, south_tab = (st.south, st.north) if cold else (st.north, st.south)
+    doy_map = _tables.doy_map(time_axis.dayofyr)
+    x, cell_dims, cell_shape = _layout.to_time_cells(xr.values_of(measure), tuple(measure.dims), require_float32=True)
+    C = x.shape[1]
+    lat = _layout.cell_latitudes(xr.coord_values(measure, "lat"), cell_dims, cell_shape)
+    thr = _threshold_cdp(threshold, measure, cell_dims)
+
+    def cells(a, name):                                             # an array with the measure's cell dims -> [C]
+        if hasattr(a, "dims") and tuple(a.dims) != tuple(cell_dims):
+            raise ValueError(f"{name} must have the measure's cell dims {tuple(cell_dims)}")
+        a = np.asarray(xr.values_of(a) if hasattr(a, "dims") else a)
+        if tuple(a.shape) != tuple(cell_shape):
+            raise ValueError(f"{name} must have the measure's cell dims {tuple(cell_dims)}")
+        return a.reshape(-1)
+    if regions is None:
+        reg = np.zeros(C, np.int32)
+        R = 1
+    else:
+        reg = cells(regions, "regions")
+        if not np.issubdtype(reg.dtype, np.integer):
+            raise ValueError("regions must be integers")
+        R = len(region_names) if region_names is not None else int(reg.max()) + 1 if reg.size and reg.max() >= 0 else 1
+        reg = np.where((reg < 0) | (reg >= R), -1, reg).astype(np.int32)
+    names = list(region_names) if region_names is not None else (["all"] if regions is None else list(range(R)))
+    w = np.cos(np.deg2rad(lat)) if weights is None else cells(weights, "weights")
+    wq = quantize_weights(w, reg, R)
+    ext = _core.extent_host(x, thr, doy_map, np.asarray(hw_definitions, dtype=np.int64).reshape(-1, 3), north, south_tab,
+                            _tables.is_south(lat), weights=wq, regions=reg, n_regions=R, cold=cold)
+    share = extent_share(ext, wq, reg, R)
+    name = "CSS" if cold else "HWS"
+    coords = {"region": names, "percentile": np.asarray(xr.coord_values(threshold, "percentile")),
+              "definition": [f"{d[0]}-{d[1]}-{d[2]}" for d in hw_definitions], "time": xr.coord_values(measure, "time")}
+    ds = xr.Dataset({name: xr.DataArray(share, dims=["region", "percentile", "definition", "time"], coords=coords)})
+    xr.set_coord_attrs(ds, "percentile", {"range": "(0, 1)"})
+    days = "cold" if cold else "hot"
+    xr.set_coord_attrs(ds, "definition", {
+        "first_number": f"Minimum number of consecutively {days} days",
+        "second_number": "Maximum number of break days after first wave",
+        "third_number": f"Minimum number of consecutively {days} days after the break"
+    })
+    kind = "Cold spell" if cold else "Heatwave"
+    ds.attrs.update({
+        "description": f"{kind} spatial extent dataset generated by Heatwave Diagnostics Package (HDP v{get_version()})",
+        "hdp_version": get_version(),
+        "hdp_type": "metric"
+    })
+    ds[name].attrs.update(EXTENT_ATTRS[name])
+    ds[name].attrs["history"] = combined_history
+    add_history(ds[name], f"Heatwave spatial extent generated by HDP v{get_version()}")
+    return ds
+
+
 _TREND_LEAD_DIMS = ("measure", "percentile", "definition")      # dims of a metric variable that are neither cells nor time
 TREND_METHOD = ("Theil-Sen slope per year with the Sen (1968) confidence interval; intercept median(y) - slope * median(x) at the "
                 "first season; two-sided Mann-Kendall test with tie-corrected variance and continuity correction")

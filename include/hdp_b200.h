@@ -17,6 +17,8 @@
  *                         threshold over the heatwave days of every season, optionally with the metrics in the same pass
  *   hdp_b200_index_heatwaves   replaces  index_heatwaves                  hdp/metric.py:11-60     (the building blocks under
  *   hdp_b200_season_metrics    replaces  heatwave_frequency / number / duration / average  hdp/metric.py:63-172   their own names)
+ *   hdp_b200_extent       (no reference counterpart) heatwave spatial extent: the weighted number of cells of each region on a
+ *                         heatwave day, for every day
  *   hdp_b200_trend        (no reference counterpart) Theil-Sen slope, its confidence interval and the Mann-Kendall test of every
  *                         season series of a metric or intensity output
  *   *_host variants       the same calls with HOST buffers (cell chunks pipelined H2D -> kernels -> D2H on three streams).
@@ -58,6 +60,7 @@ extern "C" {
 #define HDP_B200_MAX_PERCENTILES   32
 #define HDP_B200_MAX_DEFINITIONS   32
 #define HDP_B200_MAX_WINDOW        32768 /* samples pooled per day-of-year window (W * n_y) */
+#define HDP_B200_MAX_REGIONS       256   /* regions of hdp_b200_extent */
 
 int         hdp_b200_abi_version(void);
 const char *hdp_b200_strerror(int code);
@@ -291,6 +294,51 @@ int hdp_b200_compound_hot_days(const float *d_a, int64_t ld_t_a, int64_t ld_c_a,
  * shared-memory bytes per CTA}. */
 int hdp_b200_compound_plan(int P, int *info);
 
+/* ---------------------------------------------------------------------------------------------------
+ * Path 2 - heatwave spatial extent (opt-in): the daily weighted number of cells of each region that are on a heatwave day.  Same
+ * inputs as hdp_b200_metrics, plus
+ *
+ *   d_weight      u32 [C]  integer weight of every cell; NULL = 1 each (the result is then a cell count)
+ *   d_region      i32 [C]  region of every cell; NULL = every cell in region 0.  A value outside [0, R) puts the cell in no region:
+ *                          it is ignored (defined behaviour, the device input needs no validation)
+ *   R             regions, 1 <= R <= HDP_B200_MAX_REGIONS
+ *   d_ext         i64 [R, P, D, T]  ACCUMULATED (+=; the caller zeroes it, and a loop over cell ranges adds into one array):
+ *                 d_ext[r, p, d, t] += sum of w_c over the cells c of region r for which day t is a day that HWF[p, d, y, c] counts,
+ *                 y the season of c's hemisphere table that contains t
+ *   d_out         optional u16 [4, P, D, Y, C]: when given, exactly what hdp_b200_metrics writes, from the same pass
+ *
+ * "A day HWF counts": t lies in the season slice [lo, hi) after the slice semantics above and its heatwave id is > 0.  A day outside
+ * every season of a cell's hemisphere adds nothing for that cell, and a heatwave that began before the season counts from lo on.  So
+ *   sum_t d_ext[r, p, d, t] = sum_{c in r} w_c * sum_y HWF[p, d, y, c]
+ * The sums are exact int64 (u32 weights, C < 2^31), so the result depends neither on order nor on how the cells are split.  The
+ * non-empty seasons of each hemisphere's table must be pairwise disjoint after slice clamping (as for hdp_b200_intensity), else
+ * HDP_B200_ERR_UNSUPPORTED.  HDP_B200_COLD: the cold-spell days (the result is bit for bit the heatwave result on -x, -thr).
+ * HDP_B200_ONSET returns HDP_B200_ERR_INVALID.
+ * ------------------------------------------------------------------------------------------------- */
+/* h_doy_map may be NULL: the size is then an upper bound for regular daily calendars. */
+size_t hdp_b200_extent_workspace_bytes(int64_t C, int64_t T, int64_t ld_t, int64_t ld_c,
+                                       int n_doy, int P, int D, int Y, int R, const int32_t *h_doy_map);
+
+int hdp_b200_extent(const float *d_measure, int64_t C, int64_t T, int64_t ld_t, int64_t ld_c,
+                    const double *d_thr, int n_doy, int P,
+                    const int32_t *h_doy_map,
+                    const int32_t *h_defs, int D,
+                    const int32_t *h_season_north, const int32_t *h_season_south, int Y,
+                    const uint8_t *d_is_south, const uint32_t *d_weight, const int32_t *d_region, int R,
+                    int64_t *d_ext, uint16_t *d_out,
+                    void *d_workspace, size_t workspace_bytes, void *stream, int input_unit);
+
+/* Host-buffer variant (the pipeline of hdp_b200_metrics_host; the difference array stays on the device across the cell chunks).
+ * h_weight / h_region: HOST arrays as above (NULL allowed).  h_ext i64 [R, P, D, T] is written once at the end: OVERWRITTEN, not
+ * accumulated.  h_out (optional) as d_out.  Thresholds from h_thr unless d_thr (DEVICE) is given. */
+int hdp_b200_extent_host(const float *h_measure, int64_t C, int64_t T, int64_t ld_t, int64_t ld_c,
+                         const double *h_thr, const double *d_thr, int n_doy, int P,
+                         const int32_t *h_doy_map,
+                         const int32_t *h_defs, int D,
+                         const int32_t *h_season_north, const int32_t *h_season_south, int Y,
+                         const uint8_t *h_is_south, const uint32_t *h_weight, const int32_t *h_region, int R,
+                         int64_t *h_ext, uint16_t *h_out, int input_unit);
+
 /* The *_host variants keep their streams, events and device buffers (grown on demand) in a per-device context between
  * calls; this frees them.  Safe to call at any time no *_host call is running. */
 void hdp_b200_host_release(void);
@@ -394,6 +442,7 @@ int64_t hdp_b200_launch_count(void);
 #define HDP_B200_KERNEL_INTENSITY   12   /* k_intensity */
 #define HDP_B200_KERNEL_HOT_PAIR    13   /* k_hot_pair */
 #define HDP_B200_KERNEL_TREND       14   /* k_trend */
+#define HDP_B200_KERNEL_EXTENT      15   /* k_extent_prefix (the EXTENT twins of k_scan time as HDP_B200_KERNEL_SCAN) */
 void hdp_b200_timing_enable(int on);
 int  hdp_b200_timing_read(int *ids, float *ms, int cap);
 
